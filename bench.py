@@ -2,10 +2,16 @@
 """Benchmark of the rollout hot path: env-steps/s of the fused step kernel (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c5] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 One "step" = one uavenv_step launch over the whole env batch of this GPU with synthetic Bernoulli(1/2)
 actions (SURVEY.md §8d).  Prints ONE JSON line (rank 0).  N > 1: launched by torchrun, one rank per GPU,
 env batch sharded by global env id, no data-path collective (weak scaling: the per-GPU batch is fixed).
+
+--dump-outputs DIR writes what the last timed step returned to its caller as DIR/<name>.npy (float32 / float64,
+rank 0's envs): the step's (obs, reward, done, info), or with --workload c4 the last update's losses and the
+parameters it left.  Scenes and actions are seeded, so two builds run with the same arguments can be compared
+output for output.
 
 Timing: W (>= 3) warm-up steps, then exactly K timed steps; every timed step is bracketed by CUDA events on
 the launching stream and preceded by an L2 flush (a 256 MiB write) outside the bracket; per-rank time = sum
@@ -24,6 +30,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only and is left as the build left it: no __pycache__ either
 
 # BASELINE.json configs.  c3 is the configuration the 1/2/4/8-GPU env-steps/s metric is quoted on and the
 # default; c2 (4096 default-size envs, the bit-exact parity config) and c5 (large swarm) are selectable.
@@ -40,6 +47,33 @@ SCENE_SEED = 42          # configs/config.py:85 SEED
 BURN_IN_STEPS = 300      # untimed: de-synchronises the envs' decision pointers (episodes are ~2N steps long)
 POOL = 64                # pre-generated action vectors cycled through the timed steps
 L2_FLUSH_BYTES = 256 << 20
+DUMP_BYTES = 64_000_000  # --dump-outputs: above this, a fixed seeded sample of the envs is written
+
+
+def step_outputs(step_out, env_id_base):
+    """The (obs, reward, done, info) a step returned, on the host as float32 / float64 numpy arrays, one row per env;
+    a seeded sample of the envs (sorted, the same on every run) when all of them would exceed DUMP_BYTES."""
+    import numpy as np
+    obs, reward, done, info = step_out
+    host = {"obs": obs, "reward": reward, "done": done}
+    host.update(info)
+    host = {k: v.cpu().numpy() for k, v in host.items()}
+    host = {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float32) for k, v in host.items()}
+    B = len(host["obs"])
+    host["env_id"] = np.arange(env_id_base, env_id_base + B, dtype=np.float64)
+    per_env = sum(v.nbytes for v in host.values()) // B
+    if B * per_env > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(B, DUMP_BYTES // per_env, replace=False))
+        host = {k: v[keep] for k, v in host.items()}
+    return host
+
+
+def write_outputs(out_dir, arrays):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+
 
 # Algorithmic bytes per env-step of THIS design (DESIGN.md section 4.1 derives each term): io 38 (int64 action 8,
 # reward 4, done 1, info 25), header read 144 / write 124, window ring read 224 / write 56, window out 280,
@@ -180,13 +214,15 @@ def cpu_baseline(w, seconds=12.0):
     return {k: r[k] for k in ("value", "unit", "cores", "kind", "sample")}
 
 
-def measure_ppo(rank, local_rank, world, dev, B, T, K, W, with_clocks=True):
+def measure_ppo(rank, local_rank, world, dev, B, T, K, W, with_clocks=True, dump=None):
     """BASELINE.json configs[3]: end-to-end PPO samples/s = transitions collected AND trained on (K_EPOCHS = 5) per
     second.  One iteration = `T` rollout steps (tcgen05 policy forward + fused env step) followed by the PPO update (GAE
     kernel; per minibatch the hand-written bf16 forward + loss + backward, one flat NCCL gradient all-reduce at N > 1,
     fused clip + Adam - replayed as one CUDA graph).  K iterations are timed with ONE CUDA-event bracket, max over ranks.
     The gradient all-reduce (the only collective) is also timed alone, eagerly, with events around 50 calls on the
-    same 1.68 MB flat buffer.  Returns the record (rank 0) or None."""
+    same 1.68 MB flat buffer.  Returns the record (rank 0) or None; `dump` (a dict) receives the last iteration's
+    losses and the flat parameters its update left."""
+    import numpy as np
     import torch
     import uavenv_b200 as ub
     from target_allocation_ppo_transformer_b200 import parallel
@@ -223,6 +259,9 @@ def measure_ppo(rank, local_rank, world, dev, B, T, K, W, with_clocks=True):
     e1.record()
     torch.cuda.synchronize(dev); parallel.barrier()
     sampler.mark_end()
+    if dump is not None:
+        dump.update({k: np.float64(v) for k, v in stats.items()})
+        dump["policy_params"] = agent._flat_params.cpu().numpy()
     ms = parallel.reduce_scalar(e0.elapsed_time(e1), "max", dev)
     clocks = sampler.stop() if (rank == 0 and with_clocks) else None
     roll_ms = parallel.reduce_scalar(split[0].elapsed_time(split[1]), "max", dev)
@@ -272,10 +311,13 @@ def run_ppo(args):
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
     B, T = args.envs_per_gpu or PPO["envs_per_gpu"], PPO["horizon"]
-    K, W = args.steps if args.steps != 200 else 5, min(args.warmup, 3)
-    rec = measure_ppo(rank, local_rank, world, dev, B, T, K, W)
+    K, W = args.steps, min(args.warmup, 3)
+    dump = {} if args.dump_outputs and rank == 0 else None
+    rec = measure_ppo(rank, local_rank, world, dev, B, T, K, W, dump=dump)
     if rank == 0:
         print(json.dumps(rec))
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     if world > 1:
         torch.distributed.destroy_process_group()
 
@@ -283,7 +325,8 @@ def run_ppo(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default 200); with --workload c4, timed PPO iterations (default 5)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c3", choices=sorted(WORKLOADS) + ["c4"],
@@ -296,7 +339,15 @@ def main():
     ap.add_argument("--reset-episodes", type=int, default=200, help="diagnostic only: cfg.RESET_EPISODES (200)")
     ap.add_argument("--flush-mode", default="write+read", choices=["write+read", "write", "read", "sleep"],
                     help="diagnostic only: what runs between timed steps (default: the documented L2 flush)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (not with --impl reference)")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 5 if args.workload == "c4" else 200
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours: the reference arm runs on the host")
     args.warmup = max(args.warmup, 3)
     if args.workload == "c4":
         return run_ppo(args)
@@ -371,8 +422,9 @@ def main():
         for i in range(n_timed):
             flush_l2(i)
             ev[i][0].record(stream)
-            step_fn(n_warm + i)
+            out = step_fn(n_warm + i)
             ev[i][1].record(stream)
+        timed.last_out = out
         torch.cuda.synchronize(dev)
         parallel.barrier()
         raw = [a.elapsed_time(b) for a, b in ev]
@@ -410,6 +462,8 @@ def main():
     sampler.mark_begin()
     ms_dev = timed(lambda i: env.step(pool[i % POOL]), W, K)
     step_us = dict(timed.last_us)
+    # the env's output buffers still hold the last timed step: copied before anything steps the env again
+    dump = step_outputs(timed.last_out, rank * B) if args.dump_outputs and rank == 0 else None
     # the same bracket around a ~2 us kernel (the action generator): what the protocol itself costs per step
     ms_floor = timed(lambda i: env.random_actions(i, ACTION_SEED), 3, min(K, 50)) / min(K, 50)
     # --- end to end through the host-buffer entry point ----------------------------------------------------
@@ -495,6 +549,8 @@ def main():
                                               "config", "comm", "gpu_launches")}
     if rank == 0:
         print(json.dumps(out))
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
     if world > 1:
         torch.distributed.destroy_process_group()
 

@@ -5,6 +5,7 @@ Writes tests/golden/policy_net.npz: the reference TransformerActorCritic's state
 so that biases / LayerNorm affine terms are non-trivial), a batch of observation windows with realistic padding
 patterns, and the reference outputs (logits via evaluate's log-probs, values, entropy); plus the GAE returns /
 normalised advantages the reference PPOAgent.update computes on an episodic buffer (ppo.py:77-94)."""
+import hashlib
 import os
 import sys
 
@@ -40,13 +41,18 @@ def main():
         xa = net.actor_net(x)[:, -1]
         logits = net.actor_head(xa)
     sd = {k: v.detach().numpy() for k, v in net.state_dict().items()}
+    # the encoder layers' uniform draws are redrawn from the seed by tests/helpers.py: only their digests are stored
+    drawn = [k for k, v in sd.items() if ".transformer.layers." in k and v.ndim == 2]
     np.savez_compressed(os.path.join(OUT, "policy_net.npz"), obs=x.numpy(), actions=actions.numpy(),
                         logp=logp.numpy(), value=value.numpy(), entropy=ent.numpy(), logits=logits.numpy(),
-                        keys=np.array(list(sd.keys())), **{"p::" + k: v for k, v in sd.items()})
+                        keys=np.array(list(sd.keys())), init_seed=np.int64(1234),
+                        **{"p::" + k: v for k, v in sd.items() if k not in drawn},
+                        **{"sha256::" + k: np.array(hashlib.sha256(sd[k].tobytes()).hexdigest()) for k in drawn})
     print("policy_net.npz: %d tensors, %d parameters" % (len(sd), sum(v.size for v in sd.values())))
+    return sd
 
 
-def ppo_update_golden():
+def ppo_update_golden(sd):
     """One full-batch PPO update of the UNMODIFIED reference agent (agents/ppo.py:68-181) on a synthetic episodic
     buffer: records the buffer, the losses it returns and the clipped flat gradient of its single minibatch step."""
     PPOAgent, _ = ref_shim.load_agents()
@@ -54,8 +60,7 @@ def ppo_update_golden():
     saved = (cfg.BATCH_SIZE, cfg.K_EPOCHS)
     torch.manual_seed(99)
     agent = PPOAgent()
-    fx = np.load(os.path.join(OUT, "policy_net.npz"))     # initial weights = the network fixture's (stored once)
-    agent.policy.load_state_dict({str(k): torch.from_numpy(fx["p::" + str(k)]) for k in fx["keys"]})
+    agent.policy.load_state_dict({k: torch.from_numpy(v) for k, v in sd.items()})   # initial weights = the network fixture's
     agent.policy_old.load_state_dict(agent.policy.state_dict())
     g = torch.Generator().manual_seed(3)
     T = 192
@@ -102,5 +107,4 @@ def ppo_update_golden():
 
 
 if __name__ == "__main__":
-    main()
-    ppo_update_golden()
+    ppo_update_golden(main())

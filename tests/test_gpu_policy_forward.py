@@ -1,13 +1,11 @@
 """tcgen05 rollout forward (csrc/policy_forward.cu) against the fp32 PyTorch network with the reference's weights
 (tests/golden/policy_net.npz).  bf16 operands: logits / values within 3e-2 absolute, log-probs within 2e-2;
 sampling follows the returned probabilities; the library has no CPU fallback."""
-import os
-
 import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN
+from helpers import policy_fixture
 
 import uavenv_b200  # noqa: F401  (registers the package under an importable name)
 
@@ -16,9 +14,9 @@ pytestmark = pytest.mark.gpu
 
 def _net():
     import uavenv_b200 as ub
-    fx = np.load(os.path.join(GOLDEN, "policy_net.npz"))
+    fx, sd = policy_fixture()
     net = ub.TransformerActorCritic().cuda()
-    net.load_state_dict({str(k): torch.from_numpy(fx["p::" + str(k)]) for k in fx["keys"]})
+    net.load_state_dict({k: torch.from_numpy(v) for k, v in sd.items()})
     return net.eval(), fx
 
 

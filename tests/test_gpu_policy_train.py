@@ -9,6 +9,7 @@ import pytest
 import torch
 
 from conftest import GOLDEN
+from helpers import policy_fixture
 
 pytestmark = pytest.mark.gpu
 
@@ -144,10 +145,9 @@ def test_fused_update_against_the_reference_agents_update():
     2e-2 relative / absolute, clipped gradient direction cosine >= 0.99 on the recorded stride-5 sample."""
     import uavenv_b200 as ub
     fx = np.load(os.path.join(GOLDEN, "ppo_update.npz"))
-    net = np.load(os.path.join(GOLDEN, "policy_net.npz"))
     T = len(fx["rewards"])
     agent = ub.PPOAgent(num_envs=1, horizon=T, device="cuda", cfg=ub.Config(K_EPOCHS=1), minibatch_size=T, update_precision="fused")
-    sd = {str(k): torch.from_numpy(net["p::" + str(k)]) for k in net["keys"]}
+    sd = {k: torch.from_numpy(v) for k, v in policy_fixture()[1].items()}
     agent.policy.load_state_dict(sd); agent.policy_old.load_state_dict(sd)
     obs = torch.from_numpy(fx["obs"]).cuda()
     agent.buf_obs.copy_(obs[:, None]); agent.buf_action.copy_(torch.from_numpy(fx["actions"]).cuda()[:, None])

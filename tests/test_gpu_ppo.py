@@ -8,6 +8,7 @@ import pytest
 import torch
 
 from conftest import GOLDEN
+from helpers import policy_fixture
 
 pytestmark = pytest.mark.gpu
 
@@ -15,11 +16,10 @@ pytestmark = pytest.mark.gpu
 def test_single_update_matches_reference_agent():
     import uavenv_b200 as ub
     fx = np.load(os.path.join(GOLDEN, "ppo_update.npz"))
-    net = np.load(os.path.join(GOLDEN, "policy_net.npz"))
     T = len(fx["rewards"])
     cfg = ub.Config(K_EPOCHS=1)
     agent = ub.PPOAgent(num_envs=1, horizon=T, device="cuda", cfg=cfg, minibatch_size=T, update_precision="fp32")
-    sd = {str(k): torch.from_numpy(net["p::" + str(k)]) for k in net["keys"]}
+    sd = {k: torch.from_numpy(v) for k, v in policy_fixture()[1].items()}
     agent.policy.load_state_dict(sd); agent.policy_old.load_state_dict(sd)
     obs = torch.from_numpy(fx["obs"]).cuda()
     # the buffer the reference filled (its own sampled actions / log-probs / values, ppo.py:52-66)
@@ -78,9 +78,9 @@ def test_train_loop_logs_reference_columns_and_saves_reference_loadable_checkpoi
     assert np.isfinite(hist[-1]["Avg_Q0"]) and hist[-1]["Max_Coverage"] >= 1
     assert len(rows) == 3
     sd = torch.load(tmp_path / "final_model.pth", map_location="cpu")
-    fx = np.load(os.path.join(GOLDEN, "policy_net.npz"))
-    assert list(sd.keys()) == [str(k) for k in fx["keys"]]              # the keys the reference network expects
-    assert all(tuple(sd[str(k)].shape) == fx["p::" + str(k)].shape for k in fx["keys"])
+    ref = policy_fixture()[1]
+    assert list(sd.keys()) == list(ref)                                  # the keys the reference network expects
+    assert all(tuple(sd[k].shape) == ref[k].shape for k in ref)
 
 
 def test_fused_rollout_forward_drives_training():

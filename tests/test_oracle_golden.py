@@ -10,6 +10,7 @@ import numpy as np
 import pytest
 
 from conftest import GOLDEN, golden_cases
+from helpers import load_fixture
 from oracle import oracle as orc
 
 RTOL64 = 1e-12
@@ -62,7 +63,7 @@ def test_kat_composite():
 
 @pytest.mark.parametrize("case", golden_cases())
 def test_trajectory_matches_reference(case):
-    fx = np.load(os.path.join(GOLDEN, case + ".npz"))
+    fx = load_fixture(case)
     env = orc.OracleEnv(orc.cfg_from_fixture(fx))
     env.load_scene(fx)
     pf, pd, pp = env.score_matrix()

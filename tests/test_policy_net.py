@@ -1,21 +1,18 @@
 """The policy / value network mirror against golden vectors recorded from the reference network
 (oracle/gen_golden_policy.py -> tests/golden/policy_net.npz): identical state_dict keys and shapes,
 fp32 outputs within 2e-5 (same math, different kernel association)."""
-import os
-
 import numpy as np
 import torch
 
-from conftest import GOLDEN
+from helpers import policy_fixture
 
 import uavenv_b200  # noqa: F401
 from target_allocation_ppo_transformer_b200.networks.transformer_net import TransformerActorCritic
 
 
 def _load():
-    fx = np.load(os.path.join(GOLDEN, "policy_net.npz"))
-    sd = {str(k): torch.from_numpy(fx["p::" + str(k)]) for k in fx["keys"]}
-    return fx, sd
+    fx, sd = policy_fixture()
+    return fx, {k: torch.from_numpy(v) for k, v in sd.items()}
 
 
 def test_state_dict_is_interchangeable_with_the_reference():
