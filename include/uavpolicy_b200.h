@@ -5,9 +5,10 @@
  * step by PPOAgent.select_action (agents/ppo.py:52-62): for a batch of observation windows [B,5,14] it returns
  * the sampled action, its log-probability, the state value and the policy entropy.  All dense contractions run
  * on the 5th-generation tensor cores (tcgen05.mma, operands staged by TMA, fp32 accumulators in TMEM; bf16
- * operands) in hand-written kernels: the fused encoder blocks of csrc/policy_fused.cu (default) or one persistent
- * TMA-fed GEMM launch per dense layer (csrc/policy_dense.cu) with separate embedding / attention / residual + LayerNorm
- * kernels (csrc/policy_forward.cu).  No CUTLASS, cuBLAS or other library kernel is on the path.
+ * operands) in the two hand-written fused encoder-block kernels of csrc/policy_fused.cu, which keep the activations
+ * of a tile in shared memory / TMEM across the embedding, all layers and the first head layer; one more kernel
+ * (csrc/policy_forward.cu) forms the second head layers and the sample.  No CUTLASS, cuBLAS or other library kernel
+ * is on the path.
  *
  * Conventions as in uavenv_b200.h: 0 on success, negative error code otherwise; d_ = device pointers; work is
  * enqueued on the caller's stream; a handle is not thread-safe; no CPU fallback.
@@ -30,7 +31,7 @@ int uavpolicy_create(int32_t device, int32_t max_batch, uavpolicy_t **out);
 int uavpolicy_destroy(uavpolicy_t *p);
 const char *uavpolicy_last_error(const uavpolicy_t *p);
 /* version of this ABI (struct layouts, argument lists); the Python binding refuses a library that reports another */
-#define UAVPOLICY_ABI_VERSION 2
+#define UAVPOLICY_ABI_VERSION 3
 int uavpolicy_abi_version(void);
 
 /* Load the network weights from ONE flat fp32 device buffer holding every parameter in
@@ -51,11 +52,6 @@ int uavpolicy_set_weights(uavpolicy_t *p, const float *d_flat_params, void *stre
 int uavpolicy_get_action(uavpolicy_t *p, const float *d_obs, int32_t B, uint64_t seed, uint64_t step,
                          uint64_t env_id_base, int64_t *d_action, float *d_logp, float *d_value, float *d_entropy,
                          float *d_logits, void *stream);
-
-/* 1 (default): hand-written fused encoder blocks - one CTA per 25-sample tile keeps activations in shared memory /
- * TMEM across embedding, all layers and the first head layer (csrc/policy_fused.cu); 0: one tcgen05 GEMM launch per
- * dense layer (csrc/policy_gemm.cu) with separate attention / LayerNorm kernels.  Same results up to bf16 rounding. */
-int uavpolicy_set_fused(uavpolicy_t *p, int32_t fused);
 
 /* self-test of the hand-written tcgen05 path: D[128,N] (f32) = A[128,K] W[N,K]^T for one 128-row tile
  * (A, W bf16 row-major on the device; N <= 384, N % 16 == 0; K = 128 or 256). */

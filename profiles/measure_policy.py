@@ -60,19 +60,7 @@ def main():
         ms_t = timeit(run_torch, 2, 5)
         torch.backends.cuda.matmul.allow_tf32 = True
         ms_t32 = timeit(run_torch, 2, 5)
-        # the same forward as one tcgen05 GEMM launch per layer + separate attention / LayerNorm kernels (A/B path)
-        layered = ub.FusedPolicyForward(B, "cuda", fused=False)
-        layered.sync(net)
-        g2 = torch.cuda.CUDAGraph()
-        side.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(side):
-            layered.get_action(obs, 1)
-            with torch.cuda.graph(g2, stream=side):
-                layered.get_action(obs, 7)
-        torch.cuda.current_stream().wait_stream(side)
-        ms_l = timeit(g2.replay)
-        layered.close()
-        print(json.dumps({"B": B, "fused_ms": ms_f, "fused_graph_ms": ms_g, "per_layer_graph_ms": ms_l, "torch_fp32_ms": ms_t, "torch_tf32_ms": ms_t32,
+        print(json.dumps({"B": B, "fused_ms": ms_f, "fused_graph_ms": ms_g, "torch_fp32_ms": ms_t, "torch_tf32_ms": ms_t32,
                           "fused_samples_per_sec": B / (ms_g * 1e-3), "torch_samples_per_sec": B / (ms_t32 * 1e-3),
                           "fused_TFLOPs_executed": B * FLOP_LAST / (ms_g * 1e-3) / 1e12,
                           "speedup_vs_torch_tf32": ms_t32 / ms_g}))

@@ -159,7 +159,7 @@ def load_policy():
                 "stale" if os.path.isfile(path) else "missing", exc)) from exc
     L = C.CDLL(path)
     L.uavpolicy_abi_version.restype = C.c_int
-    if L.uavpolicy_abi_version() != 2:
+    if L.uavpolicy_abi_version() != 3:
         raise ImportError("libuavpolicy_b200.so ABI version mismatch")
     vp, i32, u64 = C.c_void_p, C.c_int32, C.c_uint64
     L.uavpolicy_create.argtypes = [i32, i32, C.POINTER(vp)]
@@ -168,7 +168,6 @@ def load_policy():
     L.uavpolicy_last_error.restype = C.c_char_p
     L.uavpolicy_set_weights.argtypes = [vp, vp, vp]
     L.uavpolicy_get_action.argtypes = [vp, vp, i32, u64, u64, u64, vp, vp, vp, vp, vp, vp]
-    L.uavpolicy_set_fused.argtypes = [vp, i32]
     L.uavpolicy_selftest_gemm_tile.argtypes = [vp, vp, vp, i32, i32, vp]
     i64 = C.c_int64
     L.uavpolicy_selftest_wgrad.argtypes = [vp, i64, vp, i64, i32, i32, i32, vp, vp, vp]
@@ -184,7 +183,7 @@ def load_policy():
     L.uavtrain_backward_heads.argtypes = [vp, vp, vp, vp, vp]
     L.uavtrain_ppo_loss.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, i32, C.c_float, C.c_float, C.c_float, vp, vp, vp, vp]
     for name in ("uavpolicy_create", "uavpolicy_destroy", "uavpolicy_set_weights", "uavpolicy_get_action",
-                 "uavpolicy_set_fused", "uavpolicy_selftest_gemm_tile", "uavpolicy_selftest_wgrad", "uavpolicy_selftest_dense",
+                 "uavpolicy_selftest_gemm_tile", "uavpolicy_selftest_wgrad", "uavpolicy_selftest_dense",
                  "uavpolicy_selftest_dense_ln", "uavtrain_create",
                  "uavtrain_destroy", "uavtrain_forward", "uavtrain_backward", "uavtrain_forward_heads",
                  "uavtrain_backward_heads", "uavtrain_ppo_loss"):

@@ -162,8 +162,8 @@ class PPOAgent:
         # the update's GEMMs (PyTorch autograd on the mirror network): "tf32" tensor-core math or strict "fp32"
         # or "fused": the hand-written sm_100a forward + backward of both trunks (csrc/policy_train.cu; bf16 operands,
         # fp32 accumulation and gradients), PyTorch only for the two small heads and the loss
-        if update_precision not in ("tf32", "fp32", "bf16", "fused"):
-            raise ValueError("update_precision must be 'fused', 'tf32', 'fp32' or 'bf16' (autocast)")
+        if update_precision not in ("tf32", "fp32", "fused"):
+            raise ValueError("update_precision must be 'fused', 'tf32' or 'fp32'")
         self.update_precision = update_precision
         self.trunks = None
         if update_precision == "fused":
@@ -239,10 +239,8 @@ class PPOAgent:
             self._apply_gradient()
             self._mb_sums += self._mb_stats
             return
-        else:
-            with torch.autocast("cuda", dtype=torch.bfloat16, enabled=self.update_precision == "bf16"):
-                logp, value, entropy = self.policy.evaluate(obs[idx], act[idx])
-        logp, value, entropy = logp.float(), value.float().squeeze(-1), entropy.float()
+        logp, value, entropy = self.policy.evaluate(obs[idx], act[idx])
+        value = value.squeeze(-1)
         ratio = torch.exp(logp - old_logp[idx])                             # :131
         a = self._adv[idx]
         loss_actor = -torch.min(ratio * a, torch.clamp(ratio, 1 - c.EPS_CLIP, 1 + c.EPS_CLIP) * a).mean()

@@ -394,14 +394,12 @@ int launch(const void *A, int64_t lda, const void *W, const float *bias, const v
 
 }  // namespace
 
-size_t gemm_workspace_bytes() { return 16; }   // (the hand-written kernel needs no workspace; kept for the call sites)
-
-int gemm_bias_act(const void *A, int64_t lda, const void *W, const float *bias, void *D, int M, int N, int K, int relu, void *,
-                  size_t, cudaStream_t stream) {
+int gemm_bias_act(const void *A, int64_t lda, const void *W, const float *bias, void *D, int M, int N, int K, int relu,
+                  cudaStream_t stream) {
     return launch(A, lda, W, bias, nullptr, 0, D, M, N, K, relu ? kRelu : kIdentity, stream);
 }
 
-int gemm_drelu(const void *A, int64_t lda, const void *W, const void *aux, int64_t ld_aux, void *D, int M, int N, int K, void *, size_t,
+int gemm_drelu(const void *A, int64_t lda, const void *W, const void *aux, int64_t ld_aux, void *D, int M, int N, int K,
                cudaStream_t stream) {
     return launch(A, lda, W, nullptr, aux, ld_aux, D, M, N, K, kDRelu, stream);
 }
@@ -417,9 +415,9 @@ int gemm_add_ln(const void *A, int64_t lda, const void *W, const float *bias, co
 // self-test hook: one dense product on caller-provided device buffers (act: 0 identity, 1 ReLU, 2 ReLU backward by d_aux)
 extern "C" int uavpolicy_selftest_dense(const void *d_a, int64_t lda, const void *d_w, const float *d_bias, const void *d_aux,
                                         int64_t ld_aux, void *d_out, int32_t M, int32_t N, int32_t K, int32_t act, void *stream) {
-    if (act == 2) return uavp::gemm_drelu(d_a, lda, d_w, d_aux, ld_aux, d_out, M, N, K, nullptr, 0, (cudaStream_t)stream);
+    if (act == 2) return uavp::gemm_drelu(d_a, lda, d_w, d_aux, ld_aux, d_out, M, N, K, (cudaStream_t)stream);
     if (act == 3) return -1;   // residual + LayerNorm: uavpolicy_selftest_dense_ln
-    return uavp::gemm_bias_act(d_a, lda, d_w, d_bias, d_out, M, N, K, act, nullptr, 0, (cudaStream_t)stream);
+    return uavp::gemm_bias_act(d_a, lda, d_w, d_bias, d_out, M, N, K, act, (cudaStream_t)stream);
 }
 
 // self-test hook of the fused residual + LayerNorm epilogue: d_out = LayerNorm(d_x + d_a d_w^T + d_bias) * d_gamma + d_beta,

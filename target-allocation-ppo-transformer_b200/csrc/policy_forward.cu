@@ -1,16 +1,14 @@
 // policy_forward.cu - rollout forward of TransformerActorCritic (networks/transformer_net.py:47-122) on sm_100a.
 //
-// Dense layers go through uavp::gemm_bias_act (tcgen05 / TMA / TMEM, policy_gemm.cu).  Everything between them is
-// hand-written here: embedding (K = 14 is below any tensor-core tile) + learned positions + padding mask, attention
-// over the 5-token window, residual + LayerNorm, and the two MLP heads fused with softmax, sampling, log-prob and
-// entropy.  Only the LAST token of the last encoder layer is ever read (transformer_net.py:106,114), so that layer
-// computes K/V for all five tokens but Q, out-proj, FFN and both LayerNorms for the last token only: 2.4 instead of
-// 4.0 MFLOP per sample.  Activations travel between kernels in bf16; LayerNorm / softmax / heads compute in fp32.
+// Two fused launches (policy_fused.cu) run the embedding, every encoder layer and the first head layer of both networks
+// with all dense contractions on tcgen05, and write the two [B,64] head-hidden rows in bf16.  heads_out_kernel below then
+// forms the second head layers in fp32 with softmax, the Categorical sample, log-prob and entropy.  The host side owns
+// the handle: a private fp32 copy of the parameters, the GEMM weights and biases pre-packed in the operand layouts the
+// fused kernels stage with bulk TMA, and the buffers passed between the launches.
 #include "uavpolicy_b200.h"
 
 #include <cstdarg>
 #include <cstdio>
-#include <cstring>
 #include <new>
 #include <string>
 #include <vector>
@@ -18,7 +16,6 @@
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
-#include "policy_gemm.cuh"
 #include "policy_kernels.cuh"
 #include "policy_weights.cuh"
 
@@ -39,7 +36,7 @@ __device__ __forceinline__ uint4 philox4x32(uint32_t k0, uint32_t k1, uint32_t c
     return make_uint4(c0, c1, c2, c3);
 }
 
-// head outputs (transformer_net.py:78-91 second layers; the first layers 128 -> 64 + ReLU ran as tensor-core GEMMs):
+// head outputs (transformer_net.py:78-91 second layers; the first layers 128 -> 64 + ReLU ran in the fused launches):
 // logits = W2a ha + b, value = W2c hc + b; softmax, Categorical sample (counter RNG), log-prob, entropy (:116-122).
 // One thread per sample.
 __global__ void __launch_bounds__(256) heads_out_kernel(const __nv_bfloat16 *__restrict__ Ha, const __nv_bfloat16 *__restrict__ Hc,
@@ -87,22 +84,18 @@ __global__ void __launch_bounds__(256) heads_out_kernel(const __nv_bfloat16 *__r
 struct uavpolicy {
     int device = 0, max_batch = 0;
     float *w32 = nullptr;                 // private fp32 copy of the flat parameters
-    __nv_bfloat16 *w16 = nullptr;         // bf16 copies (GEMM weights are read from here): one per block, each placed so
-    __nv_bfloat16 *w16_critic = nullptr;  // that the block's first parameter is 16 B aligned (TMA needs aligned operands)
     __nv_bfloat16 *emb2_a = nullptr, *emb2_c = nullptr;   // [128 x 32] tensor-core form of the two embedding weights
     __nv_bfloat16 *wpk = nullptr;         // GEMM weights pre-packed in canonical order (same element offsets as w32)
-    __nv_bfloat16 *bpk = nullptr;         // their biases as [N x 16] B-operands (3 layers + 2 heads), fused kernel only
+    __nv_bfloat16 *bpk = nullptr;         // their biases as [N x 16] B-operands (3 layers + 2 heads)
+    struct WPack { const __nv_bfloat16 *dst; size_t src; int N, K; };
+    std::vector<WPack> wpack;             // every GEMM weight: packed copy, its offset in w32, shape (set at create)
     BlockW actor, critic;
     HeadW actor_head, critic_head;
-    // bf16 activation workspaces (R = 5 * max_batch rows)
-    __nv_bfloat16 *Ea, *Ec, *QKV, *ATT, *T, *Y, *Hf, *X1, *Q, *AL, *T1, *Y1, *Hs, *T2, *Za, *Zc;
-    uint8_t *pad = nullptr;
+    __nv_bfloat16 *hh_actor = nullptr, *hh_critic = nullptr;   // [max_batch, 64] bf16: relu(W1 z + b1) of the two heads
     int *work_counter = nullptr;          // dynamic work-item counters of the two fused launches
     unsigned char *fused_scratch = nullptr;   // newest-token rows handed from the first fused launch to the second
-    void *gemm_ws = nullptr;
     std::vector<void *> allocs;
     bool have_weights = false;
-    bool fused = true;                    // hand-written fused tcgen05 blocks (policy_fused.cu) vs one GEMM per layer
     std::string err;
 };
 
@@ -133,24 +126,28 @@ static cudaError_t palloc(uavpolicy *p, T **ptr, size_t n) {
 constexpr size_t UPK_SIZE = (size_t)UAVPOLICY_NUM_PARAMS + 64;   // packed copies live at (offset rounded up to 8 elements)
 static inline size_t pk(size_t off) { return (off + 7) / 8 * 8; }
 
-static size_t map_block(BlockW &b, int layers, const float *w32, const __nv_bfloat16 *w16, const __nv_bfloat16 *wpk, size_t off) {
+// the [N x K] GEMM weight at element `off` of w32: its packed copy (16 B aligned for the bulk TMA copy), recorded for set_weights
+static const __nv_bfloat16 *map_weight(uavpolicy *p, size_t &off, int N, int K) {
+    const __nv_bfloat16 *dst = p->wpk + pk(off);
+    p->wpack.push_back({dst, off, N, K});
+    off += (size_t)N * K;
+    return dst;
+}
+static size_t map_block(uavpolicy *p, BlockW &b, int layers, size_t off) {
+    const float *w32 = p->w32;
     b.layers = layers;
     b.pos = w32 + off; off += S * D;
     b.emb_w = w32 + off; off += D * F;
     b.emb_b = w32 + off; off += D;
     for (int l = 0; l < layers; ++l) {
         LayerW &L = b.layer[l];
-        L.in_wp = wpk + pk(off);
-        L.in_w = w16 + off; off += 3 * D * D;
+        L.in_wp = map_weight(p, off, 3 * D, D);
         L.in_b = w32 + off; off += 3 * D;
-        L.out_wp = wpk + pk(off);
-        L.out_w = w16 + off; off += D * D;
+        L.out_wp = map_weight(p, off, D, D);
         L.out_b = w32 + off; off += D;
-        L.l1_wp = wpk + pk(off);
-        L.l1_w = w16 + off; off += FF * D;
+        L.l1_wp = map_weight(p, off, FF, D);
         L.l1_b = w32 + off; off += FF;
-        L.l2_wp = wpk + pk(off);
-        L.l2_w = w16 + off; off += D * FF;
+        L.l2_wp = map_weight(p, off, D, FF);
         L.l2_b = w32 + off; off += D;
         L.n1_w = w32 + off; off += D;
         L.n1_b = w32 + off; off += D;
@@ -159,12 +156,11 @@ static size_t map_block(BlockW &b, int layers, const float *w32, const __nv_bflo
     }
     return off;
 }
-static size_t map_head(HeadW &h, int outs, const float *w32, const __nv_bfloat16 *w16, const __nv_bfloat16 *wpk, size_t off) {
-    h.w1p = wpk + pk(off);
-    h.w1 = w16 + off; off += HID * D;
-    h.b1 = w32 + off; off += HID;
-    h.w2 = w32 + off; off += outs * HID;
-    h.b2 = w32 + off; off += outs;
+static size_t map_head(uavpolicy *p, HeadW &h, int outs, size_t off) {
+    h.w1p = map_weight(p, off, HID, D);
+    h.b1 = p->w32 + off; off += HID;
+    h.w2 = p->w32 + off; off += outs * HID;
+    h.b2 = p->w32 + off; off += outs;
     return off;
 }
 
@@ -185,17 +181,9 @@ extern "C" int uavpolicy_create(int32_t device, int32_t max_batch, uavpolicy_t *
     p->device = device; p->max_batch = max_batch;
     auto bail = [&](int rc) { g_err = p->err; for (void *q : p->allocs) cudaFree(q); delete p; return rc; };
     cudaError_t e = cudaSetDevice(device);
-    const size_t B = (size_t)max_batch, R = B * S;
     if (e == cudaSuccess) e = palloc(p, &p->w32, (size_t)UAVPOLICY_NUM_PARAMS);
-    if (e == cudaSuccess) e = palloc(p, &p->w16, 2 * ((size_t)UAVPOLICY_NUM_PARAMS + 16));
-    __nv_bfloat16 **big[] = {&p->Ea, &p->Ec, &p->ATT, &p->T, &p->Y, &p->X1};
-    for (auto b : big) if (e == cudaSuccess) e = palloc(p, b, R * D);
-    if (e == cudaSuccess) e = palloc(p, &p->QKV, R * 3 * D);
-    if (e == cudaSuccess) e = palloc(p, &p->Hf, R * FF);
-    __nv_bfloat16 **small[] = {&p->Q, &p->AL, &p->T1, &p->Y1, &p->T2, &p->Za, &p->Zc};
-    for (auto b : small) if (e == cudaSuccess) e = palloc(p, b, B * D);
-    if (e == cudaSuccess) e = palloc(p, &p->Hs, B * FF);
-    if (e == cudaSuccess) e = palloc(p, &p->pad, R);
+    if (e == cudaSuccess) e = palloc(p, &p->hh_actor, (size_t)max_batch * HID);
+    if (e == cudaSuccess) e = palloc(p, &p->hh_critic, (size_t)max_batch * HID);
     if (e == cudaSuccess) e = palloc(p, &p->work_counter, 2);
     if (e == cudaSuccess) e = palloc(p, &p->fused_scratch, uavp::fused_scratch_bytes(max_batch));
     if (e == cudaSuccess) e = cudaMemset(p->fused_scratch, 0, uavp::fused_scratch_bytes(max_batch));
@@ -203,16 +191,12 @@ extern "C" int uavpolicy_create(int32_t device, int32_t max_batch, uavpolicy_t *
     if (e == cudaSuccess) e = palloc(p, &p->bpk, (size_t)3 * uavp::kLayerBiasElems + 2 * HID * uavp::kBiasK);
     if (e == cudaSuccess) e = palloc(p, &p->emb2_a, (size_t)D * 32);
     if (e == cudaSuccess) e = palloc(p, &p->emb2_c, (size_t)D * 32);
-    if (e == cudaSuccess) { void *ws = nullptr; e = cudaMalloc(&ws, uavp::gemm_workspace_bytes()); if (e == cudaSuccess) { p->allocs.push_back(ws); p->gemm_ws = ws; } }
     if (e != cudaSuccess) { pfail(p, -2, "uavpolicy_create: %s", cudaGetErrorString(e)); return bail(-2); }
     if (uavp::fused_block_prepare() != 0) { pfail(p, -2, "uavpolicy_create: cannot reserve shared memory for the fused kernel"); return bail(-2); }
-    size_t off = map_block(p->actor, 1, p->w32, p->w16, p->wpk, 0);
-    // (the actor head's first layer starts at element 135040: 16 B aligned in the first bf16 copy)
-    off = map_head(p->actor_head, NACT, p->w32, p->w16, p->wpk, off);
-    // second bf16 copy, shifted so that element `off` (the critic block's first parameter) lands on a multiple of 8
-    p->w16_critic = p->w16 + ((size_t)UAVPOLICY_NUM_PARAMS + 15) / 8 * 8 + (8 - off % 8) % 8;
-    off = map_block(p->critic, 2, p->w32, p->w16_critic, p->wpk, off);
-    off = map_head(p->critic_head, 1, p->w32, p->w16_critic, p->wpk, off);   // 267520 elements later: still a multiple of 8
+    size_t off = map_block(p, p->actor, 1, 0);
+    off = map_head(p, p->actor_head, NACT, off);
+    off = map_block(p, p->critic, 2, off);
+    off = map_head(p, p->critic_head, 1, off);
     p->actor.emb_w2p = p->emb2_a; p->critic.emb_w2p = p->emb2_c;
     {   // bias operands: layers of the actor, then of the critic, then the two heads
         __nv_bfloat16 *q = p->bpk;
@@ -247,25 +231,14 @@ extern "C" int uavpolicy_set_weights(uavpolicy_t *p, const float *d_flat_params,
     cudaStream_t s = (cudaStream_t)stream;
     P_TRY(p, cudaSetDevice(p->device));
     P_TRY(p, cudaMemcpyAsync(p->w32, d_flat_params, (size_t)UAVPOLICY_NUM_PARAMS * sizeof(float), cudaMemcpyDeviceToDevice, s));
-    f32_to_bf16_kernel<<<(UAVPOLICY_NUM_PARAMS + 255) / 256, 256, 0, s>>>(p->w32, p->w16, UAVPOLICY_NUM_PARAMS);
-    f32_to_bf16_kernel<<<(UAVPOLICY_NUM_PARAMS + 255) / 256, 256, 0, s>>>(p->w32, p->w16_critic, UAVPOLICY_NUM_PARAMS);
-    {   // canonical-order copies of every GEMM weight for the fused kernel's bulk-TMA staging
-        auto packw = [&](const __nv_bfloat16 *dst, const __nv_bfloat16 *row_major16, int N, int K) {
-            const float *src = p->w32 + (row_major16 - (row_major16 >= p->w16_critic ? p->w16_critic : p->w16));
-            pack_canon_kernel<<<(N * K + 255) / 256, 256, 0, s>>>(src, const_cast<__nv_bfloat16 *>(dst), N, K);
-        };
-        const BlockW *blocks[2] = {&p->actor, &p->critic};
-        for (const BlockW *b : blocks)
-            for (int l = 0; l < b->layers; ++l) {
-                const LayerW &L = b->layer[l];
-                packw(L.in_wp, L.in_w, 3 * D, D); packw(L.out_wp, L.out_w, D, D);
-                packw(L.l1_wp, L.l1_w, FF, D); packw(L.l2_wp, L.l2_w, D, FF);
-            }
-        packw(p->actor_head.w1p, p->actor_head.w1, HID, D);
-        packw(p->critic_head.w1p, p->critic_head.w1, HID, D);
+    // canonical-order copies of every GEMM weight for the fused kernel's bulk-TMA staging
+    for (const uavpolicy::WPack &w : p->wpack)
+        pack_canon_kernel<<<(w.N * w.K + 255) / 256, 256, 0, s>>>(p->w32 + w.src, const_cast<__nv_bfloat16 *>(w.dst), w.N, w.K);
+    {
         auto packb = [&](const __nv_bfloat16 *dst, const float *bias, int N) {
             pack_bias_kernel<<<(N * 16 + 255) / 256, 256, 0, s>>>(bias, const_cast<__nv_bfloat16 *>(dst), N);
         };
+        const BlockW *blocks[2] = {&p->actor, &p->critic};
         for (const BlockW *b : blocks)
             for (int l = 0; l < b->layers; ++l) {
                 const LayerW &L = b->layer[l];
@@ -281,46 +254,6 @@ extern "C" int uavpolicy_set_weights(uavpolicy_t *p, const float *d_flat_params,
     return 0;
 }
 
-namespace {
-struct Ctx { uavpolicy *p; cudaStream_t s; int rc; };
-void gemm(Ctx &c, const __nv_bfloat16 *A, int64_t lda, const __nv_bfloat16 *W, const float *bias, __nv_bfloat16 *Dst, int M,
-          int N, int K, int relu) {
-    if (c.rc) return;
-    const int r = uavp::gemm_bias_act(A, lda, W, bias, Dst, M, N, K, relu, c.p->gemm_ws, uavp::gemm_workspace_bytes(), c.s);
-    if (r) c.rc = pfail(c.p, -2, "tcgen05 GEMM (M=%d N=%d K=%d) failed with %d", M, N, K, r);
-}
-void add_ln(Ctx &c, const __nv_bfloat16 *x, int64_t xs, const __nv_bfloat16 *y, const float *g, const float *b, int rows,
-            __nv_bfloat16 *out) {
-    if (c.rc) return;
-    add_ln_kernel<<<(rows * 32 + 255) / 256, 256, 0, c.s>>>(x, xs, y, g, b, rows, out);
-}
-// the LAST encoder layer of a block: only the newest token's output is needed (transformer_net.py:106,114)
-void last_layer(Ctx &c, const LayerW &L, const __nv_bfloat16 *X, int B, __nv_bfloat16 *Z) {
-    uavpolicy *p = c.p;
-    const int R = B * S;
-    gemm(c, X, D, L.in_w + D * D, L.in_b + D, p->QKV, R, 2 * D, D, 0);                 // K,V of all five tokens
-    gemm(c, X + (S - 1) * D, (int64_t)S * D, L.in_w, L.in_b, p->Q, B, D, D, 0);        // Q of the newest token
-    if (!c.rc) attn_last_kernel<<<(B * H + 255) / 256, 256, 0, c.s>>>(p->Q, p->QKV, p->pad, B, p->AL);
-    gemm(c, p->AL, D, L.out_w, L.out_b, p->T1, B, D, D, 0);
-    add_ln(c, X + (S - 1) * D, (int64_t)S * D, p->T1, L.n1_w, L.n1_b, B, p->Y1);
-    gemm(c, p->Y1, D, L.l1_w, L.l1_b, p->Hs, B, FF, D, 1);
-    gemm(c, p->Hs, FF, L.l2_w, L.l2_b, p->T2, B, D, FF, 0);
-    add_ln(c, p->Y1, D, p->T2, L.n2_w, L.n2_b, B, Z);
-}
-// an inner encoder layer: all five tokens
-void full_layer(Ctx &c, const LayerW &L, const __nv_bfloat16 *X, int B, __nv_bfloat16 *Xout) {
-    uavpolicy *p = c.p;
-    const int R = B * S;
-    gemm(c, X, D, L.in_w, L.in_b, p->QKV, R, 3 * D, D, 0);
-    if (!c.rc) attn_full_kernel<<<(B + 7) / 8, 256, 0, c.s>>>(p->QKV, p->pad, B, p->ATT);
-    gemm(c, p->ATT, D, L.out_w, L.out_b, p->T, R, D, D, 0);
-    add_ln(c, X, D, p->T, L.n1_w, L.n1_b, R, p->Y);
-    gemm(c, p->Y, D, L.l1_w, L.l1_b, p->Hf, R, FF, D, 1);
-    gemm(c, p->Hf, FF, L.l2_w, L.l2_b, p->T, R, D, FF, 0);
-    add_ln(c, p->Y, D, p->T, L.n2_w, L.n2_b, R, Xout);
-}
-}  // namespace
-
 extern "C" int uavpolicy_get_action(uavpolicy_t *p, const float *d_obs, int32_t B, uint64_t seed, uint64_t step,
                                     uint64_t env_id_base, int64_t *d_action, float *d_logp, float *d_value,
                                     float *d_entropy, float *d_logits, void *stream) {
@@ -329,37 +262,14 @@ extern "C" int uavpolicy_get_action(uavpolicy_t *p, const float *d_obs, int32_t 
     if (B <= 0 || B > p->max_batch) return pfail(p, -1, "uavpolicy_get_action: B=%d outside (0, %d]", B, p->max_batch);
     if (!p->have_weights) return pfail(p, -4, "uavpolicy_get_action before uavpolicy_set_weights");
     P_TRY(p, cudaSetDevice(p->device));
-    Ctx c{p, (cudaStream_t)stream, 0};
-    const int R = B * S;
-    if (p->fused) {
-        // two fused launches (actor block + head layer 1, critic block + head layer 1), then the per-sample outputs
-        if (uavp::launch_fused_blocks(d_obs, B, p->actor, p->actor_head, p->T1, p->critic, p->critic_head, p->T2,
-                                      p->work_counter, p->fused_scratch, c.s))
-            return pfail(p, -2, "fused block launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-        heads_out_kernel<<<(B + 255) / 256, 256, 0, c.s>>>(p->T1, p->T2, p->actor_head, p->critic_head, B, (uint32_t)seed,
-                                                           (uint32_t)(seed >> 32), step, env_id_base, d_action, d_logp, d_value,
-                                                           d_entropy, d_logits);
-        P_TRY(p, cudaGetLastError());
-        return 0;
-    }
-    embed_kernel<<<(R + kEmbTok - 1) / kEmbTok, kEmbThreads, 0, c.s>>>(d_obs, R, p->actor, p->critic, p->Ea, p->Ec, p->pad);
-    last_layer(c, p->actor.layer[0], p->Ea, B, p->Za);              // actor: 1 layer
-    full_layer(c, p->critic.layer[0], p->Ec, B, p->X1);             // critic: 2 layers
-    last_layer(c, p->critic.layer[1], p->X1, B, p->Zc);
-    if (c.rc) return c.rc;
-    // heads: first layers on the tensor cores (N = 64 is half a tile), second layers + sampling per sample
-    gemm(c, p->Za, D, p->actor_head.w1, p->actor_head.b1, p->T1, B, HID, D, 1);
-    gemm(c, p->Zc, D, p->critic_head.w1, p->critic_head.b1, p->T2, B, HID, D, 1);
-    if (c.rc) return c.rc;
-    heads_out_kernel<<<(B + 255) / 256, 256, 0, c.s>>>(p->T1, p->T2, p->actor_head, p->critic_head, B, (uint32_t)seed,
-                                                       (uint32_t)(seed >> 32), step, env_id_base, d_action, d_logp, d_value,
-                                                       d_entropy, d_logits);
+    const cudaStream_t s = (cudaStream_t)stream;
+    // two fused launches (actor block + head layer 1, critic block + head layer 1), then the per-sample outputs
+    if (uavp::launch_fused_blocks(d_obs, B, p->actor, p->actor_head, p->hh_actor, p->critic, p->critic_head, p->hh_critic,
+                                  p->work_counter, p->fused_scratch, s))
+        return pfail(p, -2, "fused block launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    heads_out_kernel<<<(B + 255) / 256, 256, 0, s>>>(p->hh_actor, p->hh_critic, p->actor_head, p->critic_head, B, (uint32_t)seed,
+                                                     (uint32_t)(seed >> 32), step, env_id_base, d_action, d_logp, d_value,
+                                                     d_entropy, d_logits);
     P_TRY(p, cudaGetLastError());
-    return 0;
-}
-
-extern "C" int uavpolicy_set_fused(uavpolicy_t *p, int32_t fused) {
-    if (!p) return -1;
-    p->fused = fused != 0;
     return 0;
 }

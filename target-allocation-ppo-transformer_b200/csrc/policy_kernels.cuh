@@ -1,6 +1,6 @@
-// policy_kernels.cuh - the hand-written (non-GEMM) kernels of the policy network shared by the rollout forward
-// (policy_forward.cu) and the PPO update (policy_train.cu): weight packing, embedding + positions + padding mask,
-// attention over the 5-token window, residual + LayerNorm.  Internal linkage: each translation unit gets its own copy.
+// policy_kernels.cuh - the hand-written (non-GEMM) kernels of the policy network outside the fused blocks: the weight
+// packing of the rollout forward (policy_forward.cu), and the embedding + positions + padding mask and the attention over
+// the 5-token window of the PPO update (policy_train.cu).  Internal linkage: each translation unit gets its own copy.
 #pragma once
 #include <cstdint>
 #include <cuda_bf16.h>
@@ -42,11 +42,6 @@ __global__ void pack_canon_kernel(const float *__restrict__ w, __nv_bfloat16 *__
     out[canon_elem(i / K, i % K, K)] = __float2bfloat16(w[i]);
 }
 
-__global__ void f32_to_bf16_kernel(const float *__restrict__ src, __nv_bfloat16 *__restrict__ dst, int n) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) dst[i] = __float2bfloat16(src[i]);
-}
-
 // embedding of both nets: E = relu(obs W^T + b) + pos (transformer_net.py:24-30,57-59) and the key-padding mask
 // (rows that are all zero, newest row never: :52-54).  One CTA = 64 tokens; thread = (net, feature pair), so a warp
 // stores 128 contiguous bytes per token.
@@ -71,6 +66,8 @@ __global__ void __launch_bounds__(kEmbThreads) embed_kernel(const float *__restr
     // obs16 / relu_mask (training only): a bf16 copy of the observation rows zero-padded to 64 columns (the B operand of
     // the embedding's weight-gradient product) and the ReLU activity bits of both networks, [R][net][4 words]:
     // word k, bit l  <->  feature 4 l + k
+    // (the update always passes both; without the null checks below nvcc schedules this kernel about 11 us slower per
+    // 131072-window minibatch on a B200, measured)
     __shared__ __align__(16) float2 s_obs[kEmbTok][F];            // every value twice: the (x, x) operand of the packed FMA
     const int t0 = blockIdx.x * kEmbTok;
     {   // the CTA's 60 x 14 floats are contiguous and 16-byte aligned: all loads of a thread go out before any is used
@@ -303,37 +300,6 @@ __global__ void attn_last_kernel(const __nv_bfloat16 *__restrict__ Q, const __nv
     const __nv_bfloat16 *base = KV + (size_t)b * S * 2 * D + h * DH;
     attend(q, base, base + D, 2 * D, pad + b * S, o);
     store16(ATT + (size_t)b * D + h * DH, o);
-}
-
-// out[r] = LayerNorm(x[r] + y[r]) * g + beta over 128 features (post-LN, eps 1e-5); one warp per row
-__global__ void add_ln_kernel(const __nv_bfloat16 *__restrict__ x, int64_t x_stride, const __nv_bfloat16 *__restrict__ y,
-                              const float *__restrict__ g, const float *__restrict__ beta, int rows,
-                              __nv_bfloat16 *__restrict__ out) {
-    const int r = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
-    if (r >= rows) return;
-    const uint2 xa = *reinterpret_cast<const uint2 *>(x + (size_t)r * x_stride + lane * 4);
-    const uint2 ya = *reinterpret_cast<const uint2 *>(y + (size_t)r * D + lane * 4);
-    float v[4];
-    {
-        const __nv_bfloat162 x0 = *reinterpret_cast<const __nv_bfloat162 *>(&xa.x), x1 = *reinterpret_cast<const __nv_bfloat162 *>(&xa.y);
-        const __nv_bfloat162 y0 = *reinterpret_cast<const __nv_bfloat162 *>(&ya.x), y1 = *reinterpret_cast<const __nv_bfloat162 *>(&ya.y);
-        v[0] = __low2float(x0) + __low2float(y0); v[1] = __high2float(x0) + __high2float(y0);
-        v[2] = __low2float(x1) + __low2float(y1); v[3] = __high2float(x1) + __high2float(y1);
-    }
-    float s = v[0] + v[1] + v[2] + v[3];
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-    const float mean = s * (1.0f / D);
-    float q = 0.0f;
-#pragma unroll
-    for (int i = 0; i < 4; ++i) { v[i] -= mean; q = fmaf(v[i], v[i], q); }
-    for (int o = 16; o > 0; o >>= 1) q += __shfl_xor_sync(0xffffffffu, q, o);
-    const float rstd = rsqrtf(q * (1.0f / D) + 1e-5f);
-    const float *gp = g + lane * 4, *bp = beta + lane * 4;   // (scalar loads: the flat parameter buffer is only 4 B aligned)
-    const __nv_bfloat162 o0 = __floats2bfloat162_rn(v[0] * rstd * gp[0] + bp[0], v[1] * rstd * gp[1] + bp[1]);
-    const __nv_bfloat162 o1 = __floats2bfloat162_rn(v[2] * rstd * gp[2] + bp[2], v[3] * rstd * gp[3] + bp[3]);
-    uint2 ov;
-    ov.x = *reinterpret_cast<const uint32_t *>(&o0); ov.y = *reinterpret_cast<const uint32_t *>(&o1);
-    *reinterpret_cast<uint2 *>(out + (size_t)r * D + lane * 4) = ov;
 }
 
 }  // namespace

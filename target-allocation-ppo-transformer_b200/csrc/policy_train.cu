@@ -562,7 +562,6 @@ struct uavtrain {
     uint32_t *relu_mask = nullptr;               // [R][2 nets][4 words] ReLU activity bits of the two embeddings
     uint8_t *pad = nullptr;
     const float *params = nullptr;               // likewise (second head layers)
-    void *gemm_ws = nullptr;
     std::vector<void *> allocs;
     std::string err;
 };
@@ -639,7 +638,7 @@ struct TCtx { uavtrain *p; cudaStream_t s; int rc; };
 
 void gemm(TCtx &c, const bf16 *A, int64_t lda, const bf16 *W, const float *bias, bf16 *Dst, int M, int N, int K, int relu) {
     if (c.rc) return;
-    const int r = uavp::gemm_bias_act(A, lda, W, bias ? bias : c.p->zeros, Dst, M, N, K, relu, c.p->gemm_ws, uavp::gemm_workspace_bytes(), c.s);
+    const int r = uavp::gemm_bias_act(A, lda, W, bias ? bias : c.p->zeros, Dst, M, N, K, relu, c.s);
     if (r) c.rc = tfail(c.p, -2, "tcgen05 GEMM (M=%d N=%d K=%d) failed with %d", M, N, K, r);
 }
 // out = LayerNorm(x + A W^T + bias) fused into the dense kernel's epilogue (policy_dense.cu), keeping x^ and 1/sigma
@@ -709,7 +708,7 @@ void ffn_ln_bwd(TCtx &c, const uavp::LayerW &L, const LayerT &T, const LayerOff 
     ln_bwd(c, dz32, dz_stride, dz16, nullptr, XH2, rstd2, L.n2_w, rows, p->dS2, g + o.n2_w, g + o.n2_b, g + o.l2_b);
     wgrad(c, p->dS2, D, Hact, FF, rows, D, FF, g + o.l2_w);
     if (!c.rc) {                                              // dH = (dS2 W2) masked by the forward's ReLU, in one GEMM
-        const int r = uavp::gemm_drelu(p->dS2, D, T.l2_t, Hact, FF, p->dH, rows, FF, D, p->gemm_ws, uavp::gemm_workspace_bytes(), c.s);
+        const int r = uavp::gemm_drelu(p->dS2, D, T.l2_t, Hact, FF, p->dH, rows, FF, D, c.s);
         if (r) c.rc = tfail(p, -2, "tcgen05 GEMM with ReLU-backward epilogue (M=%d) failed with %d", rows, r);
     }
     wgrad(c, p->dH, FF, Y1, D, rows, FF, D, g + o.l1_w, -1, g + o.l1_b);                  // + bias gradient dH^T 1
@@ -806,7 +805,6 @@ extern "C" int uavtrain_create(int32_t device, int32_t max_samples, uavtrain_t *
     if (e == cudaSuccess) e = talloc(p, &p->relu_mask, R * 8);
     if (e == cudaSuccess) e = talloc(p, &p->zeros, (size_t)3 * D);
     if (e == cudaSuccess) e = cudaMemset(p->zeros, 0, 3 * D * sizeof(float));
-    if (e == cudaSuccess) { void *ws = nullptr; e = cudaMalloc(&ws, uavp::gemm_workspace_bytes()); if (e == cudaSuccess) { p->allocs.push_back(ws); p->gemm_ws = ws; } }
     if (e != cudaSuccess) { tfail(p, -2, "uavtrain_create: %s", cudaGetErrorString(e)); return bail(-2); }
     if (uavp::wgrad_prepare() != 0) { tfail(p, -2, "uavtrain_create: cannot reserve shared memory for the weight-gradient kernel"); return bail(-2); }
     size_t arena_off = 0;

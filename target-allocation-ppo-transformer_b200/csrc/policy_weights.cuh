@@ -18,9 +18,9 @@ constexpr int kLayerBiasElems = (3 * D + D + FF + D) * kBiasK;  // bias operands
 static_assert(kBlockBase + kLayerParams + kActorHead + kBlockBase + 2 * kLayerParams + kCriticHead == UAVPOLICY_NUM_PARAMS,
               "parameter layout");
 
-struct LayerW {  // views into the fp32 copy / the bf16 copy of one encoder layer
-    const __nv_bfloat16 *in_w, *out_w, *l1_w, *l2_w;  // [384,128] [128,128] [256,128] [128,256] row-major
-    const __nv_bfloat16 *in_wp, *out_wp, *l1_wp, *l2_wp;  // the same matrices pre-packed in UMMA canonical K-major order
+struct LayerW {  // views of the parameters of one encoder layer
+    const __nv_bfloat16 *in_w, *out_w, *l1_w, *l2_w;  // [384,128] [128,128] [256,128] [128,256] bf16 row-major (PPO update)
+    const __nv_bfloat16 *in_wp, *out_wp, *l1_wp, *l2_wp;  // the same matrices pre-packed in UMMA canonical K-major order (fused kernel)
     // the four biases as [N x 16] bf16 B-operands of one more k-step (canonical order): column 0 = bf16(b), column 1 = the
     // rounding remainder, the rest zero - against an A-operand of ones the tensor core adds the bias (fused kernel only)
     const __nv_bfloat16 *in_bp = nullptr, *out_bp = nullptr, *l1_bp = nullptr, *l2_bp = nullptr;
@@ -34,7 +34,7 @@ struct BlockW {
     LayerW layer[2];
     int layers;
 };
-struct HeadW { const __nv_bfloat16 *w1, *w1p; const float *b1, *w2, *b2; const __nv_bfloat16 *b1p = nullptr; };  // w1 [64,128] bf16 (+ packed; b1p: b1 as a bias operand), rest fp32
+struct HeadW { const __nv_bfloat16 *w1p; const float *b1, *w2, *b2; const __nv_bfloat16 *b1p = nullptr; };  // w1p: W1 [64,128] packed bf16; b1p: b1 as a bias operand; rest fp32
 
 
 // fused encoder blocks (policy_fused.cu): embedding + all post-LN encoder layers + first head layer of BOTH networks for a

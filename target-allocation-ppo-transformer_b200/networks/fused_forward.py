@@ -1,11 +1,12 @@
-"""Rollout forward of the policy on the 5th-gen tensor cores (csrc/policy_forward.cu + policy_gemm.cu) behind the
+"""Rollout forward of the policy on the 5th-gen tensor cores (csrc/policy_fused.cu + policy_forward.cu) behind the
 `get_action` contract of networks/transformer_net.py:96-122.
 
     fused = FusedPolicyForward(max_batch, device); fused.sync(policy_old)
     action, logp, value, entropy = fused.get_action(obs, step)
 
 bf16 operands / fp32 accumulation: outputs agree with the fp32 network to ~1e-2 absolute (tested); gradients are
-never taken through this path - PPO's update evaluates the fp32 PyTorch mirror."""
+never taken through this path - PPO's update evaluates the network again (networks/fused_train.py or the PyTorch
+mirror, by PPOAgent's update_precision)."""
 import ctypes as C
 
 import torch
@@ -14,7 +15,7 @@ from .. import _capi
 
 
 class FusedPolicyForward:
-    def __init__(self, max_batch, device, seed=0, env_id_base=0, fused=True):
+    def __init__(self, max_batch, device, seed=0, env_id_base=0):
         self._h = None
         self.device = torch.device(device)
         if self.device.type != "cuda":
@@ -27,7 +28,6 @@ class FusedPolicyForward:
         if rc != 0:
             raise _capi.UavenvError(rc, (self._lib.uavpolicy_last_error(None) or b"").decode())
         self._h = h
-        self._lib.uavpolicy_set_fused(h, int(bool(fused)))   # False: one tcgen05 GEMM launch per layer (A/B reference)
         self.max_batch, self.seed, self.env_id_base = int(max_batch), int(seed), int(env_id_base)
         dev = self.device
         self.action = torch.zeros(max_batch, dtype=torch.int64, device=dev)

@@ -32,10 +32,10 @@ def test_policy_library_exports_every_declared_symbol_and_is_tcgen05():
     from target_allocation_ppo_transformer_b200 import _build, _capi
     L = _capi.load_policy()
     names = _declared("uavpolicy_b200.h", "uavpolicy|uavtrain")
-    assert len(names) == 19
+    assert len(names) == 18
     for name in names:
         assert hasattr(L, name), "libuavpolicy_b200.so does not export %s" % name
-    assert L.uavpolicy_abi_version() == 2
+    assert L.uavpolicy_abi_version() == 3
     sass = subprocess.run(["cuobjdump", "-sass", _build.POLICY_LIB_PATH], capture_output=True, text=True).stdout
     assert "UTCHMMA" in sass and "UTMALDG" in sass          # tcgen05.mma and TMA loads (B200_PROFILING.md)
     h = C.c_void_p()

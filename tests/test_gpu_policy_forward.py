@@ -36,12 +36,11 @@ def test_handwritten_tcgen05_gemm_tile_selftest():
         assert float((Dst - A.float() @ W.float().t()).abs().max()) < 1e-4
 
 
-@pytest.mark.parametrize("fused_kernel", [True, False])
-def test_forward_matches_fp32_network_and_reference_golden(fused_kernel):
+def test_forward_matches_fp32_network_and_reference_golden():
     from target_allocation_ppo_transformer_b200.networks.fused_forward import FusedPolicyForward
     net, fx = _net()
     obs = torch.from_numpy(fx["obs"]).cuda()
-    fused = FusedPolicyForward(256, "cuda", fused=fused_kernel)
+    fused = FusedPolicyForward(256, "cuda")
     fused.sync(net)
     a, lp, v, e = fused.get_action(obs, step=0)
     logits = fused.logits[: obs.shape[0]]
@@ -60,12 +59,11 @@ def test_forward_matches_fp32_network_and_reference_golden(fused_kernel):
     fused.close()
 
 
-@pytest.mark.parametrize("fused_kernel", [True, False])
-def test_padding_rows_and_batch_tails(fused_kernel):
+def test_padding_rows_and_batch_tails():
     """Episode starts (leading zero rows are masked keys) and batch sizes that are not tile multiples."""
     from target_allocation_ppo_transformer_b200.networks.fused_forward import FusedPolicyForward
     net, _ = _net()
-    fused = FusedPolicyForward(1000, "cuda", fused=fused_kernel)
+    fused = FusedPolicyForward(1000, "cuda")
     fused.sync(net)
     g = torch.Generator(device="cuda").manual_seed(1)
     for B in (1, 7, 24, 26, 129, 1000):
