@@ -171,6 +171,35 @@ int uavenv_recompute_objective(uavenv_t *h, double *h_max_abs_diff, void *stream
  * the env-only benchmarks (SURVEY.md §8d) */
 int uavenv_random_actions(uavenv_t *h, uint64_t action_seed, uint64_t step, int64_t *d_actions, void *stream);
 
+/* ---- per-episode records of an evaluation (csrc/uavenv_episodes.cu) ---------------------------------------------
+ * One finished episode.  ret sums the fp64 step rewards (info d_reward_f64) in step order; J_val, avg_p_dmg,
+ * avg_p_final and num_assigned are the info of the episode's last step, i.e. of its final allocation. */
+typedef struct uavenv_episode {
+    double ret;
+    float J_val, avg_p_dmg, avg_p_final;
+    int32_t length;           /* steps of the episode */
+    int32_t num_assigned;     /* covered targets N0 at the end */
+    int32_t assigns;          /* steps with action == 1 */
+    int32_t valid;            /* steps with is_valid_action == 1 (the reference's "valid assign") */
+} uavenv_episode_t;           /* 40 bytes */
+
+/* Running state of the episodes in progress: device arrays [B], zeroed by the caller before the first step, plus
+ * d_envs_complete, one device int counting the envs that have recorded their quota. */
+typedef struct uavenv_episode_acc {
+    double *d_ret;
+    int32_t *d_length, *d_assigns, *d_valid;
+    int32_t *d_episodes;      /* episodes recorded so far per env */
+    int32_t *d_envs_complete;
+} uavenv_episode_acc_t;
+
+/* Folds one step's d_actions [B], d_done [B] and info into acc (one thread per env, one launch).  When env b finishes
+ * its k-th episode (k < episodes_per_env) the record goes to d_records[b * episodes_per_env + k]; later episodes are
+ * dropped, and *d_envs_complete is incremented once, when env b records its last one.  Every info pointer must be
+ * non-NULL; argument errors return UAVENV_EINVAL before the GPU is touched. */
+int uavenv_episode_accumulate(int32_t B, const int64_t *d_actions, const uint8_t *d_done, const uavenv_info_t *info,
+                              int32_t episodes_per_env, const uavenv_episode_acc_t *acc, uavenv_episode_t *d_records,
+                              int32_t device, void *stream);
+
 /* ---- PPO rollout post-processing (agents/ppo.py:77-94) ------------------------------------------
  * GAE(gamma, lambda) over a [T,B] rollout (time-major) followed by the global advantage
  * normalisation (mean, unbiased std, +1e-7).  d_last_value[B] is V(s_T) for bootstrapping (NULL = 0,

@@ -29,10 +29,12 @@ LIBS = {
         ("ppo_gae.cu", [], ["../../include/uavenv_b200.h"]),
         ("ppo_attn.cu", [], ["../../include/uavenv_b200.h"]),
         ("ppo_optim.cu", [], ["../../include/uavenv_b200.h"]),
+        ("uavenv_episodes.cu", [], ["../../include/uavenv_b200.h"]),
     ],
     POLICY_LIB_PATH: [
         ("policy_dense.cu", [], ["policy_gemm.cuh", "tcgen05_util.cuh", "../../include/uavpolicy_b200.h"]),
-        ("policy_forward.cu", [], ["policy_kernels.cuh", "policy_weights.cuh", "../../include/uavpolicy_b200.h"]),
+        ("policy_forward.cu", [], ["policy_kernels.cuh", "policy_weights.cuh", "../../include/uavpolicy_b200.h",
+                                   "../../include/uavpolicy_eval_b200.h"]),
         ("policy_train.cu", [], ["policy_gemm.cuh", "policy_kernels.cuh", "policy_weights.cuh", "../../include/uavpolicy_b200.h"]),
         ("policy_wgrad.cu", [], ["tcgen05_util.cuh", "policy_weights.cuh", "../../include/uavpolicy_b200.h"]),
         ("policy_fused.cu", [], ["tcgen05_util.cuh", "policy_weights.cuh", "../../include/uavpolicy_b200.h"]),

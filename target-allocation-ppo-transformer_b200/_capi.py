@@ -35,6 +35,16 @@ class UavenvInfo(C.Structure):
                 ("d_avg_p_dmg", C.c_void_p), ("d_avg_p_final", C.c_void_p), ("d_reward_f64", C.c_void_p)]
 
 
+class UavenvEpisodeAcc(C.Structure):
+    _fields_ = [("d_ret", C.c_void_p), ("d_length", C.c_void_p), ("d_assigns", C.c_void_p), ("d_valid", C.c_void_p),
+                ("d_episodes", C.c_void_p), ("d_envs_complete", C.c_void_p)]
+
+
+# uavenv_episode_t (40 bytes, C layout)
+EPISODE_FIELDS = [("ret", "<f8"), ("J_val", "<f4"), ("avg_p_dmg", "<f4"), ("avg_p_final", "<f4"), ("length", "<i4"),
+                  ("num_assigned", "<i4"), ("assigns", "<i4"), ("valid", "<i4")]
+EPISODE_BYTES = 40
+
 SCENE_FIELDS = [("uav_x", "f8", "N"), ("uav_y", "f8", "N"), ("uav_vx", "f8", "N"), ("uav_vy", "f8", "N"),
                 ("uav_load", "f8", "N"), ("uav_cost", "f8", "N"), ("uav_type", "i4", "N"),
                 ("tgt_x", "f8", "M"), ("tgt_y", "f8", "M"), ("tgt_vx", "f8", "M"), ("tgt_vy", "f8", "M"),
@@ -111,6 +121,7 @@ def load():
     L.uavenv_score_matrix_f64.argtypes = [vp, vp, vp, vp]
     L.uavenv_recompute_objective.argtypes = [vp, c_f64p, vp]
     L.uavenv_random_actions.argtypes = [vp, u64, u64, vp, vp]
+    L.uavenv_episode_accumulate.argtypes = [i32, vp, vp, C.POINTER(UavenvInfo), i32, C.POINTER(UavenvEpisodeAcc), vp, i32, vp]
     L.ppo_gae_advantages.argtypes = [vp, vp, vp, vp, i32, i32, C.c_float, C.c_float, vp, vp, i32, vp, i32, vp]
     L.ppo_normalize_advantages.argtypes = [vp, i64, vp, i32, vp]
     L.ppo_attn5_forward.argtypes = [vp, i64, vp, vp, i64, vp, i64, i32, vp, i32, vp]
@@ -124,7 +135,7 @@ def load():
     for name in ("uavenv_create", "uavenv_destroy", "uavenv_reset", "uavenv_step", "uavenv_step_host",
                  "uavenv_load_scene", "uavenv_get_scene", "uavenv_get_state", "uavenv_score_matrix",
                  "uavenv_score_matrix_f64", "uavenv_recompute_objective", "uavenv_random_actions",
-                 "ppo_gae_advantages", "ppo_normalize_advantages"):
+                 "uavenv_episode_accumulate", "ppo_gae_advantages", "ppo_normalize_advantages"):
         getattr(L, name).restype = C.c_int
     if L.uavenv_abi_version() != 2:
         raise ImportError("libuavenv_b200.so ABI version mismatch")
@@ -168,6 +179,7 @@ def load_policy():
     L.uavpolicy_last_error.restype = C.c_char_p
     L.uavpolicy_set_weights.argtypes = [vp, vp, vp]
     L.uavpolicy_get_action.argtypes = [vp, vp, i32, u64, u64, u64, vp, vp, vp, vp, vp, vp]
+    L.uavpolicy_act.argtypes = [vp, vp, i32, i32, u64, u64, u64, vp, vp, vp, vp]        # include/uavpolicy_eval_b200.h
     L.uavpolicy_selftest_gemm_tile.argtypes = [vp, vp, vp, i32, i32, vp]
     i64 = C.c_int64
     L.uavpolicy_selftest_wgrad.argtypes = [vp, i64, vp, i64, i32, i32, i32, vp, vp, vp]
@@ -183,7 +195,7 @@ def load_policy():
     L.uavtrain_backward_heads.argtypes = [vp, vp, vp, vp, vp]
     L.uavtrain_ppo_loss.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, i32, C.c_float, C.c_float, C.c_float, vp, vp, vp, vp]
     for name in ("uavpolicy_create", "uavpolicy_destroy", "uavpolicy_set_weights", "uavpolicy_get_action",
-                 "uavpolicy_selftest_gemm_tile", "uavpolicy_selftest_wgrad", "uavpolicy_selftest_dense",
+                 "uavpolicy_act", "uavpolicy_selftest_gemm_tile", "uavpolicy_selftest_wgrad", "uavpolicy_selftest_dense",
                  "uavpolicy_selftest_dense_ln", "uavtrain_create",
                  "uavtrain_destroy", "uavtrain_forward", "uavtrain_backward", "uavtrain_forward_heads",
                  "uavtrain_backward_heads", "uavtrain_ppo_loss"):

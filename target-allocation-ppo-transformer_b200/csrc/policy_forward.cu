@@ -4,8 +4,10 @@
 // with all dense contractions on tcgen05, and write the two [B,64] head-hidden rows in bf16.  heads_out_kernel below then
 // forms the second head layers in fp32 with softmax, the Categorical sample, log-prob and entropy.  The host side owns
 // the handle: a private fp32 copy of the parameters, the GEMM weights and biases pre-packed in the operand layouts the
-// fused kernels stage with bulk TMA, and the buffers passed between the launches.
+// fused kernels stage with bulk TMA, and the buffers passed between the launches.  uavpolicy_act (uavpolicy_eval_b200.h)
+// runs the same launches on the actor's work items alone and actor_out_kernel in place of heads_out_kernel.
 #include "uavpolicy_b200.h"
+#include "uavpolicy_eval_b200.h"
 
 #include <cstdarg>
 #include <cstdio>
@@ -74,6 +76,46 @@ __global__ void __launch_bounds__(256) heads_out_kernel(const __nv_bfloat16 *__r
     if (logp) logp[b] = a ? lp1 : lp0;
     if (value) value[b] = vv;
     if (entropy) entropy[b] = -(p0 * lp0 + p1 * lp1);
+    if (logits_out) { logits_out[2 * b] = l0; logits_out[2 * b + 1] = l1; }
+}
+
+// uavpolicy_act: the actor half of heads_out_kernel.  The logits, the softmax and the draw are formed by the same operations
+// in the same order, so a sample (greedy = 0) is bit-identical to heads_out_kernel's for the same keys.  greedy = 1 takes
+// argmax, a tie going to action 0 (torch.argmax).  The critic's head-hidden rows are stale in this mode and are not read.
+__global__ void __launch_bounds__(256) actor_out_kernel(const __nv_bfloat16 *__restrict__ Ha, HeadW ha, int B, int greedy,
+                                                        uint32_t k0, uint32_t k1, uint64_t step, uint64_t env_base,
+                                                        int64_t *__restrict__ action, float *__restrict__ logp,
+                                                        float *__restrict__ logits_out) {
+    __shared__ float s_w[2][HID];
+    for (int i = threadIdx.x; i < HID; i += blockDim.x) { s_w[0][i] = ha.w2[i]; s_w[1][i] = ha.w2[HID + i]; }
+    __syncthreads();
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    float l0 = ha.b2[0], l1 = ha.b2[1];
+#pragma unroll
+    for (int c = 0; c < HID / DH; ++c) {
+        float xa[DH];
+        load16(Ha + (size_t)b * HID + c * DH, xa);
+#pragma unroll
+        for (int e = 0; e < DH; ++e) {
+            l0 = fmaf(s_w[0][c * DH + e], xa[e], l0);
+            l1 = fmaf(s_w[1][c * DH + e], xa[e], l1);
+        }
+    }
+    const float m = fmaxf(l0, l1), e0 = expf(l0 - m), e1 = expf(l1 - m), lse = m + logf(e0 + e1);
+    const float lp0 = l0 - lse, lp1 = l1 - lse;
+    int a;
+    if (greedy) {
+        a = l1 > l0 ? 1 : 0;
+    } else {
+        const float p1 = expf(lp1);
+        const uint64_t env = env_base + (uint64_t)b;
+        const uint4 r = philox4x32(k0, k1, (uint32_t)env, (uint32_t)step, (uint32_t)(step >> 32), 0x00B01C70u ^ (uint32_t)(env >> 32));
+        const float u = (float)(r.x >> 8) * (1.0f / 16777216.0f);
+        a = u < p1 ? 1 : 0;
+    }
+    action[b] = a;
+    if (logp) logp[b] = a ? lp1 : lp0;
     if (logits_out) { logits_out[2 * b] = l0; logits_out[2 * b + 1] = l1; }
 }
 
@@ -270,6 +312,27 @@ extern "C" int uavpolicy_get_action(uavpolicy_t *p, const float *d_obs, int32_t 
     heads_out_kernel<<<(B + 255) / 256, 256, 0, s>>>(p->hh_actor, p->hh_critic, p->actor_head, p->critic_head, B, (uint32_t)seed,
                                                      (uint32_t)(seed >> 32), step, env_id_base, d_action, d_logp, d_value,
                                                      d_entropy, d_logits);
+    P_TRY(p, cudaGetLastError());
+    return 0;
+}
+
+extern "C" int uavpolicy_act(uavpolicy_t *p, const float *d_obs, int32_t B, int32_t mode, uint64_t seed, uint64_t step,
+                             uint64_t env_id_base, int64_t *d_action, float *d_logp, float *d_logits, void *stream) {
+    // the checks that need no handle come first, so that they report their own message
+    if (!d_obs || !d_action) return pfail(p, -1, "uavpolicy_act: obs / action must be non-NULL");
+    if (B <= 0) return pfail(p, -1, "uavpolicy_act: B=%d must be > 0", B);
+    if (mode != UAVPOLICY_ACT_SAMPLE && mode != UAVPOLICY_ACT_GREEDY)
+        return pfail(p, -1, "uavpolicy_act: mode %d is neither 0 (sample) nor 1 (greedy)", mode);
+    if (!p) return pfail(nullptr, -1, "uavpolicy_act: handle is NULL");
+    if (B > p->max_batch) return pfail(p, -1, "uavpolicy_act: B=%d outside (0, %d]", B, p->max_batch);
+    if (!p->have_weights) return pfail(p, -1, "uavpolicy_act before uavpolicy_set_weights");
+    P_TRY(p, cudaSetDevice(p->device));
+    const cudaStream_t s = (cudaStream_t)stream;
+    if (uavp::launch_fused_blocks(d_obs, B, p->actor, p->actor_head, p->hh_actor, p->critic, p->critic_head, p->hh_critic,
+                                  p->work_counter, p->fused_scratch, s, /*actor_only=*/true))
+        return pfail(p, -2, "fused block launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    actor_out_kernel<<<(B + 255) / 256, 256, 0, s>>>(p->hh_actor, p->actor_head, B, mode == UAVPOLICY_ACT_GREEDY, (uint32_t)seed,
+                                                     (uint32_t)(seed >> 32), step, env_id_base, d_action, d_logp, d_logits);
     P_TRY(p, cudaGetLastError());
     return 0;
 }

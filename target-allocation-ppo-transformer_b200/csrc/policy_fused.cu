@@ -527,6 +527,13 @@ fused_heads_kernel(const float *__restrict__ obs, int B, BlockW w_actor, HeadW h
     fused_body<1>(obs, B, w_actor, head_actor, hh_actor, w_critic, head_critic, hh_critic, work_counter, scratch);
 }
 
+// actor-only forward: both work counters start at the first actor item (items are numbered critic first), so the kernels
+// above run the actor's items only and never write hh_critic
+__global__ void start_counters_kernel(int *__restrict__ work_counters, int first0, int first1) {
+    work_counters[0] = first0;
+    work_counters[1] = first1;
+}
+
 // self-test: D[128,N] (fp32) = A[128,K] W[N,K]^T with one CTA: canonical smem operands, K/16 tcgen05.mma steps
 // (N = 384 as a 256 + 128 pair), accumulator read back from TMEM.  Validates descriptors and the TMEM lane mapping.
 __global__ void __launch_bounds__(128) gemm_tile_selftest_kernel(const __nv_bfloat16 *A, const __nv_bfloat16 *W, float *D,
@@ -580,15 +587,20 @@ int fused_block_prepare() {
 size_t fused_scratch_bytes(int max_batch) { return (size_t)4 * ((max_batch + kGroupRows - 1) / kGroupRows) * kTileBytes; }
 int launch_fused_blocks(const float *d_obs, int B, const BlockW &actor, const HeadW &actor_head, __nv_bfloat16 *hh_actor,
                         const BlockW &critic, const HeadW &critic_head, __nv_bfloat16 *hh_critic, int *d_work_counters,
-                        unsigned char *d_scratch, cudaStream_t stream) {
+                        unsigned char *d_scratch, cudaStream_t stream, bool actor_only) {
     static int num_sms = 0;                       // one persistent CTA per SM of the device
     if (num_sms == 0) {
         int dev = 0;
         if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return -2;
     }
     if (actor.layers != 1 || critic.layers != 2) return -1;   // the kernels' item structure (and their staged parameter layout)
-    const int items0 = 2 * ((B + kTileSamples - 1) / kTileSamples), items1 = 2 * ((B + kGroupRows - 1) / kGroupRows);
-    if (cudaMemsetAsync(d_work_counters, 0, 2 * sizeof(int), stream) != cudaSuccess) return -2;
+    const int num_tiles = (B + kTileSamples - 1) / kTileSamples, num_groups = (B + kGroupRows - 1) / kGroupRows;
+    // items still to hand out per launch: both networks', or the actor's (the second half) alone
+    const int items0 = actor_only ? num_tiles : 2 * num_tiles, items1 = actor_only ? num_groups : 2 * num_groups;
+    if (actor_only) {
+        start_counters_kernel<<<1, 1, 0, stream>>>(d_work_counters, num_tiles, num_groups);
+        if (cudaGetLastError() != cudaSuccess) return -2;
+    } else if (cudaMemsetAsync(d_work_counters, 0, 2 * sizeof(int), stream) != cudaSuccess) return -2;
     fused_tiles_kernel<<<items0 < num_sms ? items0 : num_sms, kFusedThreads, kFusedSmem, stream>>>(
         d_obs, B, actor, actor_head, hh_actor, critic, critic_head, hh_critic, d_work_counters, d_scratch);
     {   // launched as a programmatic dependent of the first kernel (griddepcontrol.wait in its prologue)

@@ -41,9 +41,10 @@ struct HeadW { const __nv_bfloat16 *w1p; const float *b1, *w2, *b2; const __nv_b
 // batch of windows in TWO launches (per-tile work, then the newest-token rows of every 128 samples on full tiles), every GEMM
 // on tcgen05 with operands resident in shared memory.  Writes relu(W1 z_last + b1) as bf16 [B,64] per network.
 // d_work_counters: two ints; d_scratch: fused_scratch_bytes(max_batch) bytes (zero-initialised once).
+// actor_only: run the actor's work items alone (hh_critic is neither read nor written).
 int launch_fused_blocks(const float *d_obs, int B, const BlockW &actor, const HeadW &actor_head, __nv_bfloat16 *hh_actor,
                         const BlockW &critic, const HeadW &critic_head, __nv_bfloat16 *hh_critic, int *d_work_counters,
-                        unsigned char *d_scratch, cudaStream_t stream);
+                        unsigned char *d_scratch, cudaStream_t stream, bool actor_only = false);
 size_t fused_scratch_bytes(int max_batch);
 int fused_block_prepare();   // one-time kernel attribute setup; 0 on success
 

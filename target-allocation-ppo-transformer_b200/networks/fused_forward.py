@@ -3,6 +3,7 @@
 
     fused = FusedPolicyForward(max_batch, device); fused.sync(policy_old)
     action, logp, value, entropy = fused.get_action(obs, step)
+    action, logp = fused.act(obs, step, greedy=True)      # actor only: evaluation
 
 bf16 operands / fp32 accumulation: outputs agree with the fp32 network to ~1e-2 absolute (tested); gradients are
 never taken through this path - PPO's update evaluates the network again (networks/fused_train.py or the PyTorch
@@ -61,6 +62,18 @@ class FusedPolicyForward:
             C.c_void_p(self.action.data_ptr()), C.c_void_p(self.logp.data_ptr()), C.c_void_p(self.value.data_ptr()),
             C.c_void_p(self.entropy.data_ptr()), C.c_void_p(self.logits.data_ptr()), self._stream()))
         return self.action[:B], self.logp[:B], self.value[:B], self.entropy[:B]
+
+    def act(self, obs, step=0, greedy=True):
+        """(action int64 [B], log_prob [B]) from the actor alone (include/uavpolicy_eval_b200.h): the critic is not run,
+        and value / entropy are left as they were.  greedy: argmax of the logits (a tie goes to 0); otherwise a sample
+        bit-identical to get_action's for the same (seed, step, env).  self.logits is filled as by get_action."""
+        B = obs.shape[0]
+        obs = obs.contiguous()
+        self._chk(self._lib.uavpolicy_act(
+            self._h, C.c_void_p(obs.data_ptr()), B, 1 if greedy else 0, self.seed, int(step), self.env_id_base,
+            C.c_void_p(self.action.data_ptr()), C.c_void_p(self.logp.data_ptr()), C.c_void_p(self.logits.data_ptr()),
+            self._stream()))
+        return self.action[:B], self.logp[:B]
 
     def close(self):
         if getattr(self, "_h", None):
