@@ -33,9 +33,9 @@ LIBS = {
     ],
     POLICY_LIB_PATH: [
         ("policy_dense.cu", [], ["policy_gemm.cuh", "tcgen05_util.cuh", "../../include/uavpolicy_b200.h"]),
-        ("policy_forward.cu", [], ["policy_kernels.cuh", "policy_weights.cuh", "../../include/uavpolicy_b200.h",
+        ("policy_forward.cu", [], ["policy_handle.cuh", "policy_kernels.cuh", "policy_weights.cuh", "../../include/uavpolicy_b200.h",
                                    "../../include/uavpolicy_eval_b200.h"]),
-        ("policy_train.cu", [], ["policy_gemm.cuh", "policy_kernels.cuh", "policy_weights.cuh", "../../include/uavpolicy_b200.h"]),
+        ("policy_train.cu", [], ["policy_gemm.cuh", "policy_handle.cuh", "policy_kernels.cuh", "policy_weights.cuh", "../../include/uavpolicy_b200.h"]),
         ("policy_wgrad.cu", [], ["tcgen05_util.cuh", "policy_weights.cuh", "../../include/uavpolicy_b200.h"]),
         ("policy_fused.cu", [], ["tcgen05_util.cuh", "policy_weights.cuh", "../../include/uavpolicy_b200.h"]),
     ],

@@ -151,6 +151,7 @@ def check(rc, handle=None):
 
 # ---- policy rollout forward (include/uavpolicy_b200.h, lib/libuavpolicy_b200.so) ---------------------------------
 _policy_lib = None
+NUM_PARAMS = 419267   # UAVPOLICY_NUM_PARAMS: length of the flat parameter vector of include/uavpolicy_b200.h
 
 
 def load_policy():

@@ -9,15 +9,10 @@
 #include "uavpolicy_b200.h"
 #include "uavpolicy_eval_b200.h"
 
-#include <cstdarg>
-#include <cstdio>
-#include <new>
-#include <string>
-#include <vector>
-
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
+#include "policy_handle.cuh"
 #include "policy_kernels.cuh"
 #include "policy_weights.cuh"
 
@@ -38,34 +33,16 @@ __device__ __forceinline__ uint4 philox4x32(uint32_t k0, uint32_t k1, uint32_t c
     return make_uint4(c0, c1, c2, c3);
 }
 
-// head outputs (transformer_net.py:78-91 second layers; the first layers 128 -> 64 + ReLU ran in the fused launches):
-// logits = W2a ha + b, value = W2c hc + b; softmax, Categorical sample (counter RNG), log-prob, entropy (:116-122).
-// One thread per sample.
+// head outputs: logits and value (head_out), then softmax, Categorical sample (counter RNG), log-prob, entropy
+// (transformer_net.py:116-122).  One thread per sample.
 __global__ void __launch_bounds__(256) heads_out_kernel(const __nv_bfloat16 *__restrict__ Ha, const __nv_bfloat16 *__restrict__ Hc,
                                                         HeadW ha, HeadW hc, int B, uint32_t k0, uint32_t k1, uint64_t step,
                                                         uint64_t env_base, int64_t *__restrict__ action,
                                                         float *__restrict__ logp, float *__restrict__ value,
                                                         float *__restrict__ entropy, float *__restrict__ logits_out) {
-    __shared__ float s_w[3][HID];
-    for (int i = threadIdx.x; i < HID; i += blockDim.x) {
-        s_w[0][i] = ha.w2[i]; s_w[1][i] = ha.w2[HID + i]; s_w[2][i] = hc.w2[i];
-    }
-    __syncthreads();
-    const int b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= B) return;
-    float l0 = ha.b2[0], l1 = ha.b2[1], vv = hc.b2[0];
-#pragma unroll
-    for (int c = 0; c < HID / DH; ++c) {
-        float xa[DH], xc[DH];
-        load16(Ha + (size_t)b * HID + c * DH, xa);
-        load16(Hc + (size_t)b * HID + c * DH, xc);
-#pragma unroll
-        for (int e = 0; e < DH; ++e) {
-            l0 = fmaf(s_w[0][c * DH + e], xa[e], l0);
-            l1 = fmaf(s_w[1][c * DH + e], xa[e], l1);
-            vv = fmaf(s_w[2][c * DH + e], xc[e], vv);
-        }
-    }
+    int b;
+    float l0, l1, vv;
+    if (!head_out<true>(Ha, Hc, ha.w2, ha.b2, hc.w2, hc.b2, B, b, l0, l1, vv)) return;
     const float m = fmaxf(l0, l1), e0 = expf(l0 - m), e1 = expf(l1 - m), lse = m + logf(e0 + e1);
     const float lp0 = l0 - lse, lp1 = l1 - lse, p0 = expf(lp0), p1 = expf(lp1);
     const uint64_t env = env_base + (uint64_t)b;
@@ -86,22 +63,9 @@ __global__ void __launch_bounds__(256) actor_out_kernel(const __nv_bfloat16 *__r
                                                         uint32_t k0, uint32_t k1, uint64_t step, uint64_t env_base,
                                                         int64_t *__restrict__ action, float *__restrict__ logp,
                                                         float *__restrict__ logits_out) {
-    __shared__ float s_w[2][HID];
-    for (int i = threadIdx.x; i < HID; i += blockDim.x) { s_w[0][i] = ha.w2[i]; s_w[1][i] = ha.w2[HID + i]; }
-    __syncthreads();
-    const int b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= B) return;
-    float l0 = ha.b2[0], l1 = ha.b2[1];
-#pragma unroll
-    for (int c = 0; c < HID / DH; ++c) {
-        float xa[DH];
-        load16(Ha + (size_t)b * HID + c * DH, xa);
-#pragma unroll
-        for (int e = 0; e < DH; ++e) {
-            l0 = fmaf(s_w[0][c * DH + e], xa[e], l0);
-            l1 = fmaf(s_w[1][c * DH + e], xa[e], l1);
-        }
-    }
+    int b;
+    float l0, l1, unused;
+    if (!head_out<false>(Ha, nullptr, ha.w2, ha.b2, nullptr, nullptr, B, b, l0, l1, unused)) return;
     const float m = fmaxf(l0, l1), e0 = expf(l0 - m), e1 = expf(l1 - m), lse = m + logf(e0 + e1);
     const float lp0 = l0 - lse, lp1 = l1 - lse;
     int a;
@@ -123,159 +87,81 @@ __global__ void __launch_bounds__(256) actor_out_kernel(const __nv_bfloat16 *__r
 
 // ------------------------------------------------------------------------------------------------ host side
 
-struct uavpolicy {
-    int device = 0, max_batch = 0;
+struct uavpolicy : uavp::Handle {
+    int max_batch = 0;
     float *w32 = nullptr;                 // private fp32 copy of the flat parameters
     __nv_bfloat16 *emb2_a = nullptr, *emb2_c = nullptr;   // [128 x 32] tensor-core form of the two embedding weights
-    __nv_bfloat16 *wpk = nullptr;         // GEMM weights pre-packed in canonical order (same element offsets as w32)
+    __nv_bfloat16 *wpk = nullptr;         // GEMM weights pre-packed in canonical order, each at pk(its offset in w32)
     __nv_bfloat16 *bpk = nullptr;         // their biases as [N x 16] B-operands (3 layers + 2 heads)
-    struct WPack { const __nv_bfloat16 *dst; size_t src; int N, K; };
-    std::vector<WPack> wpack;             // every GEMM weight: packed copy, its offset in w32, shape (set at create)
     BlockW actor, critic;
     HeadW actor_head, critic_head;
     __nv_bfloat16 *hh_actor = nullptr, *hh_critic = nullptr;   // [max_batch, 64] bf16: relu(W1 z + b1) of the two heads
     int *work_counter = nullptr;          // dynamic work-item counters of the two fused launches
     unsigned char *fused_scratch = nullptr;   // newest-token rows handed from the first fused launch to the second
-    std::vector<void *> allocs;
     bool have_weights = false;
-    std::string err;
 };
 
-static thread_local std::string g_err;
-static int pfail(uavpolicy *p, int code, const char *fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    if (p) p->err = buf; else g_err = buf;
-    return code;
-}
-#define P_TRY(p, expr)                                                                                   \
-    do {                                                                                                 \
-        cudaError_t e_ = (expr);                                                                         \
-        if (e_ != cudaSuccess) return pfail(p, -2, "%s failed: %s", #expr, cudaGetErrorString(e_));      \
-    } while (0)
-
-template <typename T>
-static cudaError_t palloc(uavpolicy *p, T **ptr, size_t n) {
-    void *q = nullptr;
-    cudaError_t e = cudaMalloc(&q, (n ? n : 1) * sizeof(T));
-    if (e == cudaSuccess) { p->allocs.push_back(q); *ptr = static_cast<T *>(q); }
-    return e;
-}
-
 constexpr size_t UPK_SIZE = (size_t)UAVPOLICY_NUM_PARAMS + 64;   // packed copies live at (offset rounded up to 8 elements)
-static inline size_t pk(size_t off) { return (off + 7) / 8 * 8; }
-
-// the [N x K] GEMM weight at element `off` of w32: its packed copy (16 B aligned for the bulk TMA copy), recorded for set_weights
-static const __nv_bfloat16 *map_weight(uavpolicy *p, size_t &off, int N, int K) {
-    const __nv_bfloat16 *dst = p->wpk + pk(off);
-    p->wpack.push_back({dst, off, N, K});
-    off += (size_t)N * K;
-    return dst;
-}
-static size_t map_block(uavpolicy *p, BlockW &b, int layers, size_t off) {
-    const float *w32 = p->w32;
-    b.layers = layers;
-    b.pos = w32 + off; off += S * D;
-    b.emb_w = w32 + off; off += D * F;
-    b.emb_b = w32 + off; off += D;
-    for (int l = 0; l < layers; ++l) {
-        LayerW &L = b.layer[l];
-        L.in_wp = map_weight(p, off, 3 * D, D);
-        L.in_b = w32 + off; off += 3 * D;
-        L.out_wp = map_weight(p, off, D, D);
-        L.out_b = w32 + off; off += D;
-        L.l1_wp = map_weight(p, off, FF, D);
-        L.l1_b = w32 + off; off += FF;
-        L.l2_wp = map_weight(p, off, D, FF);
-        L.l2_b = w32 + off; off += D;
-        L.n1_w = w32 + off; off += D;
-        L.n1_b = w32 + off; off += D;
-        L.n2_w = w32 + off; off += D;
-        L.n2_b = w32 + off; off += D;
-    }
-    return off;
-}
-static size_t map_head(uavpolicy *p, HeadW &h, int outs, size_t off) {
-    h.w1p = map_weight(p, off, HID, D);
-    h.b1 = p->w32 + off; off += HID;
-    h.w2 = p->w32 + off; off += outs * HID;
-    h.b2 = p->w32 + off; off += outs;
-    return off;
-}
+static inline size_t pk(size_t off) { return (off + 7) / 8 * 8; }   // 16 B aligned for the bulk TMA copy
 
 extern "C" int uavpolicy_abi_version(void) { return UAVPOLICY_ABI_VERSION; }
 
-extern "C" const char *uavpolicy_last_error(const uavpolicy_t *p) { return p ? p->err.c_str() : g_err.c_str(); }
+extern "C" const char *uavpolicy_last_error(const uavpolicy_t *p) { return uavp::last_error(p); }
 
 extern "C" int uavpolicy_create(int32_t device, int32_t max_batch, uavpolicy_t **out) {
-    if (!out) return pfail(nullptr, -1, "uavpolicy_create: out is NULL");
-    *out = nullptr;
-    if (max_batch <= 0) return pfail(nullptr, -1, "uavpolicy_create: max_batch must be > 0");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        return pfail(nullptr, -2, "uavpolicy_create: no CUDA device; there is no CPU fallback");
-    if (device < 0 || device >= ndev) return pfail(nullptr, -1, "uavpolicy_create: device %d out of range", device);
-    uavpolicy *p = new (std::nothrow) uavpolicy();
-    if (!p) return pfail(nullptr, -3, "out of host memory");
-    p->device = device; p->max_batch = max_batch;
-    auto bail = [&](int rc) { g_err = p->err; for (void *q : p->allocs) cudaFree(q); delete p; return rc; };
+    uavpolicy *p;
+    if (const int rc = uavp::new_handle("uavpolicy_create", "max_batch", device, max_batch, out, p)) return rc;
+    p->max_batch = max_batch;
     cudaError_t e = cudaSetDevice(device);
-    if (e == cudaSuccess) e = palloc(p, &p->w32, (size_t)UAVPOLICY_NUM_PARAMS);
-    if (e == cudaSuccess) e = palloc(p, &p->hh_actor, (size_t)max_batch * HID);
-    if (e == cudaSuccess) e = palloc(p, &p->hh_critic, (size_t)max_batch * HID);
-    if (e == cudaSuccess) e = palloc(p, &p->work_counter, 2);
-    if (e == cudaSuccess) e = palloc(p, &p->fused_scratch, uavp::fused_scratch_bytes(max_batch));
+    if (e == cudaSuccess) e = alloc(p, &p->w32, (size_t)UAVPOLICY_NUM_PARAMS);
+    if (e == cudaSuccess) e = alloc(p, &p->hh_actor, (size_t)max_batch * HID);
+    if (e == cudaSuccess) e = alloc(p, &p->hh_critic, (size_t)max_batch * HID);
+    if (e == cudaSuccess) e = alloc(p, &p->work_counter, 2);
+    if (e == cudaSuccess) e = alloc(p, &p->fused_scratch, uavp::fused_scratch_bytes(max_batch));
     if (e == cudaSuccess) e = cudaMemset(p->fused_scratch, 0, uavp::fused_scratch_bytes(max_batch));
-    if (e == cudaSuccess) e = palloc(p, &p->wpk, (size_t)UPK_SIZE);
-    if (e == cudaSuccess) e = palloc(p, &p->bpk, (size_t)3 * uavp::kLayerBiasElems + 2 * HID * uavp::kBiasK);
-    if (e == cudaSuccess) e = palloc(p, &p->emb2_a, (size_t)D * 32);
-    if (e == cudaSuccess) e = palloc(p, &p->emb2_c, (size_t)D * 32);
-    if (e != cudaSuccess) { pfail(p, -2, "uavpolicy_create: %s", cudaGetErrorString(e)); return bail(-2); }
-    if (uavp::fused_block_prepare() != 0) { pfail(p, -2, "uavpolicy_create: cannot reserve shared memory for the fused kernel"); return bail(-2); }
-    size_t off = map_block(p, p->actor, 1, 0);
-    off = map_head(p, p->actor_head, NACT, off);
-    off = map_block(p, p->critic, 2, off);
-    off = map_head(p, p->critic_head, 1, off);
+    if (e == cudaSuccess) e = alloc(p, &p->wpk, (size_t)UPK_SIZE);
+    if (e == cudaSuccess) e = alloc(p, &p->bpk, (size_t)3 * uavp::kLayerBiasElems + 2 * HID * uavp::kBiasK);
+    if (e == cudaSuccess) e = alloc(p, &p->emb2_a, (size_t)D * 32);
+    if (e == cudaSuccess) e = alloc(p, &p->emb2_c, (size_t)D * 32);
+    if (e != cudaSuccess) return uavp::abandon_handle(p, fail(p, -2, "uavpolicy_create: %s", cudaGetErrorString(e)));
+    if (uavp::fused_block_prepare() != 0)
+        return uavp::abandon_handle(p, fail(p, -2, "uavpolicy_create: cannot reserve shared memory for the fused kernel"));
+    bind_fp32(p->actor, p->actor_head, kActorOff, p->w32);
+    bind_fp32(p->critic, p->critic_head, kCriticOff, p->w32);
     p->actor.emb_w2p = p->emb2_a; p->critic.emb_w2p = p->emb2_c;
-    {   // bias operands: layers of the actor, then of the critic, then the two heads
+    {   // packed GEMM weights, and the bias operands: layers of the actor, then of the critic, then the two heads
         __nv_bfloat16 *q = p->bpk;
+        auto packed = [&](size_t off) { return p->wpk + pk(off); };
+        const NetOff *offs[2] = {&kActorOff, &kCriticOff};
         BlockW *blocks[2] = {&p->actor, &p->critic};
-        for (BlockW *b : blocks)
-            for (int l = 0; l < b->layers; ++l) {
-                LayerW &L = b->layer[l];
+        for (int n = 0; n < 2; ++n)
+            for (int l = 0; l < blocks[n]->layers; ++l) {
+                LayerW &L = blocks[n]->layer[l];
+                const LayerOff &o = offs[n]->layer[l];
+                L.in_wp = packed(o.in_w); L.out_wp = packed(o.out_w); L.l1_wp = packed(o.l1_w); L.l2_wp = packed(o.l2_w);
                 L.in_bp = q; q += 3 * D * uavp::kBiasK;
                 L.out_bp = q; q += D * uavp::kBiasK;
                 L.l1_bp = q; q += FF * uavp::kBiasK;
                 L.l2_bp = q; q += D * uavp::kBiasK;
             }
+        p->actor_head.w1p = packed(kActorOff.head.w1); p->critic_head.w1p = packed(kCriticOff.head.w1);
         p->actor_head.b1p = q; q += HID * uavp::kBiasK;
         p->critic_head.b1p = q;
     }
-    if (off != (size_t)UAVPOLICY_NUM_PARAMS) { pfail(p, -1, "internal: parameter layout mismatch"); return bail(-1); }
     *out = p;
     return 0;
 }
 
-extern "C" int uavpolicy_destroy(uavpolicy_t *p) {
-    if (!p) return 0;
-    cudaSetDevice(p->device);
-    cudaDeviceSynchronize();
-    for (void *q : p->allocs) cudaFree(q);
-    delete p;
-    return 0;
-}
+extern "C" int uavpolicy_destroy(uavpolicy_t *p) { return uavp::destroy_handle(p); }
 
 extern "C" int uavpolicy_set_weights(uavpolicy_t *p, const float *d_flat_params, void *stream) {
     if (!p || !d_flat_params) return -1;
     cudaStream_t s = (cudaStream_t)stream;
-    P_TRY(p, cudaSetDevice(p->device));
-    P_TRY(p, cudaMemcpyAsync(p->w32, d_flat_params, (size_t)UAVPOLICY_NUM_PARAMS * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    UAVP_TRY(p, cudaSetDevice(p->device));
+    UAVP_TRY(p, cudaMemcpyAsync(p->w32, d_flat_params, (size_t)UAVPOLICY_NUM_PARAMS * sizeof(float), cudaMemcpyDeviceToDevice, s));
     // canonical-order copies of every GEMM weight for the fused kernel's bulk-TMA staging
-    for (const uavpolicy::WPack &w : p->wpack)
-        pack_canon_kernel<<<(w.N * w.K + 255) / 256, 256, 0, s>>>(p->w32 + w.src, const_cast<__nv_bfloat16 *>(w.dst), w.N, w.K);
+    for (const GemmW &w : kGemmW.w)
+        pack_canon_kernel<<<(w.N * w.K + 255) / 256, 256, 0, s>>>(p->w32 + w.off, p->wpk + pk(w.off), w.N, w.K);
     {
         auto packb = [&](const __nv_bfloat16 *dst, const float *bias, int N) {
             pack_bias_kernel<<<(N * 16 + 255) / 256, 256, 0, s>>>(bias, const_cast<__nv_bfloat16 *>(dst), N);
@@ -291,7 +177,7 @@ extern "C" int uavpolicy_set_weights(uavpolicy_t *p, const float *d_flat_params,
     }
     emb_w2_kernel<<<(D * 32 + 255) / 256, 256, 0, s>>>(p->actor.emb_w, p->actor.emb_b, p->emb2_a);
     emb_w2_kernel<<<(D * 32 + 255) / 256, 256, 0, s>>>(p->critic.emb_w, p->critic.emb_b, p->emb2_c);
-    P_TRY(p, cudaGetLastError());
+    UAVP_TRY(p, cudaGetLastError());
     p->have_weights = true;
     return 0;
 }
@@ -300,39 +186,39 @@ extern "C" int uavpolicy_get_action(uavpolicy_t *p, const float *d_obs, int32_t 
                                     uint64_t env_id_base, int64_t *d_action, float *d_logp, float *d_value,
                                     float *d_entropy, float *d_logits, void *stream) {
     if (!p) return -1;
-    if (!d_obs || !d_action) return pfail(p, -1, "uavpolicy_get_action: obs / action must be non-NULL");
-    if (B <= 0 || B > p->max_batch) return pfail(p, -1, "uavpolicy_get_action: B=%d outside (0, %d]", B, p->max_batch);
-    if (!p->have_weights) return pfail(p, -4, "uavpolicy_get_action before uavpolicy_set_weights");
-    P_TRY(p, cudaSetDevice(p->device));
+    if (!d_obs || !d_action) return fail(p, -1, "uavpolicy_get_action: obs / action must be non-NULL");
+    if (B <= 0 || B > p->max_batch) return fail(p, -1, "uavpolicy_get_action: B=%d outside (0, %d]", B, p->max_batch);
+    if (!p->have_weights) return fail(p, -4, "uavpolicy_get_action before uavpolicy_set_weights");
+    UAVP_TRY(p, cudaSetDevice(p->device));
     const cudaStream_t s = (cudaStream_t)stream;
     // two fused launches (actor block + head layer 1, critic block + head layer 1), then the per-sample outputs
     if (uavp::launch_fused_blocks(d_obs, B, p->actor, p->actor_head, p->hh_actor, p->critic, p->critic_head, p->hh_critic,
                                   p->work_counter, p->fused_scratch, s))
-        return pfail(p, -2, "fused block launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        return fail(p, -2, "fused block launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     heads_out_kernel<<<(B + 255) / 256, 256, 0, s>>>(p->hh_actor, p->hh_critic, p->actor_head, p->critic_head, B, (uint32_t)seed,
                                                      (uint32_t)(seed >> 32), step, env_id_base, d_action, d_logp, d_value,
                                                      d_entropy, d_logits);
-    P_TRY(p, cudaGetLastError());
+    UAVP_TRY(p, cudaGetLastError());
     return 0;
 }
 
 extern "C" int uavpolicy_act(uavpolicy_t *p, const float *d_obs, int32_t B, int32_t mode, uint64_t seed, uint64_t step,
                              uint64_t env_id_base, int64_t *d_action, float *d_logp, float *d_logits, void *stream) {
     // the checks that need no handle come first, so that they report their own message
-    if (!d_obs || !d_action) return pfail(p, -1, "uavpolicy_act: obs / action must be non-NULL");
-    if (B <= 0) return pfail(p, -1, "uavpolicy_act: B=%d must be > 0", B);
+    if (!d_obs || !d_action) return fail(p, -1, "uavpolicy_act: obs / action must be non-NULL");
+    if (B <= 0) return fail(p, -1, "uavpolicy_act: B=%d must be > 0", B);
     if (mode != UAVPOLICY_ACT_SAMPLE && mode != UAVPOLICY_ACT_GREEDY)
-        return pfail(p, -1, "uavpolicy_act: mode %d is neither 0 (sample) nor 1 (greedy)", mode);
-    if (!p) return pfail(nullptr, -1, "uavpolicy_act: handle is NULL");
-    if (B > p->max_batch) return pfail(p, -1, "uavpolicy_act: B=%d outside (0, %d]", B, p->max_batch);
-    if (!p->have_weights) return pfail(p, -1, "uavpolicy_act before uavpolicy_set_weights");
-    P_TRY(p, cudaSetDevice(p->device));
+        return fail(p, -1, "uavpolicy_act: mode %d is neither 0 (sample) nor 1 (greedy)", mode);
+    if (!p) return fail(p, -1, "uavpolicy_act: handle is NULL");
+    if (B > p->max_batch) return fail(p, -1, "uavpolicy_act: B=%d outside (0, %d]", B, p->max_batch);
+    if (!p->have_weights) return fail(p, -1, "uavpolicy_act before uavpolicy_set_weights");
+    UAVP_TRY(p, cudaSetDevice(p->device));
     const cudaStream_t s = (cudaStream_t)stream;
     if (uavp::launch_fused_blocks(d_obs, B, p->actor, p->actor_head, p->hh_actor, p->critic, p->critic_head, p->hh_critic,
                                   p->work_counter, p->fused_scratch, s, /*actor_only=*/true))
-        return pfail(p, -2, "fused block launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+        return fail(p, -2, "fused block launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     actor_out_kernel<<<(B + 255) / 256, 256, 0, s>>>(p->hh_actor, p->actor_head, B, mode == UAVPOLICY_ACT_GREEDY, (uint32_t)seed,
                                                      (uint32_t)(seed >> 32), step, env_id_base, d_action, d_logp, d_logits);
-    P_TRY(p, cudaGetLastError());
+    UAVP_TRY(p, cudaGetLastError());
     return 0;
 }

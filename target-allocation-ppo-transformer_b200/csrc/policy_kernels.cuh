@@ -173,6 +173,38 @@ __device__ __forceinline__ void store16(__nv_bfloat16 *p, const float *v) {
     reinterpret_cast<uint4 *>(p)[1] = make_uint4(w[4], w[5], w[6], w[7]);
 }
 
+// second head layers (transformer_net.py:78-91; the first layers 128 -> 64 + ReLU ran before) of sample b = the thread's
+// index in the grid: logits (l0, l1) = W2a ha + b2a from the bf16 hidden row Ha[b], and with kValue also the value
+// v = W2c hc + b2c from Hc[b].  The CTA stages W2 in shared memory first, so every thread calls this; it returns false
+// for the threads past B.
+template <bool kValue>
+__device__ __forceinline__ bool head_out(const __nv_bfloat16 *Ha, const __nv_bfloat16 *Hc, const float *w2a, const float *b2a,
+                                         const float *w2c, const float *b2c, int B, int &b, float &l0, float &l1, float &v) {
+    __shared__ float s_w[kValue ? 3 : 2][HID];
+    for (int i = threadIdx.x; i < HID; i += blockDim.x) {
+        s_w[0][i] = w2a[i]; s_w[1][i] = w2a[HID + i];
+        if constexpr (kValue) s_w[2][i] = w2c[i];
+    }
+    __syncthreads();
+    b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return false;
+    l0 = b2a[0]; l1 = b2a[1];
+    if constexpr (kValue) v = b2c[0];
+#pragma unroll
+    for (int c = 0; c < HID / DH; ++c) {
+        float xa[DH], xc[DH];
+        load16(Ha + (size_t)b * HID + c * DH, xa);
+        if constexpr (kValue) load16(Hc + (size_t)b * HID + c * DH, xc);
+#pragma unroll
+        for (int e = 0; e < DH; ++e) {
+            l0 = fmaf(s_w[0][c * DH + e], xa[e], l0);
+            l1 = fmaf(s_w[1][c * DH + e], xa[e], l1);
+            if constexpr (kValue) v = fmaf(s_w[2][c * DH + e], xc[e], v);
+        }
+    }
+    return true;
+}
+
 // softmax(q k^T / sqrt(16), key padding mask) v for one (sample, head, query): q, and 5 keys / values of 16 dims
 __device__ __forceinline__ void attend(const float *q, const __nv_bfloat16 *k0, const __nv_bfloat16 *v0, size_t stride,
                                        const uint8_t *pad, float *out) {

@@ -15,16 +15,11 @@
 // gradients in); uavtrain_ppo_loss turns the heads' outputs into the PPO loss statistics and those gradients.
 #include "uavpolicy_b200.h"
 
-#include <cstdarg>
-#include <cstdio>
-#include <new>
-#include <string>
-#include <vector>
-
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
 #include "policy_gemm.cuh"
+#include "policy_handle.cuh"
 #include "policy_kernels.cuh"
 #include "policy_weights.cuh"
 
@@ -37,16 +32,6 @@ int wgrad(const __nv_bfloat16 *dY, int64_t ld_dy, const __nv_bfloat16 *X, int64_
 namespace {
 using bf16 = __nv_bfloat16;
 
-__device__ __forceinline__ void unpack4(uint2 v, float *o) {
-    const __nv_bfloat162 a = *reinterpret_cast<const __nv_bfloat162 *>(&v.x), b = *reinterpret_cast<const __nv_bfloat162 *>(&v.y);
-    o[0] = __low2float(a); o[1] = __high2float(a); o[2] = __low2float(b); o[3] = __high2float(b);
-}
-__device__ __forceinline__ uint2 pack4(const float *v) {
-    const __nv_bfloat162 a = __floats2bfloat162_rn(v[0], v[1]), b = __floats2bfloat162_rn(v[2], v[3]);
-    uint2 o;
-    o.x = *reinterpret_cast<const uint32_t *>(&a); o.y = *reinterpret_cast<const uint32_t *>(&b);
-    return o;
-}
 __device__ __forceinline__ float warp_sum(float v) {
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
@@ -55,11 +40,11 @@ __device__ __forceinline__ float warp_sum(float v) {
 // ---------------------------------------------------------------------------------------------- forward extras
 
 __device__ __forceinline__ void unpack8(uint4 v, float *o) {
-    unpack4(make_uint2(v.x, v.y), o);
-    unpack4(make_uint2(v.z, v.w), o + 4);
+    unpack4f(make_uint2(v.x, v.y), o);
+    unpack4f(make_uint2(v.z, v.w), o + 4);
 }
 __device__ __forceinline__ uint4 pack8(const float *v) {
-    const uint2 a = pack4(v), b = pack4(v + 4);
+    const uint2 a = pack4f(v), b = pack4f(v + 4);
     return make_uint4(a.x, a.y, b.x, b.y);
 }
 __device__ __forceinline__ float half_warp_sum(float v) {           // over the 16 lanes that share a row
@@ -159,15 +144,15 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const void *__restrict__ dy
             const float4 t = *reinterpret_cast<const float4 *>(static_cast<const float *>(dy_) + (size_t)r * dy_stride + lane * 4);
             dy[0] = t.x; dy[1] = t.y; dy[2] = t.z; dy[3] = t.w;
         } else {
-            unpack4(*reinterpret_cast<const uint2 *>(static_cast<const bf16 *>(dy_) + (size_t)r * D + lane * 4), dy);
+            unpack4f(*reinterpret_cast<const uint2 *>(static_cast<const bf16 *>(dy_) + (size_t)r * D + lane * 4), dy);
         }
         if (add) {
             float t[4];
-            unpack4(*reinterpret_cast<const uint2 *>(add + (size_t)r * D + lane * 4), t);
+            unpack4f(*reinterpret_cast<const uint2 *>(add + (size_t)r * D + lane * 4), t);
 #pragma unroll
             for (int i = 0; i < 4; ++i) dy[i] += t[i];
         }
-        unpack4(*reinterpret_cast<const uint2 *>(xhat + (size_t)r * D + lane * 4), xh);
+        unpack4f(*reinterpret_cast<const uint2 *>(xhat + (size_t)r * D + lane * 4), xh);
         const float rs = rstd[r];
         float s1 = 0.0f, s2 = 0.0f, gd[4];
 #pragma unroll
@@ -180,7 +165,7 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(const void *__restrict__ dy
             z[i] = rs * (gd[i] - s1 - xh[i] * s2);
             ag[i] = fmaf(dy[i], xh[i], ag[i]); ab[i] += dy[i]; az[i] += z[i];
         }
-        *reinterpret_cast<uint2 *>(dz + (size_t)r * D + lane * 4) = pack4(z);
+        *reinterpret_cast<uint2 *>(dz + (size_t)r * D + lane * 4) = pack4f(z);
     }
     auto col = [](int l, int i) { return l * 4 + i; };
     block_colsum_flush<4, D>(ag, s_red, g_gamma, col);
@@ -321,12 +306,12 @@ __global__ void scatter_add_last_kernel(bf16 *__restrict__ dX, const bf16 *__res
     const int b = i / (D / 4), c = (i % (D / 4)) * 4;
     float x[4], y[4], z[4];
     bf16 *dst = dX + ((size_t)b * S + S - 1) * D + c;
-    unpack4(*reinterpret_cast<const uint2 *>(dst), x);
-    unpack4(*reinterpret_cast<const uint2 *>(t + (size_t)b * D + c), y);
-    unpack4(*reinterpret_cast<const uint2 *>(u + (size_t)b * D + c), z);
+    unpack4f(*reinterpret_cast<const uint2 *>(dst), x);
+    unpack4f(*reinterpret_cast<const uint2 *>(t + (size_t)b * D + c), y);
+    unpack4f(*reinterpret_cast<const uint2 *>(u + (size_t)b * D + c), z);
 #pragma unroll
     for (int k = 0; k < 4; ++k) x[k] += y[k] + z[k];
-    *reinterpret_cast<uint2 *>(dst) = pack4(x);
+    *reinterpret_cast<uint2 *>(dst) = pack4f(x);
 }
 
 // embedding backward: E = relu(obs W^T + b) + pos.  The forward left the ReLU activity bits (policy_kernels.cuh:
@@ -352,10 +337,10 @@ __global__ void __launch_bounds__(256) embed_mask_kernel(const bf16 *__restrict_
         for (int s = 0; s < S; ++s) {
             const size_t row = (size_t)b * S + s, off = row * D + lane * 4;
             float g[4];
-            unpack4(*reinterpret_cast<const uint2 *>(g1 + off), g);
+            unpack4f(*reinterpret_cast<const uint2 *>(g1 + off), g);
             if (g2) {
                 float t[4];
-                unpack4(*reinterpret_cast<const uint2 *>(g2 + off), t);
+                unpack4f(*reinterpret_cast<const uint2 *>(g2 + off), t);
 #pragma unroll
                 for (int f = 0; f < 4; ++f) g[f] += t[f];
             }
@@ -366,7 +351,7 @@ __global__ void __launch_bounds__(256) embed_mask_kernel(const bf16 *__restrict_
                 dpos[s][f] += g[f];
                 g[f] = ((mw[f] >> lane) & 1u) ? g[f] : 0.0f;
             }
-            *reinterpret_cast<uint2 *>(dpre + off) = pack4(g);
+            *reinterpret_cast<uint2 *>(dpre + off) = pack4f(g);
         }
     }
 #pragma unroll
@@ -382,24 +367,9 @@ __global__ void __launch_bounds__(256) head_out_kernel(const bf16 *__restrict__ 
                                                        const float *__restrict__ b2a, const float *__restrict__ w2c,
                                                        const float *__restrict__ b2c, int n, float *__restrict__ logits,
                                                        float *__restrict__ value) {
-    __shared__ float s_w[3][HID];
-    for (int i = threadIdx.x; i < HID; i += blockDim.x) { s_w[0][i] = w2a[i]; s_w[1][i] = w2a[HID + i]; s_w[2][i] = w2c[i]; }
-    __syncthreads();
-    const int b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= n) return;
-    float l0 = b2a[0], l1 = b2a[1], vv = b2c[0];
-#pragma unroll
-    for (int c = 0; c < HID / DH; ++c) {
-        float xa[DH], xc[DH];
-        load16(Ha + (size_t)b * HID + c * DH, xa);
-        load16(Hc + (size_t)b * HID + c * DH, xc);
-#pragma unroll
-        for (int e = 0; e < DH; ++e) {
-            l0 = fmaf(s_w[0][c * DH + e], xa[e], l0);
-            l1 = fmaf(s_w[1][c * DH + e], xa[e], l1);
-            vv = fmaf(s_w[2][c * DH + e], xc[e], vv);
-        }
-    }
+    int b;
+    float l0, l1, vv;
+    if (!head_out<true>(Ha, Hc, w2a, b2a, w2c, b2c, n, b, l0, l1, vv)) return;
     logits[2 * b] = l0; logits[2 * b + 1] = l1;
     value[b] = vv;
 }
@@ -532,26 +502,23 @@ __global__ void __launch_bounds__(256) ppo_loss_grad_kernel(const PpoLossArgs a,
 
 namespace {
 struct LayerT { const bf16 *in_t, *in_q_t, *in_kv_t, *out_t, *l1_t, *l2_t; };          // transposed bf16 GEMM weights
-struct LayerOff { size_t in_w, in_b, out_w, out_b, l1_w, l1_b, l2_w, l2_b, n1_w, n1_b, n2_w, n2_b; };
-struct BlockOff { size_t pos, emb_w, emb_b; LayerOff layer[2]; };
+// bf16 forms of one GEMM weight: row-major copy, transpose, and for an in_w the transposes of its Q rows and K / V rows
+struct Gemm16 { bf16 *w, *t, *q_t, *kv_t; };
+static_assert(kNumGemmW + 2 * 3 <= kMaxPrepJobs, "a conversion job per GEMM weight and two more per in_w (3 layers)");
 struct FullAct { bf16 *QKV, *ATT, *XH1, *Y1, *Hf, *XH2, *Xout; float *rstd1, *rstd2; };   // inner layer, R rows
 struct LastAct { bf16 *KV, *Q, *AL, *XH1, *Y1, *Hs, *XH2; float *rstd1, *rstd2; };        // last layer
-struct HeadOff { size_t w1, b1, w2, b2; };
 struct HeadT { bf16 *w1, *w1_t; bf16 *Z, *Hh, *dHh; };                                     // bf16 weights, feature / hidden / gradient rows
 }  // namespace
 
-struct uavtrain {
-    int device = 0, max_samples = 0, sms = 0, n = 0;
+struct uavtrain : uavp::Handle {
+    int max_samples = 0, sms = 0, n = 0;
     bf16 *arena = nullptr;                       // bf16 GEMM weights: row-major copies and transposes
+    Gemm16 g16[uavp::kNumGemmW];                 // their slices of the arena, in kGemmW order
     uavp::BlockW actor, critic;                  // fp32 members point into the caller's flat parameter buffer (set per forward)
+    uavp::HeadW actor_head, critic_head;         // likewise
     LayerT actor_t[1], critic_t[2];
-    BlockOff actor_off, critic_off;
-    HeadOff ahead_off, chead_off;
     HeadT ahead, chead;
     bool with_heads = false;                     // the last forward also ran the heads
-    PrepJobs jobs;
-    int n_jobs = 0;
-    size_t job_src_off[kMaxPrepJobs];
     bf16 *Ea, *Ec;
     LastAct la, lc;
     FullAct fc;
@@ -561,99 +528,29 @@ struct uavtrain {
     bf16 *obs16 = nullptr;                       // [R,64] bf16 observations (zero-padded): B operand of the embedding weight gradient
     uint32_t *relu_mask = nullptr;               // [R][2 nets][4 words] ReLU activity bits of the two embeddings
     uint8_t *pad = nullptr;
-    const float *params = nullptr;               // likewise (second head layers)
-    std::vector<void *> allocs;
-    std::string err;
 };
 
 namespace {
-thread_local std::string g_terr;
-int tfail(uavtrain *p, int code, const char *fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    if (p) p->err = buf; else g_terr = buf;
-    return code;
-}
-#define T_TRY(p, expr)                                                                                   \
-    do {                                                                                                 \
-        cudaError_t e_ = (expr);                                                                         \
-        if (e_ != cudaSuccess) return tfail(p, -2, "%s failed: %s", #expr, cudaGetErrorString(e_));      \
-    } while (0)
-
-template <typename T>
-cudaError_t talloc(uavtrain *p, T **ptr, size_t n) {
-    void *q = nullptr;
-    cudaError_t e = cudaMalloc(&q, (n ? n : 1) * sizeof(T));
-    if (e == cudaSuccess) { p->allocs.push_back(q); *ptr = static_cast<T *>(q); }
-    return e;
-}
-
-// lays out the bf16 weight arena of one block and records the conversion jobs; returns the new flat offset
-size_t map_train_block(uavtrain *p, uavp::BlockW &b, LayerT *lt, BlockOff &bo, int layers, size_t off, size_t &arena_off) {
-    b.layers = layers;
-    bo.pos = off; off += S * D;
-    bo.emb_w = off; off += D * F;
-    bo.emb_b = off; off += D;
-    auto take = [&](size_t elems) { bf16 *q = p->arena + arena_off; arena_off += (elems + 63) / 64 * 64; return q; };
-    auto job = [&](size_t src_off, bf16 *dst, bf16 *dst_t, int N, int K) {
-        p->job_src_off[p->n_jobs] = src_off;
-        p->jobs.job[p->n_jobs++] = PrepJob{nullptr, dst, dst_t, N, K};
-    };
-    for (int l = 0; l < layers; ++l) {
-        uavp::LayerW &L = b.layer[l];
-        LayerOff &o = bo.layer[l];
-        bf16 *in_w = take(3 * D * D), *in_t = take(3 * D * D), *in_q_t = take(D * D), *in_kv_t = take(2 * D * D);
-        bf16 *out_w = take(D * D), *out_t = take(D * D), *l1_w = take(FF * D), *l1_t = take(FF * D), *l2_w = take(D * FF), *l2_t = take(D * FF);
-        L.in_w = in_w; L.out_w = out_w; L.l1_w = l1_w; L.l2_w = l2_w;
-        L.in_wp = L.out_wp = L.l1_wp = L.l2_wp = nullptr;
-        lt[l] = LayerT{in_t, in_q_t, in_kv_t, out_t, l1_t, l2_t};
-        o.in_w = off; job(off, in_w, in_t, 3 * D, D); job(off, nullptr, in_q_t, D, D); job(off + D * D, nullptr, in_kv_t, 2 * D, D);
-        off += 3 * D * D;
-        o.in_b = off; off += 3 * D;
-        o.out_w = off; job(off, out_w, out_t, D, D); off += D * D;
-        o.out_b = off; off += D;
-        o.l1_w = off; job(off, l1_w, l1_t, FF, D); off += FF * D;
-        o.l1_b = off; off += FF;
-        o.l2_w = off; job(off, l2_w, l2_t, D, FF); off += D * FF;
-        o.l2_b = off; off += D;
-        o.n1_w = off; off += D; o.n1_b = off; off += D; o.n2_w = off; off += D; o.n2_b = off; off += D;
-    }
-    return off;
-}
-
-void bind_params(uavp::BlockW &b, const BlockOff &bo, const float *w) {
-    b.pos = w + bo.pos; b.emb_w = w + bo.emb_w; b.emb_b = w + bo.emb_b; b.emb_w2p = nullptr;
-    for (int l = 0; l < b.layers; ++l) {
-        uavp::LayerW &L = b.layer[l];
-        const LayerOff &o = bo.layer[l];
-        L.in_b = w + o.in_b; L.out_b = w + o.out_b; L.l1_b = w + o.l1_b; L.l2_b = w + o.l2_b;
-        L.n1_w = w + o.n1_w; L.n1_b = w + o.n1_b; L.n2_w = w + o.n2_w; L.n2_b = w + o.n2_b;
-    }
-}
-
 struct TCtx { uavtrain *p; cudaStream_t s; int rc; };
 
 void gemm(TCtx &c, const bf16 *A, int64_t lda, const bf16 *W, const float *bias, bf16 *Dst, int M, int N, int K, int relu) {
     if (c.rc) return;
     const int r = uavp::gemm_bias_act(A, lda, W, bias ? bias : c.p->zeros, Dst, M, N, K, relu, c.s);
-    if (r) c.rc = tfail(c.p, -2, "tcgen05 GEMM (M=%d N=%d K=%d) failed with %d", M, N, K, r);
+    if (r) c.rc = fail(c.p, -2, "tcgen05 GEMM (M=%d N=%d K=%d) failed with %d", M, N, K, r);
 }
 // out = LayerNorm(x + A W^T + bias) fused into the dense kernel's epilogue (policy_dense.cu), keeping x^ and 1/sigma
 void gemm_ln(TCtx &c, const bf16 *A, int64_t lda, const bf16 *W, const float *bias, const bf16 *x, int64_t xs, const float *g,
              const float *b, int rows, int K, bf16 *out16, bf16 *xhat, float *rstd) {
     if (c.rc) return;
     const int r = uavp::gemm_add_ln(A, lda, W, bias, x, xs, g, b, out16, xhat, rstd, rows, K, c.s);
-    if (r) c.rc = tfail(c.p, -2, "tcgen05 GEMM + LayerNorm (M=%d K=%d) failed with %d", rows, K, r);
+    if (r) c.rc = fail(c.p, -2, "tcgen05 GEMM + LayerNorm (M=%d K=%d) failed with %d", rows, K, r);
 }
 void wgrad(TCtx &c, const bf16 *dY, int64_t ld_dy, const bf16 *X, int64_t ld_x, int rows, int Nout, int Kin, float *dW,
            int nout_valid = -1, float *dbias = nullptr, int out_ld = 0, int kin_valid = 0) {
     if (c.rc) return;
     const int r = uavp::wgrad(dY, ld_dy, X, ld_x, rows, Nout, Kin, dW, nout_valid < 0 ? Nout : nout_valid, dbias, c.p->sms, c.s, out_ld,
                               kin_valid);
-    if (r) c.rc = tfail(c.p, -2, "weight-gradient kernel (rows=%d Nout=%d Kin=%d) failed with %d", rows, Nout, Kin, r);
+    if (r) c.rc = fail(c.p, -2, "weight-gradient kernel (rows=%d Nout=%d Kin=%d) failed with %d", rows, Nout, Kin, r);
 }
 void add_ln(TCtx &c, const bf16 *x, int64_t xs, const bf16 *y, const float *g, const float *b, int rows, bf16 *out16, float *out32,
             int64_t out32_stride, bf16 *xhat, float *rstd) {
@@ -701,7 +598,7 @@ void full_layer_fwd(TCtx &c, const uavp::LayerW &L, const bf16 *X, int n, FullAc
 
 // ---- backward ----------------------------------------------------------------------------------------------
 // shared tail of both layer kinds: from the gradient of the layer output down to dS1 (gradient of x + attn-proj)
-void ffn_ln_bwd(TCtx &c, const uavp::LayerW &L, const LayerT &T, const LayerOff &o, float *g, int rows, const float *dz32,
+void ffn_ln_bwd(TCtx &c, const uavp::LayerW &L, const LayerT &T, const uavp::LayerOff &o, float *g, int rows, const float *dz32,
                 int64_t dz_stride, const bf16 *dz16, const bf16 *XH2, const float *rstd2, const bf16 *Hact, const bf16 *Y1,
                 const bf16 *XH1, const float *rstd1) {
     uavtrain *p = c.p;
@@ -709,14 +606,14 @@ void ffn_ln_bwd(TCtx &c, const uavp::LayerW &L, const LayerT &T, const LayerOff 
     wgrad(c, p->dS2, D, Hact, FF, rows, D, FF, g + o.l2_w);
     if (!c.rc) {                                              // dH = (dS2 W2) masked by the forward's ReLU, in one GEMM
         const int r = uavp::gemm_drelu(p->dS2, D, T.l2_t, Hact, FF, p->dH, rows, FF, D, c.s);
-        if (r) c.rc = tfail(p, -2, "tcgen05 GEMM with ReLU-backward epilogue (M=%d) failed with %d", rows, r);
+        if (r) c.rc = fail(p, -2, "tcgen05 GEMM with ReLU-backward epilogue (M=%d) failed with %d", rows, r);
     }
     wgrad(c, p->dH, FF, Y1, D, rows, FF, D, g + o.l1_w, -1, g + o.l1_b);                  // + bias gradient dH^T 1
     gemm(c, p->dH, FF, T.l1_t, nullptr, p->tmp, rows, D, FF, 0);
     ln_bwd(c, nullptr, 0, p->tmp, p->dS2, XH1, rstd1, L.n1_w, rows, p->dS1, g + o.n1_w, g + o.n1_b, g + o.out_b);
 }
 // dX [R,128] <- gradient w.r.t. the layer input (all five tokens)
-void last_layer_bwd(TCtx &c, const uavp::LayerW &L, const LayerT &T, const LayerOff &o, float *g, const bf16 *X, int n, LastAct &A,
+void last_layer_bwd(TCtx &c, const uavp::LayerW &L, const LayerT &T, const uavp::LayerOff &o, float *g, const bf16 *X, int n, LastAct &A,
                     const float *dfeat, int64_t dfeat_stride, const bf16 *dfeat16, bf16 *dX) {
     uavtrain *p = c.p;
     const int R = n * S;
@@ -734,7 +631,7 @@ void last_layer_bwd(TCtx &c, const uavp::LayerW &L, const LayerT &T, const Layer
     if (!c.rc) scatter_add_last_kernel<<<(n * (D / 4) + 255) / 256, 256, 0, c.s>>>(dX, p->tmp, p->dS1, n);
 }
 // returns the two addends of the gradient w.r.t. the layer input: dXg (GEMM branch) and p->dS1 (residual branch)
-void full_layer_bwd(TCtx &c, const uavp::LayerW &L, const LayerT &T, const LayerOff &o, float *g, const bf16 *X, int n, FullAct &A,
+void full_layer_bwd(TCtx &c, const uavp::LayerW &L, const LayerT &T, const uavp::LayerOff &o, float *g, const bf16 *X, int n, FullAct &A,
                     const bf16 *dY, bf16 *dXg) {
     uavtrain *p = c.p;
     const int R = n * S;
@@ -748,183 +645,184 @@ void full_layer_bwd(TCtx &c, const uavp::LayerW &L, const LayerT &T, const Layer
     wgrad(c, p->dQKV, 3 * D, X, D, R, 3 * D, D, g + o.in_w, -1, g + o.in_b);                           // + bias gradient
     gemm(c, p->dQKV, 3 * D, T.in_t, nullptr, dXg, R, D, 3 * D, 0);
 }
-void embed_bwd(TCtx &c, const BlockOff &bo, int net, float *g, int n, const bf16 *g1, const bf16 *g2) {
+void embed_bwd(TCtx &c, const uavp::NetOff &o, int net, float *g, int n, const bf16 *g1, const bf16 *g2) {
     if (c.rc) return;
     uavtrain *p = c.p;
     int grid, rpw;
     row_grid(p, n, grid, rpw);                                  // (here a "row" is a window of 5 token rows)
-    embed_mask_kernel<<<grid, 256, 0, c.s>>>(g1, g2, p->relu_mask + net * 4, n, rpw, p->tmp, g + bo.pos);
-    wgrad(c, p->tmp, D, p->obs16, 64, n * S, D, 64, g + bo.emb_w, -1, g + bo.emb_b, F, F);
+    embed_mask_kernel<<<grid, 256, 0, c.s>>>(g1, g2, p->relu_mask + net * 4, n, rpw, p->tmp, g + o.pos);
+    wgrad(c, p->tmp, D, p->obs16, 64, n * S, D, 64, g + o.emb_w, -1, g + o.emb_b, F, F);
 }
 }  // namespace
 
-extern "C" const char *uavtrain_last_error(const uavtrain_t *p) { return p ? p->err.c_str() : g_terr.c_str(); }
+extern "C" const char *uavtrain_last_error(const uavtrain_t *p) { return uavp::last_error(p); }
 
 extern "C" int uavtrain_create(int32_t device, int32_t max_samples, uavtrain_t **out) {
-    if (!out) return tfail(nullptr, -1, "uavtrain_create: out is NULL");
-    *out = nullptr;
-    if (max_samples <= 0) return tfail(nullptr, -1, "uavtrain_create: max_samples must be > 0");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-        return tfail(nullptr, -2, "uavtrain_create: no CUDA device; there is no CPU fallback");
-    if (device < 0 || device >= ndev) return tfail(nullptr, -1, "uavtrain_create: device %d out of range", device);
-    uavtrain *p = new (std::nothrow) uavtrain();
-    if (!p) return tfail(nullptr, -3, "out of host memory");
-    p->device = device; p->max_samples = max_samples;
-    auto bail = [&](int rc) { g_terr = p->err; for (void *q : p->allocs) cudaFree(q); delete p; return rc; };
+    uavtrain *p;
+    if (const int rc = uavp::new_handle("uavtrain_create", "max_samples", device, max_samples, out, p)) return rc;
+    p->max_samples = max_samples;
     cudaError_t e = cudaSetDevice(device);
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(&p->sms, cudaDevAttrMultiProcessorCount, device);
     const size_t n = (size_t)max_samples, R = n * S;
-    if (e == cudaSuccess) e = talloc(p, &p->arena, (size_t)3 * (2 * 3 * D * D + 3 * D * D + 2 * D * D + 4 * FF * D) + 4 * HID * D + 64 * 64);
+    if (e == cudaSuccess) e = alloc(p, &p->arena, (size_t)3 * (2 * 3 * D * D + 3 * D * D + 2 * D * D + 4 * FF * D) + 4 * HID * D + 64 * 64);
     bf16 **rowsR128[] = {&p->Ea, &p->Ec, &p->fc.ATT, &p->fc.XH1, &p->fc.Y1, &p->fc.XH2, &p->fc.Xout, &p->T, &p->dS1, &p->dS2, &p->dXa, &p->dXb, &p->tmp};
-    for (auto b : rowsR128) if (e == cudaSuccess) e = talloc(p, b, R * D);
+    for (auto b : rowsR128) if (e == cudaSuccess) e = alloc(p, b, R * D);
     bf16 **rowsR256[] = {&p->la.KV, &p->lc.KV, &p->fc.Hf, &p->dH};
-    for (auto b : rowsR256) if (e == cudaSuccess) e = talloc(p, b, R * FF);
+    for (auto b : rowsR256) if (e == cudaSuccess) e = alloc(p, b, R * FF);
     bf16 **rowsR384[] = {&p->fc.QKV, &p->dQKV};
-    for (auto b : rowsR384) if (e == cudaSuccess) e = talloc(p, b, R * 3 * D);
+    for (auto b : rowsR384) if (e == cudaSuccess) e = alloc(p, b, R * 3 * D);
     for (LastAct *A : {&p->la, &p->lc}) {
         bf16 **rowsN128[] = {&A->Q, &A->AL, &A->XH1, &A->Y1, &A->XH2};
-        for (auto b : rowsN128) if (e == cudaSuccess) e = talloc(p, b, n * D);
-        if (e == cudaSuccess) e = talloc(p, &A->Hs, n * FF);
-        if (e == cudaSuccess) e = talloc(p, &A->rstd1, n);
-        if (e == cudaSuccess) e = talloc(p, &A->rstd2, n);
+        for (auto b : rowsN128) if (e == cudaSuccess) e = alloc(p, b, n * D);
+        if (e == cudaSuccess) e = alloc(p, &A->Hs, n * FF);
+        if (e == cudaSuccess) e = alloc(p, &A->rstd1, n);
+        if (e == cudaSuccess) e = alloc(p, &A->rstd2, n);
     }
     for (HeadT *Hd : {&p->ahead, &p->chead}) {
-        if (e == cudaSuccess) e = talloc(p, &Hd->Z, n * D);
-        if (e == cudaSuccess) e = talloc(p, &Hd->Hh, n * HID);
-        if (e == cudaSuccess) e = talloc(p, &Hd->dHh, n * D);
+        if (e == cudaSuccess) e = alloc(p, &Hd->Z, n * D);
+        if (e == cudaSuccess) e = alloc(p, &Hd->Hh, n * HID);
+        if (e == cudaSuccess) e = alloc(p, &Hd->dHh, n * D);
         if (e == cudaSuccess) e = cudaMemset(Hd->dHh, 0, n * D * sizeof(bf16));      // columns 64.. are never written again
     }
-    if (e == cudaSuccess) e = talloc(p, &p->T2, n * D);
-    if (e == cudaSuccess) e = talloc(p, &p->dQ, n * D);
-    if (e == cudaSuccess) e = talloc(p, &p->fc.rstd1, R);
-    if (e == cudaSuccess) e = talloc(p, &p->fc.rstd2, R);
-    if (e == cudaSuccess) e = talloc(p, &p->pad, R);
-    if (e == cudaSuccess) e = talloc(p, &p->loss_acc, (size_t)4);
-    if (e == cudaSuccess) e = talloc(p, &p->obs16, R * 64);
-    if (e == cudaSuccess) e = talloc(p, &p->relu_mask, R * 8);
-    if (e == cudaSuccess) e = talloc(p, &p->zeros, (size_t)3 * D);
+    if (e == cudaSuccess) e = alloc(p, &p->T2, n * D);
+    if (e == cudaSuccess) e = alloc(p, &p->dQ, n * D);
+    if (e == cudaSuccess) e = alloc(p, &p->fc.rstd1, R);
+    if (e == cudaSuccess) e = alloc(p, &p->fc.rstd2, R);
+    if (e == cudaSuccess) e = alloc(p, &p->pad, R);
+    if (e == cudaSuccess) e = alloc(p, &p->loss_acc, (size_t)4);
+    if (e == cudaSuccess) e = alloc(p, &p->obs16, R * 64);
+    if (e == cudaSuccess) e = alloc(p, &p->relu_mask, R * 8);
+    if (e == cudaSuccess) e = alloc(p, &p->zeros, (size_t)3 * D);
     if (e == cudaSuccess) e = cudaMemset(p->zeros, 0, 3 * D * sizeof(float));
-    if (e != cudaSuccess) { tfail(p, -2, "uavtrain_create: %s", cudaGetErrorString(e)); return bail(-2); }
-    if (uavp::wgrad_prepare() != 0) { tfail(p, -2, "uavtrain_create: cannot reserve shared memory for the weight-gradient kernel"); return bail(-2); }
-    size_t arena_off = 0;
-    auto map_head = [&](HeadT &Hd, HeadOff &ho, int outs, size_t off) {
-        Hd.w1 = p->arena + arena_off; arena_off += HID * D;
-        Hd.w1_t = p->arena + arena_off; arena_off += HID * D;
-        ho.w1 = off;
-        p->job_src_off[p->n_jobs] = off;
-        p->jobs.job[p->n_jobs++] = PrepJob{nullptr, Hd.w1, Hd.w1_t, HID, D};
-        off += HID * D;
-        ho.b1 = off; off += HID;
-        ho.w2 = off; off += (size_t)outs * HID;
-        ho.b2 = off; off += outs;
-        return off;
-    };
-    size_t off = map_train_block(p, p->actor, p->actor_t, p->actor_off, 1, 0, arena_off);
-    off = map_head(p->ahead, p->ahead_off, NACT, off);
-    off = map_train_block(p, p->critic, p->critic_t, p->critic_off, 2, off, arena_off);
-    off = map_head(p->chead, p->chead_off, 1, off);
-    if (off != (size_t)UAVPOLICY_NUM_PARAMS || p->n_jobs > kMaxPrepJobs) { tfail(p, -1, "internal: parameter layout mismatch"); return bail(-1); }
+    if (e != cudaSuccess) return uavp::abandon_handle(p, fail(p, -2, "uavtrain_create: %s", cudaGetErrorString(e)));
+    if (uavp::wgrad_prepare() != 0)
+        return uavp::abandon_handle(p, fail(p, -2, "uavtrain_create: cannot reserve shared memory for the weight-gradient kernel"));
+    size_t a = 0;                                               // slices 64-element aligned: TMA tensor maps are built on them
+    auto take = [&](size_t elems) { bf16 *q = p->arena + a; a += (elems + 63) / 64 * 64; return q; };
+    for (int i = 0; i < kNumGemmW; ++i) {
+        const GemmW &g = kGemmW.w[i];
+        Gemm16 &G = p->g16[i];
+        G.w = take((size_t)g.N * g.K); G.t = take((size_t)g.N * g.K);
+        if (g.N == 3 * D) { G.q_t = take(D * D); G.kv_t = take(2 * D * D); }
+    }
+    auto forms = [&](size_t off) -> const Gemm16 & { int i = 0; while (kGemmW.w[i].off != off) ++i; return p->g16[i]; };
+    const NetOff *offs[2] = {&kActorOff, &kCriticOff};
+    BlockW *blocks[2] = {&p->actor, &p->critic};
+    LayerT *lts[2] = {p->actor_t, p->critic_t};
+    HeadT *heads[2] = {&p->ahead, &p->chead};
+    for (int k = 0; k < 2; ++k) {
+        for (int l = 0; l < offs[k]->layers; ++l) {
+            const LayerOff &o = offs[k]->layer[l];
+            const Gemm16 &in = forms(o.in_w), &out = forms(o.out_w), &l1 = forms(o.l1_w), &l2 = forms(o.l2_w);
+            LayerW &L = blocks[k]->layer[l];
+            L.in_w = in.w; L.out_w = out.w; L.l1_w = l1.w; L.l2_w = l2.w;
+            lts[k][l] = LayerT{in.t, in.q_t, in.kv_t, out.t, l1.t, l2.t};
+        }
+        heads[k]->w1 = forms(offs[k]->head.w1).w;
+        heads[k]->w1_t = forms(offs[k]->head.w1).t;
+    }
     *out = p;
     return 0;
 }
 
-extern "C" int uavtrain_destroy(uavtrain_t *p) {
-    if (!p) return 0;
-    cudaSetDevice(p->device);
-    cudaDeviceSynchronize();
-    for (void *q : p->allocs) cudaFree(q);
-    delete p;
-    return 0;
-}
+extern "C" int uavtrain_destroy(uavtrain_t *p) { return uavp::destroy_handle(p); }
 
 namespace {
 int forward_impl(uavtrain *p, const float *w, const float *d_obs, int n, float *d_feat, float *d_logits, float *d_value, void *stream) {
-    if (n <= 0 || n > p->max_samples) return tfail(p, -1, "uavtrain_forward: n=%d outside (0, %d]", n, p->max_samples);
-    T_TRY(p, cudaSetDevice(p->device));
+    if (n <= 0 || n > p->max_samples) return fail(p, -1, "uavtrain_forward: n=%d outside (0, %d]", n, p->max_samples);
+    UAVP_TRY(p, cudaSetDevice(p->device));
     TCtx c{p, (cudaStream_t)stream, 0};
     const bool heads = d_logits != nullptr;
     p->n = 0;
-    bind_params(p->actor, p->actor_off, w);
-    bind_params(p->critic, p->critic_off, w);
-    for (int j = 0; j < p->n_jobs; ++j) p->jobs.job[j].src = w + p->job_src_off[j];
-    prep_weights_kernel<<<dim3(24, p->n_jobs), 256, 0, c.s>>>(p->jobs);
+    bind_fp32(p->actor, p->actor_head, kActorOff, w);
+    bind_fp32(p->critic, p->critic_head, kCriticOff, w);
+    PrepJobs jobs{};
+    int n_jobs = 0;
+    for (int i = 0; i < kNumGemmW; ++i) {
+        const GemmW &g = kGemmW.w[i];
+        const Gemm16 &G = p->g16[i];
+        jobs.job[n_jobs++] = PrepJob{w + g.off, G.w, G.t, g.N, g.K};
+        if (G.q_t) {
+            jobs.job[n_jobs++] = PrepJob{w + g.off, nullptr, G.q_t, D, D};
+            jobs.job[n_jobs++] = PrepJob{w + g.off + D * D, nullptr, G.kv_t, 2 * D, D};
+        }
+    }
+    prep_weights_kernel<<<dim3(24, n_jobs), 256, 0, c.s>>>(jobs);
     const int R = n * S;
     embed_kernel<<<(R + kEmbTok - 1) / kEmbTok, kEmbThreads, 0, c.s>>>(d_obs, R, p->actor, p->critic, p->Ea, p->Ec, p->pad, p->obs16, p->relu_mask);
     last_layer_fwd(c, p->actor.layer[0], p->Ea, n, p->la, d_feat, 2 * D, heads ? p->ahead.Z : nullptr);
     full_layer_fwd(c, p->critic.layer[0], p->Ec, n, p->fc);
     last_layer_fwd(c, p->critic.layer[1], p->fc.Xout, n, p->lc, d_feat ? d_feat + D : nullptr, 2 * D, heads ? p->chead.Z : nullptr);
     if (heads) {
-        gemm(c, p->ahead.Z, D, p->ahead.w1, w + p->ahead_off.b1, p->ahead.Hh, n, HID, D, 1);
-        gemm(c, p->chead.Z, D, p->chead.w1, w + p->chead_off.b1, p->chead.Hh, n, HID, D, 1);
+        const HeadW &ha = p->actor_head, &hc = p->critic_head;
+        gemm(c, p->ahead.Z, D, p->ahead.w1, ha.b1, p->ahead.Hh, n, HID, D, 1);
+        gemm(c, p->chead.Z, D, p->chead.w1, hc.b1, p->chead.Hh, n, HID, D, 1);
         if (!c.rc)
-            head_out_kernel<<<(n + 255) / 256, 256, 0, c.s>>>(p->ahead.Hh, p->chead.Hh, w + p->ahead_off.w2, w + p->ahead_off.b2,
-                                                              w + p->chead_off.w2, w + p->chead_off.b2, n, d_logits, d_value);
+            head_out_kernel<<<(n + 255) / 256, 256, 0, c.s>>>(p->ahead.Hh, p->chead.Hh, ha.w2, ha.b2, hc.w2, hc.b2, n, d_logits, d_value);
     }
     if (c.rc) return c.rc;
-    T_TRY(p, cudaGetLastError());
+    UAVP_TRY(p, cudaGetLastError());
     p->n = n;
     p->with_heads = heads;
-    p->params = w;
     return 0;
 }
 
 int backward_impl(uavtrain *p, const float *d_dfeat, const float *d_dlogits, const float *d_dvalue, float *g, void *stream) {
-    T_TRY(p, cudaSetDevice(p->device));
+    UAVP_TRY(p, cudaSetDevice(p->device));
     TCtx c{p, (cudaStream_t)stream, 0};
     const int n = p->n;
     const bool heads = d_dlogits != nullptr;
-    T_TRY(p, cudaMemsetAsync(g, 0, (size_t)UAVPOLICY_NUM_PARAMS * sizeof(float), c.s));
+    UAVP_TRY(p, cudaMemsetAsync(g, 0, (size_t)UAVPOLICY_NUM_PARAMS * sizeof(float), c.s));
     if (heads) {
-        const float *w = p->params;
+        const HeadOff &ao = kActorOff.head, &co = kCriticOff.head;
         const int warps = p->sms * 8 * 4, spw = max(1, (n + warps - 1) / warps);
         head_bwd_kernel<<<((n + spw - 1) / spw + 7) / 8, 256, 0, c.s>>>(
-            p->ahead.Hh, p->chead.Hh, w + p->ahead_off.w2, w + p->chead_off.w2, d_dlogits, d_dvalue, n, spw, p->ahead.dHh, p->chead.dHh,
-            g + p->ahead_off.w2, g + p->ahead_off.b2, g + p->ahead_off.b1, g + p->chead_off.w2, g + p->chead_off.b2, g + p->chead_off.b1);
-        wgrad(c, p->ahead.dHh, D, p->ahead.Z, D, n, D, D, g + p->ahead_off.w1, HID);
-        wgrad(c, p->chead.dHh, D, p->chead.Z, D, n, D, D, g + p->chead_off.w1, HID);
+            p->ahead.Hh, p->chead.Hh, p->actor_head.w2, p->critic_head.w2, d_dlogits, d_dvalue, n, spw, p->ahead.dHh, p->chead.dHh,
+            g + ao.w2, g + ao.b2, g + ao.b1, g + co.w2, g + co.b2, g + co.b1);
+        wgrad(c, p->ahead.dHh, D, p->ahead.Z, D, n, D, D, g + ao.w1, HID);
+        wgrad(c, p->chead.dHh, D, p->chead.Z, D, n, D, D, g + co.w1, HID);
         gemm(c, p->ahead.dHh, D, p->ahead.w1_t, nullptr, p->ahead.Z, n, D, HID, 0);      // dZ overwrites Z (no longer needed)
         gemm(c, p->chead.dHh, D, p->chead.w1_t, nullptr, p->chead.Z, n, D, HID, 0);
     }
     // actor: one (last) layer on the embedding
-    last_layer_bwd(c, p->actor.layer[0], p->actor_t[0], p->actor_off.layer[0], g, p->Ea, n, p->la, heads ? nullptr : d_dfeat, 2 * D,
+    last_layer_bwd(c, p->actor.layer[0], p->actor_t[0], kActorOff.layer[0], g, p->Ea, n, p->la, heads ? nullptr : d_dfeat, 2 * D,
                    heads ? p->ahead.Z : nullptr, p->dXa);
-    embed_bwd(c, p->actor_off, 0, g, n, p->dXa, nullptr);
+    embed_bwd(c, kActorOff, 0, g, n, p->dXa, nullptr);
     // critic: last layer, inner layer, embedding
-    last_layer_bwd(c, p->critic.layer[1], p->critic_t[1], p->critic_off.layer[1], g, p->fc.Xout, n, p->lc,
+    last_layer_bwd(c, p->critic.layer[1], p->critic_t[1], kCriticOff.layer[1], g, p->fc.Xout, n, p->lc,
                    heads ? nullptr : d_dfeat + D, 2 * D, heads ? p->chead.Z : nullptr, p->dXa);
-    full_layer_bwd(c, p->critic.layer[0], p->critic_t[0], p->critic_off.layer[0], g, p->Ec, n, p->fc, p->dXa, p->dXb);
-    embed_bwd(c, p->critic_off, 1, g, n, p->dXb, p->dS1);
+    full_layer_bwd(c, p->critic.layer[0], p->critic_t[0], kCriticOff.layer[0], g, p->Ec, n, p->fc, p->dXa, p->dXb);
+    embed_bwd(c, kCriticOff, 1, g, n, p->dXb, p->dS1);
     if (c.rc) return c.rc;
-    T_TRY(p, cudaGetLastError());
+    UAVP_TRY(p, cudaGetLastError());
     return 0;
 }
 }  // namespace
 
 extern "C" int uavtrain_forward(uavtrain_t *p, const float *d_flat_params, const float *d_obs, int32_t n, float *d_feat, void *stream) {
     if (!p) return -1;
-    if (!d_flat_params || !d_obs || !d_feat) return tfail(p, -1, "uavtrain_forward: NULL argument");
+    if (!d_flat_params || !d_obs || !d_feat) return fail(p, -1, "uavtrain_forward: NULL argument");
     return forward_impl(p, d_flat_params, d_obs, n, d_feat, nullptr, nullptr, stream);
 }
 
 extern "C" int uavtrain_backward(uavtrain_t *p, const float *d_dfeat, float *d_flat_grad, void *stream) {
     if (!p) return -1;
-    if (!d_dfeat || !d_flat_grad) return tfail(p, -1, "uavtrain_backward: NULL argument");
-    if (p->n <= 0 || p->with_heads) return tfail(p, -4, "uavtrain_backward without a preceding uavtrain_forward");
+    if (!d_dfeat || !d_flat_grad) return fail(p, -1, "uavtrain_backward: NULL argument");
+    if (p->n <= 0 || p->with_heads) return fail(p, -4, "uavtrain_backward without a preceding uavtrain_forward");
     return backward_impl(p, d_dfeat, nullptr, nullptr, d_flat_grad, stream);
 }
 
 extern "C" int uavtrain_forward_heads(uavtrain_t *p, const float *d_flat_params, const float *d_obs, int32_t n, float *d_logits,
                                       float *d_value, void *stream) {
     if (!p) return -1;
-    if (!d_flat_params || !d_obs || !d_logits || !d_value) return tfail(p, -1, "uavtrain_forward_heads: NULL argument");
+    if (!d_flat_params || !d_obs || !d_logits || !d_value) return fail(p, -1, "uavtrain_forward_heads: NULL argument");
     return forward_impl(p, d_flat_params, d_obs, n, nullptr, d_logits, d_value, stream);
 }
 
 extern "C" int uavtrain_backward_heads(uavtrain_t *p, const float *d_dlogits, const float *d_dvalue, float *d_flat_grad, void *stream) {
     if (!p) return -1;
-    if (!d_dlogits || !d_dvalue || !d_flat_grad) return tfail(p, -1, "uavtrain_backward_heads: NULL argument");
-    if (p->n <= 0 || !p->with_heads) return tfail(p, -4, "uavtrain_backward_heads without a preceding uavtrain_forward_heads");
+    if (!d_dlogits || !d_dvalue || !d_flat_grad) return fail(p, -1, "uavtrain_backward_heads: NULL argument");
+    if (p->n <= 0 || !p->with_heads) return fail(p, -4, "uavtrain_backward_heads without a preceding uavtrain_forward_heads");
     return backward_impl(p, nullptr, d_dlogits, d_dvalue, d_flat_grad, stream);
 }
 
@@ -933,13 +831,13 @@ extern "C" int uavtrain_ppo_loss(uavtrain_t *p, const float *d_logits, const flo
                                  float c_entropy, float *d_dlogits, float *d_dvalue, float *d_stats, void *stream) {
     if (!p) return -1;
     if (!d_logits || !d_value || !d_action || !d_old_logp || !d_adv || !d_ret || !d_old_value || !d_dlogits || !d_dvalue || n <= 0)
-        return tfail(p, -1, "uavtrain_ppo_loss: NULL argument or n <= 0");
-    T_TRY(p, cudaSetDevice(p->device));
+        return fail(p, -1, "uavtrain_ppo_loss: NULL argument or n <= 0");
+    UAVP_TRY(p, cudaSetDevice(p->device));
     cudaStream_t s = (cudaStream_t)stream;
     PpoLossArgs a{d_logits, d_value, d_old_logp, d_adv, d_ret, d_old_value, d_action, n, eps_clip, c_value, c_entropy};
-    T_TRY(p, cudaMemsetAsync(p->loss_acc, 0, 4 * sizeof(float), s));
+    UAVP_TRY(p, cudaMemsetAsync(p->loss_acc, 0, 4 * sizeof(float), s));
     ppo_loss_sums_kernel<<<min((n + 255) / 256, p->sms * 4), 256, 0, s>>>(a, p->loss_acc);
     ppo_loss_grad_kernel<<<(n + 255) / 256, 256, 0, s>>>(a, p->loss_acc, d_dlogits, d_dvalue, d_stats);
-    T_TRY(p, cudaGetLastError());
+    UAVP_TRY(p, cudaGetLastError());
     return 0;
 }

@@ -106,45 +106,6 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float *v) {
     for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
 }
 
-// cooperative ASYNC copy (cp.async 16 B, LDGSTS) of a row-major bf16 matrix [rows x K] (global, row stride ld elements)
-// into a canonical tile.  Lane mapping inside each group of 32 consecutive work items: 8 rows x 4 chunks, so a
-// quarter-warp writes one whole 128 B core-matrix column slice (bank-conflict free) and reads 64 contiguous bytes
-// of each of 8 rows.  rows % 8 == 0 and K % 32 == 0.  Complete with cp_async_wait_all() + a barrier.
-__device__ __forceinline__ void load_canon_async(unsigned char *smem_tile, const __nv_bfloat16 *g, int rows, int K, int64_t ld,
-                                                 int tid, int nthreads) {
-    const int cq_per_row = K >> 5;                  // groups of 4 chunks (32 elements) per row
-    const int items = rows * (K >> 3);
-    for (int i = tid; i < items; i += nthreads) {
-        const int grp = i >> 5, in = i & 31;
-        const int rg = grp / cq_per_row, cq = grp % cq_per_row;
-        const int r = rg * 8 + (in & 7), c = cq * 4 + (in >> 3);
-        const uint32_t dst = smem_u32(smem_tile + canon_off(r, c * 8, K));
-        const __nv_bfloat16 *src = g + (int64_t)r * ld + c * 8;
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(dst), "l"(src) : "memory");
-    }
-}
-// the same copy for a tile whose tail rows may lie beyond the matrix: rows >= valid_rows are zero-filled (cp.async
-// with a source size of 0 reads nothing and writes zeros)
-__device__ __forceinline__ void load_canon_async_zfill(unsigned char *smem_tile, const __nv_bfloat16 *g, int rows, int K,
-                                                       int64_t ld, int valid_rows, int tid, int nthreads) {
-    const int cq_per_row = K >> 5;
-    const int items = rows * (K >> 3);
-    for (int i = tid; i < items; i += nthreads) {
-        const int grp = i >> 5, in = i & 31;
-        const int rg = grp / cq_per_row, cq = grp % cq_per_row;
-        const int r = rg * 8 + (in & 7), c = cq * 4 + (in >> 3);
-        const uint32_t dst = smem_u32(smem_tile + canon_off(r, c * 8, K));
-        const bool ok = r < valid_rows;
-        const __nv_bfloat16 *src = g + (int64_t)(ok ? r : 0) * ld + c * 8;
-        const uint32_t nbytes = ok ? 16u : 0u;
-        asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(dst), "l"(src), "r"(nbytes) : "memory");
-    }
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait_group() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N) : "memory"); }
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;\n" ::: "memory"); }
-
 // 1-D bulk TMA copy global -> shared (UBLKCP) of `bytes` (multiple of 16, both sides 16 B aligned); completion is
 // signalled on the mbarrier as a transaction count.  Issued by ONE thread, which also posts the expected bytes.
 __device__ __forceinline__ void bulk_load(void *smem_dst, const void *gmem_src, uint32_t bytes, uint64_t *mbar) {
@@ -169,7 +130,8 @@ __device__ __forceinline__ void tma_load_2d(void *smem_dst, const void *tensor_m
                      smem_u32(smem_dst)), "l"(tensor_map), "r"(c0), "r"(c1), "r"(smem_u32(mbar)) : "memory");
 }
 
-// synchronous variant with zero fill of rows >= valid_rows (self-test / ragged activations)
+// cooperative copy of a row-major bf16 matrix [rows x K] (global, row stride ld elements) into a canonical tile; rows >=
+// valid_rows are zero-filled (self-test / ragged activations)
 __device__ __forceinline__ void load_canon(unsigned char *smem_tile, const __nv_bfloat16 *g, int rows, int K, int64_t ld,
                                            int valid_rows, int tid, int nthreads) {
     const int chunks_per_row = K >> 3;              // 16 B chunks

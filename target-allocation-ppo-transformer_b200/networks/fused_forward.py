@@ -15,6 +15,14 @@ import torch
 from .. import _capi
 
 
+def flatten_params(module):
+    """A TransformerActorCritic's parameters as the library's flat vector (named_parameters order); differentiable."""
+    flat = torch.cat([p.reshape(-1) for p in module.parameters()])
+    if flat.numel() != _capi.NUM_PARAMS:
+        raise ValueError("expected the %d parameters of TransformerActorCritic" % _capi.NUM_PARAMS)
+    return flat
+
+
 class FusedPolicyForward:
     def __init__(self, max_batch, device, seed=0, env_id_base=0):
         self._h = None
@@ -47,9 +55,9 @@ class FusedPolicyForward:
 
     def sync(self, module):
         """Copy the weights of a TransformerActorCritic (named_parameters order == the reference's state_dict order)."""
-        flat = torch.cat([p.detach().reshape(-1).float() for p in module.parameters()]).contiguous()
-        if flat.numel() != 419267 or flat.device != self.device:
-            raise ValueError("expected the 419267 parameters of TransformerActorCritic on %s" % self.device)
+        flat = flatten_params(module).detach().float()
+        if flat.device != self.device:
+            raise ValueError("expected the parameters of TransformerActorCritic on %s" % self.device)
         self._flat = flat
         self._chk(self._lib.uavpolicy_set_weights(self._h, C.c_void_p(flat.data_ptr()), self._stream()))
 

@@ -12,8 +12,7 @@ import ctypes as C
 import torch
 
 from .. import _capi
-
-NUM_PARAMS = 419267
+from .fused_forward import flatten_params
 
 
 class _TrunkFn(torch.autograd.Function):
@@ -34,7 +33,7 @@ class _TrunkFn(torch.autograd.Function):
         if owner._pending != dfeat.shape[0]:
             raise RuntimeError("FusedTrunks keeps the activations of ONE forward: backward must follow its forward")
         dfeat = dfeat.contiguous().float()
-        grad = torch.empty(NUM_PARAMS, device=dfeat.device, dtype=torch.float32)
+        grad = torch.empty(_capi.NUM_PARAMS, device=dfeat.device, dtype=torch.float32)
         owner._chk(owner._lib.uavtrain_backward(owner._h, C.c_void_p(dfeat.data_ptr()), C.c_void_p(grad.data_ptr()),
                                                 owner._stream()))
         owner._pending = 0
@@ -62,7 +61,7 @@ class _PolicyFn(torch.autograd.Function):
         if owner._pending != dlogits.shape[0]:
             raise RuntimeError("FusedTrunks keeps the activations of ONE forward: backward must follow its forward")
         dlogits, dvalue = dlogits.contiguous().float(), dvalue.contiguous().float()
-        grad = torch.empty(NUM_PARAMS, device=dlogits.device, dtype=torch.float32)
+        grad = torch.empty(_capi.NUM_PARAMS, device=dlogits.device, dtype=torch.float32)
         owner._chk(owner._lib.uavtrain_backward_heads(owner._h, C.c_void_p(dlogits.data_ptr()), C.c_void_p(dvalue.data_ptr()),
                                                       C.c_void_p(grad.data_ptr()), owner._stream()))
         owner._pending = 0
@@ -96,17 +95,18 @@ class FusedTrunks:
 
     def features(self, module, obs):
         """[n,2,128] fp32: last-token features of actor_net / critic_net; differentiable w.r.t. module.parameters()."""
-        flat = torch.cat([p.reshape(-1) for p in module.parameters()])
-        if flat.numel() != NUM_PARAMS or flat.dtype != torch.float32:
-            raise ValueError("expected the %d fp32 parameters of TransformerActorCritic" % NUM_PARAMS)
-        return _TrunkFn.apply(self, obs.contiguous().float(), flat)
+        return _TrunkFn.apply(self, obs.contiguous().float(), self._fp32_params(module))
 
     def logits_and_value(self, module, obs):
         """== module.logits_and_value(obs): trunks and heads in the library, differentiable w.r.t. module.parameters()."""
-        flat = torch.cat([p.reshape(-1) for p in module.parameters()])
-        if flat.numel() != NUM_PARAMS or flat.dtype != torch.float32:
-            raise ValueError("expected the %d fp32 parameters of TransformerActorCritic" % NUM_PARAMS)
-        return _PolicyFn.apply(self, obs.contiguous().float(), flat)
+        return _PolicyFn.apply(self, obs.contiguous().float(), self._fp32_params(module))
+
+    @staticmethod
+    def _fp32_params(module):
+        flat = flatten_params(module)
+        if flat.dtype != torch.float32:
+            raise ValueError("expected the fp32 parameters of TransformerActorCritic")
+        return flat
 
     def evaluate(self, module, obs, action):
         """== module.evaluate(obs, action) (transformer_net.py:124-143): (log_prob [n], value [n,1], entropy [n])."""
