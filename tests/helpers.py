@@ -93,5 +93,35 @@ def scene_from_fixture(fx, copies=1):
     return {k: np.tile(np.asarray(fx[k]), (copies, 1)) for k in SCENE_KEYS}
 
 
+LOGIT_TOL = 0.1     # of the spread of the logits (log-probs) across windows
+
+
+def logit_spread(net, logprobs=False):
+    """The smallest standard deviation across windows of a column of the actor's logits (or log-probs), fp32 network, over
+    4096 seeded random windows with 0..4 leading zero rows.  The actor's last layer is initialised with std 0.01, so the
+    logits of a young network differ across windows by a few 1e-3: an absolute tolerance of 1e-2 on them passes even an
+    actor whose trunk output is zero."""
+    import torch
+    g = torch.Generator().manual_seed(0)
+    obs = torch.rand(4096, 5, 14, generator=g)
+    obs[:, :, 13] = 1.0
+    obs[torch.arange(5)[None, :] < (torch.arange(4096) % 5)[:, None]] = 0.0
+    with torch.no_grad():
+        logits = net.actor_head(net.actor_net.forward_last(obs.to(next(net.parameters()).device)))
+    return float((torch.log_softmax(logits, -1) if logprobs else logits).std(0).min())
+
+
+def logits_close(got, ref, net, logprobs=False):
+    """(ok, error): the largest |got - ref| in units of logit_spread(net) is at most LOGIT_TOL."""
+    err = float((got.double() - ref.double()).abs().max()) / logit_spread(net, logprobs)
+    return err <= LOGIT_TOL, err
+
+
+def assert_logits_close(got, ref, net, logprobs=False, note=""):
+    ok, err = logits_close(got, ref, net, logprobs)
+    print("\n[logits_close%s] %.3f of the spread" % (note, err))
+    assert ok, ("max |error| is %.3f of the spread across windows, above %g" % (err, LOGIT_TOL), note)
+
+
 def rel_close(got, want, rtol, atol=0.0):
     np.testing.assert_allclose(np.asarray(got, np.float64), np.asarray(want, np.float64), rtol=rtol, atol=atol)

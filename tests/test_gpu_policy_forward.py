@@ -1,11 +1,12 @@
 """tcgen05 rollout forward (csrc/policy_forward.cu) against the fp32 PyTorch network with the reference's weights
-(tests/golden/policy_net.npz).  bf16 operands: logits / values within 3e-2 absolute, log-probs within 2e-2;
+(tests/golden/policy_net.npz).  bf16 operands: logits and log-probs within helpers.LOGIT_TOL of their spread across
+windows (the actor's last layer has std 0.01: an absolute tolerance would pass a zero actor trunk), values within 3e-2;
 sampling follows the returned probabilities; the library has no CPU fallback."""
 import numpy as np
 import pytest
 import torch
 
-from helpers import policy_fixture
+from helpers import assert_logits_close, policy_fixture
 
 import uavenv_b200  # noqa: F401  (registers the package under an importable name)
 
@@ -46,13 +47,13 @@ def test_forward_matches_fp32_network_and_reference_golden():
     logits = fused.logits[: obs.shape[0]]
     with torch.no_grad():
         ref_logits, ref_v = net.logits_and_value(obs)
-    assert float((logits - ref_logits).abs().max()) < 3e-2
+    assert_logits_close(logits, ref_logits, net)
     assert float((v - ref_v).abs().max()) < 3e-2 * max(1.0, float(ref_v.abs().max()))
     # against the values recorded from the UNMODIFIED reference network
-    assert float((logits.cpu() - torch.from_numpy(fx["logits"])).abs().max()) < 3e-2
+    assert_logits_close(logits.cpu(), torch.from_numpy(fx["logits"]), net)
     assert float((v.cpu() - torch.from_numpy(fx["value"])).abs().max()) < 3e-2 * max(1.0, float(np.abs(fx["value"]).max()))
     ref_lp = torch.log_softmax(ref_logits, -1).gather(-1, a[:, None]).squeeze(-1)
-    assert float((lp - ref_lp).abs().max()) < 2e-2
+    assert_logits_close(lp, ref_lp, net, logprobs=True)
     p = torch.softmax(logits, -1)
     assert torch.allclose(e, -(p * p.log()).sum(-1), atol=1e-5)
     assert set(a.tolist()) <= {0, 1}
@@ -74,7 +75,7 @@ def test_padding_rows_and_batch_tails():
         _, _, v, _ = fused.get_action(obs, step=3)
         with torch.no_grad():
             ref_logits, ref_v = net.logits_and_value(obs)
-        assert float((fused.logits[:B] - ref_logits).abs().max()) < 3e-2
+        assert_logits_close(fused.logits[:B], ref_logits, net, note=" B=%d" % B)
         assert float((v - ref_v).abs().max()) < 3e-2 * max(1.0, float(ref_v.abs().max()))
     fused.close()
 
@@ -95,7 +96,7 @@ def test_actor_work_items_of_several_tiles_at_large_batches():
         _, _, v, _ = fused.get_action(obs, step=3)
         with torch.no_grad():
             ref_logits, ref_v = net.logits_and_value(obs)
-        assert float((fused.logits[:B] - ref_logits).abs().max()) < 3e-2, B
+        assert_logits_close(fused.logits[:B], ref_logits, net, note=" B=%d" % B)
         assert float((v - ref_v).abs().max()) < 3e-2 * max(1.0, float(ref_v.abs().max())), B
     fused.close()
 
