@@ -171,6 +171,15 @@ int uavenv_recompute_objective(uavenv_t *h, double *h_max_abs_diff, void *stream
  * the env-only benchmarks (SURVEY.md §8d) */
 int uavenv_random_actions(uavenv_t *h, uint64_t action_seed, uint64_t step, int64_t *d_actions, void *stream);
 
+/* Actions of the best-target heuristic, an evaluation baseline: at the pointer (k, m) UAV k Assigns iff m is the target
+ * j* that maximises the paper reward (Eq.19) after a tentative assignment of UAV k (lowest index on a tie), and that
+ * reward is not below the current one (csrc/uavenv_kernels.cuh states the rule).  d_cache: device int64 [B], caller-owned,
+ * zeroed before the first call; it keeps j* per env keyed by (episode counter, UAV pointer), so j* is computed once per
+ * UAV row, and auto-resets, new rows and skipped calls are detected.  uavenv_reset(full_reset = 1) and uavenv_load_scene
+ * restart the episode counter at 1: zero d_cache after them unless the next call is made before the next step.
+ * d_actions: device int64 [B].  Call on the env's stream after a step and before the next one. */
+int uavenv_best_target_actions(uavenv_t *h, int64_t *d_cache, int64_t *d_actions, void *stream);
+
 /* ---- per-episode records of an evaluation (csrc/uavenv_episodes.cu) ---------------------------------------------
  * One finished episode.  ret sums the fp64 step rewards (info d_reward_f64) in step order; J_val, avg_p_dmg,
  * avg_p_final and num_assigned are the info of the episode's last step, i.e. of its final allocation. */

@@ -27,7 +27,7 @@ def __getattr__(name):  # torch / CUDA are only touched when the env classes are
     if name == "train":                      # the submodule itself is callable: ub.train(...) == ub.train.train(...)
         import importlib
         return importlib.import_module(__name__ + ".train")
-    if name in ("evaluate", "EpisodeRecorder", "load_checkpoint"):
+    if name in ("evaluate", "evaluate_baseline", "EpisodeRecorder", "load_checkpoint"):
         from . import evaluation
         return getattr(evaluation, name)
     if name in ("analyze_environment_difficulty", "record_decisions"):

@@ -121,6 +121,7 @@ def load():
     L.uavenv_score_matrix_f64.argtypes = [vp, vp, vp, vp]
     L.uavenv_recompute_objective.argtypes = [vp, c_f64p, vp]
     L.uavenv_random_actions.argtypes = [vp, u64, u64, vp, vp]
+    L.uavenv_best_target_actions.argtypes = [vp, vp, vp, vp]
     L.uavenv_episode_accumulate.argtypes = [i32, vp, vp, C.POINTER(UavenvInfo), i32, C.POINTER(UavenvEpisodeAcc), vp, i32, vp]
     L.ppo_gae_advantages.argtypes = [vp, vp, vp, vp, i32, i32, C.c_float, C.c_float, vp, vp, i32, vp, i32, vp]
     L.ppo_normalize_advantages.argtypes = [vp, i64, vp, i32, vp]
@@ -134,7 +135,7 @@ def load():
     L.ppo_attn5_backward.restype = C.c_int
     for name in ("uavenv_create", "uavenv_destroy", "uavenv_reset", "uavenv_step", "uavenv_step_host",
                  "uavenv_load_scene", "uavenv_get_scene", "uavenv_get_state", "uavenv_score_matrix",
-                 "uavenv_score_matrix_f64", "uavenv_recompute_objective", "uavenv_random_actions",
+                 "uavenv_score_matrix_f64", "uavenv_recompute_objective", "uavenv_random_actions", "uavenv_best_target_actions",
                  "uavenv_episode_accumulate", "ppo_gae_advantages", "ppo_normalize_advantages"):
         getattr(L, name).restype = C.c_int
     if L.uavenv_abi_version() != 2:

@@ -526,3 +526,13 @@ extern "C" int uavenv_random_actions(uavenv_t *h, uint64_t action_seed, uint64_t
                                                                                (uint32_t)(action_seed >> 32), step, d_actions);
     return launch_check(h, "random_actions_kernel");
 }
+
+extern "C" int uavenv_best_target_actions(uavenv_t *h, int64_t *d_cache, int64_t *d_actions, void *stream) {
+    if (!h) return UAVENV_EINVAL;
+    if (!d_cache || !d_actions) return fail(h, UAVENV_EINVAL, "uavenv_best_target_actions: cache/actions must be non-NULL device pointers");
+    if (!h->ready) return fail(h, UAVENV_ESTATE, "uavenv_best_target_actions before reset()/load_scene()");
+    CU_TRY(h, cudaSetDevice(h->device));
+    best_target_kernel<<<(h->B + kBestTargetThreads - 1) / kBestTargetThreads, kBestTargetThreads, 0, (cudaStream_t)stream>>>(
+        h->P, d_cache, d_actions);
+    return launch_check(h, "best_target_kernel");
+}

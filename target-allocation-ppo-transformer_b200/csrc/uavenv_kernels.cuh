@@ -10,6 +10,8 @@
 //   score_matrix_kernel  p_final / p_damage [B,N,M] (main.py:38-45 over mechanics.py:167-181).
 //   recompute_kernel     fresh J / N0 / sums from the per-target products, a warp per env with
 //                        shuffle reductions (uav_env.py:244-293) - drift bound for the running sums.
+//   best_target_kernel   the best-target heuristic's actions (evaluation baseline): a warp per 32 envs,
+//                        one cooperative row of pair scores when a UAV's row is entered.
 #pragma once
 
 #include "uavenv_device.cuh"
@@ -902,6 +904,86 @@ __global__ void random_actions_kernel(const __grid_constant__ Params P, uint32_t
         const uint4 r = philox4x32(s0, s1, P.env_id_base + (uint32_t)b, (uint32_t)step, (uint32_t)(step >> 32),
                                    0x00AC7101u);
         actions[b] = (int64_t)(r.x >> 31);
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Best-target heuristic (include/uavenv_b200.h, uavenv_best_target_actions).  At the pointer (k, m) of an env:
+//   prev_r    = paper_reward(J, N0) (Eq.19) from the carried header sums, as the step kernel's accept test forms it;
+//   new_r(j)  = the paper reward after tentatively assigning UAV k to target j: nh' = nh_j * (1 - p_final(k,j)),
+//               revenue += (nh_j - nh') * value_j, cost += cost_k, N0 += 1 if target j was uncovered;
+//   j*        = argmax_j new_r(j), the lowest index winning a tie;
+//   action    = Assign (1) iff m == j* and new_r(j*) >= prev_r, otherwise Skip (0).
+// Only an accepted Assign changes the scene's state, and it ends UAV k's row, so j* computed when the pointer enters row
+// k holds for the whole row.  A rejected Assign (the env's exact Eq.21 path) lets the row run out.
+//
+// The caller's cache holds one entry per env: bits 32..63 the episode counter, 16..31 the UAV pointer k, 0..15 the target
+// to assign in that row (kNoTarget: none).  An entry is recomputed when its key differs from the env's (episode, k) - an
+// auto-reset, a new row, a call skipped at the row's first step - and whenever m == 0 (the first step of every row, so a
+// reset() / load_scene(), which restart at (0, 0), never meet a stale entry on their first step).
+
+constexpr int kBestTargetThreads = 256;
+constexpr uint32_t kNoTarget = 0xffffu;
+
+__device__ __forceinline__ uint64_t best_target_key(int episode, int k) {
+    return ((uint64_t)(uint32_t)episode << 16) | (uint32_t)k;
+}
+
+// j* of env e's row k (warp-cooperative, all lanes return it): lanes = targets, as in score_matrix_kernel, pair scores as
+// in eval_pointer_pair, new_r as in the step kernel's accept test; then a shuffle arg-max
+__device__ __noinline__ uint32_t warp_best_target(const Params &P, int e, int k, int episode) {
+    const int lane = threadIdx.x & 31;
+    const Hdr h = P.header(e);
+    const int slot = h.n(I_GEN) & 1, n0 = h.n(I_NCOVERED);
+    const double rev = h.f(F_REV), cost_sum = h.f(F_COST_SUM);
+    const UavRec u = P.uav[P.uoff(slot, e) + k];                        // warp-uniform address
+    const double prev_r = paper_reward(rev - (P.omega * cost_sum), n0, P.M);
+    const double cost2 = cost_sum + u.cost;
+    const TgtRec *T = P.tgt + P.toff(slot, e);
+    double best = -INFINITY;
+    int bj = INT_MAX;
+    for (int j = lane; j < P.M; j += 32) {
+        TgtRec t = T[j];
+        const int cnt = target_view(t, episode);
+        const double pf = damage_prob(P, u, t.x, t.y, t.speed) * u.p_pen;
+        const double nh2 = t.nh * (1.0 - pf);
+        const double rev2 = rev + ((1.0 - nh2) - (1.0 - t.nh)) * t.value;
+        const double r = paper_reward(rev2 - (P.omega * cost2), n0 + (cnt == 0), P.M);
+        if (r > best) { best = r; bj = j; }                            // j ascends within a lane: the first maximum stays
+    }
+    for (int o = 16; o > 0; o >>= 1) {
+        const double ob = __shfl_xor_sync(kFullMask, best, o);
+        const int oj = __shfl_xor_sync(kFullMask, bj, o);
+        if (ob > best || (ob == best && oj < bj)) { best = ob; bj = oj; }
+    }
+    return (bj < P.M && best >= prev_r) ? (uint32_t)bj : kNoTarget;
+}
+
+__global__ void __launch_bounds__(kBestTargetThreads) best_target_kernel(const __grid_constant__ Params P, int64_t *cache,
+                                                                        int64_t *actions) {
+    const int lane = threadIdx.x & 31;
+    const int b0 = (int)(((size_t)blockIdx.x * blockDim.x + threadIdx.x) & ~(size_t)31);   // first env of this warp
+    if (b0 >= P.B) return;                                              // (uniform per warp)
+    const int b = b0 + lane;
+    const bool live = b < P.B;
+    const int bc = live ? b : P.B - 1;
+    const Hdr H = P.header(bc);
+    const int k = H.n(I_K), m = H.n(I_M), episode = H.n(I_EPISODE);
+    const bool active = live && k < P.N && (P.auto_reset || !H.n(I_FINISHED));   // a finished env without auto-reset is inert
+    uint64_t entry = (uint64_t)cache[bc];
+    const uint64_t key = best_target_key(episode, k);
+    const bool stale = active && (m == 0 || (entry >> 16) != key);
+    unsigned mask = __ballot_sync(kFullMask, stale);
+    while (mask) {
+        const int src = __ffs(mask) - 1;
+        mask &= mask - 1;
+        const int ks = __shfl_sync(kFullMask, k, src), es = __shfl_sync(kFullMask, episode, src);
+        const uint32_t j = warp_best_target(P, b0 + src, ks, es);
+        if (lane == src) entry = (key << 16) | j;
+    }
+    if (live) {
+        if (stale) cache[b] = (int64_t)entry;
+        actions[b] = (active && (uint32_t)(entry & 0xffffu) == (uint32_t)m) ? 1 : 0;
     }
 }
 

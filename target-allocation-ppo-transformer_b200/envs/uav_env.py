@@ -111,6 +111,7 @@ class UAVEnvBatched:
             self._info_c = ic
         self._actions = torch.zeros(B, dtype=torch.int64, device=dev)
         self._h_reward = self._h_done = None
+        self._best_target_cache = None        # best_target_actions' per-env entries, allocated on first use
 
     # ------------------------------------------------------------------ lifecycle
     def close(self):
@@ -141,7 +142,14 @@ class UAVEnvBatched:
             mask_ptr = C.c_void_p(env_mask.data_ptr())
         self._chk(self._lib.uavenv_reset(self._h, int(bool(full_reset)), mask_ptr, C.c_void_p(self.obs.data_ptr()),
                                          self._stream()))
+        self._forget_best_targets()
         return self.obs
+
+    def _forget_best_targets(self):
+        # a full reset or a scene load restarts the episode counter at 1: the cache key alone cannot tell the new episode 1
+        # from the old one when the first call after it comes later than the first step
+        if self._best_target_cache is not None:
+            self._best_target_cache.zero_()
 
     def _as_actions(self, actions):
         if isinstance(actions, torch.Tensor) and actions.device == self.device and actions.dtype == torch.int64 \
@@ -195,6 +203,21 @@ class UAVEnvBatched:
                                                   self._stream()))
         return out
 
+    def best_target_actions(self, out=None):
+        """Actions [B] int64 (device) of the best-target heuristic at the current pointers: UAV k Assigns iff the pointer
+        target is the one whose tentative assignment gives the highest paper reward (Eq.19; lowest index on a tie) and
+        that reward is not below the current one.  The best target is computed once per UAV row and cached on the device
+        (keyed by episode and UAV pointer); call after reset() / a step, on the env's stream."""
+        out = self._actions if out is None else out
+        if not (isinstance(out, torch.Tensor) and out.device == self.device and out.dtype == torch.int64
+                and out.is_contiguous() and out.numel() == self.num_envs):
+            raise ValueError("out must be a contiguous int64 tensor of num_envs elements on the env's device")
+        if self._best_target_cache is None:
+            self._best_target_cache = torch.zeros(self.num_envs, dtype=torch.int64, device=self.device)
+        self._chk(self._lib.uavenv_best_target_actions(self._h, C.c_void_p(self._best_target_cache.data_ptr()),
+                                                       C.c_void_p(out.data_ptr()), self._stream()))
+        return out
+
     # ------------------------------------------------------------------ scene / state access
     def _dims(self):
         return {"N": self.N, "M": self.M, "K1": self.K1, "K2": self.K2, "1": 1}
@@ -225,6 +248,7 @@ class UAVEnvBatched:
             setattr(sc, name, a.ctypes.data)
         self._chk(self._lib.uavenv_load_scene(self._h, C.byref(sc), int(first_env), int(count),
                                               C.c_void_p(self.obs.data_ptr())))
+        self._forget_best_targets()
         return self.obs[first_env:first_env + count]
 
     def get_scene(self, first_env=0, count=None):

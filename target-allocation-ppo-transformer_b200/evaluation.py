@@ -8,6 +8,9 @@ include/uavpolicy_eval_b200.h), the fused env step, and uavenv_episode_accumulat
 sums and writes a record when an episode ends.  The only host synchronisation is a poll of the completed-env counter
 every POLL_STEPS steps.
 
+ub.evaluate_baseline("best_target" | "random", ...) plays the same scenes with a rule in place of the network (the
+best-target heuristic's kernel, or the Bernoulli(1/2) action stream): reference points for a checkpoint's numbers.
+
 Scenes: the env runs with RESET_EPISODES = 1, so every episode is a fresh scene keyed (seed, global env id, scene
 index).  The default seed is not the training seed, so the evaluation plays scenes the training envs do not; two
 checkpoints evaluated with the same seed play the same scenes, and their records can be compared episode by episode.
@@ -125,6 +128,53 @@ def _summary(res, env_steps, wall):
     return s
 
 
+def _eval_setup(num_envs, episodes_per_env, config, device, env_id_base):
+    """(device, num_envs, quota, cfg, rank's first global env id, world size) of an evaluation run, arguments checked."""
+    device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    if device.type != "cuda":
+        raise RuntimeError("evaluate runs on a CUDA device (sm_100a); there is no CPU fallback")
+    if device.index is None:
+        device = torch.device("cuda", torch.cuda.current_device())
+    num_envs, quota = int(num_envs), int(episodes_per_env)
+    if num_envs <= 0 or quota <= 0:
+        raise ValueError("num_envs and episodes_per_env must be positive")
+    cfg = (config if config is not None else _global_cfg).copy(RESET_EPISODES=1)   # a fresh scene every episode
+    rank, world = _world()
+    base = rank * num_envs if env_id_base is None else int(env_id_base)
+    return device, num_envs, quota, cfg, base, world
+
+
+def _play(env, quota, act, world):
+    """Play `quota` episodes in every env of `env` with actions act(obs, step) (int64 [B] on the device); returns the
+    records of all ranks in global env order, the steps taken and the wall seconds."""
+    num_envs, device = env.num_envs, env.device
+    rec = EpisodeRecorder(env, quota)
+    max_steps = quota * env.N * env.M        # every step moves the (UAV, target) pointer: an episode ends within N * M
+    torch.cuda.synchronize(device)
+    t0 = time.perf_counter()
+    obs = env.reset(full_reset=True)
+    steps = 0
+    while steps < max_steps:
+        action = act(obs, steps)
+        obs, _, _, _ = env.step(action)
+        rec.record(action)
+        steps += 1
+        if steps % POLL_STEPS == 0 and rec.complete() == num_envs:
+            break
+    # summed over the ranks, so that all of them raise together instead of some waiting in the all-gather
+    missing = int(parallel.reduce_scalar(num_envs - rec.complete(), "sum", device))
+    if missing:
+        raise RuntimeError("%d of %d envs did not finish %d episodes within %d steps" % (
+            missing, num_envs * world, quota, max_steps))
+    raw = rec.raw
+    if world > 1:
+        parts = [torch.empty_like(raw) for _ in range(world)]
+        torch.distributed.all_gather(parts, raw)
+        raw = torch.cat(parts)
+    res = records_from_raw(raw, quota, env.M)
+    return res, steps, time.perf_counter() - t0
+
+
 def evaluate(policy, num_envs=4096, episodes_per_env=1, greedy=True, seed=DEFAULT_SEED, config=None, device=None,
              env_id_base=None):
     """Play `episodes_per_env` episodes in each of `num_envs` envs (per rank) and return per-episode numpy arrays
@@ -138,17 +188,7 @@ def evaluate(policy, num_envs=4096, episodes_per_env=1, greedy=True, seed=DEFAUL
     episodes_per_env, and the records of all ranks are all-gathered."""
     from .envs.uav_env import UAVEnvBatched
     from .networks.fused_forward import FusedPolicyForward
-    device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
-    if device.type != "cuda":
-        raise RuntimeError("evaluate runs on a CUDA device (sm_100a); there is no CPU fallback")
-    if device.index is None:
-        device = torch.device("cuda", torch.cuda.current_device())
-    num_envs, quota = int(num_envs), int(episodes_per_env)
-    if num_envs <= 0 or quota <= 0:
-        raise ValueError("num_envs and episodes_per_env must be positive")
-    cfg = (config if config is not None else _global_cfg).copy(RESET_EPISODES=1)   # a fresh scene every episode
-    rank, world = _world()
-    base = rank * num_envs if env_id_base is None else int(env_id_base)
+    device, num_envs, quota, cfg, base, world = _eval_setup(num_envs, episodes_per_env, config, device, env_id_base)
     net = load_checkpoint(policy, cfg)
     if net is policy:                            # the caller's module stays where it is: evaluate a copy on the device
         net = copy.deepcopy(net)
@@ -158,34 +198,42 @@ def evaluate(policy, num_envs=4096, episodes_per_env=1, greedy=True, seed=DEFAUL
         env = UAVEnvBatched(num_envs, device=device, seed=seed, config=cfg, env_id_base=base)
         fused = FusedPolicyForward(num_envs, device, seed=seed, env_id_base=base)
         fused.sync(net)
-        rec = EpisodeRecorder(env, quota)
-        max_steps = quota * env.N * env.M        # every step moves the (UAV, target) pointer: an episode ends within N * M
-        torch.cuda.synchronize(device)
-        t0 = time.perf_counter()
-        obs = env.reset(full_reset=True)
-        steps = 0
-        while steps < max_steps:
-            action, _ = fused.act(obs, steps, greedy=greedy)
-            obs, _, _, _ = env.step(action)
-            rec.record(action)
-            steps += 1
-            if steps % POLL_STEPS == 0 and rec.complete() == num_envs:
-                break
-        # summed over the ranks, so that all of them raise together instead of some waiting in the all-gather
-        missing = int(parallel.reduce_scalar(num_envs - rec.complete(), "sum", device))
-        if missing:
-            raise RuntimeError("%d of %d envs did not finish %d episodes within %d steps" % (
-                missing, num_envs * world, quota, max_steps))
-        raw = rec.raw
-        if world > 1:
-            parts = [torch.empty_like(raw) for _ in range(world)]
-            torch.distributed.all_gather(parts, raw)
-            raw = torch.cat(parts)
-        res = records_from_raw(raw, quota, env.M)
-        wall = time.perf_counter() - t0
+        res, steps, wall = _play(env, quota, lambda obs, step: fused.act(obs, step, greedy=greedy)[0], world)
     finally:
         if fused is not None:
             fused.close()
+        if env is not None:
+            env.close()
+    res["summary"] = _summary(res, parallel.reduce_scalar(steps * num_envs, "sum", device), wall)
+    return res
+
+
+BASELINES = ("best_target", "random")
+
+
+def evaluate_baseline(kind, num_envs=4096, episodes_per_env=1, seed=DEFAULT_SEED, config=None, device=None,
+                      env_id_base=None):
+    """Reference points for evaluate(): the same scenes played by a rule instead of a network.  Returns the same dict as
+    evaluate() (records in global env order, all-gathered under a process group, and `summary`); with an equal seed its
+    records pair episode by episode with those of evaluate(checkpoint).
+
+    kind "best_target": each UAV Assigns the target whose tentative assignment gives the highest paper reward (Eq.19),
+    if that reward is not below the current one (UAVEnvBatched.best_target_actions, one kernel per step).
+    kind "random": Bernoulli(1/2) actions keyed (seed + 1, step, global env id) - UAVEnvBatched.random_actions with
+    action_seed = seed + 1, so the action stream is not drawn with the scenes' key."""
+    from .envs.uav_env import UAVEnvBatched
+    if kind not in BASELINES:
+        raise ValueError("kind must be one of %s, got %r" % (", ".join(BASELINES), kind))
+    device, num_envs, quota, cfg, base, world = _eval_setup(num_envs, episodes_per_env, config, device, env_id_base)
+    env = None
+    try:
+        env = UAVEnvBatched(num_envs, device=device, seed=seed, config=cfg, env_id_base=base)
+
+        def act(obs, step):
+            return env.best_target_actions() if kind == "best_target" else env.random_actions(step, action_seed=seed + 1)
+
+        res, steps, wall = _play(env, quota, act, world)
+    finally:
         if env is not None:
             env.close()
     res["summary"] = _summary(res, parallel.reduce_scalar(steps * num_envs, "sum", device), wall)
