@@ -79,22 +79,32 @@ def lib_path():
     return _build.LIB_PATH
 
 
+def _open(path, override_var, abi_fn, abi_version):
+    """The library at `path`, built first when it is stale, or the build named by $override_var (timing experiments
+    only: an ablation / diagnostic build of the same ABI).  Raises ImportError on any failure."""
+    name = os.path.basename(path)
+    override = os.environ.get(override_var)
+    if override:
+        path = override
+    elif not _build.up_to_date(path):
+        try:
+            _build.build(lib=path)
+        except Exception as exc:  # no nvcc on this host, or a compile error: never load a binary older than its sources
+            raise ImportError("%s is %s and could not be (re)built (%s); there is no CPU fallback" % (
+                name, "stale" if os.path.isfile(path) else "missing", exc)) from exc
+    L = C.CDLL(path)
+    getattr(L, abi_fn).restype = C.c_int
+    if getattr(L, abi_fn)() != abi_version:
+        raise ImportError("%s ABI version mismatch" % name)
+    return L
+
+
 def load():
     """Load (building first if the sources are newer) the sm_100a library.  Raises on any failure."""
     global _lib
     if _lib is not None:
         return _lib
-    path = _build.LIB_PATH
-    override = os.environ.get("UAVENV_LIB_OVERRIDE")     # timing experiments only: an ablation build of the same ABI
-    if override:
-        path = override
-    elif not _build.up_to_date():
-        try:
-            _build.build(lib=path)
-        except Exception as exc:  # no nvcc on this host, or a compile error: never load a binary older than its sources
-            raise ImportError("libuavenv_b200.so is %s and could not be (re)built (%s); the environment has no CPU "
-                              "fallback" % ("stale" if os.path.isfile(path) else "missing", exc)) from exc
-    L = C.CDLL(path)
+    L = _open(_build.LIB_PATH, "UAVENV_LIB_OVERRIDE", "uavenv_abi_version", 2)
     vp, i32, i64, u64 = C.c_void_p, C.c_int32, C.c_int64, C.c_uint64
     L.uavenv_default_cfg.argtypes = [C.POINTER(UavenvCfg)]
     L.uavenv_default_cfg.restype = None
@@ -102,7 +112,6 @@ def load():
     L.uavenv_destroy.argtypes = [vp]
     L.uavenv_last_error.argtypes = [vp]
     L.uavenv_last_error.restype = C.c_char_p
-    L.uavenv_abi_version.restype = C.c_int
     L.uavenv_num_envs.argtypes = [vp]
     L.uavenv_num_envs.restype = i32
     L.uavenv_reset.argtypes = [vp, i32, vp, vp, vp]
@@ -138,8 +147,6 @@ def load():
                  "uavenv_score_matrix_f64", "uavenv_recompute_objective", "uavenv_random_actions", "uavenv_best_target_actions",
                  "uavenv_episode_accumulate", "ppo_gae_advantages", "ppo_normalize_advantages"):
         getattr(L, name).restype = C.c_int
-    if L.uavenv_abi_version() != 2:
-        raise ImportError("libuavenv_b200.so ABI version mismatch")
     _lib = L
     return L
 
@@ -160,20 +167,7 @@ def load_policy():
     global _policy_lib
     if _policy_lib is not None:
         return _policy_lib
-    path = _build.POLICY_LIB_PATH
-    override = os.environ.get("UAVPOLICY_LIB_OVERRIDE")   # timing experiments only: a diagnostic build of the same ABI
-    if override:
-        path = override
-    elif not _build.up_to_date(path):
-        try:
-            _build.build(lib=path)
-        except Exception as exc:
-            raise ImportError("libuavpolicy_b200.so is %s and could not be (re)built (%s)" % (
-                "stale" if os.path.isfile(path) else "missing", exc)) from exc
-    L = C.CDLL(path)
-    L.uavpolicy_abi_version.restype = C.c_int
-    if L.uavpolicy_abi_version() != 3:
-        raise ImportError("libuavpolicy_b200.so ABI version mismatch")
+    L = _open(_build.POLICY_LIB_PATH, "UAVPOLICY_LIB_OVERRIDE", "uavpolicy_abi_version", 3)
     vp, i32, u64 = C.c_void_p, C.c_int32, C.c_uint64
     L.uavpolicy_create.argtypes = [i32, i32, C.POINTER(vp)]
     L.uavpolicy_destroy.argtypes = [vp]

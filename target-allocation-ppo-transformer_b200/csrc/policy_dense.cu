@@ -330,21 +330,8 @@ __global__ void __launch_bounds__(kThreads, 1) dense_kernel(const __grid_constan
     if (warp == 1) { tc::tc_fence_after(); tc::tmem_free(tmem, tmem_cols); }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                  const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn g_encode = nullptr;
 int g_sms = 0;
 bool g_ready = false;
-
-// row-major bf16 [rows, cols] with row stride ld (elements) as a 2-D tensor map with [box_rows x 64] boxes, 128 B swizzle
-bool make_map(CUtensorMap *m, const void *base, int64_t ld, int64_t rows, int cols, int box_rows) {
-    const cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-    const cuuint64_t gstride[1] = {(cuuint64_t)ld * 2};
-    const cuuint32_t box[2] = {64, (cuuint32_t)box_rows}, estr[2] = {1, 1};
-    return g_encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(base), gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                    CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
 
 int ring_depth(int act, int K) { return act == kAddLN ? (K > 128 ? 3 : 4) : (act == kDRelu ? 4 : kRing); }
 
@@ -355,11 +342,7 @@ size_t smem_bytes(int N, int K, int act) {
 
 int prepare() {
     if (g_ready) return 0;
-    void *fn = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess || !fn)
-        return -1;
-    g_encode = reinterpret_cast<EncodeTiledFn>(fn);
+    if (!tensor_maps_available()) return -1;
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&g_sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return -1;
     if (cudaFuncSetAttribute(dense_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes(kMaxN, 128, kIdentity)) != cudaSuccess)
@@ -379,10 +362,12 @@ int launch(const void *A, int64_t lda, const void *W, const float *bias, const v
     if (act >= kDRelu && (!aux || smem_bytes(N, K, act) > smem_bytes(kMaxN, 128, kIdentity))) return -1;
     if (act == kAddLN && (N != 128 || !gamma || !beta || !xhat || !rstd)) return -1;
     CUtensorMap tm_a, tm_w, tm_d, tm_aux, tm_d2;
-    if (!make_map(&tm_a, A, lda, M, K, 128) || !make_map(&tm_w, W, K, N, K, N > 256 ? 128 : N) || !make_map(&tm_d, D, N, M, N, 128)) return -3;
-    if (act >= kDRelu) { if (!make_map(&tm_aux, aux, ld_aux, M, N, 128)) return -3; }
+    if (!make_tensor_map(&tm_a, A, lda, M, K, 128) || !make_tensor_map(&tm_w, W, K, N, K, N > 256 ? 128 : N) ||
+        !make_tensor_map(&tm_d, D, N, M, N, 128))
+        return -3;
+    if (act >= kDRelu) { if (!make_tensor_map(&tm_aux, aux, ld_aux, M, N, 128)) return -3; }
     else tm_aux = tm_d;
-    if (act == kAddLN) { if (!make_map(&tm_d2, xhat, N, M, N, 128)) return -3; }
+    if (act == kAddLN) { if (!make_tensor_map(&tm_d2, xhat, N, M, N, 128)) return -3; }
     else tm_d2 = tm_d;
     DenseArgs g;
     g.M = M; g.N = N; g.K = K; g.act = act; g.ring = ring_depth(act, K); g.bias = bias;
@@ -393,6 +378,34 @@ int launch(const void *A, int64_t lda, const void *W, const float *bias, const v
 }
 
 }  // namespace
+
+namespace {
+typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
+                                  const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+EncodeTiledFn encoder() {   // looked up on the first call
+    static const EncodeTiledFn fn = [] {
+        void *f = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        const bool ok = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) == cudaSuccess &&
+                        q == cudaDriverEntryPointSuccess;
+        return ok ? reinterpret_cast<EncodeTiledFn>(f) : nullptr;
+    }();
+    return fn;
+}
+}  // namespace
+
+bool tensor_maps_available() { return encoder() != nullptr; }
+
+bool make_tensor_map(CUtensorMap *m, const void *base, int64_t ld, int64_t rows, int cols, int box_rows) {
+    const EncodeTiledFn encode = encoder();
+    if (!encode) return false;
+    const cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
+    const cuuint64_t gstride[1] = {(cuuint64_t)ld * 2};
+    const cuuint32_t box[2] = {64, (cuuint32_t)box_rows}, estr[2] = {1, 1};
+    return encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(base), gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                  CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
 
 int gemm_bias_act(const void *A, int64_t lda, const void *W, const float *bias, void *D, int M, int N, int K, int relu,
                   cudaStream_t stream) {

@@ -12,28 +12,61 @@
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
+#include "philox.cuh"
 #include "policy_handle.cuh"
 #include "policy_kernels.cuh"
 #include "policy_weights.cuh"
+#include "tcgen05_util.cuh"
 
 namespace {
 using namespace uavp;
 
 // ------------------------------------------------------------------------------------------------ kernels
 
-__device__ __forceinline__ uint4 philox4x32(uint32_t k0, uint32_t k1, uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3) {
-#pragma unroll
-    for (int r = 0; r < 10; ++r) {
-        const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-        const uint32_t n0 = hi1 ^ c1 ^ k0, n2 = hi0 ^ c3 ^ k1;
-        c0 = n0; c1 = lo1; c2 = n2; c3 = lo0;
-        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
-    }
-    return make_uint4(c0, c1, c2, c3);
+// Weight packing (uavpolicy_set_weights): bf16 operands in the UMMA canonical K-major order the fused kernels stage
+// with one bulk TMA copy each (tc::canon_off is in bytes, hence / 2 for an element offset).
+
+// [128 x 14] fp32 embedding weight -> [128 x 32] bf16, canonical order, the 14 columns duplicated at 0.. and 16..
+// columns 14 / 15: the embedding bias as bf16 + rounding remainder (the A operand carries ones in these two columns)
+__global__ void emb_w2_kernel(const float *__restrict__ w, const float *__restrict__ b, __nv_bfloat16 *__restrict__ out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= D * 32) return;
+    const int d = i / 32, c = i % 32, j = c % 16;
+    float v = j < F ? w[d * F + j] : 0.0f;
+    if (c == 14) v = b[d];
+    if (c == 15) v = b[d] - __bfloat162float(__float2bfloat16(b[d]));
+    out[tc::canon_off(d, c, 32) / 2] = __float2bfloat16(v);
 }
 
-// head outputs: logits and value (head_out), then softmax, Categorical sample (counter RNG), log-prob, entropy
+// bias [N] fp32 -> [N x 16] bf16 B-operand in canonical order: column 0 = bf16(b), column 1 = b - bf16(b), rest zero
+__global__ void pack_bias_kernel(const float *__restrict__ b, __nv_bfloat16 *__restrict__ out, int N) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N * 16) return;
+    const int n = i / 16, c = i % 16;
+    const float hi = __bfloat162float(__float2bfloat16(b[n]));
+    out[tc::canon_off(n, c, 16) / 2] = __float2bfloat16(c == 0 ? hi : (c == 1 ? b[n] - hi : 0.0f));
+}
+
+// row-major fp32 [N x K] -> bf16 in canonical order (one bulk TMA copy then stages a whole B operand)
+__global__ void pack_canon_kernel(const float *__restrict__ w, __nv_bfloat16 *__restrict__ out, int N, int K) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N * K) return;
+    out[tc::canon_off(i / K, i % K, K) / 2] = __float2bfloat16(w[i]);
+}
+
+// log-softmax of the two logits and the Categorical sample (transformer_net.py:116-120) of env `env` at `step`: u is the
+// top 24 bits of one Philox block keyed by the seed (k0, k1).  heads_out_kernel and actor_out_kernel both draw here, so
+// a sample of uavpolicy_act is bit-identical to uavpolicy_get_action's for the same keys.
+__device__ __forceinline__ int draw_action(float l0, float l1, uint32_t k0, uint32_t k1, uint64_t step, uint64_t env, float &lp0,
+                                           float &lp1) {
+    const float m = fmaxf(l0, l1), e0 = expf(l0 - m), e1 = expf(l1 - m), lse = m + logf(e0 + e1);
+    lp0 = l0 - lse; lp1 = l1 - lse;
+    const uint4 r = philox4x32(k0, k1, (uint32_t)env, (uint32_t)step, (uint32_t)(step >> 32), 0x00B01C70u ^ (uint32_t)(env >> 32));
+    const float u = (float)(r.x >> 8) * (1.0f / 16777216.0f);   // uniform [0,1)
+    return u < expf(lp1) ? 1 : 0;                               // Categorical(probs).sample()
+}
+
+// head outputs: logits and value (head_out), then the sample (draw_action), log-prob and entropy
 // (transformer_net.py:116-122).  One thread per sample.
 __global__ void __launch_bounds__(256) heads_out_kernel(const __nv_bfloat16 *__restrict__ Ha, const __nv_bfloat16 *__restrict__ Hc,
                                                         HeadW ha, HeadW hc, int B, uint32_t k0, uint32_t k1, uint64_t step,
@@ -41,43 +74,28 @@ __global__ void __launch_bounds__(256) heads_out_kernel(const __nv_bfloat16 *__r
                                                         float *__restrict__ logp, float *__restrict__ value,
                                                         float *__restrict__ entropy, float *__restrict__ logits_out) {
     int b;
-    float l0, l1, vv;
+    float l0, l1, vv, lp0, lp1;
     if (!head_out<true>(Ha, Hc, ha.w2, ha.b2, hc.w2, hc.b2, B, b, l0, l1, vv)) return;
-    const float m = fmaxf(l0, l1), e0 = expf(l0 - m), e1 = expf(l1 - m), lse = m + logf(e0 + e1);
-    const float lp0 = l0 - lse, lp1 = l1 - lse, p0 = expf(lp0), p1 = expf(lp1);
-    const uint64_t env = env_base + (uint64_t)b;
-    const uint4 r = philox4x32(k0, k1, (uint32_t)env, (uint32_t)step, (uint32_t)(step >> 32), 0x00B01C70u ^ (uint32_t)(env >> 32));
-    const float u = (float)(r.x >> 8) * (1.0f / 16777216.0f);   // uniform [0,1)
-    const int a = u < p1 ? 1 : 0;                               // Categorical(probs).sample(), :118-120
+    const int a = draw_action(l0, l1, k0, k1, step, env_base + (uint64_t)b, lp0, lp1);
+    const float p0 = expf(lp0), p1 = expf(lp1);
     action[b] = a;
     if (logp) logp[b] = a ? lp1 : lp0;
     if (value) value[b] = vv;
-    if (entropy) entropy[b] = -(p0 * lp0 + p1 * lp1);
+    if (entropy) entropy[b] = -fmaf(p0, lp0, p1 * lp1);          // contraction written out: it fixes the rounding
     if (logits_out) { logits_out[2 * b] = l0; logits_out[2 * b + 1] = l1; }
 }
 
-// uavpolicy_act: the actor half of heads_out_kernel.  The logits, the softmax and the draw are formed by the same operations
-// in the same order, so a sample (greedy = 0) is bit-identical to heads_out_kernel's for the same keys.  greedy = 1 takes
-// argmax, a tie going to action 0 (torch.argmax).  The critic's head-hidden rows are stale in this mode and are not read.
+// uavpolicy_act: the actor half of heads_out_kernel.  greedy = 1 takes argmax, a tie going to action 0 (torch.argmax).
+// The critic's head-hidden rows are stale in this mode and are not read.
 __global__ void __launch_bounds__(256) actor_out_kernel(const __nv_bfloat16 *__restrict__ Ha, HeadW ha, int B, int greedy,
                                                         uint32_t k0, uint32_t k1, uint64_t step, uint64_t env_base,
                                                         int64_t *__restrict__ action, float *__restrict__ logp,
                                                         float *__restrict__ logits_out) {
     int b;
-    float l0, l1, unused;
+    float l0, l1, unused, lp0, lp1;
     if (!head_out<false>(Ha, nullptr, ha.w2, ha.b2, nullptr, nullptr, B, b, l0, l1, unused)) return;
-    const float m = fmaxf(l0, l1), e0 = expf(l0 - m), e1 = expf(l1 - m), lse = m + logf(e0 + e1);
-    const float lp0 = l0 - lse, lp1 = l1 - lse;
-    int a;
-    if (greedy) {
-        a = l1 > l0 ? 1 : 0;
-    } else {
-        const float p1 = expf(lp1);
-        const uint64_t env = env_base + (uint64_t)b;
-        const uint4 r = philox4x32(k0, k1, (uint32_t)env, (uint32_t)step, (uint32_t)(step >> 32), 0x00B01C70u ^ (uint32_t)(env >> 32));
-        const float u = (float)(r.x >> 8) * (1.0f / 16777216.0f);
-        a = u < p1 ? 1 : 0;
-    }
+    int a = draw_action(l0, l1, k0, k1, step, env_base + (uint64_t)b, lp0, lp1);
+    if (greedy) a = l1 > l0 ? 1 : 0;
     action[b] = a;
     if (logp) logp[b] = a ? lp1 : lp0;
     if (logits_out) { logits_out[2 * b] = l0; logits_out[2 * b + 1] = l1; }

@@ -5,6 +5,7 @@
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 
+#include "policy_kernels.cuh"
 #include "policy_weights.cuh"
 #include "tcgen05_util.cuh"
 
@@ -64,23 +65,6 @@ __device__ __forceinline__ void bulk_load2(void *s0, const void *g0, uint32_t b0
     mbar_expect_tx(mbar, b0 + b1);
     bulk_copy(s0, g0, b0, mbar);
     bulk_copy(s1, g1, b1, mbar);
-}
-
-__device__ __forceinline__ void unpack8(const uint4 &q, float *o) {   // bf16 -> fp32 is a 16-bit shift
-    const uint32_t w[4] = {q.x, q.y, q.z, q.w};
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        o[2 * i] = __uint_as_float(w[i] << 16); o[2 * i + 1] = __uint_as_float(w[i] & 0xffff0000u);
-    }
-}
-__device__ __forceinline__ uint4 pack8(const float *v) {
-    uint32_t w[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const __nv_bfloat162 t = __floats2bfloat162_rn(v[2 * i], v[2 * i + 1]);
-        w[i] = *reinterpret_cast<const uint32_t *>(&t);
-    }
-    return make_uint4(w[0], w[1], w[2], w[3]);
 }
 
 // Epilogues run on all 16 warps: warp w reads TMEM lanes 32*(w%4).. (its rows) and the column quarter w/4.

@@ -2,6 +2,7 @@
 // accumulation on tcgen05 - the hand-written persistent TMA / TMEM kernel of policy_dense.cu.
 #pragma once
 #include <cstdint>
+#include <cuda.h>
 #include <cuda_runtime.h>
 
 namespace uavp {
@@ -17,4 +18,10 @@ int gemm_drelu(const void *A, int64_t lda, const void *W, const void *aux, int64
 // normalised rows xhat (bf16 [M,128]) and rstd (fp32 [M]).  X: bf16 with row stride ldx (the residual stream).
 int gemm_add_ln(const void *A, int64_t lda, const void *W, const float *bias, const void *X, int64_t ldx, const float *gamma,
                 const float *beta, void *out, void *xhat, float *rstd, int M, int K, cudaStream_t stream);
+
+// TMA tensor maps of the dense and the weight-gradient kernels, built with the driver's cuTensorMapEncodeTiled (looked up
+// once).  tensor_maps_available: the driver provides it.  make_tensor_map: row-major bf16 [rows, cols] with row stride ld
+// (elements) as a 2-D map of [box_rows x 64] boxes with 128 B swizzle; false when the encoder is missing or rejects it.
+bool tensor_maps_available();
+bool make_tensor_map(CUtensorMap *m, const void *base, int64_t ld, int64_t rows, int cols, int box_rows);
 }  // namespace uavp

@@ -32,24 +32,240 @@ int wgrad(const __nv_bfloat16 *dY, int64_t ld_dy, const __nv_bfloat16 *X, int64_
 namespace {
 using bf16 = __nv_bfloat16;
 
-__device__ __forceinline__ float warp_sum(float v) {
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
+// ---------------------------------------------------------------------------------------------- forward kernels
+
+// embedding of both nets: E = relu(obs W^T + b) + pos (transformer_net.py:24-30,57-59) and the key-padding mask
+// (rows that are all zero, newest row never: :52-54).  One CTA = 64 tokens; thread = (net, feature pair), so a warp
+// stores 128 contiguous bytes per token.
+constexpr int kEmbTok = 60;                                   // whole windows per CTA: token i sits at position i % 5
+// packed fp32x2 arithmetic (FFMA2): both features of a thread advance with one instruction per observation column
+__device__ __forceinline__ uint64_t pack_f32x2(float lo, float hi) {
+    uint64_t r;
+    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
+    return r;
+}
+__device__ __forceinline__ void unpack_f32x2(uint64_t v, float &lo, float &hi) { asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v)); }
+__device__ __forceinline__ uint64_t fma_f32x2(uint64_t a, uint64_t b, uint64_t c) {
+    uint64_t d;
+    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
+    return d;
+}
+constexpr int kEmbThreads = 64;                               // warp 0: actor, warp 1: critic; lane = 4 features
+__global__ void __launch_bounds__(kEmbThreads) embed_kernel(const float *__restrict__ obs, int R, BlockW a, BlockW c,
+                                                            __nv_bfloat16 *__restrict__ Ea, __nv_bfloat16 *__restrict__ Ec,
+                                                            uint8_t *__restrict__ pad, __nv_bfloat16 *__restrict__ obs16 = nullptr,
+                                                            uint32_t *__restrict__ relu_mask = nullptr) {
+    // obs16 / relu_mask (training only): a bf16 copy of the observation rows zero-padded to 64 columns (the B operand of
+    // the embedding's weight-gradient product) and the ReLU activity bits of both networks, [R][net][4 words]:
+    // word k, bit l  <->  feature 4 l + k
+    // (the update always passes both; without the null checks below nvcc schedules this kernel about 11 us slower per
+    // 131072-window minibatch on a B200, measured)
+    __shared__ __align__(16) float2 s_obs[kEmbTok][F];            // every value twice: the (x, x) operand of the packed FMA
+    const int t0 = blockIdx.x * kEmbTok;
+    {   // the CTA's 60 x 14 floats are contiguous and 16-byte aligned: all loads of a thread go out before any is used
+        constexpr int kVec = kEmbTok * F / 4, kPer = (kVec + kEmbThreads - 1) / kEmbThreads;
+        const float4 *src = reinterpret_cast<const float4 *>(obs + (size_t)t0 * F);
+        const int nvec = min(kVec, (int)(((size_t)(R - t0) * F) / 4));        // R % 5 == 0 and 5 * 14 % 4 != 0: see tail below
+        float4 v[kPer];
+#pragma unroll
+        for (int k = 0; k < kPer; ++k) {
+            const int i = threadIdx.x + k * kEmbThreads;
+            v[k] = i < nvec ? src[i] : make_float4(0.f, 0.f, 0.f, 0.f);
+        }
+#pragma unroll
+        for (int k = 0; k < kPer; ++k) {
+            const int i = threadIdx.x + k * kEmbThreads;
+            if (i < kVec) {
+                float2 *dst = &s_obs[0][0] + i * 4;
+                dst[0] = make_float2(v[k].x, v[k].x); dst[1] = make_float2(v[k].y, v[k].y);
+                dst[2] = make_float2(v[k].z, v[k].z); dst[3] = make_float2(v[k].w, v[k].w);
+            }
+        }
+        const int done = nvec * 4, total = min(kEmbTok, R - t0) * F;          // at most 3 trailing floats of the last CTA
+        for (int i = done + threadIdx.x; i < total; i += kEmbThreads) { const float x = obs[(size_t)t0 * F + i]; (&s_obs[0][0])[i] = make_float2(x, x); }
+    }
+    __syncthreads();
+    if (threadIdx.x < kEmbTok && t0 + threadIdx.x < R) {
+        float sum = 0.0f;
+        for (int j = 0; j < F; ++j) sum += fabsf(s_obs[threadIdx.x][j].x);
+        pad[t0 + threadIdx.x] = (sum == 0.0f && (t0 + threadIdx.x) % S != S - 1) ? 1 : 0;
+    }
+    if (obs16) {
+        for (int i = threadIdx.x; i < kEmbTok * 32; i += kEmbThreads) {
+            const int tok = i >> 5, c2 = (i & 31) * 2;
+            if (t0 + tok < R)
+                *reinterpret_cast<__nv_bfloat162 *>(obs16 + (size_t)(t0 + tok) * 64 + c2) =
+                    __floats2bfloat162_rn(c2 < F ? s_obs[tok][c2].x : 0.0f, c2 + 1 < F ? s_obs[tok][c2 + 1].x : 0.0f);
+        }
+    }
+    const bool critic = threadIdx.x >= 32;
+    const int d = (threadIdx.x & 31) * 4;                          // features d .. d+3
+    const BlockW &w = critic ? c : a;
+    __nv_bfloat16 *E = critic ? Ec : Ea;
+    uint64_t wa[F], wb[F];                                         // (w[d], w[d+1]) and (w[d+2], w[d+3]) per observation column
+#pragma unroll
+    for (int j = 0; j < F; ++j) {
+        wa[j] = pack_f32x2(w.emb_w[d * F + j], w.emb_w[(d + 1) * F + j]);
+        wb[j] = pack_f32x2(w.emb_w[(d + 2) * F + j], w.emb_w[(d + 3) * F + j]);
+    }
+    const uint64_t ba = pack_f32x2(w.emb_b[d], w.emb_b[d + 1]), bb = pack_f32x2(w.emb_b[d + 2], w.emb_b[d + 3]);
+    float pos[S][4];
+#pragma unroll
+    for (int p = 0; p < S; ++p)
+#pragma unroll
+        for (int k = 0; k < 4; ++k) pos[p][k] = w.pos[p * D + d + k];
+    uint32_t *const mask_dst = relu_mask ? relu_mask + (critic ? 4 : 0) : nullptr;
+    for (int win = 0; win < kEmbTok / S; ++win) {                 // R is a multiple of 5: windows are never split
+        if (t0 + win * S >= R) break;
+#pragma unroll
+        for (int p = 0; p < S; ++p) {                              // p = position of the token in its window (static)
+            const int i = win * S + p, t = t0 + i;
+            uint64_t xa = ba, xb = bb;
+#pragma unroll
+            for (int j = 0; j < F; ++j) {
+                const uint64_t oo = *reinterpret_cast<const uint64_t *>(&s_obs[i][j]);     // (o_j, o_j)
+                xa = fma_f32x2(wa[j], oo, xa);
+                xb = fma_f32x2(wb[j], oo, xb);
+            }
+            float x[4];
+            unpack_f32x2(xa, x[0], x[1]);
+            unpack_f32x2(xb, x[2], x[3]);
+            if (mask_dst) {
+                unsigned m[4];
+#pragma unroll
+                for (int k = 0; k < 4; ++k) m[k] = __ballot_sync(0xffffffffu, x[k] > 0.0f);
+                if ((threadIdx.x & 31) == 0) *reinterpret_cast<uint4 *>(mask_dst + (size_t)t * 8) = make_uint4(m[0], m[1], m[2], m[3]);
+            }
+            const __nv_bfloat162 e0 = __floats2bfloat162_rn(fmaxf(x[0], 0.0f) + pos[p][0], fmaxf(x[1], 0.0f) + pos[p][1]);
+            const __nv_bfloat162 e1 = __floats2bfloat162_rn(fmaxf(x[2], 0.0f) + pos[p][2], fmaxf(x[3], 0.0f) + pos[p][3]);
+            uint2 ev;
+            ev.x = *reinterpret_cast<const uint32_t *>(&e0); ev.y = *reinterpret_cast<const uint32_t *>(&e1);
+            *reinterpret_cast<uint2 *>(E + (size_t)t * D + d) = ev;
+        }
+    }
 }
 
-// ---------------------------------------------------------------------------------------------- forward extras
+// ---- attention of an inner encoder layer (all five queries), warp = sample --------------------------------------------
+// Lane l owns 4 of the 128 feature dimensions: head h = l / 4, dimensions h*16 + (l % 4)*4 ..+4.  A token row of Q, K, V
+// or of the output is then ONE fully coalesced 256-byte warp access (8 B per lane), every element of Q / K / V is loaded
+// exactly once per sample, and the 5 x 5 score block of a head is a folded reduction: each lane forms its 4-dimension
+// partial of all 25 dot products, two xor-shuffles (lanes l^1, l^2) complete them inside the head's 4 lanes.
+// (The first version had a thread per (sample, head, query) holding 16-dimension vectors: every K / V row was re-loaded
+// five times and the register footprint capped the occupancy - 0.37-0.69 of the traffic floor.)
+struct Rows4 { uint2 t[S]; };                     // 5 token rows x this lane's 4 bf16 features, packed
+// block[i][j] = a_i . b_j over the head's 16 dimensions (every lane of the head ends with all 25 values)
+__device__ __forceinline__ void head_dots(const Rows4 &A, const Rows4 &Bm, float (*blk)[S]) {
+    float bf[S][4];
+#pragma unroll
+    for (int j = 0; j < S; ++j) unpack4f(Bm.t[j], bf[j]);
+#pragma unroll
+    for (int i = 0; i < S; ++i) {
+        float af[4];
+        unpack4f(A.t[i], af);
+#pragma unroll
+        for (int j = 0; j < S; ++j)
+            blk[i][j] = xor_sum<1, 2>(fmaf(af[0], bf[j][0], fmaf(af[1], bf[j][1], fmaf(af[2], bf[j][2], af[3] * bf[j][3]))));
+    }
+}
+// softmax over the keys of every query row, scores scaled by 1/sqrt(16), padded keys masked (transformer_net.py:52-54,63)
+__device__ __forceinline__ void head_softmax(float (*p)[S], const uint8_t *pad) {
+    bool pd[S];
+#pragma unroll
+    for (int j = 0; j < S; ++j) pd[j] = pad[j] != 0;
+#pragma unroll
+    for (int i = 0; i < S; ++i) {
+        float mx = -INFINITY, den = 0.0f;
+#pragma unroll
+        for (int j = 0; j < S; ++j) { p[i][j] = pd[j] ? -INFINITY : p[i][j] * 0.25f; mx = fmaxf(mx, p[i][j]); }
+#pragma unroll
+        for (int j = 0; j < S; ++j) { p[i][j] = __expf(p[i][j] - mx); den += p[i][j]; }
+        const float inv = 1.0f / den;
+#pragma unroll
+        for (int j = 0; j < S; ++j) p[i][j] *= inv;
+    }
+}
 
-__device__ __forceinline__ void unpack8(uint4 v, float *o) {
-    unpack4f(make_uint2(v.x, v.y), o);
-    unpack4f(make_uint2(v.z, v.w), o + 4);
+// QKV [R,384] -> ATT [R,128]
+__global__ void __launch_bounds__(256) attn_full_kernel(const __nv_bfloat16 *__restrict__ QKV, const uint8_t *__restrict__ pad, int B,
+                                                        __nv_bfloat16 *__restrict__ ATT) {
+    const int lane = threadIdx.x & 31;
+    const int nwarps = (gridDim.x * blockDim.x) >> 5;
+    for (int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; b < B; b += nwarps) {
+        const __nv_bfloat16 *base = QKV + (size_t)b * S * 3 * D + lane * 4;
+        Rows4 q, k, v;
+#pragma unroll
+        for (int t = 0; t < S; ++t) {
+            q.t[t] = *reinterpret_cast<const uint2 *>(base + (size_t)t * 3 * D);
+            k.t[t] = *reinterpret_cast<const uint2 *>(base + (size_t)t * 3 * D + D);
+            v.t[t] = *reinterpret_cast<const uint2 *>(base + (size_t)t * 3 * D + 2 * D);
+        }
+        float p[S][S];
+        head_dots(q, k, p);
+        head_softmax(p, pad + (size_t)b * S);
+        float vf[S][4];
+#pragma unroll
+        for (int j = 0; j < S; ++j) unpack4f(v.t[j], vf[j]);
+#pragma unroll
+        for (int i = 0; i < S; ++i) {
+            float o[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+#pragma unroll
+            for (int j = 0; j < S; ++j)
+#pragma unroll
+                for (int e = 0; e < 4; ++e) o[e] = fmaf(p[i][j], vf[j][e], o[e]);
+            *reinterpret_cast<uint2 *>(ATT + ((size_t)b * S + i) * D + lane * 4) = pack4f(o);
+        }
+    }
 }
-__device__ __forceinline__ uint4 pack8(const float *v) {
-    const uint2 a = pack4f(v), b = pack4f(v + 4);
-    return make_uint4(a.x, a.y, b.x, b.y);
+
+// ---- attention of the last encoder layer (newest query only), thread = (sample, head) ----------------------------------
+// normalised softmax(q k^T / sqrt(16), key padding mask) of one (sample, head) over its 5 keys (rows k0 + j * stride).
+// The backward (attn_row_grads) recomputes exactly these probabilities by calling this too.
+__device__ __forceinline__ void softmax_row(const float *q, const __nv_bfloat16 *k0, int64_t stride, const uint8_t *pad, float *p) {
+    float mx = -INFINITY;
+#pragma unroll
+    for (int j = 0; j < S; ++j) {
+        float kk[DH], s = 0.0f;
+        load16(k0 + j * stride, kk);
+#pragma unroll
+        for (int e = 0; e < DH; ++e) s = fmaf(q[e], kk[e], s);
+        p[j] = pad[j] ? -INFINITY : s * 0.25f;
+        mx = fmaxf(mx, p[j]);
+    }
+    float den = 0.0f;
+#pragma unroll
+    for (int j = 0; j < S; ++j) { p[j] = __expf(p[j] - mx); den += p[j]; }
+    const float inv = 1.0f / den;
+#pragma unroll
+    for (int j = 0; j < S; ++j) p[j] *= inv;
 }
-__device__ __forceinline__ float half_warp_sum(float v) {           // over the 16 lanes that share a row
-    for (int o = 8; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
+
+// softmax(q k^T / sqrt(16), key padding mask) v for one (sample, head, query): q, and 5 keys / values of 16 dims
+__device__ __forceinline__ void attend(const float *q, const __nv_bfloat16 *k0, const __nv_bfloat16 *v0, int64_t stride,
+                                       const uint8_t *pad, float *out) {
+    float p[S];
+    softmax_row(q, k0, stride, pad, p);
+#pragma unroll
+    for (int e = 0; e < DH; ++e) out[e] = 0.0f;
+#pragma unroll
+    for (int j = 0; j < S; ++j) {
+        float vv[DH];
+        load16(v0 + j * stride, vv);
+#pragma unroll
+        for (int e = 0; e < DH; ++e) out[e] = fmaf(p[j], vv[e], out[e]);
+    }
+}
+
+// Q [B,128], KV [R,256] -> ATT [B,128]
+__global__ void attn_last_kernel(const __nv_bfloat16 *__restrict__ Q, const __nv_bfloat16 *__restrict__ KV,
+                                 const uint8_t *__restrict__ pad, int B, __nv_bfloat16 *__restrict__ ATT) {
+    const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= B * H) return;
+    const int b = idx / H, h = idx % H;
+    float q[DH], o[DH];
+    load16(Q + (size_t)b * D + h * DH, q);
+    const __nv_bfloat16 *base = KV + (size_t)b * S * 2 * D + h * DH;
+    attend(q, base, base + D, 2 * D, pad + b * S, o);
+    store16(ATT + (size_t)b * D + h * DH, o);
 }
 
 // out = LayerNorm(x + y) * g + beta, keeping what the backward needs: the normalised row x^ (bf16) and 1/sigma.
@@ -69,11 +285,11 @@ __global__ void __launch_bounds__(256) add_ln_train_kernel(const bf16 *__restric
     float s = 0.0f;
 #pragma unroll
     for (int i = 0; i < 8; ++i) { v[i] = a[i] + b[i]; s += v[i]; }
-    const float mean = half_warp_sum(s) * (1.0f / D);
+    const float mean = xor_sum<8, 4, 2, 1>(s) * (1.0f / D);       // over the 16 lanes that share a row
     float q = 0.0f;
 #pragma unroll
     for (int i = 0; i < 8; ++i) { v[i] -= mean; q = fmaf(v[i], v[i], q); }
-    const float rstd = rsqrtf(half_warp_sum(q) * (1.0f / D) + 1e-5f);
+    const float rstd = rsqrtf(xor_sum<8, 4, 2, 1>(q) * (1.0f / D) + 1e-5f);
     if (!live) return;
     float o[8];
 #pragma unroll
@@ -183,23 +399,9 @@ struct AttnBwdArgs {
     int n;
 };
 
-// softmax row of one query over the 5 keys of (sample b, head h), and dS for that query
+// softmax row of one query over the 5 keys of (sample b, head h) (the forward's softmax_row), and dS for that query
 __device__ __forceinline__ void attn_row_grads(const AttnBwdArgs &a, int64_t b, int h, const float *q, const float *go, float *p, float *ds) {
-    const uint8_t *pad = a.pad + b * S;
-    float mx = -INFINITY;
-#pragma unroll
-    for (int j = 0; j < S; ++j) {
-        float kk[DH], s = 0.0f;
-        load16(a.k + (b * S + j) * a.kv_stride + h * DH, kk);
-#pragma unroll
-        for (int e = 0; e < DH; ++e) s = fmaf(q[e], kk[e], s);
-        p[j] = pad[j] ? -INFINITY : s * 0.25f;
-        mx = fmaxf(mx, p[j]);
-    }
-    float den = 0.0f;
-#pragma unroll
-    for (int j = 0; j < S; ++j) { p[j] = __expf(p[j] - mx); den += p[j]; }
-    const float inv = 1.0f / den;
+    softmax_row(q, a.k + b * S * a.kv_stride + h * DH, a.kv_stride, a.pad + b * S, p);
     float dot = 0.0f;
 #pragma unroll
     for (int j = 0; j < S; ++j) {
@@ -207,7 +409,6 @@ __device__ __forceinline__ void attn_row_grads(const AttnBwdArgs &a, int64_t b, 
         load16(a.v + (b * S + j) * a.kv_stride + h * DH, vv);
 #pragma unroll
         for (int e = 0; e < DH; ++e) s = fmaf(go[e], vv[e], s);
-        p[j] *= inv;
         ds[j] = s;
         dot = fmaf(p[j], s, dot);
     }
@@ -239,7 +440,7 @@ __global__ void __launch_bounds__(256) attn_bwd_last_kernel(const AttnBwdArgs a)
     store16(a.gq + b * a.q_stride + h * DH, dq);
 }
 
-// inner layer (five queries): warp = sample, lane = 4 feature dimensions of a head (policy_kernels.cuh: attn_full_kernel).
+// inner layer (five queries): warp = sample, lane = 4 feature dimensions of a head (as in attn_full_kernel above).
 // P is recomputed from Q, K; dP = dO V^T is a second folded 5 x 5 reduction; dS = P o (dP - rowsum(P o dP)) / 4; then
 // dQ = dS K, dK = dS^T Q, dV = P^T dO are plain 4-dimension FMAs per lane.  Every input row is loaded once (coalesced
 // 256 B per warp access) and every gradient row stored once.
@@ -314,8 +515,8 @@ __global__ void scatter_add_last_kernel(bf16 *__restrict__ dX, const bf16 *__res
     *reinterpret_cast<uint2 *>(dst) = pack4f(x);
 }
 
-// embedding backward: E = relu(obs W^T + b) + pos.  The forward left the ReLU activity bits (policy_kernels.cuh:
-// embed_kernel) and a bf16 copy of the observations padded to 64 columns, so what remains here is elementwise:
+// embedding backward: E = relu(obs W^T + b) + pos.  The forward left the ReLU activity bits (embed_kernel) and a bf16
+// copy of the observations padded to 64 columns, so what remains here is elementwise:
 // dPre = (g1 [+ g2]) masked -> bf16 rows, dpos = per-position column sums of the unmasked gradient (registers, lane = 4
 // features).  dW = dPre^T obs16 and db = dPre^T 1 then come from the tensor-core weight-gradient kernel (Kin = 64).
 __global__ void __launch_bounds__(256) embed_mask_kernel(const bf16 *__restrict__ g1, const bf16 *__restrict__ g2,
@@ -460,7 +661,7 @@ __global__ void __launch_bounds__(256) ppo_loss_sums_kernel(const PpoLossArgs a,
     }
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-        s[k] = warp_sum(s[k]);
+        s[k] = xor_sum<16, 8, 4, 2, 1>(s[k]);
         if ((threadIdx.x & 31) == 0) s_red[k][threadIdx.x >> 5] = s[k];
     }
     __syncthreads();

@@ -11,6 +11,7 @@
 
 #include <cuda.h>
 
+#include "policy_gemm.cuh"
 #include "policy_weights.cuh"
 #include "tcgen05_util.cuh"
 
@@ -134,30 +135,8 @@ __global__ void __launch_bounds__(kTmaThreads, 1) wgrad_tma_kernel(const __grid_
 
 }  // namespace
 
-namespace {
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                  const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn g_encode = nullptr;
-
-// row-major bf16 [rows, cols] with row stride ld (elements) as a 2-D tensor map with [64 x 64] boxes, 128 B swizzle
-bool make_map(CUtensorMap *m, const void *base, int64_t ld, int rows, int cols) {
-    const cuuint64_t gdim[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-    const cuuint64_t gstride[1] = {(cuuint64_t)ld * 2};
-    const cuuint32_t box[2] = {64, 64}, estr[2] = {1, 1};
-    return g_encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(base), gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                    CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-}  // namespace
-
 int wgrad_prepare() {
-    if (!g_encode) {
-        void *fn = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess || !fn)
-            return -1;
-        g_encode = reinterpret_cast<EncodeTiledFn>(fn);
-    }
+    if (!tensor_maps_available()) return -1;
     if (cudaFuncSetAttribute(wgrad_tma_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, WgTma<128>::kTotal) != cudaSuccess) return -1;
     if (cudaFuncSetAttribute(wgrad_tma_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, WgTma<256>::kTotal) != cudaSuccess) return -1;
     if (cudaFuncSetAttribute(wgrad_tma_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, WgTma<64>::kTotal) != cudaSuccess) return -1;
@@ -177,7 +156,7 @@ int wgrad(const __nv_bfloat16 *dY, int64_t ld_dy, const __nv_bfloat16 *X, int64_
     const int gy = Nout / 128, slabs = (rows + slab - 1) / slab;
     const int gx = max(1, min(slabs, num_sms / gy));
     CUtensorMap tm_dy, tm_x;
-    if (!g_encode || !make_map(&tm_dy, dY, ld_dy, rows, Nout) || !make_map(&tm_x, X, ld_x, rows, Kin)) return -3;
+    if (!make_tensor_map(&tm_dy, dY, ld_dy, rows, Nout, 64) || !make_tensor_map(&tm_x, X, ld_x, rows, Kin, 64)) return -3;
     if (Kin == 64) wgrad_tma_kernel<64><<<dim3(gx, gy), kTmaThreads, WgTma<64>::kTotal, stream>>>(tm_dy, tm_x, rows, dW, nout_valid, dbias, out_ld, kin_valid);
     else if (Kin == 128) wgrad_tma_kernel<128><<<dim3(gx, gy), kTmaThreads, WgTma<128>::kTotal, stream>>>(tm_dy, tm_x, rows, dW, nout_valid, dbias, out_ld, kin_valid);
     else wgrad_tma_kernel<256><<<dim3(gx, gy), kTmaThreads, WgTma<256>::kTotal, stream>>>(tm_dy, tm_x, rows, dW, nout_valid, dbias, out_ld, kin_valid);

@@ -12,7 +12,7 @@ import ctypes as C
 import torch
 
 from .. import _capi
-from .fused_forward import flatten_params
+from .fused_forward import _PolicyHandle, flatten_params
 
 
 class _TrunkFn(torch.autograd.Function):
@@ -68,30 +68,14 @@ class _PolicyFn(torch.autograd.Function):
         return None, None, grad
 
 
-class FusedTrunks:
+class FusedTrunks(_PolicyHandle):
+    _api = "uavtrain"
+
     def __init__(self, max_samples, device):
-        self._h = None
-        self.device = torch.device(device)
-        if self.device.type != "cuda":
-            raise RuntimeError("the fused PPO update runs on a CUDA device (sm_100a) only")
-        if self.device.index is None:
-            self.device = torch.device("cuda", torch.cuda.current_device())
-        self._lib = _capi.load_policy()
-        h = C.c_void_p()
-        rc = self._lib.uavtrain_create(self.device.index, int(max_samples), C.byref(h))
-        if rc != 0:
-            raise _capi.UavenvError(rc, (self._lib.uavtrain_last_error(None) or b"").decode())
-        self._h = h
+        super().__init__(max_samples, device, "the fused PPO update")
         self.max_samples = int(max_samples)
         self._pending = 0
         self._work = None
-
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-
-    def _chk(self, rc):
-        if rc != 0:
-            raise _capi.UavenvError(rc, (self._lib.uavtrain_last_error(self._h) or b"").decode())
 
     def features(self, module, obs):
         """[n,2,128] fp32: last-token features of actor_net / critic_net; differentiable w.r.t. module.parameters()."""
@@ -136,14 +120,3 @@ class FusedTrunks:
                                               C.c_void_p(dlogits), C.c_void_p(dvalue), p(stats_out) if stats_out is not None else None, s))
         self._chk(self._lib.uavtrain_backward_heads(self._h, C.c_void_p(dlogits), C.c_void_p(dvalue), p(grad_out), s))
         self._pending = 0
-
-    def close(self):
-        if getattr(self, "_h", None):
-            self._lib.uavtrain_destroy(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
