@@ -148,6 +148,13 @@ float *uavenv_obs_buffer(uavenv_t *h); /* device [B,5,14] owned by the handle */
  * in the reset(full_reset=False) state, episode 1; their first observation windows are written to
  * d_obs[B,5,14] (rows of the loaded envs only; NULL = the handle's own buffer).  Synchronous. */
 int uavenv_load_scene(uavenv_t *h, const uavenv_scene_t *scene, int32_t first_env, int32_t count, float *d_obs);
+/* the same from DEVICE arrays, with replication: d_scene holds num_scenes scenes as device structure-of-arrays (fields
+ * and layout of uavenv_scene_t, scene-major).  Scene s goes to envs first_env + s*copies + c, c in [0, copies), which are
+ * left as uavenv_load_scene leaves them (reset, episode 1); their first windows are written to d_obs (NULL = the handle's
+ * buffer).  Asynchronous on `stream`: the scene arrays must stay valid until the work enqueued there has run.  Returns
+ * UAVENV_EINVAL before the GPU is touched on a NULL required array, copies <= 0 or a range outside [0, B). */
+int uavenv_load_scene_device(uavenv_t *h, const uavenv_scene_t *d_scene, int32_t num_scenes, int32_t copies,
+                             int32_t first_env, float *d_obs, void *stream);
 /* replaces reading env.uavs / env.targets / ... (main.py:35-42, test_visualize.py:61-94). Synchronous. */
 int uavenv_get_scene(uavenv_t *h, uavenv_scene_t *scene, int32_t first_env, int32_t count);
 int uavenv_get_state(uavenv_t *h, uavenv_state_t *state, int32_t first_env, int32_t count);
@@ -179,6 +186,18 @@ int uavenv_random_actions(uavenv_t *h, uint64_t action_seed, uint64_t step, int6
  * restart the episode counter at 1: zero d_cache after them unless the next call is made before the next step.
  * d_actions: device int64 [B].  Call on the env's stream after a step and before the next one. */
 int uavenv_best_target_actions(uavenv_t *h, int64_t *d_cache, int64_t *d_actions, void *stream);
+
+/* Best-of-K read-out (a handle with auto_reset = 0, whose finished envs keep their final allocation).  For the groups
+ * g in [0, num_groups) of group_size consecutive envs starting at first_env: the member with the highest
+ * J = rev - omega * cost_sum (the value uavenv_get_state reports as J_val, bit for bit), the lowest member index winning a
+ * tie.  d_best[g] (int32, member index within the group), d_J_best[g] (its J), d_assigned_best[g*N + i] (its
+ * assigned_target_id row: Target.id, -1 = unassigned) and d_num_covered[g] (its covered-target count N0).  d_J_all
+ * [num_groups*group_size] (may be NULL) receives every member's J.  A group with a member that has not finished gets
+ * d_best = -1, d_J_best = NaN, d_num_covered = -1 and a row of -1.  All outputs are device arrays; one launch on
+ * `stream`, asynchronous.  UAVENV_EINVAL (before the GPU is touched) on a NULL output or a range outside [0, B);
+ * UAVENV_ESTATE on a handle with auto_reset = 1 or before any reset / scene load. */
+int uavenv_group_best(uavenv_t *h, int32_t first_env, int32_t num_groups, int32_t group_size, int32_t *d_best,
+                      double *d_J_best, int32_t *d_assigned_best, int32_t *d_num_covered, double *d_J_all, void *stream);
 
 /* ---- per-episode records of an evaluation (csrc/uavenv_episodes.cu) ---------------------------------------------
  * One finished episode.  ret sums the fp64 step rewards (info d_reward_f64) in step order; J_val, avg_p_dmg,

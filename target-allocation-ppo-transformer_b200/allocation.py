@@ -1,0 +1,152 @@
+"""Target allocation for given scenes with a trained policy: best-of-K sampled episodes per scene.
+
+    res = ub.allocate("runs/final_model.pth", scenes=my_scenes, samples=16)
+    res["assigned_target_id"]       # int32 [S, N]: Target.id each UAV of scene s is sent to in its best episode, -1 = none
+    res["J"], res["J_samples"]      # f64 [S] the best episode's J,  [S, K] every episode's J
+
+Each scene is played K times in K envs of one UAVEnvBatched built with auto_reset=False, so a finished episode keeps its
+final allocation on the device.  Per chunk of scenes: uavenv_load_scene_device puts every scene into its K envs (no host
+round trip), the loop act -> step runs until all of the chunk's envs are done (a poll every POLL_STEPS steps), and
+uavenv_group_best picks each scene's best episode and reads out its allocation.  Only the results cross to the host.
+
+Sampling: the actions of sample c of scene s are drawn with the key (seed, step, s*K + c) - the fused forward's
+env_id_base is set to each chunk's first sample id - so the result does not depend on how the scenes are chunked.
+"""
+import copy
+import time
+
+import torch
+
+from . import _capi
+from .configs.config import cfg as _global_cfg
+from .evaluation import DEFAULT_SEED, POLL_STEPS, _eval_setup, _stats, load_checkpoint
+
+
+def _scene_count(scenes, N):
+    if not hasattr(scenes, "get") or scenes.get("uav_x") is None:
+        raise ValueError("scenes must be a get_scene()-style dict of arrays (uav_x [S, N], ...)")
+    n = torch.as_tensor(scenes["uav_x"]).numel()
+    if n == 0 or n % N:
+        raise ValueError("scenes['uav_x'] has %d elements, not a positive multiple of NUM_UAVS = %d" % (n, N))
+    return n // N
+
+
+def allocate(policy, scenes=None, num_scenes=None, samples=1, greedy=None, seed=DEFAULT_SEED, config=None, device=None,
+             max_envs=65536):
+    """Allocate the targets of S scenes: play each scene `samples` (K) times with the policy and return the best
+    episode's allocation per scene.
+
+    policy: a TransformerActorCritic, its state_dict or a checkpoint path (see load_checkpoint), or "best_target" (the
+    best-target heuristic, deterministic: K must be 1).  scenes: a get_scene()-style dict of arrays [S, N] / [S, M] /
+    [S, K1] / [S, K2] (numpy or torch, host or device; list order, targets after the shuffle), or None with num_scenes:
+    the first-episode scenes of evaluate(..., seed=seed), scene s keyed (seed, global env id s).  greedy: argmax actions
+    (default when K == 1); otherwise actions sampled keyed (seed, step, s*K + c).  config: sizes and constants (default
+    the global cfg).  max_envs: the most envs played at once; scenes go through in chunks of max_envs // K.
+
+    Returns numpy arrays: "assigned_target_id" int32 [S, N], "J" f64 [S] (the value get_state reports as J_val),
+    "num_covered" int32 [S] (N0), "best_sample" int32 [S] (the first sample with the highest J), "J_samples" f64 [S, K];
+    and "summary": J mean / std / standard error over the scenes, mean J of all samples, K, scenes, env-steps (steps
+    times envs played), wall seconds, scenes/s and env-steps/s."""
+    K = int(samples)
+    if K <= 0:
+        raise ValueError("samples must be positive")
+    if greedy is None:
+        greedy = K == 1
+    if greedy and K > 1:
+        raise ValueError("greedy=True with samples > 1: every sample of a scene would be the same episode")
+    if isinstance(policy, str) and policy == "best_target" and K > 1:
+        raise ValueError("the best_target heuristic is deterministic: samples must be 1")
+    max_envs = int(max_envs)
+    if K > max_envs:
+        raise ValueError("samples (%d) > max_envs (%d): one scene's samples must fit one chunk" % (K, max_envs))
+    if (scenes is None) == (num_scenes is None):
+        raise ValueError("give exactly one of scenes and num_scenes")
+    N = int((config if config is not None else _global_cfg).NUM_UAVS)
+    S = _scene_count(scenes, N) if scenes is not None else int(num_scenes)
+    if S <= 0:
+        raise ValueError("num_scenes must be positive")
+    device, S, _, cfg, _, _ = _eval_setup(S, 1, config, device, 0)
+
+    from .envs.uav_env import UAVEnvBatched
+    from .networks.fused_forward import FusedPolicyForward
+    heuristic = isinstance(policy, str) and policy == "best_target"
+    net = None
+    if not heuristic:
+        net = load_checkpoint(policy, cfg)
+        if net is policy:                        # the caller's module stays where it is
+            net = copy.deepcopy(net)
+        net = net.to(device)
+    per = min(max_envs // K, S)                  # scenes per chunk
+    E = per * K
+    dev_scenes = None
+    if scenes is not None:                       # one move to the device; chunks are row slices of it
+        fields = {name for name, _, _ in _capi.SCENE_FIELDS}
+        dev_scenes = {k: torch.as_tensor(v).to(device).reshape(S, -1) for k, v in scenes.items()
+                      if k in fields and v is not None and torch.as_tensor(v).numel() > 0}
+    env = fused = None
+    parts = []
+    env_steps = 0
+    try:
+        torch.cuda.synchronize(device)
+        t0 = time.perf_counter()
+        env = UAVEnvBatched(E, device=device, seed=seed, config=cfg, auto_reset=False)
+        if heuristic:
+            def act(obs, step):
+                return env.best_target_actions()
+        else:
+            fused = FusedPolicyForward(E, device, seed=seed)
+            fused.sync(net)
+
+            def act(obs, step):
+                return fused.act(obs, step, greedy=greedy)[0]
+        limit = env.N * env.M                    # every step moves the (UAV, target) pointer: an episode ends within N * M
+        for c0 in range(0, S, per):
+            n = min(per, S - c0)
+            if dev_scenes is not None:
+                chunk = {k: v[c0:c0 + n] for k, v in dev_scenes.items()}
+            else:
+                chunk = _generated_scenes(n, c0, seed, cfg, device)
+            env.load_scene_device(chunk, copies=K, first_env=0)
+            obs = env.obs
+            if fused is not None:
+                fused.env_id_base = c0 * K       # the sample key (seed, step, global sample id)
+            done = env.done[:n * K]              # (envs past n*K hold finished episodes of the previous chunk: inert)
+            steps = 0
+            while steps < limit:
+                obs, _, _, _ = env.step(act(obs, steps))
+                steps += 1
+                if steps % POLL_STEPS == 0 and bool(done.all()):
+                    break
+            if not bool(done.all()):
+                raise RuntimeError("%d of %d envs did not finish their episode within %d steps" % (
+                    int((~done).sum()), n * K, limit))
+            env_steps += steps * E
+            parts.append(env.group_best(K, 0, n))
+        res = {k: torch.cat([p[k] for p in parts]).cpu().numpy() for k in parts[0]}
+        wall = time.perf_counter() - t0
+    finally:
+        if fused is not None:
+            fused.close()
+        if env is not None:
+            env.close()
+    out = {"assigned_target_id": res["assigned_target_id"], "J": res["J"], "num_covered": res["num_covered"],
+           "best_sample": res["best"], "J_samples": res["J_all"]}
+    s = {}
+    s["J_mean"], s["J_std"], s["J_sem"] = _stats(out["J"])
+    s["J_samples_mean"] = float(out["J_samples"].mean())
+    s["samples"], s["scenes"], s["env_steps"], s["wall_s"] = K, S, int(env_steps), float(wall)
+    s["scenes_per_s"], s["env_steps_per_s"] = S / wall, env_steps / wall
+    out["summary"] = s
+    return out
+
+
+def _generated_scenes(n, first, seed, cfg, device):
+    """The first-episode scenes of evaluate(..., seed) for global env ids [first, first + n): a full reset of envs keyed
+    (seed, global env id) (cfg carries RESET_EPISODES = 1, as evaluate's)."""
+    from .envs.uav_env import UAVEnvBatched
+    gen = UAVEnvBatched(n, device=device, seed=seed, config=cfg, auto_reset=False, env_id_base=first, with_info=False)
+    try:
+        gen.reset(full_reset=True)
+        return gen.get_scene()
+    finally:
+        gen.close()

@@ -302,16 +302,44 @@ static cudaError_t stage(std::vector<void *> &tmp, const T *host, size_t n, cons
     return cudaMemcpy(q, host, n * sizeof(T), cudaMemcpyHostToDevice);
 }
 
-extern "C" int uavenv_load_scene(uavenv_t *h, const uavenv_scene_t *sc, int32_t first_env, int32_t count,
-                                  float *d_obs) {
-    if (!h || !sc) return UAVENV_EINVAL;
-    if (first_env < 0 || count <= 0 || first_env + count > h->B)
-        return fail(h, UAVENV_EINVAL, "uavenv_load_scene: env range [%d,%d) outside [0,%d)", first_env, first_env + count, h->B);
+// the checks both scene loads make before touching the GPU
+static int check_scene_args(uavenv *h, const uavenv_scene_t *sc, int32_t num_scenes, int32_t copies, int32_t first_env,
+                            const char *what) {
+    if (num_scenes <= 0 || copies <= 0)
+        return fail(h, UAVENV_EINVAL, "%s: need num_scenes > 0 and copies > 0 (got %d, %d)", what, num_scenes, copies);
+    const int64_t end = (int64_t)first_env + (int64_t)num_scenes * copies;
+    if (first_env < 0 || end > h->B)
+        return fail(h, UAVENV_EINVAL, "%s: env range [%d,%lld) outside [0,%d)", what, first_env, (long long)end, h->B);
     const Params &P = h->P;
     if (!sc->uav_x || !sc->uav_y || !sc->uav_vx || !sc->uav_vy || !sc->uav_load || !sc->uav_cost || !sc->tgt_x ||
         !sc->tgt_y || !sc->tgt_vx || !sc->tgt_vy || !sc->tgt_value || !sc->tgt_id ||
         (P.K1 > 0 && (!sc->nfz_x || !sc->nfz_y)) || (P.K2 > 0 && (!sc->int_x || !sc->int_y || !sc->int_vx || !sc->int_vy)))
-        return fail(h, UAVENV_EINVAL, "uavenv_load_scene: a required scene array is NULL");
+        return fail(h, UAVENV_EINVAL, "%s: a required scene array is NULL", what);
+    return UAVENV_OK;
+}
+
+// the one packing path: device SoA of num_scenes scenes -> envs [first_env, first_env + num_scenes * copies), then the
+// reset of a loaded scene; enqueued on `stream`
+static int load_scene_impl(uavenv *h, const SceneSoA &s, int32_t num_scenes, int32_t copies, int32_t first_env,
+                           float *d_obs, cudaStream_t stream) {
+    const int count = num_scenes * copies;
+    const int grid = std::min((count + 3) / 4, 148 * 16);
+    pack_scene_kernel<<<grid, kResetThreads, 0, stream>>>(h->P, s, first_env, count, copies);
+    int rc = launch_check(h, "pack_scene_kernel");
+    if (rc != UAVENV_OK) return rc;
+    reset_kernel<<<grid, kResetThreads, h->reset_smem, stream>>>(h->P, 2, nullptr, first_env, count,
+                                                                 d_obs ? d_obs : h->obs_buf);
+    rc = launch_check(h, "reset_kernel");
+    if (rc == UAVENV_OK) h->ready = true;  // envs outside the range keep whatever they had (zeros until reset)
+    return rc;
+}
+
+extern "C" int uavenv_load_scene(uavenv_t *h, const uavenv_scene_t *sc, int32_t first_env, int32_t count,
+                                  float *d_obs) {
+    if (!h || !sc) return UAVENV_EINVAL;
+    int rc = check_scene_args(h, sc, count, 1, first_env, "uavenv_load_scene");
+    if (rc != UAVENV_OK) return rc;
+    const Params &P = h->P;
     CU_TRY(h, cudaSetDevice(h->device));
     std::vector<void *> tmp;
     SceneSoA s;
@@ -325,17 +353,55 @@ extern "C" int uavenv_load_scene(uavenv_t *h, const uavenv_scene_t *sc, int32_t 
     S(sc->tgt_value, m, &s.tgt_value); S(sc->tgt_id, m, &s.tgt_id);
     S(sc->nfz_x, k1, &s.nfz_x); S(sc->nfz_y, k1, &s.nfz_y); S(sc->nfz_radius, k1, &s.nfz_radius);
     S(sc->int_x, k2, &s.int_x); S(sc->int_y, k2, &s.int_y); S(sc->int_vx, k2, &s.int_vx); S(sc->int_vy, k2, &s.int_vy);
-    int rc = UAVENV_OK;
+    rc = UAVENV_OK;
     if (e == cudaSuccess) {
-        const int grid = std::min((count + 3) / 4, 148 * 16);
-        pack_scene_kernel<<<grid, kResetThreads>>>(P, s, first_env, count);
-        reset_kernel<<<grid, kResetThreads, h->reset_smem>>>(P, 2, nullptr, first_env, count, d_obs ? d_obs : h->obs_buf);
+        rc = load_scene_impl(h, s, count, 1, first_env, d_obs, nullptr);
         e = cudaDeviceSynchronize();
     }
     for (void *p : tmp) cudaFree(p);
-    if (e != cudaSuccess) rc = fail(h, UAVENV_ECUDA, "uavenv_load_scene: %s", cudaGetErrorString(e));
-    else h->ready = true;  // envs outside the range keep whatever they had (zeros until reset)
-    return rc;
+    if (rc != UAVENV_OK) return rc;
+    if (e != cudaSuccess) return fail(h, UAVENV_ECUDA, "uavenv_load_scene: %s", cudaGetErrorString(e));
+    return UAVENV_OK;
+}
+
+extern "C" int uavenv_load_scene_device(uavenv_t *h, const uavenv_scene_t *d_scene, int32_t num_scenes, int32_t copies,
+                                         int32_t first_env, float *d_obs, void *stream) {
+    if (!h || !d_scene) return UAVENV_EINVAL;
+    int rc = check_scene_args(h, d_scene, num_scenes, copies, first_env, "uavenv_load_scene_device");
+    if (rc != UAVENV_OK) return rc;
+    CU_TRY(h, cudaSetDevice(h->device));
+    const uavenv_scene_t &c = *d_scene;
+    SceneSoA s;
+    s.uav_x = c.uav_x; s.uav_y = c.uav_y; s.uav_vx = c.uav_vx; s.uav_vy = c.uav_vy; s.uav_load = c.uav_load;
+    s.uav_cost = c.uav_cost; s.uav_type = c.uav_type;
+    s.tgt_x = c.tgt_x; s.tgt_y = c.tgt_y; s.tgt_vx = c.tgt_vx; s.tgt_vy = c.tgt_vy; s.tgt_value = c.tgt_value;
+    s.tgt_id = c.tgt_id;
+    s.nfz_x = c.nfz_x; s.nfz_y = c.nfz_y; s.nfz_radius = c.nfz_radius;
+    s.int_x = c.int_x; s.int_y = c.int_y; s.int_vx = c.int_vx; s.int_vy = c.int_vy;
+    return load_scene_impl(h, s, num_scenes, copies, first_env, d_obs, (cudaStream_t)stream);
+}
+
+extern "C" int uavenv_group_best(uavenv_t *h, int32_t first_env, int32_t num_groups, int32_t group_size, int32_t *d_best,
+                                  double *d_J_best, int32_t *d_assigned_best, int32_t *d_num_covered, double *d_J_all,
+                                  void *stream) {
+    if (!h) return UAVENV_EINVAL;
+    if (!d_best || !d_J_best || !d_assigned_best || !d_num_covered)
+        return fail(h, UAVENV_EINVAL, "uavenv_group_best: best / J_best / assigned_best / num_covered must be non-NULL");
+    if (num_groups <= 0 || group_size <= 0)
+        return fail(h, UAVENV_EINVAL, "uavenv_group_best: need num_groups > 0 and group_size > 0 (got %d, %d)", num_groups,
+                    group_size);
+    const int64_t end = (int64_t)first_env + (int64_t)num_groups * group_size;
+    if (first_env < 0 || end > h->B)
+        return fail(h, UAVENV_EINVAL, "uavenv_group_best: env range [%d,%lld) outside [0,%d)", first_env, (long long)end, h->B);
+    if (h->P.auto_reset)
+        return fail(h, UAVENV_ESTATE, "uavenv_group_best: the handle restarts finished envs (auto_reset = 1); final "
+                    "allocations are kept with auto_reset = 0 only");
+    if (!h->ready) return fail(h, UAVENV_ESTATE, "uavenv_group_best before reset()/load_scene()");
+    CU_TRY(h, cudaSetDevice(h->device));
+    const int grid = (num_groups + 7) / 8;                               // a warp per group, 8 per CTA
+    group_best_kernel<<<grid, kGroupBestThreads, 0, (cudaStream_t)stream>>>(h->P, first_env, num_groups, group_size, d_best,
+                                                                           d_J_best, d_assigned_best, d_num_covered, d_J_all);
+    return launch_check(h, "group_best_kernel");
 }
 
 template <typename T>

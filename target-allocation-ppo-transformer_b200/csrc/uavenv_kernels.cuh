@@ -6,12 +6,15 @@
 //                        generation, uav_env.py:65-182) -> pair score + observation row of the new
 //                        pointer pair (mechanics.py:167-241) -> [B,5,14] window.
 //   reset_kernel         UAVEnv.reset for a masked subset (uav_env.py:42-63), one warp per env.
-//   pack_scene_kernel    scene injection (host SoA -> device records) + per-scene derived values.
+//   pack_scene_kernel    scene injection (device SoA -> records, each scene into `copies` consecutive envs) +
+//                        per-scene derived values.
 //   score_matrix_kernel  p_final / p_damage [B,N,M] (main.py:38-45 over mechanics.py:167-181).
 //   recompute_kernel     fresh J / N0 / sums from the per-target products, a warp per env with
 //                        shuffle reductions (uav_env.py:244-293) - drift bound for the running sums.
 //   best_target_kernel   the best-target heuristic's actions (evaluation baseline): a warp per 32 envs,
 //                        one cooperative row of pair scores when a UAV's row is entered.
+//   group_best_kernel    the best finished member of each group of consecutive envs (best-of-K allocation):
+//                        a warp per group, shuffle arg-max over J, coalesced copy of the winner's allocation.
 #pragma once
 
 #include "uavenv_device.cuh"
@@ -739,7 +742,8 @@ __global__ void __launch_bounds__(kResetThreads) reset_kernel(const __grid_const
 }
 
 // ------------------------------------------------------------------------------------------------
-// Scene injection: staged SoA (device copies of the host arrays, env-major) -> records.
+// Scene injection: device SoA (scene-major) -> records.  Env first_env + e of the range receives scene e / copies, so
+// every replica of a scene is packed from the same values by the same instructions: the copies are bit-identical.
 
 struct SceneSoA {
     const double *uav_x, *uav_y, *uav_vx, *uav_vy, *uav_load, *uav_cost;
@@ -750,10 +754,12 @@ struct SceneSoA {
 };
 
 __global__ void __launch_bounds__(kResetThreads) pack_scene_kernel(const __grid_constant__ Params P,
-                                                                    const SceneSoA s, int first_env, int count) {
+                                                                    const SceneSoA s, int first_env, int count,
+                                                                    int copies) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, wpb = blockDim.x >> 5;
-    for (int e = blockIdx.x * wpb + warp; e < count; e += gridDim.x * wpb) {
-        const int b = first_env + e;
+    for (int env = blockIdx.x * wpb + warp; env < count; env += gridDim.x * wpb) {
+        const int b = first_env + env;
+        const int e = env / copies;    // the scene
         const int slot = P.header(b).n(I_GEN) & 1;
         for (int i = lane; i < P.K1; i += 32) {
             NfzRec z; z.x = s.nfz_x[(size_t)e * P.K1 + i]; z.y = s.nfz_y[(size_t)e * P.K1 + i];
@@ -984,6 +990,52 @@ __global__ void __launch_bounds__(kBestTargetThreads) best_target_kernel(const _
     if (live) {
         if (stale) cache[b] = (int64_t)entry;
         actions[b] = (active && (uint32_t)(entry & 0xffffu) == (uint32_t)m) ? 1 : 0;
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Best member of each group of group_size consecutive envs (include/uavenv_b200.h, uavenv_group_best): one warp per group.
+// Lanes stride over the members (a warp's 32 loads of one header field hit one tile row), keep their first maximum of
+// J = rev - omega * cost_sum (the expression uavenv_get_state evaluates, so the bits agree under -fmad=false), and a
+// shuffle arg-max with the lower index winning a tie picks the group's member.  The warp then copies the winner's
+// assigned[] row along the UAV index.  A group with an unfinished member reports best = -1, J = NaN, N0 = -1 and a row
+// of -1.
+
+constexpr int kGroupBestThreads = 256;
+
+__global__ void __launch_bounds__(kGroupBestThreads) group_best_kernel(const __grid_constant__ Params P, int first_env,
+                                                                      int num_groups, int group_size, int32_t *best,
+                                                                      double *J_best, int32_t *assigned_best,
+                                                                      int32_t *num_covered, double *J_all) {
+    const int lane = threadIdx.x & 31;
+    const int g = (int)(((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+    if (g >= num_groups) return;                                            // (uniform per warp)
+    const int b0 = first_env + g * group_size;
+    double bJ = -INFINITY;
+    int bi = INT_MAX;
+    bool unfinished = false;
+    for (int i = lane; i < group_size; i += 32) {
+        const Hdr H = P.header(b0 + i);
+        const double J = H.f(F_REV) - (P.omega * H.f(F_COST_SUM));
+        if (J_all) J_all[(size_t)g * group_size + i] = J;
+        unfinished |= H.n(I_FINISHED) == 0;
+        if (bi == INT_MAX || J > bJ) { bJ = J; bi = i; }           // i ascends within a lane: the first maximum stays
+    }
+    for (int o = 16; o > 0; o >>= 1) {
+        const double oJ = __shfl_xor_sync(kFullMask, bJ, o);
+        const int oi = __shfl_xor_sync(kFullMask, bi, o);
+        if (oi != INT_MAX && (bi == INT_MAX || oJ > bJ || (oJ == bJ && oi < bi))) { bJ = oJ; bi = oi; }
+    }
+    unfinished = __any_sync(kFullMask, unfinished);
+    const Hdr W = P.header(b0 + bi);                                 // (member 0 always exists: bi is a member)
+    const int kptr = unfinished ? 0 : W.n(I_K);                      // slots at / past the pointer are stale
+    const int32_t *src = P.assigned + (size_t)(b0 + bi) * P.N;
+    int32_t *dst = assigned_best + (size_t)g * P.N;
+    for (int k = lane; k < P.N; k += 32) dst[k] = k < kptr ? src[k] : -1;
+    if (lane == 0) {
+        best[g] = unfinished ? -1 : bi;
+        J_best[g] = unfinished ? __longlong_as_double(0x7ff8000000000000ll) : bJ;
+        num_covered[g] = unfinished ? -1 : W.n(I_NCOVERED);
     }
 }
 

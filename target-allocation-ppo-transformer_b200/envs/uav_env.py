@@ -18,6 +18,7 @@ from ..configs.config import Config, cfg as _global_cfg
 from .entities import build_entities
 
 _NP = {"f8": np.float64, "i4": np.int32, "u1": np.uint8}
+_TORCH = {"f8": torch.float64, "i4": torch.int32}
 
 
 class _Discrete:           # stand-in for gym.spaces.Discrete (envs/uav_env.py:18); gym is not a dependency
@@ -222,10 +223,9 @@ class UAVEnvBatched:
     def _dims(self):
         return {"N": self.N, "M": self.M, "K1": self.K1, "K2": self.K2, "1": 1}
 
-    def load_scene(self, scene, first_env=0):
-        """Inject scenes (dict of arrays named as include/uavenv_b200.h:uavenv_scene, list order; one env
-        ([N]) or several ([count,N])) into envs [first_env, first_env+count); they are left reset
-        (episode 1).  Returns their first observation windows (a view of self.obs)."""
+    def _scene_struct(self, scene, array):
+        """(scene count, the arrays to keep alive, a UavenvScene of their addresses) of a scene dict named as
+        _capi.SCENE_FIELDS; array(value, kind) -> (contiguous array, element count, address)."""
         dims = self._dims()
         count = None
         keep, sc = [], _capi.UavenvScene()
@@ -234,22 +234,70 @@ class UAVEnvBatched:
                 if name in ("uav_type", "nfz_radius") or dims[dim] == 0:
                     continue
                 raise KeyError("scene is missing %r" % name)
-            a = np.ascontiguousarray(np.asarray(scene[name], dtype=_NP[kind]))
             if dims[dim] == 0:
                 continue
-            c = a.size // dims[dim]
-            if a.size != c * dims[dim] or c == 0:
-                raise ValueError("scene[%r] has %d elements, not a multiple of %d" % (name, a.size, dims[dim]))
+            a, n, ptr = array(scene[name], kind)
+            c = n // dims[dim]
+            if n != c * dims[dim] or c == 0:
+                raise ValueError("scene[%r] has %d elements, not a multiple of %d" % (name, n, dims[dim]))
             if count is None:
                 count = c
             elif c != count:
-                raise ValueError("scene arrays disagree on the number of envs")
+                raise ValueError("scene arrays disagree on the number of scenes")
             keep.append(a)
-            setattr(sc, name, a.ctypes.data)
+            setattr(sc, name, ptr)
+        return count, keep, sc
+
+    def load_scene(self, scene, first_env=0):
+        """Inject scenes (dict of arrays named as include/uavenv_b200.h:uavenv_scene, list order; one env
+        ([N]) or several ([count,N])) into envs [first_env, first_env+count); they are left reset
+        (episode 1).  Returns their first observation windows (a view of self.obs)."""
+        def host(v, kind):
+            a = np.ascontiguousarray(np.asarray(v, dtype=_NP[kind]))
+            return a, a.size, a.ctypes.data
+
+        count, keep, sc = self._scene_struct(scene, host)
         self._chk(self._lib.uavenv_load_scene(self._h, C.byref(sc), int(first_env), int(count),
                                               C.c_void_p(self.obs.data_ptr())))
         self._forget_best_targets()
         return self.obs[first_env:first_env + count]
+
+    def load_scene_device(self, scene, copies=1, first_env=0):
+        """Inject S scenes given as device tensors (dict named as _capi.SCENE_FIELDS, shapes [S,N] / [S,M] / [S,K1] /
+        [S,K2]; host tensors or numpy arrays are moved to the env's device first) into envs [first_env, first_env +
+        S*copies): scene s goes to envs first_env + s*copies + c, c in [0, copies), left reset (episode 1).  No host
+        round trip and no synchronisation: the packing runs on the env's stream.  Returns the loaded envs' first
+        observation windows (a view of self.obs)."""
+        def device(v, kind):
+            t = torch.as_tensor(v).to(device=self.device, dtype=_TORCH[kind]).contiguous()
+            return t, t.numel(), t.data_ptr()
+
+        # (a copy made here is freed in stream order when `keep` goes: the packing has read it by then)
+        count, keep, sc = self._scene_struct(scene, device)
+        self._chk(self._lib.uavenv_load_scene_device(self._h, C.byref(sc), int(count), int(copies), int(first_env),
+                                                     C.c_void_p(self.obs.data_ptr()), self._stream()))
+        self._forget_best_targets()
+        return self.obs[first_env:first_env + count * int(copies)]
+
+    def group_best(self, group_size, first_env=0, num_groups=None):
+        """The best member of each group of `group_size` consecutive envs from first_env (an env built with
+        auto_reset=False, after its episodes have finished): highest J (= get_state()["J_val"], bit for bit), lowest
+        member index on a tie.  Returns device tensors {"best": int32 [G] member index (-1: a member has not finished),
+        "J": f64 [G], "assigned_target_id": int32 [G,N] (Target.id, -1 = unassigned), "num_covered": int32 [G],
+        "J_all": f64 [G, group_size] every member's J}.  One launch on the env's stream."""
+        group_size = int(group_size)
+        if num_groups is None:
+            num_groups = (self.num_envs - int(first_env)) // max(group_size, 1)
+        G, dev = int(num_groups), self.device
+        out = {"best": torch.empty(G, dtype=torch.int32, device=dev), "J": torch.empty(G, dtype=torch.float64, device=dev),
+               "assigned_target_id": torch.empty(G, self.N, dtype=torch.int32, device=dev),
+               "num_covered": torch.empty(G, dtype=torch.int32, device=dev),
+               "J_all": torch.empty(G, group_size, dtype=torch.float64, device=dev)}
+        self._chk(self._lib.uavenv_group_best(self._h, int(first_env), G, group_size,
+                                              *(C.c_void_p(out[k].data_ptr()) for k in ("best", "J", "assigned_target_id",
+                                                                                        "num_covered", "J_all")),
+                                              self._stream()))
+        return out
 
     def get_scene(self, first_env=0, count=None):
         count = self.num_envs - first_env if count is None else count

@@ -109,15 +109,17 @@ def _world():
     return 0, 1
 
 
-def _summary(res, env_steps, wall):
-    def stats(x):
-        x = np.asarray(x, np.float64).reshape(-1)
-        std = float(x.std(ddof=1)) if x.size > 1 else 0.0
-        return float(x.mean()), std, std / np.sqrt(x.size)
+def _stats(x):
+    """(mean, sample std, standard error of the mean) of all values of x."""
+    x = np.asarray(x, np.float64).reshape(-1)
+    std = float(x.std(ddof=1)) if x.size > 1 else 0.0
+    return float(x.mean()), std, std / np.sqrt(x.size)
 
+
+def _summary(res, env_steps, wall):
     s = {}
     for key in ("return", "J", "coverage"):
-        s[key + "_mean"], s[key + "_std"], s[key + "_sem"] = stats(res[key])
+        s[key + "_mean"], s[key + "_std"], s[key + "_sem"] = _stats(res[key])
     s["valid_assign_rate"] = float(res["valid"].sum()) / max(int(res["assigns"].sum()), 1)
     s["length_mean"] = float(res["length"].mean())
     s["episodes"] = int(res["length"].size)
