@@ -20,6 +20,7 @@
 #ifndef UAVENV_B200_H
 #define UAVENV_B200_H
 
+#include <stddef.h>
 #include <stdint.h>
 
 #ifdef __cplusplus
@@ -198,6 +199,39 @@ int uavenv_best_target_actions(uavenv_t *h, int64_t *d_cache, int64_t *d_actions
  * UAVENV_ESTATE on a handle with auto_reset = 1 or before any reset / scene load. */
 int uavenv_group_best(uavenv_t *h, int32_t first_env, int32_t num_groups, int32_t group_size, int32_t *d_best,
                       double *d_J_best, int32_t *d_assigned_best, int32_t *d_num_covered, double *d_J_all, void *stream);
+
+/* Steepest-ascent local search on allocations of the scenes held by envs first_env + s*env_stride, s in [0, count).
+ * Row s of d_assigned_in [count*N] (group_best's layout: Target.id, -1 = none) is the start; the search maximises
+ *   J = sum_j value_j * (1 - prod_{k -> j} (1 - p[k][j])) - omega * sum_{k assigned} cost_k
+ * with p[k][j] = damage_prob(uav k, target j) * p_pen_k in fp64, list order (the bits of uavenv_score_matrix_f64's
+ * p_final).  t(k) is UAV k's target position (-1 = none), nh_j the product over the UAVs on j and nh_excl_k the product
+ * over the OTHER UAVs on t(k), each taken in ascending UAV index (never by dividing by 1 - p: p can be 1).  Candidates:
+ *   move (k, b), b in {-1} u [0, M), b != a = t(k):
+ *     gain = ([a>=0] v_a (nh_a - nh_excl_k) + [b>=0] (v_b nh_b) p[k][b]) + (omega c_k) ([a>=0] - [b>=0])
+ *   swap (k1 < k2), a1 = t(k1) != a2 = t(k2), either may be -1; k1 takes a2 and k2 takes a1:
+ *     gain = ([a1>=0] v_a1 (nh_a1 - nh_excl_k1 (1 - p[k2][a1])) + [a2>=0] v_a2 (nh_a2 - nh_excl_k2 (1 - p[k1][a2])))
+ *            + (omega (c_k1 - c_k2)) ([a1>=0] - [a2>=0])     (the cost term is 0 unless one side is -1)
+ * in that operation order.  Candidate order: moves before swaps, moves by ascending k then b from -1 up, swaps by
+ * (k1, k2) lexicographic; the first candidate with the largest gain wins an exact tie.  A round applies the winner iff its
+ * gain > 1e-12 * max(1, |J_run|), where J_run is J_in plus the gains applied so far; after a move the products of the
+ * touched targets and their UAVs are recomputed from scratch.  The search stops when no candidate qualifies
+ * (d_converged = 1: the row is a local optimum) or when a qualifying candidate is found after max_moves applied moves
+ * (d_converged = 0).  Outputs per s: d_assigned_out row (may be d_assigned_in), d_J_in (may be NULL) and d_J_out - J from
+ * scratch: products in ascending UAV index, targets summed in list order, then minus omega times the assigned UAVs'
+ * costs summed in UAV order -, d_num_covered (N0, distinct targets), d_moves (applied moves).  A row holding an id below
+ * -1 or one that is not a Target.id of its scene gets moves = -1, J_in = J_out = NaN, N0 = -1, converged = 0 and a row of
+ * -1; other rows are unaffected.  max_moves = 0 returns the input rows with their J.  d_workspace: device memory of
+ * uavenv_improve_workspace_bytes(h) bytes, not needed (may be NULL) when that is 0.  One launch on `stream`,
+ * asynchronous; results do not depend on count, env_stride or the launch.  UAVENV_EINVAL (before the GPU is touched) on
+ * a NULL required pointer or workspace, count <= 0, env_stride <= 0, max_moves < 0 or an env outside [0, B);
+ * UAVENV_ESTATE before any reset / scene load. */
+int uavenv_improve_allocation(uavenv_t *h, int32_t first_env, int32_t count, int32_t env_stride,
+                              const int32_t *d_assigned_in, int32_t max_moves, int32_t *d_assigned_out, double *d_J_in,
+                              double *d_J_out, int32_t *d_num_covered, int32_t *d_moves, uint8_t *d_converged,
+                              void *d_workspace, void *stream);
+/* bytes of the workspace uavenv_improve_allocation needs: 0 when p[N][M] fits the kernel's shared memory (N*M <= 8192),
+ * otherwise N*M*8 per SM of the handle's device (L2-resident slices). */
+size_t uavenv_improve_workspace_bytes(const uavenv_t *h);
 
 /* ---- per-episode records of an evaluation (csrc/uavenv_episodes.cu) ---------------------------------------------
  * One finished episode.  ret sums the fp64 step rewards (info d_reward_f64) in step order; J_val, avg_p_dmg,

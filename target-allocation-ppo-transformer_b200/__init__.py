@@ -30,9 +30,9 @@ def __getattr__(name):  # torch / CUDA are only touched when the env classes are
     if name in ("evaluate", "evaluate_baseline", "EpisodeRecorder", "load_checkpoint"):
         from . import evaluation
         return getattr(evaluation, name)
-    if name == "allocate":
-        from .allocation import allocate
-        return allocate
+    if name in ("allocate", "improve_allocation"):
+        from . import allocation
+        return getattr(allocation, name)
     if name in ("analyze_environment_difficulty", "record_decisions"):
         from . import diagnostics
         return getattr(diagnostics, name)

@@ -4,6 +4,9 @@
     res["assigned_target_id"]       # int32 [S, N]: Target.id each UAV of scene s is sent to in its best episode, -1 = none
     res["J"], res["J_samples"]      # f64 [S] the best episode's J,  [S, K] every episode's J
 
+    pol = ub.improve_allocation(my_scenes, res["assigned_target_id"])   # local search from any allocation
+    pol["assigned_target_id"], pol["J"], pol["J_before"]
+
 Each scene is played K times in K envs of one UAVEnvBatched built with auto_reset=False, so a finished episode keeps its
 final allocation on the device.  Per chunk of scenes: uavenv_load_scene_device puts every scene into its K envs (no host
 round trip), the loop act -> step runs until all of the chunk's envs are done (a poll every POLL_STEPS steps), and
@@ -11,6 +14,11 @@ uavenv_group_best picks each scene's best episode and reads out its allocation. 
 
 Sampling: the actions of sample c of scene s are drawn with the key (seed, step, s*K + c) - the fused forward's
 env_id_base is set to each chunk's first sample id - so the result does not depend on how the scenes are chunked.
+
+Local search (improve_allocation, allocate(improve=True)): uavenv_improve_allocation moves one UAV or swaps two while J
+rises (steepest ascent; the rule is in include/uavenv_b200.h), on the device, a scene per CTA.  allocate runs it on the
+first env of each scene's group right after group_best - every member holds the same scene - so no second scene load
+is needed.
 """
 import copy
 import time
@@ -31,8 +39,21 @@ def _scene_count(scenes, N):
     return n // N
 
 
+def _device_scenes(scenes, S, device):
+    """The scene arrays on the device as [S, ...] tensors (one move; chunks are row slices of them)."""
+    fields = {name for name, _, _ in _capi.SCENE_FIELDS}
+    return {k: torch.as_tensor(v).to(device).reshape(S, -1) for k, v in scenes.items()
+            if k in fields and v is not None and torch.as_tensor(v).numel() > 0}
+
+
+def _max_moves(max_moves):
+    if max_moves is not None and int(max_moves) < 0:
+        raise ValueError("max_moves must be >= 0 (or None: 16 * NUM_UAVS)")
+    return None if max_moves is None else int(max_moves)
+
+
 def allocate(policy, scenes=None, num_scenes=None, samples=1, greedy=None, seed=DEFAULT_SEED, config=None, device=None,
-             max_envs=65536):
+             max_envs=65536, improve=False):
     """Allocate the targets of S scenes: play each scene `samples` (K) times with the policy and return the best
     episode's allocation per scene.
 
@@ -42,11 +63,15 @@ def allocate(policy, scenes=None, num_scenes=None, samples=1, greedy=None, seed=
     the first-episode scenes of evaluate(..., seed=seed), scene s keyed (seed, global env id s).  greedy: argmax actions
     (default when K == 1); otherwise actions sampled keyed (seed, step, s*K + c).  config: sizes and constants (default
     the global cfg).  max_envs: the most envs played at once; scenes go through in chunks of max_envs // K.
+    improve: polish each scene's best allocation with the local search of improve_allocation (cap 16 * N moves).
 
     Returns numpy arrays: "assigned_target_id" int32 [S, N], "J" f64 [S] (the value get_state reports as J_val),
     "num_covered" int32 [S] (N0), "best_sample" int32 [S] (the first sample with the highest J), "J_samples" f64 [S, K];
     and "summary": J mean / std / standard error over the scenes, mean J of all samples, K, scenes, env-steps (steps
-    times envs played), wall seconds, scenes/s and env-steps/s."""
+    times envs played), wall seconds, scenes/s and env-steps/s.  With improve=True, "assigned_target_id", "J" and
+    "num_covered" are those of the improved allocation, and "J_before_improve" f64 [S] (the best episode's J), "moves"
+    int32 [S] and "converged" bool [S] (False: the move cap stopped the search) are added; "best_sample" and "J_samples"
+    stay those of the episodes."""
     K = int(samples)
     if K <= 0:
         raise ValueError("samples must be positive")
@@ -80,9 +105,7 @@ def allocate(policy, scenes=None, num_scenes=None, samples=1, greedy=None, seed=
     E = per * K
     dev_scenes = None
     if scenes is not None:                       # one move to the device; chunks are row slices of it
-        fields = {name for name, _, _ in _capi.SCENE_FIELDS}
-        dev_scenes = {k: torch.as_tensor(v).to(device).reshape(S, -1) for k, v in scenes.items()
-                      if k in fields and v is not None and torch.as_tensor(v).numel() > 0}
+        dev_scenes = _device_scenes(scenes, S, device)
     env = fused = None
     parts = []
     env_steps = 0
@@ -121,7 +144,13 @@ def allocate(policy, scenes=None, num_scenes=None, samples=1, greedy=None, seed=
                 raise RuntimeError("%d of %d envs did not finish their episode within %d steps" % (
                     int((~done).sum()), n * K, limit))
             env_steps += steps * E
-            parts.append(env.group_best(K, 0, n))
+            part = env.group_best(K, 0, n)
+            if improve:                          # on env g*K of each group: the scene, bit for bit, of every member
+                pol = env.improve_allocation(part["assigned_target_id"], first_env=0, env_stride=K)
+                part["J_before_improve"] = part["J"]
+                for k in ("assigned_target_id", "J", "num_covered", "moves", "converged"):
+                    part[k] = pol[k]
+            parts.append(part)
         res = {k: torch.cat([p[k] for p in parts]).cpu().numpy() for k in parts[0]}
         wall = time.perf_counter() - t0
     finally:
@@ -131,13 +160,72 @@ def allocate(policy, scenes=None, num_scenes=None, samples=1, greedy=None, seed=
             env.close()
     out = {"assigned_target_id": res["assigned_target_id"], "J": res["J"], "num_covered": res["num_covered"],
            "best_sample": res["best"], "J_samples": res["J_all"]}
+    if improve:
+        for k in ("J_before_improve", "moves", "converged"):
+            out[k] = res[k]
     s = {}
     s["J_mean"], s["J_std"], s["J_sem"] = _stats(out["J"])
     s["J_samples_mean"] = float(out["J_samples"].mean())
+    if improve:
+        s["J_before_improve_mean"] = float(out["J_before_improve"].mean())
+        s["moves_mean"] = float(out["moves"].mean())
     s["samples"], s["scenes"], s["env_steps"], s["wall_s"] = K, S, int(env_steps), float(wall)
     s["scenes_per_s"], s["env_steps_per_s"] = S / wall, env_steps / wall
     out["summary"] = s
     return out
+
+
+def improve_allocation(scenes, assigned_target_id, max_moves=None, config=None, device=None, max_envs=65536):
+    """Polish given allocations of S scenes to a local optimum of J: steepest ascent over single-UAV moves (to another
+    target or to none) and swaps of two UAVs' targets, one applied per round, until no candidate raises J by more than
+    1e-12 * max(1, |J|) or max_moves moves have been applied (the exact rule is in include/uavenv_b200.h).
+
+    scenes: a get_scene()-style dict of arrays (as allocate takes them).  assigned_target_id: int [S, N], the Target.id
+    each UAV is sent to (-1 = none): a user's allocation, the reference's, or allocate's.  max_moves: cap on applied
+    moves per scene (None: 16 * N).  config: sizes and omega (default the global cfg).  max_envs: scenes per launch.
+
+    Returns numpy arrays: "assigned_target_id" int32 [S, N], "J" f64 [S] after and "J_before" f64 [S] before the search,
+    "num_covered" int32 [S] (N0 after), "moves" int32 [S] (moves applied), "converged" bool [S] (True: the result is a
+    local optimum; False: the cap was reached first); and "summary": mean J before and after, mean moves, converged
+    fraction, scenes, wall seconds and scenes/s.  A row holding an id that is not a Target.id of its scene comes back
+    as a row of -1 with J NaN, num_covered -1 and moves -1."""
+    max_moves = _max_moves(max_moves)
+    max_envs = int(max_envs)
+    if max_envs <= 0:
+        raise ValueError("max_envs must be positive")
+    N = int((config if config is not None else _global_cfg).NUM_UAVS)
+    S = _scene_count(scenes, N)
+    asg = torch.as_tensor(assigned_target_id)
+    if asg.dtype.is_floating_point or asg.dtype == torch.bool or asg.dtype.is_complex:
+        raise ValueError("assigned_target_id must be an integer array of Target.ids")
+    if asg.numel() != S * N:
+        raise ValueError("assigned_target_id has %d elements, scenes hold %d x NUM_UAVS = %d" % (asg.numel(), S, S * N))
+    device, S, _, cfg, _, _ = _eval_setup(S, 1, config, device, 0)
+    from .envs.uav_env import UAVEnvBatched
+    dev_scenes = _device_scenes(scenes, S, device)
+    asg = asg.to(device=device, dtype=torch.int32).reshape(S, N)
+    per = min(max_envs, S)
+    env = None
+    parts = []
+    try:
+        torch.cuda.synchronize(device)
+        t0 = time.perf_counter()
+        env = UAVEnvBatched(per, device=device, seed=0, config=cfg, auto_reset=False, with_info=False)
+        for c0 in range(0, S, per):
+            n = min(per, S - c0)
+            env.load_scene_device({k: v[c0:c0 + n] for k, v in dev_scenes.items()}, copies=1, first_env=0)
+            parts.append(env.improve_allocation(asg[c0:c0 + n], first_env=0, env_stride=1, max_moves=max_moves))
+        res = {k: torch.cat([p[k] for p in parts]).cpu().numpy() for k in parts[0]}
+        wall = time.perf_counter() - t0
+    finally:
+        if env is not None:
+            env.close()
+    ok = res["moves"] >= 0                       # rows with valid ids (the means skip the flagged ones)
+    mean = (lambda x: float(x[ok].mean())) if ok.any() else (lambda x: float("nan"))
+    res["summary"] = {"J_before_mean": mean(res["J_before"]), "J_mean": mean(res["J"]), "moves_mean": mean(res["moves"]),
+                      "converged_frac": float(res["converged"].mean()), "scenes": S, "invalid_rows": int((~ok).sum()),
+                      "wall_s": float(wall), "scenes_per_s": S / wall}
+    return res
 
 
 def _generated_scenes(n, first, seed, cfg, device):

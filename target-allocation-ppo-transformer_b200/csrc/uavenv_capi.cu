@@ -602,3 +602,53 @@ extern "C" int uavenv_best_target_actions(uavenv_t *h, int64_t *d_cache, int64_t
         h->P, d_cache, d_actions);
     return launch_check(h, "best_target_kernel");
 }
+
+// ---- local search on allocations ----------------------------------------------------------------
+
+static int improve_sms(const uavenv *h) {
+    int sms = 0;
+    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, h->device) != cudaSuccess) return 0;
+    return sms;
+}
+
+extern "C" size_t uavenv_improve_workspace_bytes(const uavenv_t *h) {
+    if (!h || improve_p_in_smem(h->P.N, h->P.M)) return 0;
+    return (size_t)improve_sms(h) * h->P.N * h->P.M * sizeof(double);    // one p[N][M] slice per SM
+}
+
+extern "C" int uavenv_improve_allocation(uavenv_t *h, int32_t first_env, int32_t count, int32_t env_stride,
+                                         const int32_t *d_assigned_in, int32_t max_moves, int32_t *d_assigned_out,
+                                         double *d_J_in, double *d_J_out, int32_t *d_num_covered, int32_t *d_moves,
+                                         uint8_t *d_converged, void *d_workspace, void *stream) {
+    if (!h) return UAVENV_EINVAL;
+    if (!d_assigned_in || !d_assigned_out || !d_J_out || !d_num_covered || !d_moves || !d_converged)
+        return fail(h, UAVENV_EINVAL, "uavenv_improve_allocation: assigned_in / assigned_out / J_out / num_covered / "
+                    "moves / converged must be non-NULL");
+    const bool p_smem = improve_p_in_smem(h->P.N, h->P.M);
+    if (!p_smem && !d_workspace)
+        return fail(h, UAVENV_EINVAL, "uavenv_improve_allocation: N*M = %d needs a workspace of "
+                    "uavenv_improve_workspace_bytes() bytes", h->P.N * h->P.M);
+    if (count <= 0 || env_stride <= 0 || max_moves < 0)
+        return fail(h, UAVENV_EINVAL, "uavenv_improve_allocation: need count > 0, env_stride > 0 and max_moves >= 0 "
+                    "(got %d, %d, %d)", count, env_stride, max_moves);
+    const int64_t last = (int64_t)first_env + (int64_t)(count - 1) * env_stride;
+    if (first_env < 0 || last >= h->B)
+        return fail(h, UAVENV_EINVAL, "uavenv_improve_allocation: envs %d .. %lld outside [0,%d)", first_env,
+                    (long long)last, h->B);
+    if (!h->ready) return fail(h, UAVENV_ESTATE, "uavenv_improve_allocation before reset()/load_scene()");
+    CU_TRY(h, cudaSetDevice(h->device));
+    const int sms = improve_sms(h);
+    if (sms <= 0) return fail(h, UAVENV_ECUDA, "uavenv_improve_allocation: no multiprocessor count for device %d", h->device);
+    const size_t smem = improve_smem_bytes(h->P.N, h->P.M);
+    CU_TRY(h, cudaFuncSetAttribute(improve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int per_sm = 1;                          // the workspace holds one slice per SM: one CTA per SM on that path
+    if (p_smem) CU_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, improve_kernel, kImproveThreads, smem));
+    const int grid = std::min(count, sms * std::max(per_sm, 1));
+    ImproveIO io;
+    io.assigned_in = d_assigned_in; io.assigned_out = d_assigned_out; io.J_in = d_J_in; io.J_out = d_J_out;
+    io.num_covered = d_num_covered; io.moves = d_moves; io.converged = d_converged;
+    io.workspace = p_smem ? nullptr : static_cast<double *>(d_workspace);
+    io.first_env = first_env; io.count = count; io.env_stride = env_stride; io.max_moves = max_moves;
+    improve_kernel<<<grid, kImproveThreads, smem, (cudaStream_t)stream>>>(h->P, io);
+    return launch_check(h, "improve_kernel");
+}

@@ -15,6 +15,8 @@
 //                        one cooperative row of pair scores when a UAV's row is entered.
 //   group_best_kernel    the best finished member of each group of consecutive envs (best-of-K allocation):
 //                        a warp per group, shuffle arg-max over J, coalesced copy of the winner's allocation.
+//   improve_kernel       steepest-ascent local search (UAV moves and swaps) on given allocations: persistent CTAs,
+//                        a scene per CTA, block arg-max over the candidates of a round.
 #pragma once
 
 #include "uavenv_device.cuh"
@@ -1036,6 +1038,227 @@ __global__ void __launch_bounds__(kGroupBestThreads) group_best_kernel(const __g
         best[g] = unfinished ? -1 : bi;
         J_best[g] = unfinished ? __longlong_as_double(0x7ff8000000000000ll) : bJ;
         num_covered[g] = unfinished ? -1 : W.n(I_NCOVERED);
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Local search on allocations (include/uavenv_b200.h, uavenv_improve_allocation; the rule is stated there and in
+// DESIGN §4.9).  Persistent CTAs, one scene at a time per CTA.  The CTA computes its scene's p[N][M] once (warps over UAV
+// rows, lanes over targets, score_matrix_kernel's expression) into shared memory when N*M*8 <= kImproveSmemPBytes,
+// otherwise into its slice of the caller's workspace (L2-resident: one slice per SM).  t[N], nh[M], nh_excl[N], the
+// values and costs live in shared memory.  A round:
+//   1. every thread scores a strided share of the N*(M+1) moves and N*(N-1)/2 swaps in candidate order, keeping its
+//      first maximum, with the old targets of its best candidate packed beside it;
+//   2. a warp-shuffle arg-max, then every warp reduces the 8 warp winners itself (no second barrier): largest gain,
+//      lowest candidate index on an exact tie;
+//   3. if the winner qualifies, every thread knows the new allocation t' from the winner alone, so the products of the two
+//      touched targets (nh) and of their UAVs (nh_excl) are recomputed from scratch over t' in ascending UAV order while
+//      thread 0 writes t.  Two barriers per round.
+
+constexpr int kImproveThreads = 256;
+constexpr int kImproveWarps = kImproveThreads / 32;
+#ifndef UAV_IMPROVE_SMEM_P_BYTES
+#define UAV_IMPROVE_SMEM_P_BYTES (64 * 1024)
+#endif
+constexpr size_t kImproveSmemPBytes = UAV_IMPROVE_SMEM_P_BYTES;   // p in shared memory up to this size (64x64: 32 KB)
+
+struct ImproveIO {
+    const int32_t *assigned_in;  // [count][N] Target.id, -1 = none
+    int32_t *assigned_out;       // [count][N] (may alias assigned_in: a CTA reads its row before it writes it)
+    double *J_in, *J_out;        // [count] (J_in may be NULL)
+    int32_t *num_covered, *moves;
+    uint8_t *converged;
+    double *workspace;           // [gridDim.x][N*M] when p does not fit shared memory, else NULL
+    int32_t first_env, count, env_stride, max_moves;
+};
+
+__host__ __device__ __forceinline__ bool improve_p_in_smem(int N, int M) {
+    return (size_t)N * M * sizeof(double) <= kImproveSmemPBytes;
+}
+__host__ __device__ __forceinline__ size_t improve_smem_bytes(int N, int M) {
+    return (improve_p_in_smem(N, M) ? (size_t)N * M * sizeof(double) : 0) + (size_t)(2 * M + 2 * N) * sizeof(double) +
+           (size_t)(N + M) * sizeof(int32_t);
+}
+
+// prod over UAVs i != skip with t'(i) == j, ascending i, of (1 - p[i][j]); t' is t with t'(k1) = n1 and t'(k2) = n2.
+// (t[k1] / t[k2] may be rewritten concurrently: their loaded values are never used)
+__device__ __forceinline__ double improve_prod(const double *p, const int32_t *t, int N, int M, int j, int skip, int k1,
+                                               int n1, int k2, int n2) {
+    double q = 1.0;
+    for (int i = 0; i < N; ++i) {
+        const int ti = i == k1 ? n1 : (i == k2 ? n2 : t[i]);
+        if (ti == j && i != skip) q *= 1.0 - p[(size_t)i * M + j];
+    }
+    return q;
+}
+
+// J of the allocation t from its products: targets summed in list order, then the assigned UAVs' costs in UAV order
+__device__ __forceinline__ double improve_J(const double *nh, const double *val, const double *cost, const int32_t *t,
+                                            int N, int M, double omega) {
+    double rev = 0.0, c = 0.0;
+    for (int j = 0; j < M; ++j) rev += (1.0 - nh[j]) * val[j];
+    for (int k = 0; k < N; ++k) if (t[k] >= 0) c += cost[k];
+    return rev - (omega * c);
+}
+
+__global__ void __launch_bounds__(kImproveThreads) improve_kernel(const __grid_constant__ Params P, const ImproveIO io) {
+    extern __shared__ __align__(16) unsigned char improve_smem[];
+    __shared__ double red_g[kImproveWarps];
+    __shared__ int red_i[kImproveWarps], red_o[kImproveWarps];
+    __shared__ double sh_J;
+    __shared__ int sh_n0;
+    const int N = P.N, M = P.M, M1 = M + 1;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const double omega = P.omega;
+    const bool p_smem = improve_p_in_smem(N, M);
+    double *sd = reinterpret_cast<double *>(improve_smem);
+    double *p = p_smem ? sd : io.workspace + (size_t)blockIdx.x * N * M;
+    double *nh = sd + (p_smem ? (size_t)N * M : 0), *val = nh + M, *nhx = val + M, *cost = nhx + N;
+    int32_t *t = reinterpret_cast<int32_t *>(cost + N), *ids = t + N;
+    const int n_moves = N * M1, n_swaps = N * (N - 1) / 2;
+    const int dq = kImproveThreads / M1, dr = kImproveThreads % M1;     // a thread's stride through the moves
+    int s1 = 0, r0 = tid;                                                // its first swap (lexicographic index tid)
+    while (s1 < N - 1 && r0 >= N - 1 - s1) { r0 -= N - 1 - s1; ++s1; }
+    const int s2 = s1 + 1 + r0;
+
+    for (int s = blockIdx.x; s < io.count; s += gridDim.x) {
+        const int b = io.first_env + s * io.env_stride;
+        const int slot = P.header(b).n(I_GEN) & 1;
+        const UavRec *U = P.uav + P.uoff(slot, b);
+        const TgtRec *T = P.tgt + P.toff(slot, b);
+        for (int j = tid; j < M; j += kImproveThreads) { val[j] = T[j].value; ids[j] = T[j].id; }
+        for (int k = tid; k < N; k += kImproveThreads) cost[k] = U[k].cost;
+        for (int k = warp; k < N; k += kImproveWarps) {
+            const UavRec u = U[k];                                           // warp-uniform address
+            for (int j = lane; j < M; j += 32) {
+                const double tx = T[j].x, ty = T[j].y, ts = T[j].speed;
+                p[(size_t)k * M + j] = damage_prob(P, u, tx, ty, ts) * u.p_pen;
+            }
+        }
+        if (tid == 0) sh_n0 = 0;
+        __syncthreads();
+        const int32_t *row = io.assigned_in + (size_t)s * N;
+        bool bad = false;
+        for (int k = tid; k < N; k += kImproveThreads) {
+            const int id = row[k];
+            int pos = -1;
+            if (id < -1) bad = true;
+            else if (id >= 0) {
+                for (int j = 0; j < M; ++j) if (ids[j] == id) { pos = j; break; }
+                bad |= pos < 0;
+            }
+            t[k] = pos;
+        }
+        if (__syncthreads_or(bad)) {
+            for (int k = tid; k < N; k += kImproveThreads) io.assigned_out[(size_t)s * N + k] = -1;
+            if (tid == 0) {
+                const double nan = __longlong_as_double(0x7ff8000000000000ll);
+                if (io.J_in) io.J_in[s] = nan;
+                io.J_out[s] = nan; io.num_covered[s] = -1; io.moves[s] = -1; io.converged[s] = 0;
+            }
+            __syncthreads();
+            continue;
+        }
+        for (int j = tid; j < M; j += kImproveThreads) nh[j] = improve_prod(p, t, N, M, j, -1, -1, 0, -1, 0);
+        for (int k = tid; k < N; k += kImproveThreads)
+            nhx[k] = t[k] >= 0 ? improve_prod(p, t, N, M, t[k], k, -1, 0, -1, 0) : 1.0;
+        __syncthreads();
+        if (tid == 0) {
+            sh_J = improve_J(nh, val, cost, t, N, M, omega);
+            if (io.J_in) io.J_in[s] = sh_J;
+        }
+        __syncthreads();
+        double J = sh_J;                                                     // running J: the threshold's scale
+        int moves = 0;
+        bool conv = false;
+        for (;;) {
+            double bg = -INFINITY;
+            int bi = INT_MAX, bo = 0;                                        // gain, candidate index, packed old targets
+            int k = tid / M1, r = tid % M1;
+            for (int idx = tid; idx < n_moves; idx += kImproveThreads) {
+                const int a = t[k], bt = r - 1;
+                if (bt != a) {
+                    double ga = 0.0, gb = 0.0;
+                    if (a >= 0) ga = val[a] * (nh[a] - nhx[k]);
+                    if (bt >= 0) gb = (val[bt] * nh[bt]) * p[(size_t)k * M + bt];
+                    const double g = (ga + gb) + ((omega * cost[k]) * (double)((a >= 0) - (bt >= 0)));
+                    if (g > bg) { bg = g; bi = idx; bo = a + 1; }
+                }
+                k += dq; r += dr;
+                if (r >= M1) { r -= M1; ++k; }
+            }
+            int k1 = s1, k2 = s2;
+            for (int idx = tid; idx < n_swaps; idx += kImproveThreads) {
+                const int a1 = t[k1], a2 = t[k2];
+                if (a1 != a2) {
+                    double g1 = 0.0, g2 = 0.0;
+                    if (a1 >= 0) g1 = val[a1] * (nh[a1] - (nhx[k1] * (1.0 - p[(size_t)k2 * M + a1])));
+                    if (a2 >= 0) g2 = val[a2] * (nh[a2] - (nhx[k2] * (1.0 - p[(size_t)k1 * M + a2])));
+                    const double g = (g1 + g2) + ((omega * (cost[k1] - cost[k2])) * (double)((a1 >= 0) - (a2 >= 0)));
+                    if (g > bg) { bg = g; bi = n_moves + idx; bo = (a1 + 1) | ((a2 + 1) << 16); }
+                }
+                k2 += kImproveThreads;
+                while (k2 >= N && k1 < N) { ++k1; k2 += k1 + 1 - N; }    // overflow into the next row, which starts at k1 + 1
+            }
+            for (int o = 16; o > 0; o >>= 1) {
+                const double og = __shfl_xor_sync(kFullMask, bg, o);
+                const int oi = __shfl_xor_sync(kFullMask, bi, o), oo = __shfl_xor_sync(kFullMask, bo, o);
+                if (og > bg || (og == bg && oi < bi)) { bg = og; bi = oi; bo = oo; }
+            }
+            if (lane == 0) { red_g[warp] = bg; red_i[warp] = bi; red_o[warp] = bo; }
+            __syncthreads();
+            bg = red_g[0]; bi = red_i[0]; bo = red_o[0];
+            for (int w = 1; w < kImproveWarps; ++w) {
+                const double og = red_g[w];
+                const int oi = red_i[w];
+                if (og > bg || (og == bg && oi < bi)) { bg = og; bi = oi; bo = red_o[w]; }
+            }
+            if (!(bg > 1e-12 * fmax(1.0, fabs(J)))) { conv = true; break; }  // (uniform: every thread holds the winner)
+            if (moves >= io.max_moves) break;
+            ++moves;
+            J += bg;
+            int n1, n2 = 0, ja, jb;                                          // t'(k1) = n1, t'(k2) = n2; touched ja, jb
+            if (bi < n_moves) {
+                k1 = bi / M1; n1 = bi % M1 - 1; k2 = -1;
+                ja = bo - 1; jb = n1;
+            } else {
+                int q = bi - n_moves;
+                k1 = 0;
+                while (q >= N - 1 - k1) { q -= N - 1 - k1; ++k1; }
+                k2 = k1 + 1 + q;
+                ja = (bo & 0xffff) - 1; jb = (bo >> 16) - 1;
+                n1 = jb; n2 = ja;
+            }
+            for (int kk = tid; kk < N; kk += kImproveThreads) {
+                const int tk = kk == k1 ? n1 : (kk == k2 ? n2 : t[kk]);
+                if (tk < 0) nhx[kk] = 1.0;
+                else if (tk == ja || tk == jb) nhx[kk] = improve_prod(p, t, N, M, tk, kk, k1, n1, k2, n2);
+            }
+            if (tid == kImproveThreads - 1 && ja >= 0) nh[ja] = improve_prod(p, t, N, M, ja, -1, k1, n1, k2, n2);
+            if (tid == kImproveThreads - 2 && jb >= 0) nh[jb] = improve_prod(p, t, N, M, jb, -1, k1, n1, k2, n2);
+            if (tid == 0) { t[k1] = n1; if (k2 >= 0) t[k2] = n2; }
+            __syncthreads();
+        }
+        // outputs: t, nh are final (last written before the round's barrier)
+        int first = 0;                                                       // UAVs that are the first on their target
+        for (int kk = tid; kk < N; kk += kImproveThreads) {
+            const int tk = t[kk];
+            io.assigned_out[(size_t)s * N + kk] = tk >= 0 ? ids[tk] : -1;
+            if (tk >= 0) {
+                bool f = true;
+                for (int i = 0; i < kk && f; ++i) f = t[i] != tk;
+                first += f;
+            }
+        }
+        if (first) atomicAdd(&sh_n0, first);
+        if (tid == 0) {
+            io.J_out[s] = improve_J(nh, val, cost, t, N, M, omega);
+            io.moves[s] = moves;
+            io.converged[s] = conv ? 1 : 0;
+        }
+        __syncthreads();
+        if (tid == 0) io.num_covered[s] = sh_n0;
+        __syncthreads();                                                     // before the next scene reuses shared memory
     }
 }
 

@@ -113,6 +113,7 @@ class UAVEnvBatched:
         self._actions = torch.zeros(B, dtype=torch.int64, device=dev)
         self._h_reward = self._h_done = None
         self._best_target_cache = None        # best_target_actions' per-env entries, allocated on first use
+        self._improve_workspace = None        # improve_allocation's p slices (large N*M only), allocated on first use
 
     # ------------------------------------------------------------------ lifecycle
     def close(self):
@@ -297,6 +298,36 @@ class UAVEnvBatched:
                                               *(C.c_void_p(out[k].data_ptr()) for k in ("best", "J", "assigned_target_id",
                                                                                         "num_covered", "J_all")),
                                               self._stream()))
+        return out
+
+    def improve_allocation(self, assigned, first_env=0, env_stride=1, max_moves=None):
+        """Steepest-ascent local search (single-UAV moves and two-UAV swaps, include/uavenv_b200.h:
+        uavenv_improve_allocation) on the allocations assigned [S, N] (Target.id, -1 = none; moved to the device) of the
+        scenes held by envs first_env + s * env_stride.  max_moves: cap on applied moves per scene (None: 16 * N).
+        Returns device tensors {"assigned_target_id": int32 [S,N], "J": f64 [S], "J_before": f64 [S], "num_covered":
+        int32 [S] (N0), "moves": int32 [S], "converged": bool [S] (False: the cap stopped the search before a local
+        optimum)}.  A row with an id that is not a Target.id of its scene gets moves -1, J NaN, N0 -1 and a row of -1.
+        One launch on the env's stream."""
+        a = torch.as_tensor(assigned).to(device=self.device, dtype=torch.int32).contiguous()
+        if a.numel() == 0 or a.numel() % self.N:
+            raise ValueError("assigned has %d elements, not a positive multiple of N = %d" % (a.numel(), self.N))
+        S, dev = a.numel() // self.N, self.device
+        max_moves = 16 * self.N if max_moves is None else int(max_moves)
+        ws = int(self._lib.uavenv_improve_workspace_bytes(self._h))
+        if ws and (self._improve_workspace is None or self._improve_workspace.numel() < ws):
+            self._improve_workspace = torch.empty(ws, dtype=torch.uint8, device=dev)
+        out = {"assigned_target_id": torch.empty(S, self.N, dtype=torch.int32, device=dev),
+               "J": torch.empty(S, dtype=torch.float64, device=dev),
+               "J_before": torch.empty(S, dtype=torch.float64, device=dev),
+               "num_covered": torch.empty(S, dtype=torch.int32, device=dev),
+               "moves": torch.empty(S, dtype=torch.int32, device=dev),
+               "converged": torch.empty(S, dtype=torch.uint8, device=dev)}
+        self._chk(self._lib.uavenv_improve_allocation(
+            self._h, int(first_env), S, int(env_stride), C.c_void_p(a.data_ptr()), max_moves,
+            *(C.c_void_p(out[k].data_ptr()) for k in ("assigned_target_id", "J_before", "J", "num_covered", "moves",
+                                                      "converged")),
+            C.c_void_p(self._improve_workspace.data_ptr() if ws else None), self._stream()))
+        out["converged"] = out["converged"].view(torch.bool)
         return out
 
     def get_scene(self, first_env=0, count=None):
