@@ -1,8 +1,10 @@
 """Local search on allocations (uavenv_improve_allocation, ub.improve_allocation, ub.allocate(improve=True)): every applied
-move against an fp64 numpy re-implementation of the rule in include/uavenv_b200.h, local optimality at 64x64 (p in shared
-memory) and 256x256 (p in the workspace), max_moves = 0, determinism and layout independence, flagged rows, argument
-checks, and allocate's improve path.  The CPU tests at the end need no GPU."""
+move against an fp64 numpy re-implementation of the rule in include/uavenv_b200.h (at the configs, at every shape class
+of the candidate walk and of p's home, on a CTA's later scenes, on exact ties and under a cap that stops mid-search),
+local optimality at 64x64 (p in shared memory) and 256x256 (p in the workspace), max_moves = 0, determinism and layout
+independence, flagged rows, argument checks, and allocate's improve path.  The CPU tests at the end need no GPU."""
 import ctypes as C
+import math
 import os
 import re
 
@@ -30,11 +32,8 @@ CONFIGS = {"30x10": {}, "30x10_omega05": {"COST_WEIGHT_OMEGA": 0.5}, "hard_omega
 # ---- the fp64 reference of the search rule ---------------------------------------------------------------------------
 
 def _prod(p, t, j, skip=-1):
-    q = 1.0
-    for i in range(len(t)):
-        if t[i] == j and i != skip:
-            q *= 1.0 - p[i, j]
-    return q
+    """Product over UAVs i != skip on target j of (1 - p[i, j]) in ascending i (math.prod multiplies in order)."""
+    return math.prod((1.0 - p[[i for i in range(len(t)) if t[i] == j and i != skip], j]).tolist(), start=1.0)
 
 
 def _J(nh, val, cost, t, omega):
@@ -71,18 +70,21 @@ def _gains(p, t, nh, nhx, val, cost, omega):
     return np.concatenate([mv.reshape(-1), sw[iu]]), iu
 
 
-def ref_search(p, val, cost, omega, t0, max_moves):
+def ref_search(p, val, cost, omega, t0, max_moves, last_wins_tie=False):
     """(t, moves, converged, J_in, J_out, near, kinds) of the search from t0 (target positions, -1 = none).  kinds counts
-    moves to -1 and swaps with an unassigned side."""
+    moves to -1, swaps with an unassigned side and applied rounds whose best gain two or more candidates reach exactly
+    ("ties", their candidate indices in "tied").  last_wins_tie gives an exact tie to the highest candidate index: a
+    mutant of the rule, for showing that a test meets ties."""
     N, M = p.shape
     t = list(int(x) for x in t0)
     nh = np.array([_prod(p, t, j) for j in range(M)])
     nhx = np.array([_prod(p, t, t[k], k) if t[k] >= 0 else 1.0 for k in range(N)])
     J_in = _J(nh, val, cost, t, omega)
-    J, moves, near, kinds = J_in, 0, False, {"to_none": 0, "swap_none": 0, "moves": 0, "swaps": 0}
+    J, moves, near = J_in, 0, False
+    kinds = {"to_none": 0, "swap_none": 0, "moves": 0, "swaps": 0, "ties": 0, "tied": []}
     while True:
         g, iu = _gains(p, t, nh, nhx, val, cost, omega)
-        c = int(np.argmax(g))
+        c = g.size - 1 - int(np.argmax(g[::-1])) if last_wins_tie else int(np.argmax(g))
         best = g[c]
         if not best > 1e-12 * max(1.0, abs(J)):
             conv = True
@@ -93,6 +95,9 @@ def ref_search(p, val, cost, omega, t0, max_moves):
         second = np.max(np.delete(g, c)) if g.size > 1 else -np.inf
         # (an exact tie is no exclusion: both sides compute the same bits, and the candidate order decides)
         near |= bool(0.0 < best - second <= NEAR * max(abs(best), abs(second)))
+        if second == best:
+            kinds["ties"] += 1
+            kinds["tied"].append(np.flatnonzero(g == best))
         moves += 1
         J += best
         if c < N * (M + 1):
@@ -179,14 +184,43 @@ def _bits(x):
 
 # ---- 1: move by move against the reference -----------------------------------------------------------------------------
 
+def _check(got, scenes, pf, rows, omega, max_moves, label, kinds=None, idx=None):
+    """Checks the kernel's results got (entry i: scene idx[i], default every scene) of a search from rows [S, N] against
+    ref_search: J_before to 1e-12 for every scene; the rows, moves, converged, N0 exactly and J to 1e-12.  A scene in
+    which some round's two best gains lie within NEAR without being equal may differ (a last-bit difference could pick
+    either) and is then left out.  Returns (the scenes that matched, the scenes with such a near tie), and adds the
+    reference's counts of the matched scenes to kinds."""
+    idx = list(range(len(rows))) if idx is None else list(idx)
+    pos = _positions(np.asarray(rows)[idx], scenes["tgt_id"][idx])
+    kept, nears = [], []
+    for i, s in enumerate(idx):
+        t, moves, conv, J_in, J_out, near, kd = ref_search(pf[s], scenes["tgt_value"][s], scenes["uav_cost"][s], omega,
+                                                           pos[i], max_moves)
+        assert got["J_before"][i] == pytest.approx(J_in, rel=1e-12, abs=1e-12), (label, s)
+        want = np.where(t >= 0, scenes["tgt_id"][s][np.maximum(t, 0)], -1)
+        ok = {"rows": np.array_equal(got["assigned_target_id"][i], want),
+              "moves": got["moves"][i] == moves and bool(got["converged"][i]) == conv,
+              "J": got["J"][i] == pytest.approx(J_out, rel=1e-12, abs=1e-12),
+              "N0": got["num_covered"][i] == len(set(t[t >= 0].tolist()))}
+        if near:
+            nears.append(s)
+            if not all(ok.values()):
+                continue
+        assert all(ok.values()), (label, s, ok, got["moves"][i], moves)
+        kept.append(s)
+        for k in kinds or ():
+            kinds[k] += kd[k]
+    return kept, nears
+
+
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", sorted(CONFIGS))
 def test_search_equals_fp64_reference(name):
     """Final rows, move counts and converged flags equal the reference's exactly and J to 1e-12, from empty, random and
     allocate() allocations; scenes whose two best gains of some round lie within NEAR (but are not equal) are counted and
-    left out.  With omega > 0 moves to none occur; swaps with an unassigned side need a UAV whose cost outweighs a
-    positive contribution, which the default scenes have at omega = 0.5 (HARD_MODE's p_final is almost everywhere 0 at
-    30 x 10, so there every gain is a cost and single moves to none always win)."""
+    left out when they differ.  With omega > 0 moves to none occur; swaps with an unassigned side need a UAV whose cost
+    outweighs a positive contribution, which the default scenes have at omega = 0.5 (HARD_MODE's p_final is almost
+    everywhere 0 at 30 x 10, so there every gain is a cost and single moves to none always win)."""
     cfg = ub.Config(**CONFIGS[name])
     S, omega = 48, float(cfg.COST_WEIGHT_OMEGA)
     scenes = _scenes(S, 71, cfg)
@@ -196,26 +230,12 @@ def test_search_equals_fp64_reference(name):
     inputs = {"empty": np.full((S, N), -1, np.int32), "random": _random_rows(scenes, rng),
               "allocate": ub.allocate(_net(2), scenes=scenes, samples=2, seed=4, config=cfg)["assigned_target_id"]}
     kinds = {"to_none": 0, "swap_none": 0, "moves": 0, "swaps": 0}
-    excluded = 0
+    excluded = near = 0
     for label, rows in inputs.items():
-        got = _np(env.improve_allocation(rows))
-        pos = _positions(rows, scenes["tgt_id"])
-        for s in range(S):
-            t, moves, conv, J_in, J_out, near, kd = ref_search(pf[s], scenes["tgt_value"][s], scenes["uav_cost"][s], omega,
-                                                               pos[s], 16 * N)
-            for k in kinds:
-                kinds[k] += kd[k]
-            assert got["J_before"][s] == pytest.approx(J_in, rel=1e-12, abs=1e-12), (label, s)
-            if near:
-                excluded += 1
-                continue
-            want = np.where(t >= 0, scenes["tgt_id"][s][np.maximum(t, 0)], -1)
-            assert np.array_equal(got["assigned_target_id"][s], want), (label, s)
-            assert got["moves"][s] == moves and bool(got["converged"][s]) == conv, (label, s)
-            assert got["J"][s] == pytest.approx(J_out, rel=1e-12, abs=1e-12), (label, s)
-            assert got["num_covered"][s] == len(set(t[t >= 0].tolist())), (label, s)
-    print("\n[improve %s] moves %d (to none %d), swaps %d (an unassigned side %d), near-tie scenes excluded %d of %d" % (
-        name, kinds["moves"], kinds["to_none"], kinds["swaps"], kinds["swap_none"], excluded, 3 * S))
+        kept, nears = _check(_np(env.improve_allocation(rows)), scenes, pf, rows, omega, 16 * N, label, kinds)
+        excluded, near = excluded + S - len(kept), near + len(nears)
+    print("\n[improve %s] moves %d (to none %d), swaps %d (an unassigned side %d), near-tie scenes %d, excluded %d of %d" % (
+        name, kinds["moves"], kinds["to_none"], kinds["swaps"], kinds["swap_none"], near, excluded, 3 * S))
     # HARD_MODE's p_final is almost everywhere ~0, so its gains are costs apart by terms of ~1e-10: most near-ties are there
     assert excluded <= max(2, 3 * S // 8)
     assert kinds["moves"] > 0
@@ -223,6 +243,174 @@ def test_search_equals_fp64_reference(name):
         assert kinds["to_none"] > 0
     if name == "30x10_omega05":
         assert kinds["swap_none"] > 0
+    env.close()
+
+
+# Shapes at which the kernel's candidate walk or p's home changes.  Each of the 256 threads steps through the moves by
+# dq UAV rows and dr targets, divmod(256, M + 1), and through the swaps by 256, skipping whole short rows; p is in shared
+# memory while N * M * 8 <= 64 KB, else in the workspace.  (N, M, omega, scenes per input, p in, dq, dr)
+SHAPES = [(1, 7, 0.25, 48, "shared", 32, 0),            # no swaps at all
+          (8, 300, 0.25, 32, "shared", 0, 256),         # M + 1 > 256; fewer swaps (28) than threads
+          (16, 255, 0.25, 32, "shared", 1, 0),          # M + 1 = 256
+          (40, 63, 0.25, 32, "shared", 4, 0),           # M + 1 = 64 divides 256
+          (64, 64, 0.25, 24, "shared", 3, 61),          # the largest square on the shared path
+          (64, 64, 2.0, 24, "shared", 3, 61),           # moves to none and swaps with an unassigned side are common
+          (128, 64, 0.25, 12, "shared", 3, 61),         # N * M * 8 = 64 KB: the last shape on the shared path
+          (129, 64, 0.25, 12, "workspace", 3, 61),      # the first shapes on the workspace path
+          (64, 129, 0.25, 12, "workspace", 1, 126),
+          (300, 4, 0.25, 10, "shared", 51, 1),          # N > 256: the per-UAV loops take two passes; 44 850 swaps
+          (256, 256, 0.25, 10, "workspace", 0, 256)]    # BASELINE config 5
+
+
+def _shape_id(N, M, omega, S, path, dq, dr):
+    return "%dx%d%s-%s-dq%d-dr%d" % (N, M, "" if omega == 0.25 else "_omega%g" % omega, path, dq, dr)
+
+
+def _perturbed(rows, ids, rng, frac=0.05):
+    """rows with max(1, round(frac * N)) UAVs of each scene put on a random target or none."""
+    rows = rows.copy()
+    S, N = rows.shape
+    n = max(1, round(frac * N))
+    for s in range(S):
+        pos = rng.integers(-1, ids.shape[1], n)
+        rows[s, rng.choice(N, n, replace=False)] = np.where(pos >= 0, ids[s][np.maximum(pos, 0)], -1)
+    return rows
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("N,M,omega,S,path,dq,dr", [pytest.param(*c, id=_shape_id(*c)) for c in SHAPES])
+def test_shape_classes_equal_fp64_reference(N, M, omega, S, path, dq, dr):
+    """test_search_equals_fp64_reference's exact comparison where the candidate walk and p's home change form, from
+    empty rows, random rows, a pile-up (every UAV on the first target: the longest products) and a perturbed optimum
+    (the kernel's result for the random rows with ~5 % of the UAVs moved: gains near the threshold)."""
+    assert divmod(256, M + 1) == (dq, dr)
+    cfg = ub.Config(NUM_UAVS=N, NUM_TARGETS=M, COST_WEIGHT_OMEGA=omega)
+    scenes = _scenes(S, 61, cfg)
+    env, pf = _loaded(scenes, cfg)
+    assert (env._lib.uavenv_improve_workspace_bytes(env._h) == 0) == (path == "shared")
+    ids, rng = scenes["tgt_id"], np.random.default_rng(1000 * N + M)
+    rows = {"empty": np.full((S, N), -1, np.int32), "random": _random_rows(scenes, rng, p_none=0.5),
+            "pileup": np.ascontiguousarray(np.repeat(ids[:, :1], N, axis=1))}
+    kinds = {"to_none": 0, "swap_none": 0, "moves": 0, "swaps": 0}
+    got, excluded = {}, 0
+    for label in ("empty", "random", "pileup", "perturbed"):
+        if label == "perturbed":
+            rows[label] = _perturbed(got["random"]["assigned_target_id"], ids, rng)
+        got[label] = _np(env.improve_allocation(rows[label]))
+        kept, nears = _check(got[label], scenes, pf, rows[label], omega, 16 * N, label, kinds)
+        excluded += S - len(kept)
+        print("\n[improve %s] %s: %d of %d scenes equal (%d with a near tie), %d excluded, moves/scene %.1f" % (
+            _shape_id(N, M, omega, S, path, dq, dr), label, len(kept), S, len(nears), S - len(kept),
+            got[label]["moves"].mean()), end="")
+    print("\n  moves %d (to none %d), swaps %d (an unassigned side %d)" % (
+        kinds["moves"], kinds["to_none"], kinds["swaps"], kinds["swap_none"]))
+    assert excluded <= max(2, 4 * S // 8)
+    assert kinds["moves"] > 0 and (kinds["swaps"] > 0) == (N > 1)
+    if omega == 2.0:
+        assert kinds["to_none"] > 0 and kinds["swap_none"] > 0
+    env.close()
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("shape,waves,extra", [((256, 256), 2, 7), ((64, 64), 8, 50)], ids=["256x256", "64x64"])
+def test_later_scenes_of_a_cta_equal_fp64_reference(shape, waves, extra):
+    """A persistent CTA reuses its workspace slice (256x256: the grid is one CTA per SM) or its shared memory (64x64: at
+    most 8 CTAs per SM) for its next scene.  waves * SMs + extra scenes in one call, so the last ones are some CTA's
+    second or later scene; the scenes around each multiple of the SM count, the last and a few random ones equal the
+    reference, and each alone in a call (the first scene of CTA 0) gives the same bits."""
+    N, M = shape
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    S, omega = waves * sms + extra, 0.25
+    cfg = ub.Config(NUM_UAVS=N, NUM_TARGETS=M, COST_WEIGHT_OMEGA=omega)
+    scenes = _scenes(S, 37, cfg)
+    env, pf = _loaded(scenes, cfg)
+    rng = np.random.default_rng(N)
+    rows = _random_rows(scenes, rng, p_none=0.5)
+    got = _np(env.improve_allocation(rows))
+    sub = sorted({0, S - 1} | {c * sms + d for c in range(1, waves + 1) for d in (-1, 0, 1)} |
+                 set(rng.choice(S, 4, replace=False).tolist()))
+    kept, nears = _check({k: v[sub] for k, v in got.items()}, scenes, pf, rows, omega, 16 * N, "later scenes", idx=sub)
+    print("\n[improve %dx%d, %d scenes, %d SMs] %d of %d checked scenes equal (%d with a near tie)" % (
+        N, M, S, sms, len(kept), len(sub), len(nears)))
+    assert len(sub) - len(kept) <= max(2, len(sub) // 8)
+    for s in sub:
+        one = _np(env.improve_allocation(rows[s:s + 1], first_env=s))
+        for k in got:
+            if got[k].dtype == np.float64:
+                assert np.array_equal(_bits(got[k][s:s + 1]), _bits(one[k])), (k, s)
+            else:
+                assert np.array_equal(got[k][s:s + 1], one[k]), (k, s)
+    env.close()
+
+
+@pytest.mark.gpu
+def test_exact_ties_go_to_the_lowest_candidate_index():
+    """Generated 64x63 scenes (M + 1 = 64) in which UAVs 1 and 4 copy UAV 0 and target 40 copies target 3's position,
+    velocity and value (keeping its id).  Equal candidates of UAVs 0, 1 and 4 are 64 (other warps) and 256 (the same
+    thread) apart, so the in-thread first maximum, the warp arg-max and the cross-warp reduction each meet exact ties;
+    the rounds where each does are counted from the reference's tied candidates.  The kernel equals the reference, and a
+    reference that gives a tie to the highest index does not."""
+    N, M, S, omega = 64, 63, 64, 0.25
+    cfg = ub.Config(NUM_UAVS=N, NUM_TARGETS=M, COST_WEIGHT_OMEGA=omega)
+    scenes = _scenes(S, 43, cfg)
+    for f in scenes:
+        if f.startswith("uav_"):
+            scenes[f][:, [1, 4]] = scenes[f][:, :1]
+        elif f.startswith("tgt_") and f != "tgt_id":
+            scenes[f][:, 40] = scenes[f][:, 3]
+    env, pf = _loaded(scenes, cfg)
+    for a, b in ((pf[:, 0], pf[:, 1]), (pf[:, 0], pf[:, 4]), (pf[:, :, 3], pf[:, :, 40])):
+        assert np.array_equal(_bits(a), _bits(b))
+    rows = {"empty": np.full((S, N), -1, np.int32), "random": _random_rows(scenes, np.random.default_rng(9), p_none=0.5)}
+    kinds = {"ties": 0, "tied": []}
+    compared = rejected = 0
+    for label in rows:
+        got = _np(env.improve_allocation(rows[label]))
+        kept, _ = _check(got, scenes, pf, rows[label], omega, 16 * N, label, kinds)
+        pos = _positions(rows[label], scenes["tgt_id"])
+        for s in kept:
+            t, moves, *_ = ref_search(pf[s], scenes["tgt_value"][s], scenes["uav_cost"][s], omega, pos[s], 16 * N,
+                                      last_wins_tie=True)
+            want = np.where(t >= 0, scenes["tgt_id"][s][np.maximum(t, 0)], -1)
+            rejected += not (np.array_equal(got["assigned_target_id"][s], want) and got["moves"][s] == moves)
+        compared += len(kept)
+    n_moves, stage = N * (M + 1), {"thread": 0, "warp": 0, "block": 0}
+    for c in kinds["tied"]:
+        th = np.where(c < n_moves, c, c - n_moves) % 256                   # the thread that scores candidate c
+        w = th // 32
+        stage["thread"] += len(np.unique(th)) < len(th)
+        stage["warp"] += any(len(np.unique(th[w == x])) > 1 for x in np.unique(w))
+        stage["block"] += len(np.unique(w)) > 1
+    print("\n[improve ties 64x63] %d of %d scenes equal; %d rounds with an exact tie (in a thread %d, in a warp "
+          "%d, across warps %d); the highest-index-wins reference disagrees on %d scenes" % (
+              compared, 2 * S, kinds["ties"], stage["thread"], stage["warp"], stage["block"], rejected))
+    assert 2 * S - compared <= max(2, 2 * S // 8)
+    assert kinds["ties"] >= 8 and min(stage.values()) > 0
+    assert rejected > 0
+    env.close()
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("shape", [(64, 64), (256, 256)], ids=["64x64", "256x256"])
+def test_cap_stops_at_the_reference_state_mid_search(shape):
+    """max_moves = half the reference's moves from random rows: the rows, J, N0 and moves after exactly that many moves,
+    converged = False."""
+    N, M = shape
+    S, omega = 16 if N == 64 else 8, 0.25
+    cfg = ub.Config(NUM_UAVS=N, NUM_TARGETS=M, COST_WEIGHT_OMEGA=omega)
+    scenes = _scenes(S, 53, cfg)
+    env, pf = _loaded(scenes, cfg)
+    rows = _random_rows(scenes, np.random.default_rng(3), p_none=0.5)
+    pos = _positions(rows, scenes["tgt_id"])
+    compared = 0
+    for s in range(S):
+        cap = ref_search(pf[s], scenes["tgt_value"][s], scenes["uav_cost"][s], omega, pos[s], 16 * N)[1] // 2
+        assert cap > 0
+        got = _np(env.improve_allocation(rows[s:s + 1], first_env=s, max_moves=cap))
+        assert got["moves"][0] == cap and not got["converged"][0]
+        compared += len(_check(got, scenes, pf, rows, omega, cap, "cap %d" % cap, idx=[s])[0])
+    print("\n[improve %dx%d cap] %d of %d scenes equal" % (N, M, compared, S))
+    assert S - compared <= max(2, S // 8)
     env.close()
 
 
