@@ -204,6 +204,19 @@ static int launch_check(uavenv *h, const char *what) {
     return UAVENV_OK;
 }
 
+static int check_ready(uavenv *h, const char *what) {
+    return h->ready ? UAVENV_OK : fail(h, UAVENV_ESTATE, "%s before reset()/load_scene()", what);
+}
+
+// envs first_env + i * stride, i in [0, count), must exist; 64-bit arithmetic, so that no int32 argument wraps the test
+static int check_env_range(uavenv *h, int64_t first_env, int64_t count, int64_t stride, const char *what) {
+    const int64_t end = first_env + (count - 1) * stride + 1;
+    if (count <= 0 || first_env < 0 || end > h->B)
+        return fail(h, UAVENV_EINVAL, "%s: env range [%lld,%lld) empty or outside [0,%d)", what, (long long)first_env,
+                    (long long)end, h->B);
+    return UAVENV_OK;
+}
+
 extern "C" int uavenv_reset(uavenv_t *h, int32_t full_reset, const uint8_t *d_env_mask, float *d_obs, void *stream) {
     if (!h) return UAVENV_EINVAL;
     if (!full_reset && !h->ready)
@@ -224,7 +237,7 @@ static int launch_step(uavenv_t *h, const void *d_actions, int action_bytes, flo
     if (!h) return UAVENV_EINVAL;
     if (!d_actions || !d_obs || !d_reward || !d_done)
         return fail(h, UAVENV_EINVAL, "uavenv_step: actions/obs/reward/done must be non-NULL device pointers");
-    if (!h->ready) return fail(h, UAVENV_ESTATE, "uavenv_step before reset()/load_scene()");
+    if (int rc = check_ready(h, "uavenv_step")) return rc;
     StepIO io;
     io.actions = d_actions; io.action_bytes = action_bytes; io.obs = d_obs; io.reward = d_reward; io.done = d_done;
     // actions that live in (mapped) host memory are fetched with ONE bulk copy per CTA instead of one 32 B read per warp
@@ -291,14 +304,14 @@ extern "C" int uavenv_step_host_i8(uavenv_t *h, const int8_t *h_actions, float *
 // ---- scene injection / readback ----------------------------------------------------------------
 
 template <typename T>
-static cudaError_t stage(std::vector<void *> &tmp, const T *host, size_t n, const T **dev) {
+static cudaError_t stage(std::vector<void *> &tmp, const T *host, size_t n, T **dev) {
     *dev = nullptr;
     if (!host || n == 0) return cudaSuccess;
     void *q = nullptr;
     cudaError_t e = cudaMalloc(&q, n * sizeof(T));
     if (e != cudaSuccess) return e;
     tmp.push_back(q);
-    *dev = static_cast<const T *>(q);
+    *dev = static_cast<T *>(q);
     return cudaMemcpy(q, host, n * sizeof(T), cudaMemcpyHostToDevice);
 }
 
@@ -307,9 +320,7 @@ static int check_scene_args(uavenv *h, const uavenv_scene_t *sc, int32_t num_sce
                             const char *what) {
     if (num_scenes <= 0 || copies <= 0)
         return fail(h, UAVENV_EINVAL, "%s: need num_scenes > 0 and copies > 0 (got %d, %d)", what, num_scenes, copies);
-    const int64_t end = (int64_t)first_env + (int64_t)num_scenes * copies;
-    if (first_env < 0 || end > h->B)
-        return fail(h, UAVENV_EINVAL, "%s: env range [%d,%lld) outside [0,%d)", what, first_env, (long long)end, h->B);
+    if (int rc = check_env_range(h, first_env, (int64_t)num_scenes * copies, 1, what)) return rc;
     const Params &P = h->P;
     if (!sc->uav_x || !sc->uav_y || !sc->uav_vx || !sc->uav_vy || !sc->uav_load || !sc->uav_cost || !sc->tgt_x ||
         !sc->tgt_y || !sc->tgt_vx || !sc->tgt_vy || !sc->tgt_value || !sc->tgt_id ||
@@ -320,7 +331,7 @@ static int check_scene_args(uavenv *h, const uavenv_scene_t *sc, int32_t num_sce
 
 // the one packing path: device SoA of num_scenes scenes -> envs [first_env, first_env + num_scenes * copies), then the
 // reset of a loaded scene; enqueued on `stream`
-static int load_scene_impl(uavenv *h, const SceneSoA &s, int32_t num_scenes, int32_t copies, int32_t first_env,
+static int load_scene_impl(uavenv *h, const uavenv_scene_t &s, int32_t num_scenes, int32_t copies, int32_t first_env,
                            float *d_obs, cudaStream_t stream) {
     const int count = num_scenes * copies;
     const int grid = std::min((count + 3) / 4, 148 * 16);
@@ -337,13 +348,11 @@ static int load_scene_impl(uavenv *h, const SceneSoA &s, int32_t num_scenes, int
 extern "C" int uavenv_load_scene(uavenv_t *h, const uavenv_scene_t *sc, int32_t first_env, int32_t count,
                                   float *d_obs) {
     if (!h || !sc) return UAVENV_EINVAL;
-    int rc = check_scene_args(h, sc, count, 1, first_env, "uavenv_load_scene");
-    if (rc != UAVENV_OK) return rc;
+    if (int rc = check_scene_args(h, sc, count, 1, first_env, "uavenv_load_scene")) return rc;
     const Params &P = h->P;
     CU_TRY(h, cudaSetDevice(h->device));
     std::vector<void *> tmp;
-    SceneSoA s;
-    std::memset(&s, 0, sizeof s);
+    uavenv_scene_t s{};
     const size_t n = (size_t)count * P.N, m = (size_t)count * P.M, k1 = (size_t)count * P.K1, k2 = (size_t)count * P.K2;
     cudaError_t e = cudaSuccess;
     auto S = [&](auto host, size_t cnt, auto dev) { if (e == cudaSuccess) e = stage(tmp, host, cnt, dev); };
@@ -353,7 +362,7 @@ extern "C" int uavenv_load_scene(uavenv_t *h, const uavenv_scene_t *sc, int32_t 
     S(sc->tgt_value, m, &s.tgt_value); S(sc->tgt_id, m, &s.tgt_id);
     S(sc->nfz_x, k1, &s.nfz_x); S(sc->nfz_y, k1, &s.nfz_y); S(sc->nfz_radius, k1, &s.nfz_radius);
     S(sc->int_x, k2, &s.int_x); S(sc->int_y, k2, &s.int_y); S(sc->int_vx, k2, &s.int_vx); S(sc->int_vy, k2, &s.int_vy);
-    rc = UAVENV_OK;
+    int rc = UAVENV_OK;
     if (e == cudaSuccess) {
         rc = load_scene_impl(h, s, count, 1, first_env, d_obs, nullptr);
         e = cudaDeviceSynchronize();
@@ -367,18 +376,9 @@ extern "C" int uavenv_load_scene(uavenv_t *h, const uavenv_scene_t *sc, int32_t 
 extern "C" int uavenv_load_scene_device(uavenv_t *h, const uavenv_scene_t *d_scene, int32_t num_scenes, int32_t copies,
                                          int32_t first_env, float *d_obs, void *stream) {
     if (!h || !d_scene) return UAVENV_EINVAL;
-    int rc = check_scene_args(h, d_scene, num_scenes, copies, first_env, "uavenv_load_scene_device");
-    if (rc != UAVENV_OK) return rc;
+    if (int rc = check_scene_args(h, d_scene, num_scenes, copies, first_env, "uavenv_load_scene_device")) return rc;
     CU_TRY(h, cudaSetDevice(h->device));
-    const uavenv_scene_t &c = *d_scene;
-    SceneSoA s;
-    s.uav_x = c.uav_x; s.uav_y = c.uav_y; s.uav_vx = c.uav_vx; s.uav_vy = c.uav_vy; s.uav_load = c.uav_load;
-    s.uav_cost = c.uav_cost; s.uav_type = c.uav_type;
-    s.tgt_x = c.tgt_x; s.tgt_y = c.tgt_y; s.tgt_vx = c.tgt_vx; s.tgt_vy = c.tgt_vy; s.tgt_value = c.tgt_value;
-    s.tgt_id = c.tgt_id;
-    s.nfz_x = c.nfz_x; s.nfz_y = c.nfz_y; s.nfz_radius = c.nfz_radius;
-    s.int_x = c.int_x; s.int_y = c.int_y; s.int_vx = c.int_vx; s.int_vy = c.int_vy;
-    return load_scene_impl(h, s, num_scenes, copies, first_env, d_obs, (cudaStream_t)stream);
+    return load_scene_impl(h, *d_scene, num_scenes, copies, first_env, d_obs, (cudaStream_t)stream);
 }
 
 extern "C" int uavenv_group_best(uavenv_t *h, int32_t first_env, int32_t num_groups, int32_t group_size, int32_t *d_best,
@@ -390,13 +390,11 @@ extern "C" int uavenv_group_best(uavenv_t *h, int32_t first_env, int32_t num_gro
     if (num_groups <= 0 || group_size <= 0)
         return fail(h, UAVENV_EINVAL, "uavenv_group_best: need num_groups > 0 and group_size > 0 (got %d, %d)", num_groups,
                     group_size);
-    const int64_t end = (int64_t)first_env + (int64_t)num_groups * group_size;
-    if (first_env < 0 || end > h->B)
-        return fail(h, UAVENV_EINVAL, "uavenv_group_best: env range [%d,%lld) outside [0,%d)", first_env, (long long)end, h->B);
+    if (int rc = check_env_range(h, first_env, (int64_t)num_groups * group_size, 1, "uavenv_group_best")) return rc;
     if (h->P.auto_reset)
         return fail(h, UAVENV_ESTATE, "uavenv_group_best: the handle restarts finished envs (auto_reset = 1); final "
                     "allocations are kept with auto_reset = 0 only");
-    if (!h->ready) return fail(h, UAVENV_ESTATE, "uavenv_group_best before reset()/load_scene()");
+    if (int rc = check_ready(h, "uavenv_group_best")) return rc;
     CU_TRY(h, cudaSetDevice(h->device));
     const int grid = (num_groups + 7) / 8;                               // a warp per group, 8 per CTA
     group_best_kernel<<<grid, kGroupBestThreads, 0, (cudaStream_t)stream>>>(h->P, first_env, num_groups, group_size, d_best,
@@ -410,44 +408,46 @@ static cudaError_t fetch(std::vector<T> &v, const T *dev, size_t n) {
     return n ? cudaMemcpy(v.data(), dev, n * sizeof(T), cudaMemcpyDeviceToHost) : cudaSuccess;
 }
 
+// the header tiles covering envs [first, first + count): env first + i's is header_at(tiles.data(), first % 32 + i)
+static cudaError_t fetch_headers(const Params &P, size_t first, size_t count, std::vector<unsigned char> &tiles) {
+    return fetch(tiles, P.hdr + first / 32 * kEnvTileBytes, ((first + count + 31) / 32 - first / 32) * kEnvTileBytes);
+}
+
+// envs [first, first + count) of a double-buffered [2 slots][B][per] array, each env's `per` elements taken from the
+// storage slot of its current scene (I_GEN & 1; tiles from fetch_headers)
+template <typename T>
+static cudaError_t fetch_current(std::vector<T> &v, const T *dev, size_t per, const Params &P,
+                                 std::vector<unsigned char> &tiles, size_t first, size_t count) {
+    v.resize(count * per);
+    std::vector<T> s;
+    for (int slot = 0; slot < 2; ++slot) {
+        const cudaError_t e = fetch(s, dev + ((size_t)slot * P.B + first) * per, count * per);
+        if (e != cudaSuccess) return e;
+        for (size_t i = 0; i < count; ++i)
+            if ((header_at(tiles.data(), (int)(first % 32 + i)).n(I_GEN) & 1) == slot)
+                std::copy(s.begin() + i * per, s.begin() + (i + 1) * per, v.begin() + i * per);
+    }
+    return cudaSuccess;
+}
+
 extern "C" int uavenv_get_scene(uavenv_t *h, uavenv_scene_t *sc, int32_t first_env, int32_t count) {
     if (!h || !sc) return UAVENV_EINVAL;
-    if (first_env < 0 || count <= 0 || first_env + count > h->B)
-        return fail(h, UAVENV_EINVAL, "uavenv_get_scene: env range outside [0,%d)", h->B);
+    if (int rc = check_env_range(h, first_env, count, 1, "uavenv_get_scene")) return rc;
     const Params &P = h->P;
     CU_TRY(h, cudaSetDevice(h->device));
     CU_TRY(h, cudaDeviceSynchronize());
     const size_t n = (size_t)count * P.N, m = (size_t)count * P.M, k1 = (size_t)count * P.K1, k2 = (size_t)count * P.K2;
-    // both storage slots are fetched; each env's current slot (I_GEN & 1) selects
-    const size_t B = (size_t)h->B, fe = (size_t)first_env, ce = (size_t)count;
-    std::vector<UavRec> U(n); std::vector<TgtRec> T(m); std::vector<int32_t> ty(n); std::vector<double2> tv(m), uv(n);
-    std::vector<NfzRec> Z(k1); std::vector<IntRec> I(k2);
-    {
-        const size_t t0 = fe / 32, t1 = (fe + ce + 31) / 32;
-        std::vector<unsigned char> tiles;
-        CU_TRY(h, fetch(tiles, P.hdr + t0 * kEnvTileBytes, (t1 - t0) * kEnvTileBytes));
-        std::vector<UavRec> U2; std::vector<TgtRec> T2; std::vector<int32_t> ty2; std::vector<double2> tv2, uv2;
-        std::vector<NfzRec> Z2; std::vector<IntRec> I2;
-        for (int slot = 0; slot < 2; ++slot) {
-            CU_TRY(h, fetch(U2, P.uav + (slot * B + fe) * P.N, n));
-            CU_TRY(h, fetch(T2, P.tgt + (slot * B + fe) * P.M, m));
-            CU_TRY(h, fetch(ty2, P.uav_type + (slot * B + fe) * P.N, n));
-            CU_TRY(h, fetch(tv2, P.tgt_vel + (slot * B + fe) * P.M, m));
-            CU_TRY(h, fetch(uv2, P.uav_vel + (slot * B + fe) * P.N, n));
-            CU_TRY(h, fetch(Z2, P.nfz + (slot * B + fe) * P.K1, k1));
-            CU_TRY(h, fetch(I2, P.intc + (slot * B + fe) * P.K2, k2));
-            for (size_t e = 0; e < ce; ++e) {
-                if ((header_at(tiles.data(), (int)(fe + e - t0 * 32)).n(I_GEN) & 1) != slot) continue;
-                std::copy(U2.begin() + e * P.N, U2.begin() + (e + 1) * P.N, U.begin() + e * P.N);
-                std::copy(ty2.begin() + e * P.N, ty2.begin() + (e + 1) * P.N, ty.begin() + e * P.N);
-                std::copy(uv2.begin() + e * P.N, uv2.begin() + (e + 1) * P.N, uv.begin() + e * P.N);
-                std::copy(T2.begin() + e * P.M, T2.begin() + (e + 1) * P.M, T.begin() + e * P.M);
-                std::copy(tv2.begin() + e * P.M, tv2.begin() + (e + 1) * P.M, tv.begin() + e * P.M);
-                std::copy(Z2.begin() + e * P.K1, Z2.begin() + (e + 1) * P.K1, Z.begin() + e * P.K1);
-                std::copy(I2.begin() + e * P.K2, I2.begin() + (e + 1) * P.K2, I.begin() + e * P.K2);
-            }
-        }
-    }
+    std::vector<unsigned char> tiles;
+    CU_TRY(h, fetch_headers(P, first_env, count, tiles));
+    std::vector<UavRec> U; std::vector<TgtRec> T; std::vector<int32_t> ty; std::vector<double2> tv, uv;
+    std::vector<NfzRec> Z; std::vector<IntRec> I;
+    CU_TRY(h, fetch_current(U, P.uav, P.N, P, tiles, first_env, count));
+    CU_TRY(h, fetch_current(T, P.tgt, P.M, P, tiles, first_env, count));
+    CU_TRY(h, fetch_current(ty, P.uav_type, P.N, P, tiles, first_env, count));
+    CU_TRY(h, fetch_current(tv, P.tgt_vel, P.M, P, tiles, first_env, count));
+    CU_TRY(h, fetch_current(uv, P.uav_vel, P.N, P, tiles, first_env, count));
+    CU_TRY(h, fetch_current(Z, P.nfz, P.K1, P, tiles, first_env, count));
+    CU_TRY(h, fetch_current(I, P.intc, P.K2, P, tiles, first_env, count));
     for (size_t i = 0; i < n; ++i) {
         if (sc->uav_x) sc->uav_x[i] = U[i].x;
         if (sc->uav_y) sc->uav_y[i] = U[i].y;
@@ -481,8 +481,7 @@ extern "C" int uavenv_get_scene(uavenv_t *h, uavenv_scene_t *sc, int32_t first_e
 
 extern "C" int uavenv_get_state(uavenv_t *h, uavenv_state_t *st, int32_t first_env, int32_t count) {
     if (!h || !st) return UAVENV_EINVAL;
-    if (first_env < 0 || count <= 0 || first_env + count > h->B)
-        return fail(h, UAVENV_EINVAL, "uavenv_get_state: env range outside [0,%d)", h->B);
+    if (int rc = check_env_range(h, first_env, count, 1, "uavenv_get_state")) return rc;
     const Params &P = h->P;
     CU_TRY(h, cudaSetDevice(h->device));
     CU_TRY(h, cudaDeviceSynchronize());
@@ -491,36 +490,31 @@ extern "C" int uavenv_get_state(uavenv_t *h, uavenv_state_t *st, int32_t first_e
         return dst ? cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost) : cudaSuccess;
     };
     CU_TRY(h, D2H(st->assigned_target_id, P.assigned + f * P.N, c * P.N * 4));
-    // header tiles covering [first_env, first_env + count)
-    const size_t t0 = f / 32, t1 = (f + c + 31) / 32;
     std::vector<unsigned char> tiles;
-    CU_TRY(h, fetch(tiles, P.hdr + t0 * kEnvTileBytes, (t1 - t0) * kEnvTileBytes));
+    CU_TRY(h, fetch_headers(P, f, c, tiles));
     for (size_t i = 0; i < c; ++i) {
-        const Hdr hv = header_at(tiles.data(), (int)(f + i - t0 * 32));
+        const Hdr hv = header_at(tiles.data(), (int)(f % 32 + i));
         if (st->uav_idx) st->uav_idx[i] = hv.n(I_K);
         if (st->target_idx) st->target_idx[i] = hv.n(I_M);
         if (st->episode) st->episode[i] = hv.n(I_EPISODE);
         if (st->scene_index) st->scene_index[i] = hv.n(I_GEN) >> 1;
         if (st->finished) st->finished[i] = (uint8_t)(hv.n(I_FINISHED) != 0);
-        if (st->J_val) st->J_val[i] = hv.f(F_REV) - (P.omega * hv.f(F_COST_SUM));
+        if (st->J_val) st->J_val[i] = objective(P, hv.f(F_REV), hv.f(F_COST_SUM));
         // UAV slots at / past the decision pointer have not decided in this episode (a restart does not clear them)
         if (st->assigned_target_id)
             for (int32_t k = std::max(hv.n(I_K), 0); k < P.N; ++k) st->assigned_target_id[i * P.N + k] = -1;
     }
     if (st->lock_count || st->not_hit || st->not_hit_pure) {
         std::vector<TgtRec> T;
-        for (int slot = 0; slot < 2; ++slot) {
-            CU_TRY(h, fetch(T, P.tgt + ((size_t)slot * h->B + f) * P.M, c * P.M));
-            for (size_t e = 0; e < c; ++e) {
-                const Hdr hv = header_at(tiles.data(), (int)(f + e - t0 * 32));
-                if ((hv.n(I_GEN) & 1) != slot) continue;
-                for (size_t j = e * P.M; j < (e + 1) * P.M; ++j) {
-                    TgtRec t = T[j];                       // as the env sees it in its current episode
-                    const int cnt = target_view(t, hv.n(I_EPISODE));
-                    if (st->lock_count) st->lock_count[j] = cnt;
-                    if (st->not_hit) st->not_hit[j] = t.nh;
-                    if (st->not_hit_pure) st->not_hit_pure[j] = t.nh_pure;
-                }
+        CU_TRY(h, fetch_current(T, P.tgt, P.M, P, tiles, f, c));
+        for (size_t e = 0; e < c; ++e) {
+            const int episode = header_at(tiles.data(), (int)(f % 32 + e)).n(I_EPISODE);
+            for (size_t j = e * P.M; j < (e + 1) * P.M; ++j) {
+                TgtRec t = T[j];                           // as the env sees it in its current episode
+                const int cnt = target_view(t, episode);
+                if (st->lock_count) st->lock_count[j] = cnt;
+                if (st->not_hit) st->not_hit[j] = t.nh;
+                if (st->not_hit_pure) st->not_hit_pure[j] = t.nh_pure;
             }
         }
     }
@@ -529,8 +523,7 @@ extern "C" int uavenv_get_state(uavenv_t *h, uavenv_state_t *st, int32_t first_e
 
 extern "C" int uavenv_set_episode_counters(uavenv_t *h, const int32_t *h_episode, int32_t first_env, int32_t count) {
     if (!h || !h_episode) return UAVENV_EINVAL;
-    if (first_env < 0 || count <= 0 || first_env + count > h->B)
-        return fail(h, UAVENV_EINVAL, "uavenv_set_episode_counters: env range outside [0,%d)", h->B);
+    if (int rc = check_env_range(h, first_env, count, 1, "uavenv_set_episode_counters")) return rc;
     for (int32_t i = 0; i < count; ++i)
         if (h_episode[i] < 1) return fail(h, UAVENV_EINVAL, "uavenv_set_episode_counters: counters are 1-based");
     const Params &P = h->P;
@@ -554,7 +547,7 @@ template <typename OutT>
 static int score_matrix_impl(uavenv *h, OutT *pf, OutT *pd, void *stream) {
     if (!h) return UAVENV_EINVAL;
     if (!pf && !pd) return fail(h, UAVENV_EINVAL, "uavenv_score_matrix: both outputs NULL");
-    if (!h->ready) return fail(h, UAVENV_ESTATE, "uavenv_score_matrix before reset()/load_scene()");
+    if (int rc = check_ready(h, "uavenv_score_matrix")) return rc;
     CU_TRY(h, cudaSetDevice(h->device));
     const size_t warps = (size_t)h->B * ((h->P.M + 31) / 32);          // one warp per (env, 32-target chunk)
     const int grid = (int)std::min<size_t>((warps + 7) / 8, (size_t)148 * 32);
@@ -570,7 +563,7 @@ extern "C" int uavenv_score_matrix_f64(uavenv_t *h, double *pf, double *pd, void
 
 extern "C" int uavenv_recompute_objective(uavenv_t *h, double *h_max_abs_diff, void *stream) {
     if (!h) return UAVENV_EINVAL;
-    if (!h->ready) return fail(h, UAVENV_ESTATE, "uavenv_recompute_objective before reset()/load_scene()");
+    if (int rc = check_ready(h, "uavenv_recompute_objective")) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     CU_TRY(h, cudaSetDevice(h->device));
     CU_TRY(h, cudaMemsetAsync(h->d_scratch, 0, sizeof(double), s));
@@ -596,7 +589,7 @@ extern "C" int uavenv_random_actions(uavenv_t *h, uint64_t action_seed, uint64_t
 extern "C" int uavenv_best_target_actions(uavenv_t *h, int64_t *d_cache, int64_t *d_actions, void *stream) {
     if (!h) return UAVENV_EINVAL;
     if (!d_cache || !d_actions) return fail(h, UAVENV_EINVAL, "uavenv_best_target_actions: cache/actions must be non-NULL device pointers");
-    if (!h->ready) return fail(h, UAVENV_ESTATE, "uavenv_best_target_actions before reset()/load_scene()");
+    if (int rc = check_ready(h, "uavenv_best_target_actions")) return rc;
     CU_TRY(h, cudaSetDevice(h->device));
     best_target_kernel<<<(h->B + kBestTargetThreads - 1) / kBestTargetThreads, kBestTargetThreads, 0, (cudaStream_t)stream>>>(
         h->P, d_cache, d_actions);
@@ -631,11 +624,8 @@ extern "C" int uavenv_improve_allocation(uavenv_t *h, int32_t first_env, int32_t
     if (count <= 0 || env_stride <= 0 || max_moves < 0)
         return fail(h, UAVENV_EINVAL, "uavenv_improve_allocation: need count > 0, env_stride > 0 and max_moves >= 0 "
                     "(got %d, %d, %d)", count, env_stride, max_moves);
-    const int64_t last = (int64_t)first_env + (int64_t)(count - 1) * env_stride;
-    if (first_env < 0 || last >= h->B)
-        return fail(h, UAVENV_EINVAL, "uavenv_improve_allocation: envs %d .. %lld outside [0,%d)", first_env,
-                    (long long)last, h->B);
-    if (!h->ready) return fail(h, UAVENV_ESTATE, "uavenv_improve_allocation before reset()/load_scene()");
+    if (int rc = check_env_range(h, first_env, count, env_stride, "uavenv_improve_allocation")) return rc;
+    if (int rc = check_ready(h, "uavenv_improve_allocation")) return rc;
     CU_TRY(h, cudaSetDevice(h->device));
     const int sms = improve_sms(h);
     if (sms <= 0) return fail(h, UAVENV_ECUDA, "uavenv_improve_allocation: no multiprocessor count for device %d", h->device);

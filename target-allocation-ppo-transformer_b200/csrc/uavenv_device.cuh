@@ -61,6 +61,10 @@ __host__ __device__ __forceinline__ int target_view(TgtRec &t, int episode) {
     t.nh = 1.0; t.nh_pure = 1.0; t.lock_cost = 0.0;
     return 0;
 }
+// an empty lock list for record T[j] (indexed: a TgtRec & form changes reset_kernel's register allocation)
+__host__ __device__ __forceinline__ void clear_locks(TgtRec *T, int j) {
+    T[j].nh = 1.0; T[j].nh_pure = 1.0; T[j].lock_cost = 0.0; T[j].lock_tag = 0;
+}
 
 struct NfzRec { double x, y, radius; };            // envs/entities.py:52-55
 struct IntRec { double x, y, vx, vy; };            // envs/entities.py:58-61 + velocity (uav_env.py:168)
@@ -150,6 +154,8 @@ struct Params {
     __host__ __device__ __forceinline__ Hdr header(int b) const { return header_at(hdr, b); }
     __host__ __device__ __forceinline__ size_t uoff(int slot, int b) const { return ((size_t)slot * B + b) * N; }
     __host__ __device__ __forceinline__ size_t toff(int slot, int b) const { return ((size_t)slot * B + b) * M; }
+    __host__ __device__ __forceinline__ size_t zoff(int slot, int b) const { return ((size_t)slot * B + b) * K1; }
+    __host__ __device__ __forceinline__ size_t ioff(int slot, int b) const { return ((size_t)slot * B + b) * K2; }
     // ring element (slot, feature pair f) of env b: ring(b)[slot * 224 + f * 32]
     __host__ __device__ __forceinline__ float2 *ring(int b) const {
         return reinterpret_cast<float2 *>(hdr + (size_t)(b >> 5) * kEnvTileBytes + kHdrTileBytes) + (b & 31);
@@ -212,6 +218,14 @@ __device__ __forceinline__ double damage_prob(const Params &P, const UavRec &u, 
     return clip01(e_angle * term * u.load);                        // :112-114
 }
 
+// envs/mechanics.py:167-181 calc_advantage: p_final of UAV u on the target at (tx, ty) moving at tspeed (*pd = p_damage)
+__device__ __forceinline__ double pair_score(const Params &P, const UavRec &u, double tx, double ty, double tspeed,
+                                             double *pd = nullptr) {
+    const double d = damage_prob(P, u, tx, ty, tspeed);
+    if (pd) *pd = d;
+    return d * u.p_pen;                                            // :179
+}
+
 // envs/mechanics.py:118-163 calc_penetration_prob (Eq.5-6): depends on the UAV only
 __device__ __forceinline__ double penetration_prob(const Params &P, const NfzRec *Z, const IntRec *I, const UavRec &u) {
     double p = 1.0;
@@ -244,9 +258,6 @@ __device__ __forceinline__ void finish_uav(const Params &P, const NfzRec *Z, con
     finish_uav_kinematics(u, vx, vy);
     u.p_pen = penetration_prob(P, Z, I, u);
 }
-__device__ __forceinline__ void finish_uav(const Params &P, int slot, int b, UavRec &u, double vx, double vy) {
-    finish_uav(P, P.nfz + ((size_t)slot * P.B + b) * P.K1, P.intc + ((size_t)slot * P.B + b) * P.K2, u, vx, vy);
-}
 
 // envs/mechanics.py:185-241 get_state_vector (Eq.15): fp64 features, cast to f32, then the power-of-two
 // scalings applied in f32 exactly as the reference does (:235-239).
@@ -272,9 +283,26 @@ __device__ __forceinline__ void state_vector(double cost, double value, double c
     o[13] = 1.0f;  // float(uav.available): the pointer UAV is always unassigned (uav_env.py:317-324)
 }
 
+// envs/uav_env.py:268 _calc_J_X: J from the revenue and the summed cost of the assigned UAVs (every J of the library)
+__host__ __device__ __forceinline__ double objective(const Params &P, double rev, double cost) { return rev - (P.omega * cost); }
+
 // envs/uav_env.py:271-293 _calculate_paper_reward (Eq.19) from the running aggregates
 __device__ __forceinline__ double paper_reward(double J, int n0, int M) {
     return (n0 == M) ? 2.0 * J : J * ((double)n0 / (double)M);
+}
+
+// X' = X + (UAV -> target) (uav_env.py:308-313) from the carried aggregates: only the target's product nh, the revenue,
+// the cost sum and N0 change.  (nh, value, lock_cnt: the target; pf: the pair's p_final; ucost: the UAV's cost)
+struct Tentative { double nh2, rev2, cost2, new_r; int n02; };
+__device__ __forceinline__ Tentative tentative_assign(const Params &P, double rev, double cost_sum, int n0, double nh,
+                                                      double value, int lock_cnt, double pf, double ucost) {
+    Tentative x;
+    x.nh2 = nh * (1.0 - pf);
+    x.rev2 = rev + ((1.0 - x.nh2) - (1.0 - nh)) * value;
+    x.cost2 = cost_sum + ucost;
+    x.n02 = n0 + (lock_cnt == 0);
+    x.new_r = paper_reward(objective(P, x.rev2, x.cost2), x.n02, P.M);   // :313
+    return x;
 }
 
 }  // namespace uavk

@@ -19,6 +19,7 @@
 //                        a scene per CTA, block arg-max over the candidates of a round.
 #pragma once
 
+#include "uavenv_b200.h"
 #include "uavenv_device.cuh"
 
 namespace uavk {
@@ -56,6 +57,19 @@ __device__ __forceinline__ double warp_sum(double v) {
     return v;
 }
 
+// Shuffle arg-max of (best, bi) over the warp, every lane ending with the winner (best_target, group_best): the larger
+// value wins, on equal values the lower index; index INT_MAX means "no candidate" and never beats a real one.  Branching
+// on the index first keeps each step's compare chain as short as the unguarded rule's (best_target's row is latency-bound).
+__device__ __forceinline__ void warp_argmax(double &best, int &bi) {
+    for (int o = 16; o > 0; o >>= 1) {
+        const double ob = __shfl_xor_sync(kFullMask, best, o);
+        const int oi = __shfl_xor_sync(kFullMask, bi, o);
+        if (oi < bi ? (ob >= best || bi == INT_MAX) : (ob > best && oi != INT_MAX)) { best = ob; bi = oi; }
+    }
+}
+
+__device__ __forceinline__ double quiet_nan() { return __longlong_as_double(0x7ff8000000000000ll); }
+
 // position of element i in a sort of keys[0..n) by (key, index): a uniformly random permutation
 __device__ __forceinline__ int rank_of(const uint32_t *keys, int n, int i) {
     const uint32_t ki = keys[i];
@@ -73,9 +87,7 @@ __device__ __forceinline__ void warp_clear_allocation(const Params &P, int slot,
     int32_t *asg = P.assigned + (size_t)b * P.N;
     for (int i = lane; i < P.N; i += 32) asg[i] = -1;
     TgtRec *T = P.tgt + P.toff(slot, b);
-    for (int j = lane; j < P.M; j += 32) {
-        T[j].nh = 1.0; T[j].nh_pure = 1.0; T[j].lock_cost = 0.0; T[j].lock_tag = 0;
-    }
+    for (int j = lane; j < P.M; j += 32) clear_locks(T, j);
 }
 
 // ---- _generate_scene (envs/uav_env.py:65-173) with the counter RNG, in independent chunks of 32 entities ----
@@ -158,7 +170,7 @@ __device__ void warp_generate_chunk(const Params &P, int slot, int b, uint32_t s
             const double vx = (u53(v.x, v.y) - 0.5) * 0.03, vy = (u53(v.z, v.w) - 0.5) * 0.03;  // :139
             t.speed = sqrt(vx * vx + vy * vy);
             t.value = value;
-            t.nh = 1.0; t.nh_pure = 1.0; t.lock_cost = 0.0; t.lock_tag = 0; t.id = i;
+            clear_locks(&t, 0); t.id = i;
             P.tgt[P.toff(slot, b) + pos] = t;
             P.tgt_vel[P.toff(slot, b) + pos] = make_double2(vx, vy);
         }
@@ -203,8 +215,8 @@ __device__ void warp_generate_chunk(const Params &P, int slot, int b, uint32_t s
 // whole scene in one go (reset(), and the fallback when the next scene was not pre-generated in time)
 __device__ __noinline__ void warp_generate_scene(const Params &P, int slot, int b, uint32_t scene, uint32_t *s_keys) {
     const int nchunks = scene_chunks(P);
-    NfzRec *Z = P.nfz + ((size_t)slot * P.B + b) * P.K1;
-    IntRec *I = P.intc + ((size_t)slot * P.B + b) * P.K2;
+    NfzRec *Z = P.nfz + P.zoff(slot, b);
+    IntRec *I = P.intc + P.ioff(slot, b);
     warp_generate_obstacles(P, b, scene, Z, I);
     __threadfence_block();  // obstacles visible to the UAV chunks of this warp
     __syncwarp();
@@ -315,8 +327,8 @@ __device__ __noinline__ void pregen_service(const Params &P, int service_cta, in
     const int scene = gen >> 1, slot = (gen & 1) ^ 1;
     // the obstacles: chunk 0 generates them (in its shared-memory scratch) and writes the records; the p_pen jobs run in a
     // later launch and read those records - nobody else needs them
-    NfzRec *Zg = P.nfz + ((size_t)slot * P.B + eb) * P.K1;
-    IntRec *Ig = P.intc + ((size_t)slot * P.B + eb) * P.K2;
+    NfzRec *Zg = P.nfz + P.zoff(slot, eb);
+    IntRec *Ig = P.intc + P.ioff(slot, eb);
     const NfzRec *Z = Zg;
     const IntRec *I = Ig;
     if (chunk == 0) {
@@ -339,14 +351,21 @@ __device__ __noinline__ void pregen_service(const Params &P, int service_cta, in
 __device__ __forceinline__ void eval_pointer_pair(const Params &P, const UavRec &u, const TgtRec &t, double cost_sum,
                                                   double covered_val, double total_cost, double total_val,
                                                   double &pf, double &pd, float *row) {
-    pd = damage_prob(P, u, t.x, t.y, t.speed);
-    pf = pd * u.p_pen;                                                  // mechanics.py:179
+    pf = pair_score(P, u, t.x, t.y, t.speed, &pd);
     const double inv_tc = 1.0 / (total_cost + 1e-6);
     const double chi_c = cost_sum * inv_tc;                             // uav_env.py:195-196
     const double chi_v = covered_val / (total_val + 1e-6);              // :198-200
     const double chi_mc = t.lock_cost * inv_tc;                         // :202-206
     const double P_prev = 1.0 - t.nh, P_pure = 1.0 - t.nh_pure;         // :226-227
     state_vector(u.cost, t.value, chi_c, chi_v, chi_mc, pf, pd, P_prev, P_prev * t.value, P_pure, row);
+}
+
+// the decision pointers, counters and running sums of an env; age = valid rows of its observation window
+__device__ __forceinline__ void store_progress(const Hdr &h, int k, int m, int nA, int n0, int age, double rev, double cost_sum,
+                                               double covered_val, double sum_pd, double sum_pf) {
+    h.n(I_K) = k; h.n(I_M) = m; h.n(I_NASSIGNED) = nA; h.n(I_NCOVERED) = n0; h.n(I_AGE) = age;
+    h.f(F_REV) = rev; h.f(F_COST_SUM) = cost_sum; h.f(F_COVERED_VAL) = covered_val;
+    h.f(F_SUM_PD) = sum_pd; h.f(F_SUM_PF) = sum_pf;
 }
 
 // capture the new current pair in the header (the next step's accept rule reads only these)
@@ -401,8 +420,8 @@ __device__ __noinline__ void exact_rewards(const Params &P, int slot, int b, int
         rev += (1.0 - nh) * value;                                    // :264-265
         rev2 += (1.0 - (j == m ? nh2 : nh)) * value;
     }
-    prev_r = paper_reward(rev - (P.omega * cost_sum), n0, P.M);       // :268, :287-291
-    new_r = paper_reward(rev2 - (P.omega * cost2), n02, P.M);
+    prev_r = paper_reward(objective(P, rev, cost_sum), n0, P.M);      // :268, :287-291
+    new_r = paper_reward(objective(P, rev2, cost2), n02, P.M);
 }
 
 // restart bookkeeping of the finished envs in mask (their scene is in slot_of[lane]): stores only
@@ -524,32 +543,28 @@ __global__ void __launch_bounds__(kStepThreads, 512 / kStepThreads) step_kernel(
     if (live) {
         double reward = 0.0;
         if (!was_finished) {
-            double prev_r = paper_reward(rev - (P.omega * cost_sum), n0, M);            // :301
+            double prev_r = paper_reward(objective(P, rev, cost_sum), n0, M);           // :301
             double cur_r = prev_r;
             bool advance_uav = false;
             if (action == 1) {                                                           // :306
-                // tentative X' (:308-310): only target m's product, the cost sum and N0 change
-                const double nh2 = c_nh * (1.0 - c_pf);
-                const double rev2 = rev + ((1.0 - nh2) - (1.0 - c_nh)) * c_value;
-                const double cost2 = cost_sum + c_ucost;
-                const int n02 = n0 + (c_lock_cnt == 0);
-                double new_r = paper_reward(rev2 - (P.omega * cost2), n02, M);          // :313
+                const Tentative x = tentative_assign(P, rev, cost_sum, n0, c_nh, c_value, c_lock_cnt, c_pf, c_ucost);
+                double new_r = x.new_r;
                 // the carried sums differ from the reference's fresh sums by O(1e-14) relative: inside the tie band the
                 // decision (and the reward) come from the exact re-summation.  Only with a cost term: at omega = 0 an Assign
                 // can only grow one term of J and N0, so new_r >= prev_r holds under rounding in the reference's summation
                 // and in the carried one alike (and near-ties are the NORM there once a target's product has underflowed)
                 if (P.omega != 0.0 && fabs(new_r - prev_r) <= P.tie_band * fmax(fabs(new_r), fabs(prev_r)))
-                    exact_rewards(P, slot, b, episode_new - 1, m, nh2, cost_sum, cost2, n0, n02, prev_r, new_r);
+                    exact_rewards(P, slot, b, episode_new - 1, m, x.nh2, cost_sum, x.cost2, n0, x.n02, prev_r, new_r);
                 if (new_r >= prev_r) {                                                   // :317 (Eq.21)
                     reward = new_r - prev_r;                                             // :321
                     cur_r = new_r;
                     TgtRec *tp = P.tgt + P.toff(slot, b) + m;
-                    tp->nh = nh2; tp->nh_pure = c_nhp * (1.0 - c_pd);
+                    tp->nh = x.nh2; tp->nh_pure = c_nhp * (1.0 - c_pd);
                     tp->lock_cost = c_lock_cost + c_ucost; tp->lock_tag = make_tag(c_lock_cnt + 1, episode_new - 1);
                     tp->id = c_tid;   // (unchanged value: the record's second 32 B sector is then written WHOLE - no fill read)
                     P.assigned[(size_t)b * N + k] = c_tid;                               // :308
-                    rev = rev2; cost_sum = cost2;
-                    if (c_lock_cnt == 0) { covered_val += c_value; n0 = n02; }
+                    rev = x.rev2; cost_sum = x.cost2;
+                    if (c_lock_cnt == 0) { covered_val += c_value; n0 = x.n02; }
                     sum_pd += c_pd; sum_pf += c_pf; nA += 1;
                     advance_uav = true;                                                  // :324-325
                 }
@@ -570,7 +585,7 @@ __global__ void __launch_bounds__(kStepThreads, 512 / kStepThreads) step_kernel(
         io.reward[b] = (float)reward;
         io.done[b] = done ? 1 : 0;
         if (io.reward_f64) io.reward_f64[b] = reward;
-        if (io.J_val) io.J_val[b] = (float)(rev - (P.omega * cost_sum));                 // :427
+        if (io.J_val) io.J_val[b] = (float)objective(P, rev, cost_sum);                  // :427
         if (io.num_assigned) io.num_assigned[b] = n0;                                    // :428
         if (io.avg_p_dmg) io.avg_p_dmg[b] = nA > 0 ? (float)(sum_pd / nA) : 0.0f;        // :409
         if (io.avg_p_final) io.avg_p_final[b] = nA > 0 ? (float)(sum_pf / nA) : 0.0f;    // :416
@@ -639,20 +654,15 @@ __global__ void __launch_bounds__(kStepThreads, 512 / kStepThreads) step_kernel(
                 dsth[f * 32] = v;
                 *reinterpret_cast<float2 *>(tile + (kSeqLen - 1) * kStateDim + 2 * f) = v;
             }
-            H.n(I_K) = k; H.n(I_M) = m; H.n(I_NASSIGNED) = nA; H.n(I_NCOVERED) = n0; H.n(I_AGE) = nprev + 1;
-            H.f(F_REV) = rev; H.f(F_COST_SUM) = cost_sum; H.f(F_COVERED_VAL) = covered_val;
-            H.f(F_SUM_PD) = sum_pd; H.f(F_SUM_PF) = sum_pf;
+            store_progress(H, k, m, nA, n0, nprev + 1, rev, cost_sum, covered_val, sum_pd, sum_pf);
         }
     }
     cp_async_wait_all();
     if (inert) {
 #pragma unroll
         for (int f = 0; f < kObsFloats; f += 2) *reinterpret_cast<float2 *>(tile + f) = make_float2(0.f, 0.f);
-        if (!was_finished) {  // the step that finished the episode: freeze the final pointers
-            H.n(I_K) = k; H.n(I_M) = m; H.n(I_NASSIGNED) = nA; H.n(I_NCOVERED) = n0; H.n(I_AGE) = 0;
-            H.f(F_REV) = rev; H.f(F_COST_SUM) = cost_sum; H.f(F_COVERED_VAL) = covered_val;
-            H.f(F_SUM_PD) = sum_pd; H.f(F_SUM_PF) = sum_pf;
-        }
+        if (!was_finished)  // the step that finished the episode: freeze the final pointers
+            store_progress(H, k, m, nA, n0, 0, rev, cost_sum, covered_val, sum_pd, sum_pf);
     }
     // ---- window out: one TMA bulk store per warp (32 x 280 B contiguous in obs) ------------------------
     fence_proxy_async_smem();
@@ -723,9 +733,7 @@ __global__ void __launch_bounds__(kResetThreads) reset_kernel(const __grid_const
             const TgtRec t = P.tgt[P.toff(slot, b)];       // (just cleared)
             eval_pointer_pair(P, u, t, 0.0, 0.0, total_cost, total_val, pf, pd, row);
             store_current_pair(H, u, t, 0, pf, pd);
-            H.n(I_K) = 0; H.n(I_M) = 0; H.n(I_NASSIGNED) = 0; H.n(I_NCOVERED) = 0; H.n(I_AGE) = 1;
-            H.f(F_REV) = 0.0; H.f(F_COST_SUM) = 0.0; H.f(F_COVERED_VAL) = 0.0;
-            H.f(F_SUM_PD) = 0.0; H.f(F_SUM_PF) = 0.0;
+            store_progress(H, 0, 0, 0, 0, 1, 0.0, 0.0, 0.0, 0.0, 0.0);
             H.n(I_FINISHED) = 0;
             H.n(I_EPISODE) = (mode == 0) ? H.n(I_EPISODE) + 1 : 1;
             const uint32_t head = P.step_ctr[0] % (uint32_t)kSeqLen;
@@ -744,19 +752,11 @@ __global__ void __launch_bounds__(kResetThreads) reset_kernel(const __grid_const
 }
 
 // ------------------------------------------------------------------------------------------------
-// Scene injection: device SoA (scene-major) -> records.  Env first_env + e of the range receives scene e / copies, so
+// Scene injection: device uavenv_scene_t -> records.  Env first_env + e of the range receives scene e / copies, so
 // every replica of a scene is packed from the same values by the same instructions: the copies are bit-identical.
 
-struct SceneSoA {
-    const double *uav_x, *uav_y, *uav_vx, *uav_vy, *uav_load, *uav_cost;
-    const int32_t *uav_type;
-    const double *tgt_x, *tgt_y, *tgt_vx, *tgt_vy, *tgt_value;
-    const int32_t *tgt_id;
-    const double *nfz_x, *nfz_y, *nfz_radius, *int_x, *int_y, *int_vx, *int_vy;
-};
-
 __global__ void __launch_bounds__(kResetThreads) pack_scene_kernel(const __grid_constant__ Params P,
-                                                                    const SceneSoA s, int first_env, int count,
+                                                                    const uavenv_scene_t s, int first_env, int count,
                                                                     int copies) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, wpb = blockDim.x >> 5;
     for (int env = blockIdx.x * wpb + warp; env < count; env += gridDim.x * wpb) {
@@ -766,12 +766,12 @@ __global__ void __launch_bounds__(kResetThreads) pack_scene_kernel(const __grid_
         for (int i = lane; i < P.K1; i += 32) {
             NfzRec z; z.x = s.nfz_x[(size_t)e * P.K1 + i]; z.y = s.nfz_y[(size_t)e * P.K1 + i];
             z.radius = s.nfz_radius ? s.nfz_radius[(size_t)e * P.K1 + i] : 0.0;
-            P.nfz[((size_t)slot * P.B + b) * P.K1 + i] = z;
+            P.nfz[P.zoff(slot, b) + i] = z;
         }
         for (int i = lane; i < P.K2; i += 32) {
             IntRec r; r.x = s.int_x[(size_t)e * P.K2 + i]; r.y = s.int_y[(size_t)e * P.K2 + i];
             r.vx = s.int_vx[(size_t)e * P.K2 + i]; r.vy = s.int_vy[(size_t)e * P.K2 + i];
-            P.intc[((size_t)slot * P.B + b) * P.K2 + i] = r;
+            P.intc[P.ioff(slot, b) + i] = r;
         }
         __syncwarp();
         double cost_part = 0.0, val_part = 0.0;
@@ -780,7 +780,7 @@ __global__ void __launch_bounds__(kResetThreads) pack_scene_kernel(const __grid_
             UavRec u;
             u.x = s.uav_x[g]; u.y = s.uav_y[g];
             u.load = s.uav_load[g]; u.cost = s.uav_cost[g];
-            finish_uav(P, slot, b, u, s.uav_vx[g], s.uav_vy[g]);
+            finish_uav(P, P.nfz + P.zoff(slot, b), P.intc + P.ioff(slot, b), u, s.uav_vx[g], s.uav_vy[g]);
             P.uav[P.uoff(slot, b) + i] = u;
             P.uav_vel[P.uoff(slot, b) + i] = make_double2(s.uav_vx[g], s.uav_vy[g]);
             P.uav_type[P.uoff(slot, b) + i] = s.uav_type ? s.uav_type[g] : 1;
@@ -793,7 +793,7 @@ __global__ void __launch_bounds__(kResetThreads) pack_scene_kernel(const __grid_
             const double vx = s.tgt_vx[g], vy = s.tgt_vy[g];
             t.speed = sqrt(vx * vx + vy * vy);
             t.value = s.tgt_value[g];
-            t.nh = 1.0; t.nh_pure = 1.0; t.lock_cost = 0.0; t.lock_tag = 0; t.id = s.tgt_id[g];
+            clear_locks(&t, 0); t.id = s.tgt_id[g];
             P.tgt[P.toff(slot, b) + j] = t;
             P.tgt_vel[P.toff(slot, b) + j] = make_double2(vx, vy);
             val_part += t.value;
@@ -831,10 +831,11 @@ __global__ void __launch_bounds__(256) score_matrix_kernel(const __grid_constant
 #pragma unroll 2
         for (int k = 0; k < P.N; ++k) {
             const UavRec u = U[k];                                    // warp-uniform address
-            const double pd = damage_prob(P, u, tx, ty, ts);
+            double pd;
+            const double pf = pair_score(P, u, tx, ty, ts, &pd);
             if (ok) {
                 if (p_damage) p_damage[out0 + (size_t)k * P.M] = (OutT)pd;
-                if (p_final) p_final[out0 + (size_t)k * P.M] = (OutT)(pd * u.p_pen);
+                if (p_final) p_final[out0 + (size_t)k * P.M] = (OutT)pf;
             }
         }
     }
@@ -866,15 +867,11 @@ __global__ void __launch_bounds__(256) recompute_kernel(const __grid_constant__ 
         const UavRec *U = P.uav + P.uoff(slot, b);
         const int32_t *asg = P.assigned + (size_t)b * P.N;
         for (int i = lane; i < min(P.N, kptr); i += 32) if (asg[i] >= 0) cost += U[i].cost;   // slots at / past the pointer are stale
-        for (int o = 16; o > 0; o >>= 1) {
-            rev += __shfl_xor_sync(0xffffffffu, rev, o);
-            cval += __shfl_xor_sync(0xffffffffu, cval, o);
-            cost += __shfl_xor_sync(0xffffffffu, cost, o);
-            n0 += __shfl_xor_sync(0xffffffffu, n0, o);
-        }
+        rev = warp_sum(rev); cval = warp_sum(cval); cost = warp_sum(cost);
+        n0 = (int)__reduce_add_sync(kFullMask, (unsigned)n0);
         if (lane == 0) {
-            const double J_fresh = rev - (P.omega * cost);
-            const double J_run = P.header(b).f(F_REV) - (P.omega * P.header(b).f(F_COST_SUM));
+            const double J_fresh = objective(P, rev, cost);
+            const double J_run = objective(P, P.header(b).f(F_REV), P.header(b).f(F_COST_SUM));
             worst = fmax(worst, fabs(J_fresh - J_run));
             if (n0 != P.header(b).n(I_NCOVERED)) worst = fmax(worst, 1e30);  // integer state must agree exactly
             if (fix) { P.header(b).f(F_REV) = rev; P.header(b).f(F_COST_SUM) = cost; P.header(b).f(F_COVERED_VAL) = cval; }
@@ -937,33 +934,26 @@ __device__ __forceinline__ uint64_t best_target_key(int episode, int k) {
     return ((uint64_t)(uint32_t)episode << 16) | (uint32_t)k;
 }
 
-// j* of env e's row k (warp-cooperative, all lanes return it): lanes = targets, as in score_matrix_kernel, pair scores as
-// in eval_pointer_pair, new_r as in the step kernel's accept test; then a shuffle arg-max
+// j* of env e's row k (warp-cooperative, all lanes return it): lanes = targets, as in score_matrix_kernel, pair scores
+// (pair_score) and new_r (tentative_assign) as in the step kernel; then a shuffle arg-max
 __device__ __noinline__ uint32_t warp_best_target(const Params &P, int e, int k, int episode) {
     const int lane = threadIdx.x & 31;
     const Hdr h = P.header(e);
     const int slot = h.n(I_GEN) & 1, n0 = h.n(I_NCOVERED);
     const double rev = h.f(F_REV), cost_sum = h.f(F_COST_SUM);
     const UavRec u = P.uav[P.uoff(slot, e) + k];                        // warp-uniform address
-    const double prev_r = paper_reward(rev - (P.omega * cost_sum), n0, P.M);
-    const double cost2 = cost_sum + u.cost;
+    const double prev_r = paper_reward(objective(P, rev, cost_sum), n0, P.M);
     const TgtRec *T = P.tgt + P.toff(slot, e);
     double best = -INFINITY;
     int bj = INT_MAX;
     for (int j = lane; j < P.M; j += 32) {
         TgtRec t = T[j];
         const int cnt = target_view(t, episode);
-        const double pf = damage_prob(P, u, t.x, t.y, t.speed) * u.p_pen;
-        const double nh2 = t.nh * (1.0 - pf);
-        const double rev2 = rev + ((1.0 - nh2) - (1.0 - t.nh)) * t.value;
-        const double r = paper_reward(rev2 - (P.omega * cost2), n0 + (cnt == 0), P.M);
+        const double pf = pair_score(P, u, t.x, t.y, t.speed);
+        const double r = tentative_assign(P, rev, cost_sum, n0, t.nh, t.value, cnt, pf, u.cost).new_r;
         if (r > best) { best = r; bj = j; }                            // j ascends within a lane: the first maximum stays
     }
-    for (int o = 16; o > 0; o >>= 1) {
-        const double ob = __shfl_xor_sync(kFullMask, best, o);
-        const int oj = __shfl_xor_sync(kFullMask, bj, o);
-        if (ob > best || (ob == best && oj < bj)) { best = ob; bj = oj; }
-    }
+    warp_argmax(best, bj);
     return (bj < P.M && best >= prev_r) ? (uint32_t)bj : kNoTarget;
 }
 
@@ -998,10 +988,9 @@ __global__ void __launch_bounds__(kBestTargetThreads) best_target_kernel(const _
 // ------------------------------------------------------------------------------------------------
 // Best member of each group of group_size consecutive envs (include/uavenv_b200.h, uavenv_group_best): one warp per group.
 // Lanes stride over the members (a warp's 32 loads of one header field hit one tile row), keep their first maximum of
-// J = rev - omega * cost_sum (the expression uavenv_get_state evaluates, so the bits agree under -fmad=false), and a
-// shuffle arg-max with the lower index winning a tie picks the group's member.  The warp then copies the winner's
-// assigned[] row along the UAV index.  A group with an unfinished member reports best = -1, J = NaN, N0 = -1 and a row
-// of -1.
+// J = objective(rev, cost_sum) (uavenv_get_state's J), and a shuffle arg-max picks the group's member.  The warp then
+// copies the winner's assigned[] row along the UAV index.  A group with an unfinished member reports best = -1, J = NaN,
+// N0 = -1 and a row of -1.
 
 constexpr int kGroupBestThreads = 256;
 
@@ -1018,16 +1007,12 @@ __global__ void __launch_bounds__(kGroupBestThreads) group_best_kernel(const __g
     bool unfinished = false;
     for (int i = lane; i < group_size; i += 32) {
         const Hdr H = P.header(b0 + i);
-        const double J = H.f(F_REV) - (P.omega * H.f(F_COST_SUM));
+        const double J = objective(P, H.f(F_REV), H.f(F_COST_SUM));
         if (J_all) J_all[(size_t)g * group_size + i] = J;
         unfinished |= H.n(I_FINISHED) == 0;
         if (bi == INT_MAX || J > bJ) { bJ = J; bi = i; }           // i ascends within a lane: the first maximum stays
     }
-    for (int o = 16; o > 0; o >>= 1) {
-        const double oJ = __shfl_xor_sync(kFullMask, bJ, o);
-        const int oi = __shfl_xor_sync(kFullMask, bi, o);
-        if (oi != INT_MAX && (bi == INT_MAX || oJ > bJ || (oJ == bJ && oi < bi))) { bJ = oJ; bi = oi; }
-    }
+    warp_argmax(bJ, bi);
     unfinished = __any_sync(kFullMask, unfinished);
     const Hdr W = P.header(b0 + bi);                                 // (member 0 always exists: bi is a member)
     const int kptr = unfinished ? 0 : W.n(I_K);                      // slots at / past the pointer are stale
@@ -1036,7 +1021,7 @@ __global__ void __launch_bounds__(kGroupBestThreads) group_best_kernel(const __g
     for (int k = lane; k < P.N; k += 32) dst[k] = k < kptr ? src[k] : -1;
     if (lane == 0) {
         best[g] = unfinished ? -1 : bi;
-        J_best[g] = unfinished ? __longlong_as_double(0x7ff8000000000000ll) : bJ;
+        J_best[g] = unfinished ? quiet_nan() : bJ;
         num_covered[g] = unfinished ? -1 : W.n(I_NCOVERED);
     }
 }
@@ -1093,12 +1078,12 @@ __device__ __forceinline__ double improve_prod(const double *p, const int32_t *t
 }
 
 // J of the allocation t from its products: targets summed in list order, then the assigned UAVs' costs in UAV order
-__device__ __forceinline__ double improve_J(const double *nh, const double *val, const double *cost, const int32_t *t,
-                                            int N, int M, double omega) {
+__device__ __forceinline__ double improve_J(const Params &P, const double *nh, const double *val, const double *cost,
+                                            const int32_t *t, int N, int M) {
     double rev = 0.0, c = 0.0;
     for (int j = 0; j < M; ++j) rev += (1.0 - nh[j]) * val[j];
     for (int k = 0; k < N; ++k) if (t[k] >= 0) c += cost[k];
-    return rev - (omega * c);
+    return objective(P, rev, c);
 }
 
 __global__ void __launch_bounds__(kImproveThreads) improve_kernel(const __grid_constant__ Params P, const ImproveIO io) {
@@ -1132,7 +1117,7 @@ __global__ void __launch_bounds__(kImproveThreads) improve_kernel(const __grid_c
             const UavRec u = U[k];                                           // warp-uniform address
             for (int j = lane; j < M; j += 32) {
                 const double tx = T[j].x, ty = T[j].y, ts = T[j].speed;
-                p[(size_t)k * M + j] = damage_prob(P, u, tx, ty, ts) * u.p_pen;
+                p[(size_t)k * M + j] = pair_score(P, u, tx, ty, ts);
             }
         }
         if (tid == 0) sh_n0 = 0;
@@ -1152,7 +1137,7 @@ __global__ void __launch_bounds__(kImproveThreads) improve_kernel(const __grid_c
         if (__syncthreads_or(bad)) {
             for (int k = tid; k < N; k += kImproveThreads) io.assigned_out[(size_t)s * N + k] = -1;
             if (tid == 0) {
-                const double nan = __longlong_as_double(0x7ff8000000000000ll);
+                const double nan = quiet_nan();
                 if (io.J_in) io.J_in[s] = nan;
                 io.J_out[s] = nan; io.num_covered[s] = -1; io.moves[s] = -1; io.converged[s] = 0;
             }
@@ -1164,7 +1149,7 @@ __global__ void __launch_bounds__(kImproveThreads) improve_kernel(const __grid_c
             nhx[k] = t[k] >= 0 ? improve_prod(p, t, N, M, t[k], k, -1, 0, -1, 0) : 1.0;
         __syncthreads();
         if (tid == 0) {
-            sh_J = improve_J(nh, val, cost, t, N, M, omega);
+            sh_J = improve_J(P, nh, val, cost, t, N, M);
             if (io.J_in) io.J_in[s] = sh_J;
         }
         __syncthreads();
@@ -1200,6 +1185,7 @@ __global__ void __launch_bounds__(kImproveThreads) improve_kernel(const __grid_c
                 k2 += kImproveThreads;
                 while (k2 >= N && k1 < N) { ++k1; k2 += k1 + 1 - N; }    // overflow into the next row, which starts at k1 + 1
             }
+            // (not warp_argmax: its INT_MAX guard here and in the cross-warp pass cost 1.5-3 % of the kernel, B200 at 1000 W)
             for (int o = 16; o > 0; o >>= 1) {
                 const double og = __shfl_xor_sync(kFullMask, bg, o);
                 const int oi = __shfl_xor_sync(kFullMask, bi, o), oo = __shfl_xor_sync(kFullMask, bo, o);
@@ -1252,7 +1238,7 @@ __global__ void __launch_bounds__(kImproveThreads) improve_kernel(const __grid_c
         }
         if (first) atomicAdd(&sh_n0, first);
         if (tid == 0) {
-            io.J_out[s] = improve_J(nh, val, cost, t, N, M, omega);
+            io.J_out[s] = improve_J(P, nh, val, cost, t, N, M);
             io.moves[s] = moves;
             io.converged[s] = conv ? 1 : 0;
         }

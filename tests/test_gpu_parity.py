@@ -322,6 +322,14 @@ def test_error_paths():
         env.step(torch.zeros(7, dtype=torch.int64, device="cuda"))
     with pytest.raises(KeyError):
         env.load_scene({"uav_x": np.zeros(30)})
+    # an env range whose end does not fit int32 (1 + INT32_MAX) is refused, not wrapped into [0, B)
+    import ctypes as C
+    from target_allocation_ppo_transformer_b200._capi import UavenvScene, UavenvState
+    L, einval = env._lib, -1                                             # UAVENV_EINVAL (include/uavenv_b200.h)
+    assert L.uavenv_get_scene(env._h, C.byref(UavenvScene()), 1, 2**31 - 1) == einval
+    assert L.uavenv_get_state(env._h, C.byref(UavenvState()), 1, 2**31 - 1) == einval
+    assert L.uavenv_set_episode_counters(env._h, C.byref(C.c_int32(1)), 1, 2**31 - 1) == einval
+    assert b"outside" in L.uavenv_last_error(env._h)
     env.close()
 
 
