@@ -112,7 +112,8 @@ void uavenv_default_cfg(uavenv_cfg_t *cfg);
 int uavenv_create(const uavenv_cfg_t *cfg, int32_t num_envs, int32_t device, uint64_t seed,
                   uint64_t env_id_base, uavenv_t **out);
 int uavenv_destroy(uavenv_t *h);
-/* message of the last failure on this handle (h may be NULL: last creation failure) */
+/* message of the last failure on this handle; with h NULL, of this thread's last failure that had no handle: a
+ * uavenv_create, or a call without a handle (uavenv_episode_accumulate, the ppo_* entry points) */
 const char *uavenv_last_error(const uavenv_t *h);
 int uavenv_abi_version(void);
 int32_t uavenv_num_envs(const uavenv_t *h);

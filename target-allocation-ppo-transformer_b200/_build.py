@@ -25,17 +25,18 @@ COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-I", os.path
 # operation order: no FMA contraction there.
 LIBS = {
     LIB_PATH: [
-        ("uavenv_capi.cu", ["-fmad=false"], ["philox.cuh", "uavenv_device.cuh", "uavenv_kernels.cuh", "../../include/uavenv_b200.h"]),
-        ("ppo_gae.cu", [], ["../../include/uavenv_b200.h"]),
-        ("ppo_attn.cu", [], ["../../include/uavenv_b200.h"]),
-        ("ppo_optim.cu", [], ["../../include/uavenv_b200.h"]),
-        ("uavenv_episodes.cu", [], ["../../include/uavenv_b200.h"]),
+        ("uavenv_capi.cu", ["-fmad=false"], ["handle.cuh", "philox.cuh", "uavenv_device.cuh", "uavenv_kernels.cuh",
+                                             "../../include/uavenv_b200.h"]),
+        ("ppo_gae.cu", [], ["handle.cuh", "../../include/uavenv_b200.h"]),
+        ("ppo_attn.cu", [], ["handle.cuh", "../../include/uavenv_b200.h"]),
+        ("ppo_optim.cu", [], ["handle.cuh", "../../include/uavenv_b200.h"]),
+        ("uavenv_episodes.cu", [], ["handle.cuh", "../../include/uavenv_b200.h"]),
     ],
     POLICY_LIB_PATH: [
         ("policy_dense.cu", [], ["policy_gemm.cuh", "tcgen05_util.cuh", "../../include/uavpolicy_b200.h"]),
-        ("policy_forward.cu", [], ["philox.cuh", "policy_handle.cuh", "policy_kernels.cuh", "policy_weights.cuh", "tcgen05_util.cuh",
+        ("policy_forward.cu", [], ["handle.cuh", "philox.cuh", "policy_kernels.cuh", "policy_weights.cuh", "tcgen05_util.cuh",
                                    "../../include/uavpolicy_b200.h", "../../include/uavpolicy_eval_b200.h"]),
-        ("policy_train.cu", [], ["policy_gemm.cuh", "policy_handle.cuh", "policy_kernels.cuh", "policy_weights.cuh", "../../include/uavpolicy_b200.h"]),
+        ("policy_train.cu", [], ["handle.cuh", "policy_gemm.cuh", "policy_kernels.cuh", "policy_weights.cuh", "../../include/uavpolicy_b200.h"]),
         ("policy_wgrad.cu", [], ["policy_gemm.cuh", "tcgen05_util.cuh", "policy_weights.cuh", "../../include/uavpolicy_b200.h"]),
         ("policy_fused.cu", [], ["policy_kernels.cuh", "tcgen05_util.cuh", "policy_weights.cuh", "../../include/uavpolicy_b200.h"]),
     ],

@@ -6,6 +6,8 @@ missing and cannot be built, or when it reports a failure, an exception is raise
 import ctypes as C
 import os
 
+import torch
+
 from . import _build
 
 STATE_DIM = 14
@@ -157,10 +159,53 @@ def load():
     return L
 
 
-def check(rc, handle=None):
+def check(rc, handle=None, last_error=None):
+    """Raises UavenvError with the library's message when rc != 0: last_error(handle), by default the env library's
+    uavenv_last_error, which with no handle reports this thread's last create or handle-free call that failed."""
     if rc != 0:
-        msg = load().uavenv_last_error(handle)
+        msg = (last_error or load().uavenv_last_error)(handle)
         raise UavenvError(rc, msg.decode() if msg else "(no message)")
+
+
+def cuda_device(device, what):
+    """The torch.device `what` runs on: `device` (None: the current CUDA device), which must be a CUDA device."""
+    dev = torch.device("cuda" if device is None else device)
+    if dev.type != "cuda" or not torch.cuda.is_available():
+        raise RuntimeError("%s runs on a CUDA device (sm_100a) only; there is no CPU fallback" % what)
+    return torch.device("cuda", torch.cuda.current_device()) if dev.index is None else dev
+
+
+class Handle:
+    """One library handle on a CUDA device: created with <prefix>_create, every call checked through
+    <prefix>_last_error, work enqueued on the device's current stream, <prefix>_destroy on close."""
+
+    def __init__(self, load_lib, prefix, device, what):
+        self._h = None
+        self.device = cuda_device(device, what)
+        self._lib, self._prefix = load_lib(), prefix
+        self._last_error = getattr(self._lib, prefix + "_last_error")
+
+    def _create(self, *args):
+        h = C.c_void_p()
+        self._chk(getattr(self._lib, self._prefix + "_create")(*args, C.byref(h)))
+        self._h = h
+
+    def _stream(self):
+        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def _chk(self, rc):
+        check(rc, self._h, self._last_error)
+
+    def close(self):
+        if getattr(self, "_h", None):
+            getattr(self._lib, self._prefix + "_destroy")(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 # ---- policy rollout forward (include/uavpolicy_b200.h, lib/libuavpolicy_b200.so) ---------------------------------

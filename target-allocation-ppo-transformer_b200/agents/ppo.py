@@ -41,15 +41,11 @@ def compute_gae(rewards, values, dones, last_value=None, gamma=0.998, lam=0.95, 
     distributed = group is not None or (torch.distributed.is_available() and torch.distributed.is_initialized()
                                         and torch.distributed.get_world_size() > 1)
     local_norm = int(bool(normalize) and not distributed)
-    rc = lib.ppo_gae_advantages(_ptr(rewards), _ptr(values), _ptr(dones_u8), _ptr(last_value), T, B, float(gamma),
-                                float(lam), _ptr(returns), _ptr(adv), local_norm, _ptr(stats), dev.index, stream)
-    if rc != 0:
-        raise _capi.UavenvError(rc, "ppo_gae_advantages failed")
+    _capi.check(lib.ppo_gae_advantages(_ptr(rewards), _ptr(values), _ptr(dones_u8), _ptr(last_value), T, B, float(gamma),
+                                       float(lam), _ptr(returns), _ptr(adv), local_norm, _ptr(stats), dev.index, stream))
     if normalize and distributed:
         torch.distributed.all_reduce(stats, group=group)
-        rc = lib.ppo_normalize_advantages(_ptr(adv), T * B, _ptr(stats), dev.index, stream)
-        if rc != 0:
-            raise _capi.UavenvError(rc, "ppo_normalize_advantages failed")
+        _capi.check(lib.ppo_normalize_advantages(_ptr(adv), T * B, _ptr(stats), dev.index, stream))
     if squeeze:
         returns, adv = returns[:, 0], adv[:, 0]
     return returns, adv
@@ -58,9 +54,7 @@ def compute_gae(rewards, values, dones, last_value=None, gamma=0.998, lam=0.95, 
 def normalize_advantages(adv, stats):
     lib = _capi.load()
     stream = C.c_void_p(torch.cuda.current_stream(adv.device).cuda_stream)
-    rc = lib.ppo_normalize_advantages(_ptr(adv), adv.numel(), _ptr(stats), adv.device.index, stream)
-    if rc != 0:
-        raise _capi.UavenvError(rc, "ppo_normalize_advantages failed")
+    _capi.check(lib.ppo_normalize_advantages(_ptr(adv), adv.numel(), _ptr(stats), adv.device.index, stream))
     return adv
 
 
@@ -267,13 +261,11 @@ class PPOAgent:
             self._flat_grad.mul_(torch.clamp(c.GRAD_NORM_CLIP / (norm + 1e-6), max=1.0))
             self.optimizer.step()
             return
-        rc = _capi.load().ppo_clip_adam_step(
+        _capi.check(_capi.load().ppo_clip_adam_step(
             _ptr(self._flat_params), _ptr(self._flat_grad), _ptr(self._exp_avg), _ptr(self._exp_avg_sq), self.num_params,
             self._seg_end, self._seg_lr, len(self._seg_lr), 1.0 / self.world, float(c.GRAD_NORM_CLIP), 0.9, 0.999, 1e-8,
             _ptr(self._adam_step), _ptr(self._norm_partials), _ptr(self.grad_norm), self.device.index,
-            C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream))
-        if rc != 0:
-            raise _capi.UavenvError(rc, "ppo_clip_adam_step failed")
+            C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
 
     def launches_per_minibatch(self):
         """Own kernels launched by one minibatch step (bench.py's gpu_launches claim)."""

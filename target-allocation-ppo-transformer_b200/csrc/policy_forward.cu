@@ -13,7 +13,7 @@
 #include <cuda_runtime.h>
 
 #include "philox.cuh"
-#include "policy_handle.cuh"
+#include "handle.cuh"
 #include "policy_kernels.cuh"
 #include "policy_weights.cuh"
 #include "tcgen05_util.cuh"
@@ -105,7 +105,7 @@ __global__ void __launch_bounds__(256) actor_out_kernel(const __nv_bfloat16 *__r
 
 // ------------------------------------------------------------------------------------------------ host side
 
-struct uavpolicy : uavp::Handle {
+struct uavpolicy : capi::Handle {
     int max_batch = 0;
     float *w32 = nullptr;                 // private fp32 copy of the flat parameters
     __nv_bfloat16 *emb2_a = nullptr, *emb2_c = nullptr;   // [128 x 32] tensor-core form of the two embedding weights
@@ -124,11 +124,12 @@ static inline size_t pk(size_t off) { return (off + 7) / 8 * 8; }   // 16 B alig
 
 extern "C" int uavpolicy_abi_version(void) { return UAVPOLICY_ABI_VERSION; }
 
-extern "C" const char *uavpolicy_last_error(const uavpolicy_t *p) { return uavp::last_error(p); }
+extern "C" const char *uavpolicy_last_error(const uavpolicy_t *p) { return capi::last_error(p); }
 
 extern "C" int uavpolicy_create(int32_t device, int32_t max_batch, uavpolicy_t **out) {
     uavpolicy *p;
-    if (const int rc = uavp::new_handle("uavpolicy_create", "max_batch", device, max_batch, out, p)) return rc;
+    if (const int rc = capi::check_create_args("uavpolicy_create", "max_batch", max_batch, out)) return rc;
+    if (const int rc = capi::new_handle("uavpolicy_create", device, p)) return rc;
     p->max_batch = max_batch;
     cudaError_t e = cudaSetDevice(device);
     if (e == cudaSuccess) e = alloc(p, &p->w32, (size_t)UAVPOLICY_NUM_PARAMS);
@@ -141,9 +142,9 @@ extern "C" int uavpolicy_create(int32_t device, int32_t max_batch, uavpolicy_t *
     if (e == cudaSuccess) e = alloc(p, &p->bpk, (size_t)3 * uavp::kLayerBiasElems + 2 * HID * uavp::kBiasK);
     if (e == cudaSuccess) e = alloc(p, &p->emb2_a, (size_t)D * 32);
     if (e == cudaSuccess) e = alloc(p, &p->emb2_c, (size_t)D * 32);
-    if (e != cudaSuccess) return uavp::abandon_handle(p, fail(p, -2, "uavpolicy_create: %s", cudaGetErrorString(e)));
+    if (e != cudaSuccess) return capi::abandon_handle(p, fail(p, -2, "uavpolicy_create: %s", cudaGetErrorString(e)));
     if (uavp::fused_block_prepare() != 0)
-        return uavp::abandon_handle(p, fail(p, -2, "uavpolicy_create: cannot reserve shared memory for the fused kernel"));
+        return capi::abandon_handle(p, fail(p, -2, "uavpolicy_create: cannot reserve shared memory for the fused kernel"));
     bind_fp32(p->actor, p->actor_head, kActorOff, p->w32);
     bind_fp32(p->critic, p->critic_head, kCriticOff, p->w32);
     p->actor.emb_w2p = p->emb2_a; p->critic.emb_w2p = p->emb2_c;
@@ -170,13 +171,13 @@ extern "C" int uavpolicy_create(int32_t device, int32_t max_batch, uavpolicy_t *
     return 0;
 }
 
-extern "C" int uavpolicy_destroy(uavpolicy_t *p) { return uavp::destroy_handle(p); }
+extern "C" int uavpolicy_destroy(uavpolicy_t *p) { return capi::destroy_handle(p); }
 
 extern "C" int uavpolicy_set_weights(uavpolicy_t *p, const float *d_flat_params, void *stream) {
     if (!p || !d_flat_params) return -1;
     cudaStream_t s = (cudaStream_t)stream;
-    UAVP_TRY(p, cudaSetDevice(p->device));
-    UAVP_TRY(p, cudaMemcpyAsync(p->w32, d_flat_params, (size_t)UAVPOLICY_NUM_PARAMS * sizeof(float), cudaMemcpyDeviceToDevice, s));
+    CU_TRY(p, cudaSetDevice(p->device));
+    CU_TRY(p, cudaMemcpyAsync(p->w32, d_flat_params, (size_t)UAVPOLICY_NUM_PARAMS * sizeof(float), cudaMemcpyDeviceToDevice, s));
     // canonical-order copies of every GEMM weight for the fused kernel's bulk-TMA staging
     for (const GemmW &w : kGemmW.w)
         pack_canon_kernel<<<(w.N * w.K + 255) / 256, 256, 0, s>>>(p->w32 + w.off, p->wpk + pk(w.off), w.N, w.K);
@@ -195,7 +196,7 @@ extern "C" int uavpolicy_set_weights(uavpolicy_t *p, const float *d_flat_params,
     }
     emb_w2_kernel<<<(D * 32 + 255) / 256, 256, 0, s>>>(p->actor.emb_w, p->actor.emb_b, p->emb2_a);
     emb_w2_kernel<<<(D * 32 + 255) / 256, 256, 0, s>>>(p->critic.emb_w, p->critic.emb_b, p->emb2_c);
-    UAVP_TRY(p, cudaGetLastError());
+    CU_TRY(p, cudaGetLastError());
     p->have_weights = true;
     return 0;
 }
@@ -207,7 +208,7 @@ extern "C" int uavpolicy_get_action(uavpolicy_t *p, const float *d_obs, int32_t 
     if (!d_obs || !d_action) return fail(p, -1, "uavpolicy_get_action: obs / action must be non-NULL");
     if (B <= 0 || B > p->max_batch) return fail(p, -1, "uavpolicy_get_action: B=%d outside (0, %d]", B, p->max_batch);
     if (!p->have_weights) return fail(p, -4, "uavpolicy_get_action before uavpolicy_set_weights");
-    UAVP_TRY(p, cudaSetDevice(p->device));
+    CU_TRY(p, cudaSetDevice(p->device));
     const cudaStream_t s = (cudaStream_t)stream;
     // two fused launches (actor block + head layer 1, critic block + head layer 1), then the per-sample outputs
     if (uavp::launch_fused_blocks(d_obs, B, p->actor, p->actor_head, p->hh_actor, p->critic, p->critic_head, p->hh_critic,
@@ -216,7 +217,7 @@ extern "C" int uavpolicy_get_action(uavpolicy_t *p, const float *d_obs, int32_t 
     heads_out_kernel<<<(B + 255) / 256, 256, 0, s>>>(p->hh_actor, p->hh_critic, p->actor_head, p->critic_head, B, (uint32_t)seed,
                                                      (uint32_t)(seed >> 32), step, env_id_base, d_action, d_logp, d_value,
                                                      d_entropy, d_logits);
-    UAVP_TRY(p, cudaGetLastError());
+    CU_TRY(p, cudaGetLastError());
     return 0;
 }
 
@@ -230,13 +231,13 @@ extern "C" int uavpolicy_act(uavpolicy_t *p, const float *d_obs, int32_t B, int3
     if (!p) return fail(p, -1, "uavpolicy_act: handle is NULL");
     if (B > p->max_batch) return fail(p, -1, "uavpolicy_act: B=%d outside (0, %d]", B, p->max_batch);
     if (!p->have_weights) return fail(p, -1, "uavpolicy_act before uavpolicy_set_weights");
-    UAVP_TRY(p, cudaSetDevice(p->device));
+    CU_TRY(p, cudaSetDevice(p->device));
     const cudaStream_t s = (cudaStream_t)stream;
     if (uavp::launch_fused_blocks(d_obs, B, p->actor, p->actor_head, p->hh_actor, p->critic, p->critic_head, p->hh_critic,
                                   p->work_counter, p->fused_scratch, s, /*actor_only=*/true))
         return fail(p, -2, "fused block launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     actor_out_kernel<<<(B + 255) / 256, 256, 0, s>>>(p->hh_actor, p->actor_head, B, mode == UAVPOLICY_ACT_GREEDY, (uint32_t)seed,
                                                      (uint32_t)(seed >> 32), step, env_id_base, d_action, d_logp, d_logits);
-    UAVP_TRY(p, cudaGetLastError());
+    CU_TRY(p, cudaGetLastError());
     return 0;
 }

@@ -19,7 +19,7 @@
 #include <cuda_runtime.h>
 
 #include "policy_gemm.cuh"
-#include "policy_handle.cuh"
+#include "handle.cuh"
 #include "policy_kernels.cuh"
 #include "policy_weights.cuh"
 
@@ -711,7 +711,7 @@ struct LastAct { bf16 *KV, *Q, *AL, *XH1, *Y1, *Hs, *XH2; float *rstd1, *rstd2; 
 struct HeadT { bf16 *w1, *w1_t; bf16 *Z, *Hh, *dHh; };                                     // bf16 weights, feature / hidden / gradient rows
 }  // namespace
 
-struct uavtrain : uavp::Handle {
+struct uavtrain : capi::Handle {
     int max_samples = 0, sms = 0, n = 0;
     bf16 *arena = nullptr;                       // bf16 GEMM weights: row-major copies and transposes
     Gemm16 g16[uavp::kNumGemmW];                 // their slices of the arena, in kGemmW order
@@ -856,11 +856,12 @@ void embed_bwd(TCtx &c, const uavp::NetOff &o, int net, float *g, int n, const b
 }
 }  // namespace
 
-extern "C" const char *uavtrain_last_error(const uavtrain_t *p) { return uavp::last_error(p); }
+extern "C" const char *uavtrain_last_error(const uavtrain_t *p) { return capi::last_error(p); }
 
 extern "C" int uavtrain_create(int32_t device, int32_t max_samples, uavtrain_t **out) {
     uavtrain *p;
-    if (const int rc = uavp::new_handle("uavtrain_create", "max_samples", device, max_samples, out, p)) return rc;
+    if (const int rc = capi::check_create_args("uavtrain_create", "max_samples", max_samples, out)) return rc;
+    if (const int rc = capi::new_handle("uavtrain_create", device, p)) return rc;
     p->max_samples = max_samples;
     cudaError_t e = cudaSetDevice(device);
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(&p->sms, cudaDevAttrMultiProcessorCount, device);
@@ -895,9 +896,9 @@ extern "C" int uavtrain_create(int32_t device, int32_t max_samples, uavtrain_t *
     if (e == cudaSuccess) e = alloc(p, &p->relu_mask, R * 8);
     if (e == cudaSuccess) e = alloc(p, &p->zeros, (size_t)3 * D);
     if (e == cudaSuccess) e = cudaMemset(p->zeros, 0, 3 * D * sizeof(float));
-    if (e != cudaSuccess) return uavp::abandon_handle(p, fail(p, -2, "uavtrain_create: %s", cudaGetErrorString(e)));
+    if (e != cudaSuccess) return capi::abandon_handle(p, fail(p, -2, "uavtrain_create: %s", cudaGetErrorString(e)));
     if (uavp::wgrad_prepare() != 0)
-        return uavp::abandon_handle(p, fail(p, -2, "uavtrain_create: cannot reserve shared memory for the weight-gradient kernel"));
+        return capi::abandon_handle(p, fail(p, -2, "uavtrain_create: cannot reserve shared memory for the weight-gradient kernel"));
     size_t a = 0;                                               // slices 64-element aligned: TMA tensor maps are built on them
     auto take = [&](size_t elems) { bf16 *q = p->arena + a; a += (elems + 63) / 64 * 64; return q; };
     for (int i = 0; i < kNumGemmW; ++i) {
@@ -926,12 +927,12 @@ extern "C" int uavtrain_create(int32_t device, int32_t max_samples, uavtrain_t *
     return 0;
 }
 
-extern "C" int uavtrain_destroy(uavtrain_t *p) { return uavp::destroy_handle(p); }
+extern "C" int uavtrain_destroy(uavtrain_t *p) { return capi::destroy_handle(p); }
 
 namespace {
 int forward_impl(uavtrain *p, const float *w, const float *d_obs, int n, float *d_feat, float *d_logits, float *d_value, void *stream) {
     if (n <= 0 || n > p->max_samples) return fail(p, -1, "uavtrain_forward: n=%d outside (0, %d]", n, p->max_samples);
-    UAVP_TRY(p, cudaSetDevice(p->device));
+    CU_TRY(p, cudaSetDevice(p->device));
     TCtx c{p, (cudaStream_t)stream, 0};
     const bool heads = d_logits != nullptr;
     p->n = 0;
@@ -962,18 +963,18 @@ int forward_impl(uavtrain *p, const float *w, const float *d_obs, int n, float *
             head_out_kernel<<<(n + 255) / 256, 256, 0, c.s>>>(p->ahead.Hh, p->chead.Hh, ha.w2, ha.b2, hc.w2, hc.b2, n, d_logits, d_value);
     }
     if (c.rc) return c.rc;
-    UAVP_TRY(p, cudaGetLastError());
+    CU_TRY(p, cudaGetLastError());
     p->n = n;
     p->with_heads = heads;
     return 0;
 }
 
 int backward_impl(uavtrain *p, const float *d_dfeat, const float *d_dlogits, const float *d_dvalue, float *g, void *stream) {
-    UAVP_TRY(p, cudaSetDevice(p->device));
+    CU_TRY(p, cudaSetDevice(p->device));
     TCtx c{p, (cudaStream_t)stream, 0};
     const int n = p->n;
     const bool heads = d_dlogits != nullptr;
-    UAVP_TRY(p, cudaMemsetAsync(g, 0, (size_t)UAVPOLICY_NUM_PARAMS * sizeof(float), c.s));
+    CU_TRY(p, cudaMemsetAsync(g, 0, (size_t)UAVPOLICY_NUM_PARAMS * sizeof(float), c.s));
     if (heads) {
         const HeadOff &ao = kActorOff.head, &co = kCriticOff.head;
         const int warps = p->sms * 8 * 4, spw = max(1, (n + warps - 1) / warps);
@@ -995,7 +996,7 @@ int backward_impl(uavtrain *p, const float *d_dfeat, const float *d_dlogits, con
     full_layer_bwd(c, p->critic.layer[0], p->critic_t[0], kCriticOff.layer[0], g, p->Ec, n, p->fc, p->dXa, p->dXb);
     embed_bwd(c, kCriticOff, 1, g, n, p->dXb, p->dS1);
     if (c.rc) return c.rc;
-    UAVP_TRY(p, cudaGetLastError());
+    CU_TRY(p, cudaGetLastError());
     return 0;
 }
 }  // namespace
@@ -1033,12 +1034,12 @@ extern "C" int uavtrain_ppo_loss(uavtrain_t *p, const float *d_logits, const flo
     if (!p) return -1;
     if (!d_logits || !d_value || !d_action || !d_old_logp || !d_adv || !d_ret || !d_old_value || !d_dlogits || !d_dvalue || n <= 0)
         return fail(p, -1, "uavtrain_ppo_loss: NULL argument or n <= 0");
-    UAVP_TRY(p, cudaSetDevice(p->device));
+    CU_TRY(p, cudaSetDevice(p->device));
     cudaStream_t s = (cudaStream_t)stream;
     PpoLossArgs a{d_logits, d_value, d_old_logp, d_adv, d_ret, d_old_value, d_action, n, eps_clip, c_value, c_entropy};
-    UAVP_TRY(p, cudaMemsetAsync(p->loss_acc, 0, 4 * sizeof(float), s));
+    CU_TRY(p, cudaMemsetAsync(p->loss_acc, 0, 4 * sizeof(float), s));
     ppo_loss_sums_kernel<<<min((n + 255) / 256, p->sms * 4), 256, 0, s>>>(a, p->loss_acc);
     ppo_loss_grad_kernel<<<(n + 255) / 256, 256, 0, s>>>(a, p->loss_acc, d_dlogits, d_dvalue, d_stats);
-    UAVP_TRY(p, cudaGetLastError());
+    CU_TRY(p, cudaGetLastError());
     return 0;
 }

@@ -9,6 +9,8 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
+#include "handle.cuh"
+
 namespace {
 constexpr int S = 5, H = 8, DH = 16;
 
@@ -118,32 +120,44 @@ __global__ void __launch_bounds__(256) attn5_backward_kernel(AttnArgs a, const f
     if (NQ == S) store16(gq + (b * S + t) * a.q_stride + h * DH, dq);
     else if (t == 0) store16(gq + b * a.q_stride + h * DH, dq);
 }
+
+// the checks forward and backward make on the window geometry
+int check_shape(const char *fn, int64_t n, int32_t num_queries, int64_t q_stride, int64_t kv_stride) {
+    if (n <= 0) return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: n must be > 0 (got %lld)", fn, (long long)n);
+    if (num_queries != 1 && num_queries != 5)
+        return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: num_queries %d is neither 1 nor 5", fn, num_queries);
+    if ((q_stride | kv_stride) % 4)
+        return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: q_stride %lld and kv_stride %lld must be multiples of 4", fn,
+                                  (long long)q_stride, (long long)kv_stride);
+    return UAVENV_OK;
+}
 }  // namespace
 
 extern "C" int ppo_attn5_forward(const float *d_q, int64_t q_stride, const float *d_k, const float *d_v, int64_t kv_stride,
                                  const uint8_t *d_pad, int64_t n, int32_t num_queries, float *d_out, int32_t device, void *stream) {
-    if (!d_q || !d_k || !d_v || !d_pad || !d_out || n <= 0 || (num_queries != 1 && num_queries != 5)) return UAVENV_EINVAL;
-    if ((q_stride | kv_stride) % 4) return UAVENV_EINVAL;
-    if (cudaSetDevice(device) != cudaSuccess) return UAVENV_ECUDA;
+    if (!d_q || !d_k || !d_v || !d_pad || !d_out)
+        return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: q / k / v / pad / out must be non-NULL", __func__);
+    if (int rc = check_shape(__func__, n, num_queries, q_stride, kv_stride)) return rc;
+    if (int rc = capi::check_cuda<uavenv>(cudaSetDevice(device), __func__, "cudaSetDevice")) return rc;
     AttnArgs a{d_q, d_k, d_v, q_stride, kv_stride, d_pad, n};
     const int64_t threads = n * H * num_queries;
     const unsigned grid = (unsigned)((threads + 255) / 256);
     if (num_queries == 5) attn5_forward_kernel<5><<<grid, 256, 0, (cudaStream_t)stream>>>(a, d_out);
     else attn5_forward_kernel<1><<<grid, 256, 0, (cudaStream_t)stream>>>(a, d_out);
-    return cudaGetLastError() == cudaSuccess ? UAVENV_OK : UAVENV_ECUDA;
+    return capi::check_cuda<uavenv>(cudaGetLastError(), __func__, "attn5_forward_kernel launch");
 }
 
 extern "C" int ppo_attn5_backward(const float *d_q, int64_t q_stride, const float *d_k, const float *d_v, int64_t kv_stride,
                                   const uint8_t *d_pad, int64_t n, int32_t num_queries, const float *d_grad_out, float *d_grad_q,
                                   float *d_grad_k, float *d_grad_v, int32_t device, void *stream) {
-    if (!d_q || !d_k || !d_v || !d_pad || !d_grad_out || !d_grad_q || !d_grad_k || !d_grad_v || n <= 0 ||
-        (num_queries != 1 && num_queries != 5))
-        return UAVENV_EINVAL;
-    if ((q_stride | kv_stride) % 4) return UAVENV_EINVAL;
-    if (cudaSetDevice(device) != cudaSuccess) return UAVENV_ECUDA;
+    if (!d_q || !d_k || !d_v || !d_pad || !d_grad_out || !d_grad_q || !d_grad_k || !d_grad_v)
+        return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: q / k / v / pad / grad_out / grad_q / grad_k / grad_v must be "
+                                  "non-NULL", __func__);
+    if (int rc = check_shape(__func__, n, num_queries, q_stride, kv_stride)) return rc;
+    if (int rc = capi::check_cuda<uavenv>(cudaSetDevice(device), __func__, "cudaSetDevice")) return rc;
     AttnArgs a{d_q, d_k, d_v, q_stride, kv_stride, d_pad, n};
     const unsigned grid = (unsigned)((n * H * S + 255) / 256);
     if (num_queries == 5) attn5_backward_kernel<5><<<grid, 256, 0, (cudaStream_t)stream>>>(a, d_grad_out, d_grad_q, d_grad_k, d_grad_v);
     else attn5_backward_kernel<1><<<grid, 256, 0, (cudaStream_t)stream>>>(a, d_grad_out, d_grad_q, d_grad_k, d_grad_v);
-    return cudaGetLastError() == cudaSuccess ? UAVENV_OK : UAVENV_ECUDA;
+    return capi::check_cuda<uavenv>(cudaGetLastError(), __func__, "attn5_backward_kernel launch");
 }

@@ -16,6 +16,8 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
+#include "handle.cuh"
+
 namespace {
 
 constexpr int kCols = 32;       // env columns per CTA (one per lane)
@@ -118,30 +120,40 @@ __global__ void normalize_kernel(float *__restrict__ adv, int64_t n, const doubl
 
 extern "C" int ppo_normalize_advantages(float *d_advantages, int64_t n, const double *d_adv_stats, int32_t device,
                                         void *stream) {
-    if (!d_advantages || !d_adv_stats || n <= 0) return UAVENV_EINVAL;
-    if (cudaSetDevice(device) != cudaSuccess) return UAVENV_ECUDA;
+    if (!d_advantages || !d_adv_stats)
+        return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: advantages / adv_stats must be non-NULL", __func__);
+    if (n <= 0) return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: n must be > 0 (got %lld)", __func__, (long long)n);
+    if (int rc = capi::check_cuda<uavenv>(cudaSetDevice(device), __func__, "cudaSetDevice")) return rc;
     const int grid = (int)std::min<int64_t>((n + 255) / 256, 148 * 16);
     normalize_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(d_advantages, n, d_adv_stats);
-    return cudaGetLastError() == cudaSuccess ? UAVENV_OK : UAVENV_ECUDA;
+    return capi::check_cuda<uavenv>(cudaGetLastError(), __func__, "normalize_kernel launch");
 }
 
 extern "C" int ppo_gae_advantages(const float *d_rewards, const float *d_values, const uint8_t *d_dones,
                                   const float *d_last_value, int32_t T, int32_t B, float gamma, float lam,
                                   float *d_returns, float *d_advantages, int32_t normalize, double *d_adv_stats,
                                   int32_t device, void *stream) {
-    if (!d_rewards || !d_values || !d_dones || !d_returns || !d_advantages || T <= 0 || B <= 0) return UAVENV_EINVAL;
-    if (normalize && !d_adv_stats) return UAVENV_EINVAL;  // the statistics buffer is caller-owned (no hidden allocation)
-    if (cudaSetDevice(device) != cudaSuccess) return UAVENV_ECUDA;
+    if (!d_rewards || !d_values || !d_dones || !d_returns || !d_advantages)
+        return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: rewards / values / dones / returns / advantages must be non-NULL",
+                                  __func__);
+    if (T <= 0 || B <= 0)
+        return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: need T > 0 and B > 0 (got %d, %d)", __func__, T, B);
+    if (normalize && !d_adv_stats)  // the statistics buffer is caller-owned (no hidden allocation)
+        return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: normalize needs adv_stats", __func__);
+    if (int rc = capi::check_cuda<uavenv>(cudaSetDevice(device), __func__, "cudaSetDevice")) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     // chunks: as many warps as keep every chunk >= 4 steps, at most 32
     int W = std::max(1, std::min(kMaxChunks, T / 4));
     const int chunk_len = (T + W - 1) / W;
     W = (T + chunk_len - 1) / chunk_len;
-    if (d_adv_stats && cudaMemsetAsync(d_adv_stats, 0, 3 * sizeof(double), s) != cudaSuccess) return UAVENV_ECUDA;
+    if (d_adv_stats) {
+        const cudaError_t e = cudaMemsetAsync(d_adv_stats, 0, 3 * sizeof(double), s);
+        if (int rc = capi::check_cuda<uavenv>(e, __func__, "cudaMemsetAsync")) return rc;
+    }
     const int grid = (B + kCols - 1) / kCols;
     gae_kernel<<<grid, kCols * W, 0, s>>>(d_rewards, d_values, d_dones, d_last_value, T, B, chunk_len, (double)gamma,
                                           (double)lam, d_returns, d_advantages, d_adv_stats);
-    if (cudaGetLastError() != cudaSuccess) return UAVENV_ECUDA;
+    if (int rc = capi::check_cuda<uavenv>(cudaGetLastError(), __func__, "gae_kernel launch")) return rc;
     if (normalize) return ppo_normalize_advantages(d_advantages, (int64_t)T * B, d_adv_stats, device, stream);
     return UAVENV_OK;
 }

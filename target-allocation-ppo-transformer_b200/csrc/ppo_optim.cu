@@ -10,6 +10,8 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
+#include "handle.cuh"
+
 namespace {
 
 constexpr int kThreads = 256;
@@ -98,25 +100,32 @@ extern "C" int ppo_clip_adam_step(float *d_params, float *d_grad, float *d_exp_a
                                   const int64_t *seg_end, const float *seg_lr, int32_t num_segments, float grad_scale,
                                   float max_norm, float beta1, float beta2, float eps, int64_t *d_step,
                                   double *d_partials, float *d_norm_out, int32_t device, void *stream) {
-    if (!d_params || !d_grad || !d_exp_avg || !d_exp_avg_sq || !seg_end || !seg_lr || !d_step || !d_partials || n <= 0)
-        return UAVENV_EINVAL;
-    if (num_segments < 1 || num_segments > PPO_OPTIM_MAX_GROUPS) return UAVENV_EINVAL;
+    if (!d_params || !d_grad || !d_exp_avg || !d_exp_avg_sq || !seg_end || !seg_lr || !d_step || !d_partials)
+        return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: params / grad / exp_avg / exp_avg_sq / seg_end / seg_lr / step / "
+                                  "partials must be non-NULL", __func__);
+    if (n <= 0) return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: n must be > 0 (got %lld)", __func__, (long long)n);
+    if (num_segments < 1 || num_segments > PPO_OPTIM_MAX_GROUPS)
+        return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: num_segments %d outside [1, %d]", __func__, num_segments,
+                                  PPO_OPTIM_MAX_GROUPS);
     Segs segs;
     segs.n = num_segments;
     for (int i = 0; i < PPO_OPTIM_MAX_GROUPS; ++i) {
         segs.end[i] = i < num_segments ? seg_end[i] : n;
         segs.lr[i] = i < num_segments ? seg_lr[i] : 0.f;
-        if (i > 0 && i < num_segments && seg_end[i] < seg_end[i - 1]) return UAVENV_EINVAL;
+        if (i > 0 && i < num_segments && seg_end[i] < seg_end[i - 1])
+            return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: seg_end decreases at segment %d", __func__, i);
     }
-    if (segs.end[num_segments - 1] != n) return UAVENV_EINVAL;
-    if (cudaSetDevice(device) != cudaSuccess) return UAVENV_ECUDA;
+    if (segs.end[num_segments - 1] != n)
+        return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: the last seg_end (%lld) is not n (%lld)", __func__,
+                                  (long long)segs.end[num_segments - 1], (long long)n);
+    if (int rc = capi::check_cuda<uavenv>(cudaSetDevice(device), __func__, "cudaSetDevice")) return rc;
     cudaStream_t s = (cudaStream_t)stream;
     const int nparts = (int)std::min<int64_t>(kMaxParts, (n + 4 * kThreads - 1) / (4 * kThreads));
     sumsq_kernel<<<nparts, kThreads, 0, s>>>(d_grad, n, grad_scale, d_partials, d_step);
     const int grid = (int)std::min<int64_t>((n + kThreads - 1) / kThreads, 148 * 8);
     adam_kernel<<<grid, kThreads, 0, s>>>(d_params, d_grad, d_exp_avg, d_exp_avg_sq, n, segs, grad_scale, max_norm, beta1,
                                           beta2, eps, d_partials, nparts, d_step, d_norm_out);
-    return cudaGetLastError() == cudaSuccess ? UAVENV_OK : UAVENV_ECUDA;
+    return capi::check_cuda<uavenv>(cudaGetLastError(), __func__, "sumsq_kernel / adam_kernel launch");
 }
 
 extern "C" int ppo_optim_partials(void) { return kMaxParts; }

@@ -4,24 +4,21 @@
 #include "uavenv_b200.h"
 
 #include <algorithm>
-#include <cstdarg>
-#include <cstdio>
 #include <cstdlib>
 #include <cstring>
-#include <new>
-#include <string>
 #include <vector>
 
+#include "handle.cuh"
 #include "uavenv_kernels.cuh"
 
 using namespace uavk;
+using capi::fail;
 
-struct uavenv {
+struct uavenv : capi::Handle {
     uavenv_cfg_t cfg;
-    int32_t B = 0, device = 0;
+    int32_t B = 0;
     uint64_t seed = 0, env_id_base = 0;
     Params P;
-    std::vector<void *> allocs;
     float *obs_buf = nullptr;        // [B,5,14] handle-owned window buffer
     int64_t *d_actions = nullptr;    // staging for uavenv_step_host
     float *d_reward = nullptr;
@@ -30,36 +27,7 @@ struct uavenv {
     size_t reset_smem = 0;
     int n_service = 0;
     bool ready = false;              // reset() or load_scene() happened
-    std::string err;
 };
-
-static thread_local std::string g_create_err;
-
-static int fail(uavenv *h, int code, const char *fmt, ...) {
-    char buf[512];
-    va_list ap;
-    va_start(ap, fmt);
-    vsnprintf(buf, sizeof buf, fmt, ap);
-    va_end(ap);
-    if (h) h->err = buf; else g_create_err = buf;
-    return code;
-}
-
-#define CU_TRY(h, expr)                                                                              \
-    do {                                                                                             \
-        cudaError_t e_ = (expr);                                                                     \
-        if (e_ != cudaSuccess)                                                                       \
-            return fail(h, e_ == cudaErrorMemoryAllocation ? UAVENV_ENOMEM : UAVENV_ECUDA,           \
-                        "%s failed: %s", #expr, cudaGetErrorString(e_));                             \
-    } while (0)
-
-template <typename T>
-static cudaError_t dev_alloc(uavenv *h, T **p, size_t n) {
-    void *q = nullptr;
-    cudaError_t e = cudaMalloc(&q, std::max<size_t>(n, 1) * sizeof(T));
-    if (e == cudaSuccess) { h->allocs.push_back(q); *p = static_cast<T *>(q); }
-    return e;
-}
 
 extern "C" void uavenv_default_cfg(uavenv_cfg_t *c) {
     if (!c) return;
@@ -79,7 +47,7 @@ extern "C" void uavenv_default_cfg(uavenv_cfg_t *c) {
 
 extern "C" int uavenv_abi_version(void) { return UAVENV_ABI_VERSION; }
 extern "C" int32_t uavenv_num_envs(const uavenv_t *h) { return h ? h->B : 0; }
-extern "C" const char *uavenv_last_error(const uavenv_t *h) { return h ? h->err.c_str() : g_create_err.c_str(); }
+extern "C" const char *uavenv_last_error(const uavenv_t *h) { return capi::last_error(h); }
 extern "C" float *uavenv_obs_buffer(uavenv_t *h) { return h ? h->obs_buf : nullptr; }
 
 static int create_impl(uavenv *h) {
@@ -105,29 +73,29 @@ static int create_impl(uavenv *h) {
     P.seed_lo = (uint32_t)h->seed; P.seed_hi = (uint32_t)(h->seed >> 32);
     P.env_id_base = (uint32_t)h->env_id_base;
     // scene storage is double-buffered (current scene + the pre-generated next one)
-    CU_TRY(h, dev_alloc(h, &P.uav, 2 * B * N));
-    CU_TRY(h, dev_alloc(h, &P.tgt, 2 * B * M));
-    CU_TRY(h, dev_alloc(h, &P.assigned, B * N));
-    CU_TRY(h, dev_alloc(h, &P.uav_type, 2 * B * N));
-    CU_TRY(h, dev_alloc(h, &P.uav_vel, 2 * B * N));
-    CU_TRY(h, dev_alloc(h, &P.tgt_vel, 2 * B * M));
-    CU_TRY(h, dev_alloc(h, &P.nfz, 2 * B * K1));
-    CU_TRY(h, dev_alloc(h, &P.intc, 2 * B * K2));
+    CU_TRY(h, capi::alloc(h, &P.uav, 2 * B * N));
+    CU_TRY(h, capi::alloc(h, &P.tgt, 2 * B * M));
+    CU_TRY(h, capi::alloc(h, &P.assigned, B * N));
+    CU_TRY(h, capi::alloc(h, &P.uav_type, 2 * B * N));
+    CU_TRY(h, capi::alloc(h, &P.uav_vel, 2 * B * N));
+    CU_TRY(h, capi::alloc(h, &P.tgt_vel, 2 * B * M));
+    CU_TRY(h, capi::alloc(h, &P.nfz, 2 * B * K1));
+    CU_TRY(h, capi::alloc(h, &P.intc, 2 * B * K2));
     // pre-generation service: one CTA per 1024 envs (only when scenes are ever regenerated, and when a warp's
     // shared-memory scratch holds the scene's obstacles)
     const size_t n_svc = (B + kServiceEnvsPerCta - 1) / kServiceEnvsPerCta;
     h->n_service = (c.auto_reset && c.reset_episodes > 0 &&
                     K1 * sizeof(NfzRec) + K2 * sizeof(IntRec) <= (size_t)kServiceScratchPerWarp) ? (int)n_svc : 0;
-    CU_TRY(h, dev_alloc(h, &P.svc_ctr, n_svc));
+    CU_TRY(h, capi::alloc(h, &P.svc_ctr, n_svc));
     CU_TRY(h, cudaMemset(P.svc_ctr, 0, n_svc * sizeof(uint32_t)));
-    CU_TRY(h, dev_alloc(h, &P.q_count, 2));
+    CU_TRY(h, capi::alloc(h, &P.q_count, 2));
     CU_TRY(h, cudaMemset(P.q_count, 0, 2 * sizeof(uint32_t)));
-    CU_TRY(h, dev_alloc(h, &P.q_env, 2 * B));
-    CU_TRY(h, dev_alloc(h, &P.q_gen, 2 * B));
-    CU_TRY(h, dev_alloc(h, &P.q_done, 2 * B));
+    CU_TRY(h, capi::alloc(h, &P.q_env, 2 * B));
+    CU_TRY(h, capi::alloc(h, &P.q_gen, 2 * B));
+    CU_TRY(h, capi::alloc(h, &P.q_done, 2 * B));
     const size_t tiles = (B + 31) / 32;
-    CU_TRY(h, dev_alloc(h, &P.step_ctr, 2));
-    CU_TRY(h, dev_alloc(h, &P.hdr, tiles * kEnvTileBytes));
+    CU_TRY(h, capi::alloc(h, &P.step_ctr, 2));
+    CU_TRY(h, capi::alloc(h, &P.hdr, tiles * kEnvTileBytes));
     {   // headers start zeroed, with "no scene prepared" in the service-owned words
         std::vector<unsigned char> init(tiles * kEnvTileBytes, 0);
         for (size_t b = 0; b < tiles * 32; ++b) {
@@ -138,11 +106,11 @@ static int create_impl(uavenv *h) {
     }
     CU_TRY(h, cudaMemset(P.step_ctr, 0, 2 * sizeof(uint32_t)));
     CU_TRY(h, cudaMemset(P.assigned, 0xff, B * N * sizeof(int32_t)));
-    CU_TRY(h, dev_alloc(h, &h->obs_buf, B * kObsFloats));
-    CU_TRY(h, dev_alloc(h, &h->d_actions, B));
-    CU_TRY(h, dev_alloc(h, &h->d_reward, B));
-    CU_TRY(h, dev_alloc(h, &h->d_done, B));
-    CU_TRY(h, dev_alloc(h, &h->d_scratch, 1));
+    CU_TRY(h, capi::alloc(h, &h->obs_buf, B * kObsFloats));
+    CU_TRY(h, capi::alloc(h, &h->d_actions, B));
+    CU_TRY(h, capi::alloc(h, &h->d_reward, B));
+    CU_TRY(h, capi::alloc(h, &h->d_done, B));
+    CU_TRY(h, capi::alloc(h, &h->d_scratch, 1));
     // per-warp scratch of the scene generator: max(N,M) sort keys, for the 4 warps of a CTA
     h->reset_smem = (size_t)std::max(kWarpsPerCta, kResetThreads / 32) * std::max(N, M) * sizeof(uint32_t);
     if (h->reset_smem > 8 * 1024) {
@@ -160,43 +128,23 @@ static int create_impl(uavenv *h) {
 
 extern "C" int uavenv_create(const uavenv_cfg_t *cfg, int32_t num_envs, int32_t device, uint64_t seed,
                              uint64_t env_id_base, uavenv_t **out) {
-    if (!cfg || !out) return fail(nullptr, UAVENV_EINVAL, "uavenv_create: cfg/out is NULL");
-    *out = nullptr;
-    if (num_envs <= 0) return fail(nullptr, UAVENV_EINVAL, "uavenv_create: num_envs must be > 0 (got %d)", num_envs);
+    if (!cfg) return fail<uavenv>(nullptr, UAVENV_EINVAL, "uavenv_create: cfg is NULL");
+    if (int rc = capi::check_create_args("uavenv_create", "num_envs", num_envs, out)) return rc;
     if (cfg->num_uavs <= 0 || cfg->num_targets <= 0 || cfg->num_nfz < 0 || cfg->num_interceptors < 0)
-        return fail(nullptr, UAVENV_EINVAL, "uavenv_create: need num_uavs > 0, num_targets > 0, obstacles >= 0");
+        return fail<uavenv>(nullptr, UAVENV_EINVAL, "uavenv_create: need num_uavs > 0, num_targets > 0, obstacles >= 0");
     if (cfg->num_uavs > 8192 || cfg->num_targets > 8192)
-        return fail(nullptr, UAVENV_EINVAL, "uavenv_create: num_uavs / num_targets above 8192 are not supported");
+        return fail<uavenv>(nullptr, UAVENV_EINVAL, "uavenv_create: num_uavs / num_targets above 8192 are not supported");
     if (env_id_base + (uint64_t)num_envs > 0xffffffffull)
-        return fail(nullptr, UAVENV_EINVAL, "uavenv_create: global env ids must fit 32 bits");
-    int ndev = 0;
-    cudaError_t e = cudaGetDeviceCount(&ndev);
-    if (e != cudaSuccess || ndev == 0)
-        return fail(nullptr, UAVENV_ECUDA, "uavenv_create: no CUDA device (%s); there is no CPU fallback",
-                    e != cudaSuccess ? cudaGetErrorString(e) : "device count 0");
-    if (device < 0 || device >= ndev) return fail(nullptr, UAVENV_EINVAL, "uavenv_create: device %d out of range", device);
-    uavenv *h = new (std::nothrow) uavenv();
-    if (!h) return fail(nullptr, UAVENV_ENOMEM, "uavenv_create: out of host memory");
-    h->cfg = *cfg; h->B = num_envs; h->device = device; h->seed = seed; h->env_id_base = env_id_base;
-    int rc = create_impl(h);
-    if (rc != UAVENV_OK) {
-        g_create_err = h->err;
-        for (void *p : h->allocs) cudaFree(p);
-        delete h;
-        return rc;
-    }
+        return fail<uavenv>(nullptr, UAVENV_EINVAL, "uavenv_create: global env ids must fit 32 bits");
+    uavenv *h;
+    if (int rc = capi::new_handle("uavenv_create", device, h)) return rc;
+    h->cfg = *cfg; h->B = num_envs; h->seed = seed; h->env_id_base = env_id_base;
+    if (int rc = create_impl(h)) return capi::abandon_handle(h, rc);
     *out = h;
     return UAVENV_OK;
 }
 
-extern "C" int uavenv_destroy(uavenv_t *h) {
-    if (!h) return UAVENV_OK;
-    cudaSetDevice(h->device);
-    cudaDeviceSynchronize();
-    for (void *p : h->allocs) cudaFree(p);
-    delete h;
-    return UAVENV_OK;
-}
+extern "C" int uavenv_destroy(uavenv_t *h) { return capi::destroy_handle(h); }
 
 static int launch_check(uavenv *h, const char *what) {
     cudaError_t e = cudaGetLastError();

@@ -8,6 +8,8 @@
 #include <cstdint>
 #include <cuda_runtime.h>
 
+#include "handle.cuh"
+
 static_assert(sizeof(uavenv_episode_t) == 40, "uavenv_episode_t layout");
 
 namespace {
@@ -49,16 +51,20 @@ __global__ void __launch_bounds__(256) episode_accumulate_kernel(int B, const in
 extern "C" int uavenv_episode_accumulate(int32_t B, const int64_t *d_actions, const uint8_t *d_done, const uavenv_info_t *info,
                                          int32_t episodes_per_env, const uavenv_episode_acc_t *acc, uavenv_episode_t *d_records,
                                          int32_t device, void *stream) {
-    if (B <= 0 || episodes_per_env <= 0 || !d_actions || !d_done || !info || !acc || !d_records) return UAVENV_EINVAL;
+    if (B <= 0 || episodes_per_env <= 0)
+        return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: need B > 0 and episodes_per_env > 0 (got %d, %d)", __func__, B,
+                                  episodes_per_env);
+    if (!d_actions || !d_done || !info || !acc || !d_records)
+        return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: actions / done / info / acc / records must be non-NULL", __func__);
     if (!info->d_reward_f64 || !info->d_J_val || !info->d_avg_p_dmg || !info->d_avg_p_final || !info->d_num_assigned ||
         !info->d_is_valid_action)
-        return UAVENV_EINVAL;
+        return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: every array of info must be non-NULL", __func__);
     if (!acc->d_ret || !acc->d_length || !acc->d_assigns || !acc->d_valid || !acc->d_episodes || !acc->d_envs_complete)
-        return UAVENV_EINVAL;
-    if (cudaSetDevice(device) != cudaSuccess) return UAVENV_ECUDA;
+        return capi::fail<uavenv>(nullptr, UAVENV_EINVAL, "%s: every array of acc must be non-NULL", __func__);
+    if (int rc = capi::check_cuda<uavenv>(cudaSetDevice(device), __func__, "cudaSetDevice")) return rc;
     const InfoIn in = {info->d_reward_f64, info->d_J_val, info->d_avg_p_dmg, info->d_avg_p_final, info->d_num_assigned,
                        info->d_is_valid_action};
     episode_accumulate_kernel<<<(B + 255) / 256, 256, 0, (cudaStream_t)stream>>>(B, d_actions, d_done, in, episodes_per_env, *acc,
                                                                                   d_records);
-    return cudaGetLastError() == cudaSuccess ? UAVENV_OK : UAVENV_ECUDA;
+    return capi::check_cuda<uavenv>(cudaGetLastError(), __func__, "episode_accumulate_kernel launch");
 }

@@ -39,7 +39,7 @@ class _Box:                # stand-in for gym.spaces.Box (envs/uav_env.py:21-24)
         self.low, self.high, self.shape, self.dtype = -np.inf, np.inf, tuple(shape), np.float32
 
 
-class UAVEnvBatched:
+class UAVEnvBatched(_capi.Handle):
     """B independent UAV->target allocation envs on one B200.
 
     reset(full_reset=True) -> obs[B,5,14] f32 (CUDA)
@@ -54,15 +54,8 @@ class UAVEnvBatched:
 
     def __init__(self, num_envs, device=None, seed=None, config=None, auto_reset=True, env_id_base=0,
                  with_info=True, tie_band=1e-12):
-        self._h = None
-        if not torch.cuda.is_available():
-            raise RuntimeError("UAVEnvBatched needs a CUDA device (sm_100a); there is no CPU fallback")
+        super().__init__(_capi.load, "uavenv", device, "UAVEnvBatched")
         self.cfg = (config if config is not None else _global_cfg).copy()
-        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
-        if self.device.type != "cuda":
-            raise ValueError("device must be a CUDA device")
-        if self.device.index is None:
-            self.device = torch.device("cuda", torch.cuda.current_device())
         self.num_envs = int(num_envs)
         self.seed = int(self.cfg.SEED if seed is None else seed)
         self.env_id_base = int(env_id_base)
@@ -71,12 +64,8 @@ class UAVEnvBatched:
         self.K1, self.K2 = int(self.cfg.NUM_NFZ), int(self.cfg.NUM_INTERCEPTORS)
         self.action_space = _Discrete(self.cfg.ACTION_DIM)
         self.observation_space = _Box((self.cfg.SEQ_LEN, self.cfg.STATE_DIM))
-        self._lib = _capi.load()
         ccfg = self.cfg.to_c(auto_reset=self.auto_reset, tie_band=tie_band)
-        h = C.c_void_p()
-        _capi.check(self._lib.uavenv_create(C.byref(ccfg), self.num_envs, self.device.index, self.seed,
-                                            self.env_id_base, C.byref(h)))
-        self._h = h
+        self._create(C.byref(ccfg), self.num_envs, self.device.index, self.seed, self.env_id_base)
         B, dev = self.num_envs, self.device
         self.obs = torch.zeros(B, _capi.SEQ_LEN, _capi.STATE_DIM, dtype=torch.float32, device=dev)
         # per-step outputs are carved out of ONE allocation (8-byte aligned slices): fewer distinct pages per launch
@@ -114,24 +103,6 @@ class UAVEnvBatched:
         self._h_reward = self._h_done = None
         self._best_target_cache = None        # best_target_actions' per-env entries, allocated on first use
         self._improve_workspace = None        # improve_allocation's p slices (large N*M only), allocated on first use
-
-    # ------------------------------------------------------------------ lifecycle
-    def close(self):
-        if getattr(self, "_h", None):
-            self._lib.uavenv_destroy(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-
-    def _chk(self, rc):
-        _capi.check(rc, self._h)
 
     # ------------------------------------------------------------------ reset / step
     def reset(self, full_reset=True, env_mask=None):

@@ -132,14 +132,10 @@ def _summary(res, env_steps, wall):
 
 def _eval_setup(num_envs, episodes_per_env, config, device, env_id_base):
     """(device, num_envs, quota, cfg, rank's first global env id, world size) of an evaluation run, arguments checked."""
-    device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
-    if device.type != "cuda":
-        raise RuntimeError("evaluate runs on a CUDA device (sm_100a); there is no CPU fallback")
-    if device.index is None:
-        device = torch.device("cuda", torch.cuda.current_device())
     num_envs, quota = int(num_envs), int(episodes_per_env)
     if num_envs <= 0 or quota <= 0:
         raise ValueError("num_envs and episodes_per_env must be positive")
+    device = _capi.cuda_device(device, "evaluate")
     cfg = (config if config is not None else _global_cfg).copy(RESET_EPISODES=1)   # a fresh scene every episode
     rank, world = _world()
     base = rank * num_envs if env_id_base is None else int(env_id_base)

@@ -30,10 +30,8 @@ class _Attention5(torch.autograd.Function):
         out = torch.empty(n, nq, 128, dtype=torch.float32, device=q.device)
         lib = _capi.load()
         stream = C.c_void_p(torch.cuda.current_stream(q.device).cuda_stream)
-        rc = lib.ppo_attn5_forward(_ptr(q), _rows(q), _ptr(k), _ptr(v), _rows(k), _ptr(pad_u8), n, nq, _ptr(out),
-                                   q.device.index, stream)
-        if rc != 0:
-            raise _capi.UavenvError(rc, "ppo_attn5_forward failed")
+        _capi.check(lib.ppo_attn5_forward(_ptr(q), _rows(q), _ptr(k), _ptr(v), _rows(k), _ptr(pad_u8), n, nq, _ptr(out),
+                                          q.device.index, stream))
         ctx.save_for_backward(q, k, v, pad_u8)
         return out
 
@@ -48,10 +46,8 @@ class _Attention5(torch.autograd.Function):
             gq, gk, gv = (torch.empty_strided(t.shape, t.stride(), dtype=t.dtype, device=t.device) for t in (q, k, v))
         lib = _capi.load()
         stream = C.c_void_p(torch.cuda.current_stream(q.device).cuda_stream)
-        rc = lib.ppo_attn5_backward(_ptr(q), _rows(q), _ptr(k), _ptr(v), _rows(k), _ptr(pad_u8), n, nq, _ptr(grad_out),
-                                    _ptr(gq), _ptr(gk), _ptr(gv), q.device.index, stream)
-        if rc != 0:
-            raise _capi.UavenvError(rc, "ppo_attn5_backward failed")
+        _capi.check(lib.ppo_attn5_backward(_ptr(q), _rows(q), _ptr(k), _ptr(v), _rows(k), _ptr(pad_u8), n, nq,
+                                           _ptr(grad_out), _ptr(gq), _ptr(gk), _ptr(gv), q.device.index, stream))
         return gq, gk, gv, None
 
 

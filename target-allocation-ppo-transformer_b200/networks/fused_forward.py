@@ -23,48 +23,10 @@ def flatten_params(module):
     return flat
 
 
-class _PolicyHandle:
-    """One handle of the policy library on a CUDA device: created with <_api>_create, every call checked through
-    <_api>_last_error, work enqueued on the device's current stream, <_api>_destroy on close.  _api is "uavpolicy"
-    (FusedPolicyForward) or "uavtrain" (networks/fused_train.py: FusedTrunks)."""
-    _api = None
-
-    def __init__(self, size, device, what):
-        self._h = None
-        self.device = torch.device(device)
-        if self.device.type != "cuda":
-            raise RuntimeError("%s runs on a CUDA device (sm_100a) only" % what)
-        if self.device.index is None:
-            self.device = torch.device("cuda", torch.cuda.current_device())
-        self._lib = _capi.load_policy()
-        h = C.c_void_p()
-        self._chk(getattr(self._lib, self._api + "_create")(self.device.index, int(size), C.byref(h)))
-        self._h = h
-
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-
-    def _chk(self, rc):
-        if rc != 0:
-            raise _capi.UavenvError(rc, (getattr(self._lib, self._api + "_last_error")(self._h) or b"").decode())
-
-    def close(self):
-        if getattr(self, "_h", None):
-            getattr(self._lib, self._api + "_destroy")(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-
-class FusedPolicyForward(_PolicyHandle):
-    _api = "uavpolicy"
-
+class FusedPolicyForward(_capi.Handle):
     def __init__(self, max_batch, device, seed=0, env_id_base=0):
-        super().__init__(max_batch, device, "the fused policy forward")
+        super().__init__(_capi.load_policy, "uavpolicy", device, "the fused policy forward")
+        self._create(self.device.index, int(max_batch))
         self.max_batch, self.seed, self.env_id_base = int(max_batch), int(seed), int(env_id_base)
         dev = self.device
         self.action = torch.zeros(max_batch, dtype=torch.int64, device=dev)

@@ -12,7 +12,7 @@ import ctypes as C
 import torch
 
 from .. import _capi
-from .fused_forward import _PolicyHandle, flatten_params
+from .fused_forward import flatten_params
 
 
 class _TrunkFn(torch.autograd.Function):
@@ -68,11 +68,10 @@ class _PolicyFn(torch.autograd.Function):
         return None, None, grad
 
 
-class FusedTrunks(_PolicyHandle):
-    _api = "uavtrain"
-
+class FusedTrunks(_capi.Handle):
     def __init__(self, max_samples, device):
-        super().__init__(max_samples, device, "the fused PPO update")
+        super().__init__(_capi.load_policy, "uavtrain", device, "the fused PPO update")
+        self._create(self.device.index, int(max_samples))
         self.max_samples = int(max_samples)
         self._pending = 0
         self._work = None

@@ -87,6 +87,49 @@ def test_create_validates_arguments_without_gpu():
     assert isinstance(_capi.UavenvError(-1, "x"), RuntimeError)
 
 
+def test_handle_free_calls_report_their_arguments_without_gpu():
+    """Every entry point without a handle leaves its failure in uavenv_last_error(NULL), naming itself and the argument;
+    _capi.check raises it."""
+    from target_allocation_ppo_transformer_b200 import _capi
+    L = ub.load_library()
+    p = 64                            # never dereferenced: validation fails first
+
+    def message(rc):
+        assert rc == -1
+        return L.uavenv_last_error(None).decode()
+
+    def gae(rewards=p, T=4, B=8, normalize=0, stats=None):
+        return L.ppo_gae_advantages(rewards, p, p, None, T, B, 0.99, 0.95, p, p, normalize, stats, 0, None)
+
+    assert message(gae(rewards=None)).startswith("ppo_gae_advantages: rewards /")
+    assert message(gae(T=0)) == "ppo_gae_advantages: need T > 0 and B > 0 (got 0, 8)"
+    assert message(gae(B=-1)) == "ppo_gae_advantages: need T > 0 and B > 0 (got 4, -1)"
+    assert message(gae(normalize=1)) == "ppo_gae_advantages: normalize needs adv_stats"
+    assert message(L.ppo_normalize_advantages(p, 8, None, 0, None)).startswith("ppo_normalize_advantages: advantages /")
+    assert message(L.ppo_normalize_advantages(p, 0, p, 0, None)) == "ppo_normalize_advantages: n must be > 0 (got 0)"
+
+    def attn(q=p, n=8, nq=5, q_stride=128):
+        return L.ppo_attn5_forward(q, q_stride, p, p, 384, p, n, nq, p, 0, None)
+
+    assert message(attn(q=None)).startswith("ppo_attn5_forward: q /")
+    assert message(attn(n=0)) == "ppo_attn5_forward: n must be > 0 (got 0)"
+    assert message(attn(nq=3)) == "ppo_attn5_forward: num_queries 3 is neither 1 nor 5"
+    assert "multiples of 4" in message(attn(q_stride=130))
+
+    def adam(params=p, n=10, ends=(4, 10), num_segments=None):
+        seg_end, seg_lr = (C.c_int64 * len(ends))(*ends), (C.c_float * len(ends))(*[1e-3] * len(ends))
+        return L.ppo_clip_adam_step(params, p, p, p, n, seg_end, seg_lr, len(ends) if num_segments is None else num_segments,
+                                    1.0, 0.5, 0.9, 0.999, 1e-8, p, p, None, 0, None)
+
+    assert message(adam(params=None)).startswith("ppo_clip_adam_step: params /")
+    assert message(adam(n=0, ends=(0,))) == "ppo_clip_adam_step: n must be > 0 (got 0)"
+    assert message(adam(num_segments=0)).startswith("ppo_clip_adam_step: num_segments 0 outside [1, ")
+    assert message(adam(ends=(6, 4, 10))) == "ppo_clip_adam_step: seg_end decreases at segment 1"
+    assert message(adam(ends=(4, 9))) == "ppo_clip_adam_step: the last seg_end (9) is not n (10)"
+    with pytest.raises(_capi.UavenvError, match="error -1: ppo_normalize_advantages: n must be > 0"):
+        _capi.check(L.ppo_normalize_advantages(p, 0, p, 0, None))
+
+
 def test_config_mirror_reads_like_the_reference():
     cfg = ub.Config()
     assert cfg.UAV_GEN_X_RANGE == (60, 90) and cfg.GAMMA == 0.998 and cfg.GAE_LAMBDA == 0.95

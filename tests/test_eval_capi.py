@@ -62,16 +62,22 @@ def test_episode_accumulate_validates_arguments_without_gpu():
         return L.uavenv_episode_accumulate(B, actions, done, C.byref(ic) if info else None, quota,
                                            C.byref(ac) if acc else None, records, 0, None)
 
-    assert call(B=0) == -1
-    assert call(quota=0) == -1 and call(quota=-1) == -1
-    assert call(actions=None) == -1 and call(done=None) == -1 and call(records=None) == -1
-    assert call(info=False) == -1 and call(acc=False) == -1
+    def rejected(**kw):               # -1, with a message for uavenv_last_error(NULL) that names the function
+        assert L.ppo_normalize_advantages(None, 1, None, 0, None) == -1       # another message in between
+        rc, msg = call(**kw), L.uavenv_last_error(None)
+        return rc == -1 and msg.startswith(b"uavenv_episode_accumulate: ")
+
+    assert rejected(B=0)
+    assert rejected(quota=0) and rejected(quota=-1)
+    assert rejected(actions=None) and rejected(done=None) and rejected(records=None)
+    assert rejected(info=False) and rejected(acc=False)
     for name in info_fields:
-        assert call(info_null=name) == -1, name
+        assert rejected(info_null=name), name
     for name in acc_fields:
-        assert call(acc_null=name) == -1, name
+        assert rejected(acc_null=name), name
     if not torch.cuda.is_available():
         assert call() == -2           # valid arguments: the device is needed
+        assert L.uavenv_last_error(None).startswith(b"uavenv_episode_accumulate: cudaSetDevice failed")
 
 
 def test_evaluate_refuses_a_cpu_device():
