@@ -230,9 +230,40 @@ int uavenv_improve_allocation(uavenv_t *h, int32_t first_env, int32_t count, int
                               const int32_t *d_assigned_in, int32_t max_moves, int32_t *d_assigned_out, double *d_J_in,
                               double *d_J_out, int32_t *d_num_covered, int32_t *d_moves, uint8_t *d_converged,
                               void *d_workspace, void *stream);
-/* bytes of the workspace uavenv_improve_allocation needs: 0 when p[N][M] fits the kernel's shared memory (N*M <= 8192),
+/* bytes of the workspace uavenv_improve_allocation and uavenv_upper_bound need: 0 when p[N][M] fits the kernel's shared memory (N*M <= 8192),
  * otherwise N*M*8 per SM of the handle's device (L2-resident slices). */
 size_t uavenv_improve_workspace_bytes(const uavenv_t *h);
+
+/* Certified upper bound on the best J of the scenes held by envs first_env + s*env_stride, s in [0, count): no
+ * allocation of scene s has J above d_bound[s].  With a_kj = min(-log1p(-p[k][j]), A), A = 40 (p as in
+ * uavenv_improve_allocation; the cap keeps a finite where p = 1) and x_kj in {0,1}, sum_j x_kj <= 1, every allocation has
+ *   J(x) <= F(x) + sum_j v_j e^-A,   F(x) = sum_j v_j (1 - exp(-sum_k a_kj x_kj)) - omega sum_k c_k sum_j x_kj
+ * (where a cap is active, exp(-sum_k a_kj x_kj) <= e^-A, so target j loses at most v_j e^-A).  F is concave, so over the
+ * relaxation x_kj in [0,1], sum_j x_kj <= 1, every feasible x gives F* <= F(x) + max_{vertex y} grad F(x).(y - x) =: U;
+ * U is a valid bound at every feasible x, whatever the step sizes that reached it.  x enters only through
+ * s_j = sum_k a_kj x_kj and C = sum_k c_k sum_j x_kj, which the iteration keeps (never x), in fp64:
+ *   start s = 0, C = 0 (the empty allocation).  Iteration t = 1, 2, ...:
+ *     nh_j = exp(-s_j), w_j = v_j nh_j;  F = sum_j v_j (1 - nh_j) - omega C, targets in list order;
+ *     g_kj = w_j a_kj - omega c_k; UAV k picks j*_k = argmax_j g_kj (lowest j on a tie) if that maximum is > 0, else none;
+ *     U_t = (F + sum_{k picks} g_kj*) - (sum_j w_j s_j - omega C), both sums in ascending index;
+ *     stop if U_t - F <= 1e-9 max(1, |U_t|) (the relaxation is solved) or t = iters;
+ *     sigma_j = sum_{k picks j} a_kj and C_sigma = sum_{k picks} c_k in ascending k; d = sigma - s, dC = C_sigma - C;
+ *     gamma in [0,1] (every gamma keeps x feasible: validity never depends on it) maximises the concave
+ *     phi(gamma) = F(s + gamma d, C + gamma dC) by: gamma = 1 if phi'(1) >= 0; otherwise lo = 0, hi = 1, gamma = 1 and
+ *     up to 10 times { c = gamma - phi'(gamma)/phi''(gamma); stop if c == gamma (converged: without this test a
+ *     sub-ulp step would land on the bracket end and send gamma to the midpoint); the midpoint of (lo, hi) unless
+ *     lo < c < hi; gamma = c; phi'(gamma) > 0 ? lo = gamma : hi = gamma }, with phi'(gamma) = sum_j (v_j e_j) d_j - omega dC and
+ *     -phi''(gamma) = sum_j ((v_j e_j) d_j) d_j, e_j = exp(-(s_j + gamma d_j)), each reduced over targets in a fixed
+ *     order (csrc/uavenv_kernels.cuh, block_sum2);
+ *     s += gamma d, C += gamma dC.
+ * Outputs per s: d_bound = min_t U_t + (sum_j v_j) e^-A + 1e-12 (sum_j v_j + omega sum_k c_k) (the last term covers fp64
+ * rounding), d_relaxed = F at the last iterate (d_bound - d_relaxed shows whether more iterations would help) and
+ * d_iters = the iterations run (<= iters; iteration t takes no step when it stops).  d_workspace as for
+ * uavenv_improve_allocation (uavenv_improve_workspace_bytes).  One launch on `stream`, asynchronous; results do not depend
+ * on count, env_stride or the launch.  UAVENV_EINVAL (before the GPU is touched) on a NULL output or required workspace,
+ * count <= 0, env_stride <= 0, iters < 1 or an env outside [0, B); UAVENV_ESTATE before any reset / scene load. */
+int uavenv_upper_bound(uavenv_t *h, int32_t first_env, int32_t count, int32_t env_stride, int32_t iters, double *d_bound,
+                       double *d_relaxed, int32_t *d_iters, void *d_workspace, void *stream);
 
 /* ---- per-episode records of an evaluation (csrc/uavenv_episodes.cu) ---------------------------------------------
  * One finished episode.  ret sums the fp64 step rewards (info d_reward_f64) in step order; J_val, avg_p_dmg,

@@ -30,7 +30,7 @@ def __getattr__(name):  # torch / CUDA are only touched when the env classes are
     if name in ("evaluate", "evaluate_baseline", "EpisodeRecorder", "load_checkpoint"):
         from . import evaluation
         return getattr(evaluation, name)
-    if name in ("allocate", "improve_allocation"):
+    if name in ("allocate", "improve_allocation", "upper_bound"):
         from . import allocation
         return getattr(allocation, name)
     if name in ("analyze_environment_difficulty", "record_decisions"):

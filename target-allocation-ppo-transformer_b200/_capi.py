@@ -129,6 +129,7 @@ def load():
     L.uavenv_improve_allocation.argtypes = [vp, i32, i32, i32, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp]
     L.uavenv_improve_workspace_bytes.argtypes = [vp]
     L.uavenv_improve_workspace_bytes.restype = C.c_size_t
+    L.uavenv_upper_bound.argtypes = [vp, i32, i32, i32, i32, vp, vp, vp, vp, vp]
     L.uavenv_get_scene.argtypes = [vp, C.POINTER(UavenvScene), i32, i32]
     L.uavenv_get_state.argtypes = [vp, C.POINTER(UavenvState), i32, i32]
     L.uavenv_set_episode_counters.argtypes = [vp, vp, i32, i32]
@@ -153,7 +154,7 @@ def load():
                  "uavenv_load_scene", "uavenv_get_scene", "uavenv_get_state", "uavenv_score_matrix",
                  "uavenv_score_matrix_f64", "uavenv_recompute_objective", "uavenv_random_actions", "uavenv_best_target_actions",
                  "uavenv_episode_accumulate", "ppo_gae_advantages", "ppo_normalize_advantages",
-                 "uavenv_load_scene_device", "uavenv_group_best", "uavenv_improve_allocation"):
+                 "uavenv_load_scene_device", "uavenv_group_best", "uavenv_improve_allocation", "uavenv_upper_bound"):
         getattr(L, name).restype = C.c_int
     _lib = L
     return L

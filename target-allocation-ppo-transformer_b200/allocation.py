@@ -7,6 +7,9 @@
     pol = ub.improve_allocation(my_scenes, res["assigned_target_id"])   # local search from any allocation
     pol["assigned_target_id"], pol["J"], pol["J_before"]
 
+    ub_ = ub.upper_bound(my_scenes)     # certified: no allocation of scene s beats ub_["bound"][s]
+    gap = ub_["bound"] - pol["J"]       # how far an allocation can be from the optimum, at most
+
 Each scene is played K times in K envs of one UAVEnvBatched built with auto_reset=False, so a finished episode keeps its
 final allocation on the device.  Per chunk of scenes: uavenv_load_scene_device puts every scene into its K envs (no host
 round trip), the loop act -> step runs until all of the chunk's envs are done (a poll every POLL_STEPS steps), and
@@ -19,6 +22,10 @@ Local search (improve_allocation, allocate(improve=True)): uavenv_improve_alloca
 rises (steepest ascent; the rule is in include/uavenv_b200.h), on the device, a scene per CTA.  allocate runs it on the
 first env of each scene's group right after group_best - every member holds the same scene - so no second scene load
 is needed.
+
+Upper bound (upper_bound, allocate(bound=True)): uavenv_upper_bound runs Frank-Wolfe on the concave relaxation of J and
+returns min_t of its duality bound plus a stated margin, a value no allocation of the scene exceeds (the rule and its
+proof are in include/uavenv_b200.h).  allocate runs it on the same env as the local search.
 """
 import copy
 import time
@@ -53,7 +60,7 @@ def _max_moves(max_moves):
 
 
 def allocate(policy, scenes=None, num_scenes=None, samples=1, greedy=None, seed=DEFAULT_SEED, config=None, device=None,
-             max_envs=65536, improve=False):
+             max_envs=65536, improve=False, bound=False):
     """Allocate the targets of S scenes: play each scene `samples` (K) times with the policy and return the best
     episode's allocation per scene.
 
@@ -64,6 +71,7 @@ def allocate(policy, scenes=None, num_scenes=None, samples=1, greedy=None, seed=
     (default when K == 1); otherwise actions sampled keyed (seed, step, s*K + c).  config: sizes and constants (default
     the global cfg).  max_envs: the most envs played at once; scenes go through in chunks of max_envs // K.
     improve: polish each scene's best allocation with the local search of improve_allocation (cap 16 * N moves).
+    bound: also compute each scene's certified upper bound on J (upper_bound, 256 iterations).
 
     Returns numpy arrays: "assigned_target_id" int32 [S, N], "J" f64 [S] (the value get_state reports as J_val),
     "num_covered" int32 [S] (N0), "best_sample" int32 [S] (the first sample with the highest J), "J_samples" f64 [S, K];
@@ -71,7 +79,8 @@ def allocate(policy, scenes=None, num_scenes=None, samples=1, greedy=None, seed=
     times envs played), wall seconds, scenes/s and env-steps/s.  With improve=True, "assigned_target_id", "J" and
     "num_covered" are those of the improved allocation, and "J_before_improve" f64 [S] (the best episode's J), "moves"
     int32 [S] and "converged" bool [S] (False: the move cap stopped the search) are added; "best_sample" and "J_samples"
-    stay those of the episodes."""
+    stay those of the episodes.  With bound=True, "J_bound" f64 [S] (upper_bound's "bound") is added, and the summary
+    gains "J_bound_mean" and "gap_mean" (the mean of J_bound - J)."""
     K = int(samples)
     if K <= 0:
         raise ValueError("samples must be positive")
@@ -150,6 +159,8 @@ def allocate(policy, scenes=None, num_scenes=None, samples=1, greedy=None, seed=
                 part["J_before_improve"] = part["J"]
                 for k in ("assigned_target_id", "J", "num_covered", "moves", "converged"):
                     part[k] = pol[k]
+            if bound:
+                part["J_bound"] = env.upper_bound(first_env=0, count=n, env_stride=K)["bound"]
             parts.append(part)
         res = {k: torch.cat([p[k] for p in parts]).cpu().numpy() for k in parts[0]}
         wall = time.perf_counter() - t0
@@ -163,12 +174,17 @@ def allocate(policy, scenes=None, num_scenes=None, samples=1, greedy=None, seed=
     if improve:
         for k in ("J_before_improve", "moves", "converged"):
             out[k] = res[k]
+    if bound:
+        out["J_bound"] = res["J_bound"]
     s = {}
     s["J_mean"], s["J_std"], s["J_sem"] = _stats(out["J"])
     s["J_samples_mean"] = float(out["J_samples"].mean())
     if improve:
         s["J_before_improve_mean"] = float(out["J_before_improve"].mean())
         s["moves_mean"] = float(out["moves"].mean())
+    if bound:
+        s["J_bound_mean"] = float(out["J_bound"].mean())
+        s["gap_mean"] = float((out["J_bound"] - out["J"]).mean())
     s["samples"], s["scenes"], s["env_steps"], s["wall_s"] = K, S, int(env_steps), float(wall)
     s["scenes_per_s"], s["env_steps_per_s"] = S / wall, env_steps / wall
     out["summary"] = s
@@ -225,6 +241,51 @@ def improve_allocation(scenes, assigned_target_id, max_moves=None, config=None, 
     res["summary"] = {"J_before_mean": mean(res["J_before"]), "J_mean": mean(res["J"]), "moves_mean": mean(res["moves"]),
                       "converged_frac": float(res["converged"].mean()), "scenes": S, "invalid_rows": int((~ok).sum()),
                       "wall_s": float(wall), "scenes_per_s": S / wall}
+    return res
+
+
+def upper_bound(scenes, iters=256, config=None, device=None, max_envs=65536):
+    """Certified upper bound on the best J of each of S scenes: no allocation of scene s has J above "bound"[s], so
+    bound - J is at most how far an allocation's J is from the optimum.  Frank-Wolfe on the concave relaxation of J for
+    at most `iters` iterations (fewer when the relaxation is solved first); the rule, and why the bound holds whatever
+    the iteration does, are in include/uavenv_b200.h (uavenv_upper_bound).
+
+    scenes: a get_scene()-style dict of arrays (as allocate takes them).  iters: iteration cap (>= 1).  config: sizes
+    and omega (default the global cfg).  max_envs: scenes per launch.
+
+    Returns numpy arrays: "bound" f64 [S], "relaxed" f64 [S] (the relaxation's value at the last iterate: bound -
+    relaxed shows whether more iterations would tighten the bound), "iters" int32 [S] (iterations run); and "summary":
+    mean bound, mean relaxed value, mean iterations, scenes, wall seconds and scenes/s."""
+    iters = int(iters)
+    if iters < 1:
+        raise ValueError("iters must be >= 1")
+    max_envs = int(max_envs)
+    if max_envs <= 0:
+        raise ValueError("max_envs must be positive")
+    N = int((config if config is not None else _global_cfg).NUM_UAVS)
+    S = _scene_count(scenes, N)
+    device, S, _, cfg, _, _ = _eval_setup(S, 1, config, device, 0)
+    from .envs.uav_env import UAVEnvBatched
+    dev_scenes = _device_scenes(scenes, S, device)
+    per = min(max_envs, S)
+    env = None
+    parts = []
+    try:
+        torch.cuda.synchronize(device)
+        t0 = time.perf_counter()
+        env = UAVEnvBatched(per, device=device, seed=0, config=cfg, auto_reset=False, with_info=False)
+        for c0 in range(0, S, per):
+            n = min(per, S - c0)
+            env.load_scene_device({k: v[c0:c0 + n] for k, v in dev_scenes.items()}, copies=1, first_env=0)
+            parts.append(env.upper_bound(first_env=0, count=n, iters=iters))
+        res = {k: torch.cat([p[k] for p in parts]).cpu().numpy() for k in parts[0]}
+        wall = time.perf_counter() - t0
+    finally:
+        if env is not None:
+            env.close()
+    res["summary"] = {"bound_mean": float(res["bound"].mean()), "relaxed_mean": float(res["relaxed"].mean()),
+                      "iters_mean": float(res["iters"].mean()), "scenes": S, "wall_s": float(wall),
+                      "scenes_per_s": S / wall}
     return res
 
 

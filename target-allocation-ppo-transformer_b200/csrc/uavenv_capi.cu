@@ -590,3 +590,35 @@ extern "C" int uavenv_improve_allocation(uavenv_t *h, int32_t first_env, int32_t
     improve_kernel<<<grid, kImproveThreads, smem, (cudaStream_t)stream>>>(h->P, io);
     return launch_check(h, "improve_kernel");
 }
+
+// ---- upper bound on the best allocation ----------------------------------------------------------------------------
+
+extern "C" int uavenv_upper_bound(uavenv_t *h, int32_t first_env, int32_t count, int32_t env_stride, int32_t iters,
+                                  double *d_bound, double *d_relaxed, int32_t *d_iters, void *d_workspace, void *stream) {
+    if (!h) return UAVENV_EINVAL;
+    if (!d_bound || !d_relaxed || !d_iters)
+        return fail(h, UAVENV_EINVAL, "uavenv_upper_bound: bound / relaxed / iters must be non-NULL");
+    const bool a_smem = improve_p_in_smem(h->P.N, h->P.M);
+    if (!a_smem && !d_workspace)
+        return fail(h, UAVENV_EINVAL, "uavenv_upper_bound: N*M = %d needs a workspace of "
+                    "uavenv_improve_workspace_bytes() bytes", h->P.N * h->P.M);
+    if (count <= 0 || env_stride <= 0 || iters < 1)
+        return fail(h, UAVENV_EINVAL, "uavenv_upper_bound: need count > 0, env_stride > 0 and iters >= 1 (got %d, %d, %d)",
+                    count, env_stride, iters);
+    if (int rc = check_env_range(h, first_env, count, env_stride, "uavenv_upper_bound")) return rc;
+    if (int rc = check_ready(h, "uavenv_upper_bound")) return rc;
+    CU_TRY(h, cudaSetDevice(h->device));
+    const int sms = improve_sms(h);
+    if (sms <= 0) return fail(h, UAVENV_ECUDA, "uavenv_upper_bound: no multiprocessor count for device %d", h->device);
+    const size_t smem = bound_smem_bytes(h->P.N, h->P.M);
+    CU_TRY(h, cudaFuncSetAttribute(bound_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int per_sm = 1;                          // the workspace holds one slice per SM: one CTA per SM on that path
+    if (a_smem) CU_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, bound_kernel, kBoundThreads, smem));
+    const int grid = std::min(count, sms * std::max(per_sm, 1));
+    BoundIO io;
+    io.bound = d_bound; io.relaxed = d_relaxed; io.iters = d_iters;
+    io.workspace = a_smem ? nullptr : static_cast<double *>(d_workspace);
+    io.first_env = first_env; io.count = count; io.env_stride = env_stride; io.max_iters = iters;
+    bound_kernel<<<grid, kBoundThreads, smem, (cudaStream_t)stream>>>(h->P, io);
+    return launch_check(h, "bound_kernel");
+}

@@ -17,6 +17,8 @@
 //                        a warp per group, shuffle arg-max over J, coalesced copy of the winner's allocation.
 //   improve_kernel       steepest-ascent local search (UAV moves and swaps) on given allocations: persistent CTAs,
 //                        a scene per CTA, block arg-max over the candidates of a round.
+//   bound_kernel         certified upper bound on each scene's best J (Frank-Wolfe on the concave relaxation):
+//                        improve_kernel's launch shape, a warp-per-UAV arg-max and fixed-order reductions per iteration.
 #pragma once
 
 #include "uavenv_b200.h"
@@ -1065,6 +1067,20 @@ __host__ __device__ __forceinline__ size_t improve_smem_bytes(int N, int M) {
            (size_t)(N + M) * sizeof(int32_t);
 }
 
+// out[k][j] = f(p[k][j]) for the scene's N x M pairs, p = pair_score (uavenv_score_matrix_f64's p_final bits): warps over
+// UAV rows, lanes over targets.  The local search keeps p itself, the upper bound a = min(-log1p(-p), A).
+template <int kWarps, typename F>
+__device__ __forceinline__ void fill_pair_matrix(const Params &P, const UavRec *U, const TgtRec *T, double *out, F f) {
+    const int lane = threadIdx.x & 31, M = P.M;
+    for (int k = threadIdx.x >> 5; k < P.N; k += kWarps) {
+        const UavRec u = U[k];                                               // warp-uniform address
+        for (int j = lane; j < M; j += 32) {
+            const double tx = T[j].x, ty = T[j].y, ts = T[j].speed;
+            out[(size_t)k * M + j] = f(pair_score(P, u, tx, ty, ts));
+        }
+    }
+}
+
 // prod over UAVs i != skip with t'(i) == j, ascending i, of (1 - p[i][j]); t' is t with t'(k1) = n1 and t'(k2) = n2.
 // (t[k1] / t[k2] may be rewritten concurrently: their loaded values are never used)
 __device__ __forceinline__ double improve_prod(const double *p, const int32_t *t, int N, int M, int j, int skip, int k1,
@@ -1113,13 +1129,7 @@ __global__ void __launch_bounds__(kImproveThreads) improve_kernel(const __grid_c
         const TgtRec *T = P.tgt + P.toff(slot, b);
         for (int j = tid; j < M; j += kImproveThreads) { val[j] = T[j].value; ids[j] = T[j].id; }
         for (int k = tid; k < N; k += kImproveThreads) cost[k] = U[k].cost;
-        for (int k = warp; k < N; k += kImproveWarps) {
-            const UavRec u = U[k];                                           // warp-uniform address
-            for (int j = lane; j < M; j += 32) {
-                const double tx = T[j].x, ty = T[j].y, ts = T[j].speed;
-                p[(size_t)k * M + j] = pair_score(P, u, tx, ty, ts);
-            }
-        }
+        fill_pair_matrix<kImproveWarps>(P, U, T, p, [](double x) { return x; });
         if (tid == 0) sh_n0 = 0;
         __syncthreads();
         const int32_t *row = io.assigned_in + (size_t)s * N;
@@ -1244,6 +1254,161 @@ __global__ void __launch_bounds__(kImproveThreads) improve_kernel(const __grid_c
         }
         __syncthreads();
         if (tid == 0) io.num_covered[s] = sh_n0;
+        __syncthreads();                                                     // before the next scene reuses shared memory
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// Upper bound on the best J of a scene (include/uavenv_b200.h, uavenv_upper_bound; the rule and its validity argument
+// are stated there and in DESIGN §4.10): Frank-Wolfe on the concave relaxation of J.  Persistent CTAs, one scene at a
+// time per CTA, with improve_kernel's launch shape and its home for the N x M matrix (a = min(-log1p(-p), A) in shared
+// memory when improve_p_in_smem, else in the CTA's workspace slice).  An iteration:
+//   1. nh_j = exp(-s_j) and w_j = v_j nh_j per target; barrier;
+//   2. a warp per UAV row: g_kj = w_j a_kj - omega c_k, lanes keep their first maximum, warp_argmax; thread 0 then sums
+//      F and sum_j w_j s_j in list order; barrier;
+//   3. a thread per target: sigma_j over the picking UAVs in ascending k, d_j = sigma_j - s_j (into nh's storage); thread
+//      0 sums the picked gradients and costs in ascending k and forms U_t; barrier;
+//   4. the line search: each evaluation of phi' and phi'' is one block_sum2 (one barrier); s_j += gamma d_j.
+// Every sum has a fixed order, so the bits depend on the scene alone.
+
+constexpr int kBoundThreads = 256;
+constexpr int kBoundWarps = kBoundThreads / 32;
+constexpr double kBoundAmax = 40.0;   // a = min(-log1p(-p), A): finite where p = 1
+constexpr int kBoundNewton = 10;      // safeguarded Newton steps of the line search
+
+struct BoundIO {
+    double *bound, *relaxed;   // [count]
+    int32_t *iters;            // [count]
+    double *workspace;         // [gridDim.x][N*M] when a does not fit shared memory, else NULL
+    int32_t first_env, count, env_stride, max_iters;
+};
+
+__host__ __device__ __forceinline__ size_t bound_smem_bytes(int N, int M) {
+    return (improve_p_in_smem(N, M) ? (size_t)N * M * sizeof(double) : 0) + (size_t)(4 * M + 2 * N) * sizeof(double) +
+           (size_t)N * sizeof(int32_t);
+}
+
+// (sum of x1, sum of x2) over the CTA in a fixed order: each thread's strided share of targets (added in ascending j,
+// from 0), warp_sum, then the warps' totals from warp 0 up, read by every thread.  red[2][2][kBoundWarps] alternates
+// halves by `par`, so one barrier per call suffices (a half is rewritten only after the next call's barrier).
+__device__ __forceinline__ void block_sum2(double x1, double x2, double (*red)[2][kBoundWarps], int &par, double &r1,
+                                           double &r2) {
+    const int warp = threadIdx.x >> 5;
+    x1 = warp_sum(x1); x2 = warp_sum(x2);
+    if ((threadIdx.x & 31) == 0) { red[par][0][warp] = x1; red[par][1][warp] = x2; }
+    __syncthreads();
+    r1 = red[par][0][0]; r2 = red[par][1][0];
+    for (int w = 1; w < kBoundWarps; ++w) { r1 += red[par][0][w]; r2 += red[par][1][w]; }
+    par ^= 1;
+}
+
+__global__ void __launch_bounds__(kBoundThreads) bound_kernel(const __grid_constant__ Params P, const BoundIO io) {
+    extern __shared__ __align__(16) unsigned char bound_smem[];
+    __shared__ double red[2][2][kBoundWarps];
+    __shared__ double sh_F, sh_U, sh_dC, sh_margin;
+    const int N = P.N, M = P.M;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const double omega = P.omega;
+    const bool a_smem = improve_p_in_smem(N, M);
+    double *sd = reinterpret_cast<double *>(bound_smem);
+    double *a = a_smem ? sd : io.workspace + (size_t)blockIdx.x * N * M;
+    double *s = sd + (a_smem ? (size_t)N * M : 0), *w = s + M, *nh = w + M, *val = nh + M, *cost = val + M, *gp = cost + N;
+    double *d = nh;                                                          // d_j replaces nh_j once F is summed
+    int32_t *pick = reinterpret_cast<int32_t *>(gp + N);
+    int par = 0;
+
+    for (int sc = blockIdx.x; sc < io.count; sc += gridDim.x) {
+        const int b = io.first_env + sc * io.env_stride;
+        const int slot = P.header(b).n(I_GEN) & 1;
+        const UavRec *U = P.uav + P.uoff(slot, b);
+        const TgtRec *T = P.tgt + P.toff(slot, b);
+        for (int j = tid; j < M; j += kBoundThreads) { val[j] = T[j].value; s[j] = 0.0; }
+        for (int k = tid; k < N; k += kBoundThreads) cost[k] = U[k].cost;
+        fill_pair_matrix<kBoundWarps>(P, U, T, a, [](double p) { return fmin(-log1p(-p), kBoundAmax); });
+        __syncthreads();
+        if (tid == 0) {
+            double tv = 0.0, tc = 0.0;                                       // list order, UAV order
+            for (int j = 0; j < M; ++j) tv += val[j];
+            for (int k = 0; k < N; ++k) tc += cost[k];
+            sh_margin = tv * exp(-kBoundAmax) + 1e-12 * (tv + omega * tc);
+        }
+        double C = 0.0, best = INFINITY, F = 0.0;
+        int t = 0;
+        for (;;) {
+            ++t;
+            for (int j = tid; j < M; j += kBoundThreads) {
+                const double e = exp(-s[j]);
+                nh[j] = e; w[j] = val[j] * e;
+            }
+            __syncthreads();
+            for (int k = warp; k < N; k += kBoundWarps) {
+                const double ock = omega * cost[k];
+                const double *ak = a + (size_t)k * M;
+                double bg = -INFINITY;
+                int bj = INT_MAX;
+                for (int j = lane; j < M; j += 32) {
+                    const double g = w[j] * ak[j] - ock;
+                    if (g > bg) { bg = g; bj = j; }
+                }
+                warp_argmax(bg, bj);
+                if (lane == 0) { pick[k] = bg > 0.0 ? bj : -1; gp[k] = bg > 0.0 ? bg : 0.0; }
+            }
+            if (tid == 0) {
+                double rev = 0.0, lin = 0.0;
+                for (int j = 0; j < M; ++j) { rev += val[j] * (1.0 - nh[j]); lin += w[j] * s[j]; }
+                sh_F = objective(P, rev, C);
+                sh_U = lin;                                                  // sum_j w_j s_j until step 3
+            }
+            __syncthreads();
+            for (int j = tid; j < M; j += kBoundThreads) {
+                double sg = 0.0;
+                for (int k = 0; k < N; ++k) if (pick[k] == j) sg += a[(size_t)k * M + j];
+                d[j] = sg - s[j];
+            }
+            if (tid == 0) {
+                double G = 0.0, Cs = 0.0;
+                for (int k = 0; k < N; ++k) { G += gp[k]; if (pick[k] >= 0) Cs += cost[k]; }
+                sh_U = (sh_F + G) - objective(P, sh_U, C);
+                sh_dC = Cs - C;
+            }
+            __syncthreads();
+            F = sh_F;
+            const double Ut = sh_U, dC = sh_dC;
+            best = fmin(best, Ut);
+            if (Ut - F <= 1e-9 * fmax(1.0, fabs(Ut)) || t >= io.max_iters) break;   // (uniform)
+            // line search on phi(gamma) = F(s + gamma d, C + gamma dC): phi' = sum_j (v_j e_j) d_j - omega dC and
+            // phi'' = -sum_j ((v_j e_j) d_j) d_j with e_j = exp(-(s_j + gamma d_j))
+            double gam = 1.0, p1, p2;
+            auto eval = [&](double g) {
+                double x1 = 0.0, x2 = 0.0;
+                for (int j = tid; j < M; j += kBoundThreads) {
+                    const double q = (val[j] * exp(-(s[j] + g * d[j]))) * d[j];
+                    x1 += q; x2 += q * d[j];
+                }
+                double r1, r2;
+                block_sum2(x1, x2, red, par, r1, r2);
+                p1 = r1 - omega * dC; p2 = r2;                               // p2 = -phi''
+            };
+            eval(1.0);
+            if (p1 < 0.0) {
+                double lo = 0.0, hi = 1.0;
+                for (int i = 0; i < kBoundNewton; ++i) {
+                    double c = gam + p1 / p2;
+                    if (c == gam) break;         // converged: a step below gamma's last bit (or phi' = 0 exactly)
+                    if (!(c > lo && c < hi)) c = 0.5 * (lo + hi);
+                    gam = c;
+                    eval(gam);
+                    if (p1 > 0.0) lo = gam; else hi = gam;
+                }
+            }
+            for (int j = tid; j < M; j += kBoundThreads) s[j] = s[j] + gam * d[j];
+            C = C + gam * dC;
+        }
+        if (tid == 0) {
+            io.bound[sc] = best + sh_margin;
+            io.relaxed[sc] = F;
+            io.iters[sc] = t;
+        }
         __syncthreads();                                                     // before the next scene reuses shared memory
     }
 }

@@ -102,7 +102,7 @@ class UAVEnvBatched(_capi.Handle):
         self._actions = torch.zeros(B, dtype=torch.int64, device=dev)
         self._h_reward = self._h_done = None
         self._best_target_cache = None        # best_target_actions' per-env entries, allocated on first use
-        self._improve_workspace = None        # improve_allocation's p slices (large N*M only), allocated on first use
+        self._improve_workspace = None        # improve_allocation's / upper_bound's N x M slices (large N*M only), on first use
 
     # ------------------------------------------------------------------ reset / step
     def reset(self, full_reset=True, env_mask=None):
@@ -284,9 +284,7 @@ class UAVEnvBatched(_capi.Handle):
             raise ValueError("assigned has %d elements, not a positive multiple of N = %d" % (a.numel(), self.N))
         S, dev = a.numel() // self.N, self.device
         max_moves = 16 * self.N if max_moves is None else int(max_moves)
-        ws = int(self._lib.uavenv_improve_workspace_bytes(self._h))
-        if ws and (self._improve_workspace is None or self._improve_workspace.numel() < ws):
-            self._improve_workspace = torch.empty(ws, dtype=torch.uint8, device=dev)
+        ws = self._workspace()
         out = {"assigned_target_id": torch.empty(S, self.N, dtype=torch.int32, device=dev),
                "J": torch.empty(S, dtype=torch.float64, device=dev),
                "J_before": torch.empty(S, dtype=torch.float64, device=dev),
@@ -297,8 +295,34 @@ class UAVEnvBatched(_capi.Handle):
             self._h, int(first_env), S, int(env_stride), C.c_void_p(a.data_ptr()), max_moves,
             *(C.c_void_p(out[k].data_ptr()) for k in ("assigned_target_id", "J_before", "J", "num_covered", "moves",
                                                       "converged")),
-            C.c_void_p(self._improve_workspace.data_ptr() if ws else None), self._stream()))
+            C.c_void_p(ws.data_ptr() if ws is not None else None), self._stream()))
         out["converged"] = out["converged"].view(torch.bool)
+        return out
+
+    def _workspace(self):
+        """The workspace of improve_allocation and upper_bound (uavenv_improve_workspace_bytes), or None when 0."""
+        ws = int(self._lib.uavenv_improve_workspace_bytes(self._h))
+        if ws and (self._improve_workspace is None or self._improve_workspace.numel() < ws):
+            self._improve_workspace = torch.empty(ws, dtype=torch.uint8, device=self.device)
+        return self._improve_workspace if ws else None
+
+    def upper_bound(self, first_env=0, count=None, env_stride=1, iters=256):
+        """Certified upper bound on the best J of the scenes held by envs first_env + s * env_stride, s in [0, count)
+        (count None: as many as fit): Frank-Wolfe on the concave relaxation of J for at most `iters` iterations
+        (include/uavenv_b200.h: uavenv_upper_bound states the rule and why the bound is valid).  Returns device tensors
+        {"bound": f64 [S] (no allocation of the scene has a higher J), "relaxed": f64 [S] (the relaxation's value at the
+        last iterate), "iters": int32 [S] (iterations run)}.  One launch on the env's stream."""
+        first_env, env_stride = int(first_env), int(env_stride)
+        if count is None:
+            count = (self.num_envs - first_env + env_stride - 1) // max(env_stride, 1)
+        S, dev = int(count), self.device
+        out = {"bound": torch.empty(max(S, 0), dtype=torch.float64, device=dev),
+               "relaxed": torch.empty(max(S, 0), dtype=torch.float64, device=dev),
+               "iters": torch.empty(max(S, 0), dtype=torch.int32, device=dev)}
+        ws = self._workspace()
+        self._chk(self._lib.uavenv_upper_bound(
+            self._h, first_env, S, env_stride, int(iters), *(C.c_void_p(out[k].data_ptr()) for k in ("bound", "relaxed", "iters")),
+            C.c_void_p(ws.data_ptr() if ws is not None else None), self._stream()))
         return out
 
     def get_scene(self, first_env=0, count=None):
